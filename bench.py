@@ -49,7 +49,7 @@ CONFIGS = {
     "cfg2s": dict(n_seqs=40, seq_len=5_000_000, shared=0.10, div=0.01, reads=2_000_000, read_len=150,
                   flags={}, label="cfg2s: 200 Mbp chunk (40 x 5 Mbp), 150 bp reads, default flags"),
 }
-CACHE_DIR = os.environ.get("MTSV_B200_CACHE", "/tmp/mtsv_b200_cache")
+CACHE_DIR = os.environ.get("MTSV_B200_CACHE", os.path.join(tempfile.gettempdir(), "mtsv_b200_cache"))
 
 
 def log(*a):
@@ -445,8 +445,9 @@ def parity_gate(args, w):
     return parity
 
 
-def time_device(w, steps, warmup, n=None, profile=True):
-    """Device-resident leg: reads already in HBM, results left there.  Returns (ms, stats, stage_ms, launches)."""
+def time_device(w, steps, warmup, n=None, profile=True, on_last=None):
+    """Device-resident leg: reads already in HBM, results left there.  Returns (ms, stats, stage_ms, launches).
+    on_last: called after the timed region with what the last timed step returned (device hits, offsets, count)."""
     import torch
     from mtsv_tools_b200 import load_library
     lib = load_library()
@@ -464,8 +465,9 @@ def time_device(w, steps, warmup, n=None, profile=True):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     stage_ms, stats = {}, None
     e0.record(w.stream)
+    last = None
     for _ in range(steps):
-        step()
+        last = step()
         if profile:
             stats = w.gix.last_batch_stats()
             for k, v in stats["ms"].items():
@@ -475,10 +477,51 @@ def time_device(w, steps, warmup, n=None, profile=True):
     w.ctx.barrier()
     ms = e0.elapsed_time(e1)
     launches = lib.mtsvgpu_launch_count() - launches0
+    if on_last is not None:
+        on_last(last)  # (before any other call on the handle: the results live in its buffers until then)
     w.gix.set_profiling(False)
     if stats is None:
         stats = w.gix.last_batch_stats()
     return ms, stats, {k: v / steps for k, v in stage_ms.items()}, int(launches)
+
+
+DUMP_READS = 1 << 16
+DUMP_BYTES = 64 << 20
+
+
+def _device_array(ptr, shape, typestr, dev):
+    """A torch view of memory the library owns on `dev` (no copy)."""
+    import torch
+
+    class View:
+        __cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
+    return torch.as_tensor(View(), device=dev)
+
+
+def dump_outputs(out_dir, w, last):
+    """Writes what the timed device-resident call returned in its last step as float64 .npy files under out_dir:
+    a fixed, seeded sample of DUMP_READS reads (whole reads, in read order, cut where DUMP_BYTES would be exceeded).
+    read_index: the sampled reads; hit_count: hits of each; tax_id, gi, offset, edit: their hits, read by read."""
+    import torch
+    from mtsv_tools_b200.index import HIT_DTYPE
+    d_hits, d_off, n_hits = last
+    n = w.n_reads
+    off = _device_array(d_off, (n + 1,), "<i8", w.ctx.dev).cpu().numpy().astype(np.int64)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_READS), replace=False))
+    cnt = off[idx + 1] - off[idx]
+    keep = np.cumsum(2 * 8 + 4 * 8 * cnt) <= DUMP_BYTES
+    idx, cnt = idx[keep], cnt[keep]
+    pos = np.repeat(off[idx] - np.cumsum(cnt) + cnt, cnt) + np.arange(int(cnt.sum()))
+    hits = np.zeros(0, dtype=HIT_DTYPE)
+    if len(pos):
+        rows = _device_array(d_hits, (int(n_hits), HIT_DTYPE.itemsize), "|u1", w.ctx.dev)
+        hits = rows[torch.from_numpy(pos).to(w.ctx.dev)].cpu().numpy().reshape(-1).view(HIT_DTYPE)
+    os.makedirs(out_dir, exist_ok=True)
+    cols = {"read_index": idx, "hit_count": cnt}
+    cols.update((f, hits[f]) for f in ("tax_id", "gi", "offset", "edit"))
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    log("outputs of the last timed step: %d of %d reads, %d hits -> %s" % (len(idx), n, len(hits), out_dir))
 
 
 def time_e2e(w, steps, n=None):
@@ -680,8 +723,10 @@ def cpu_baseline(args, w, seconds):
                 (2 * c["bs_steps"] + c["lf_steps"] + c["rows_located"] + c["window_bytes"] / 128.0) / ns}
 
 
-def measure(args, name, cfg, ctx, steps, warmup, ragged=False, n_reads=None, cpu_seconds=None, full=False):
+def measure(args, name, cfg, ctx, steps, warmup, ragged=False, n_reads=None, cpu_seconds=None, full=False,
+            dump_dir=None):
     """One workload on this rank set: parity gate, device-resident leg, end-to-end leg, CPU baseline.
+    dump_dir: rank 0 writes there what the last step of the device-resident leg computed (dump_outputs).
     Returns (summary dict on rank 0 / None elsewhere, Workload)."""
     w = Workload(args, name, cfg, ctx, ragged=ragged, n_reads=n_reads)
     parity = parity_gate(args, w) if (ctx.rank == 0 and not args.no_parity) else None
@@ -692,7 +737,8 @@ def measure(args, name, cfg, ctx, steps, warmup, ragged=False, n_reads=None, cpu
     # `value`: the call as a user makes it (no per-stage timers; the library then runs its slices on two lanes).
     # A second, identical leg with the per-stage CUDA-event timers on (one lane, so that kernels are timed alone)
     # gives the stage times and the roofline's kernel durations; its own step time is reported beside them.
-    ms, _, _, launches = time_device(w, steps, max(3, warmup), profile=False)
+    dump = (lambda last: dump_outputs(dump_dir, w, last)) if dump_dir and ctx.rank == 0 else None
+    ms, _, _, launches = time_device(w, steps, max(3, warmup), profile=False, on_last=dump)
     ms_prof, stats, per_step, _ = time_device(w, 1 if args.no_profile else steps, 2, profile=True)
     prof_steps = 1 if args.no_profile else steps
     e2e_ms, h2d, d2h = time_e2e(w, steps)
@@ -743,7 +789,7 @@ def run_gpu_arm(args, name, cfg, ctx):
     numa = bind_to_gpu_numa_node(ctx.local_rank) if ctx.world > 1 else "single rank: unbound"
     log("rank %d: host affinity: %s" % (ctx.rank, numa))
     world = ctx.world
-    m, w = measure(args, name, cfg, ctx, args.steps, args.warmup, full=True)
+    m, w = measure(args, name, cfg, ctx, args.steps, args.warmup, full=True, dump_dir=args.dump_outputs)
     roofline, roofline_mem = rooflines(w, m["_stats"], m["stages_ms_per_step"], m["profiled_leg"]["ms_per_step"], m["clocks"])
     L = w.L
     line = {
@@ -1136,7 +1182,14 @@ def main():
     ap.add_argument("--no-chunk-oracle", action="store_true", help="chunk mode: skip the CPU-oracle check of chunk 0")
     ap.add_argument("--hybrid-chunks", type=int, default=0, help="chunk mode: chunks per copy of the database (< N: hybrid)")
     ap.add_argument("--only-main", action="store_true", help="only the headline workload (no side configs / legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (a seeded sample of the reads' hits, float64 .npy, "
+                         "at most 64 MB) to DIR, to compare two builds on identical inputs (reads mode)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode == "chunk" or args.impl == "reference"):
+        ap.error("--dump-outputs writes the outputs of the reads mode of this implementation")
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -166,16 +166,18 @@ def _long_pair(rng, max_edits=40):
 
 def test_ssw_word_kernel_emulation(oracle, emul):
     """Reads >= 254 bases: ssw_align falls to sw_sse2_word once SW reaches 254, and that kernel is not textbook
-    SW (core.cuh).  The cell-for-cell emulation must reproduce the reference's own ssw.c (oracle/_ref) score;
-    the banded lower bound must never exceed it; the device's accept decision must equal `score >= L - 2k`."""
-    if not oracle.ssw_ref_available():
-        pytest.skip("oracle/_ref/libssw_ref.so not built")
-    rng = random.Random(7)
+    SW (core.cuh).  The cell-for-cell emulation must reproduce the reference's own ssw.c score (stored in
+    tests/golden/ssw_scores.npz, and ssw.c itself when oracle/_ref is built); the banded lower bound must never exceed
+    it; the device's accept decision must equal `score >= L - 2k`."""
+    from tests.golden.make_ssw_golden import PATH, long_sw_pairs
+    scores = np.load(PATH)["long_scores"]
+    have_ref = oracle.ssw_ref_available()
     n_word = n_diff = n_band_ok = n_band_short = 0
-    for it in range(1200):
-        read, tx = _long_pair(rng)
+    for it, (read, tx) in enumerate(long_sw_pairs()):
         L = len(read)
-        ref_score = oracle.ssw_score(read, tx, 1)
+        ref_score = int(scores[it])
+        if have_ref:
+            assert oracle.ssw_score(read, tx, 1) == ref_score, it
         w, e = emul.ssw_scores(read, tx)
         assert (w if e >= 254 else e) == ref_score, (it, L, len(tx), ref_score, w, e)
         assert w <= e
@@ -262,19 +264,19 @@ def _borderline_long_reads(ref_cat, n, read_len, k, seed):
 
 
 def test_pipeline_reads_of_254_bases_and_more(oracle, emul, small_ref, small_index):
-    """The oracle runs the reference's own ssw.c (16-bit kernel for these reads); the per-item device logic
-    must reject exactly the candidates it rejects (edit distance within budget but SSW score below L - 2k)."""
-    if not oracle.ssw_ref_available():
-        pytest.skip("oracle/_ref/libssw_ref.so not built")
+    """What the oracle answers with the reference's own ssw.c (16-bit kernel for these reads; stored in
+    tests/golden/ssw_scores.npz, and ssw.c itself when oracle/_ref is built): the per-item device logic must reject
+    exactly the candidates it rejects (edit distance within budget but SSW score below L - 2k)."""
+    from tests.golden.make_ssw_golden import EMUL_CASES, PATH, expected_hits, long_read_batch
+    golden = np.load(PATH)
     L = oracle.lib()
     n_changed = 0
-    for read_len, rate, frac in ((254, 0.13, 0.11), (300, 0.13, 0.12), (300, 0.05, 0.045), (420, 0.10, 0.09)):
-        rl = _long_reads(small_ref[0], 150, read_len, seed=read_len + int(rate * 100), edit_frac=frac)
-        k = int(np.ceil(read_len * rate))
-        rl += _borderline_long_reads(small_ref[0], 150, read_len, k, seed=read_len)
-        reads = oracle.pack_seqs(rl)
-        p = oracle.default_params(edit_rate=rate)
-        h1, o1 = small_index.bin_reads(reads, p, threads=4)  # real ssw.c
+    for i, case in enumerate(EMUL_CASES):
+        reads = long_read_batch(oracle, small_ref[0], case, ragged=False)
+        p = oracle.default_params(edit_rate=case[1])
+        o1, h1 = expected_hits(golden, "emul%d" % i)
+        if oracle.ssw_ref_available():
+            _same(h1, o1, *small_index.bin_reads(reads, p, threads=4))  # real ssw.c
         e = emul.EmulIndex(small_index, sa_rate=1, ktab_k=6)
         h2, o2 = e.bin_reads(reads[0], reads[1], p)
         _same(h1, o1, h2, o2)

@@ -355,37 +355,33 @@ def test_verifier_fast_and_legacy_paths_agree(oracle, small_ref, small_index):
 
 
 def test_pipeline_reads_longer_than_253(oracle, small_ref, small_index):
-    """Reads of 254-3000 bp (per-lane verifier with 4-64 words + the SW re-check).  The oracle runs the
-    reference's own ssw.c, whose 16-bit kernel (used once SW reaches 254) is not textbook SW: candidates with
-    edit <= k can still fail `score >= L - 2k`.  ssw_band_kernel / ssw_full_kernel must reject exactly those.
+    """Reads of 254-3000 bp (per-lane verifier with 4-64 words + the SW re-check) against what the oracle answers
+    with the reference's own ssw.c (tests/golden/ssw_scores.npz; and ssw.c itself when oracle/_ref is built), whose
+    16-bit kernel (used once SW reaches 254) is not textbook SW: candidates with edit <= k can still fail
+    `score >= L - 2k`.  ssw_band_kernel / ssw_full_kernel must reject exactly those.
     Includes reads built to sit on that threshold (tests/test_emul_parity.py::_borderline_long_reads)."""
-    from tests.test_emul_parity import _borderline_long_reads, _long_reads
+    from tests.golden.make_ssw_golden import GPU_CASES, PATH, expected_hits, long_read_batch
+    golden = np.load(PATH)
     L = oracle.lib()
     have_ref = oracle.ssw_ref_available()
     n_changed = 0
     with _gpu_index(small_index) as g:
-        for read_len, rate, frac, n in ((254, 0.13, 0.11, 300), (300, 0.13, 0.12, 400), (300, 0.05, 0.045, 300),
-                                        (420, 0.10, 0.09, 300), (700, 0.13, 0.10, 200), (1500, 0.13, 0.08, 100),
-                                        (3000, 0.13, 0.05, 60)):
-            rl = _long_reads(small_ref[0], n, read_len, seed=read_len + int(rate * 100), edit_frac=frac)
-            k = int(np.ceil(read_len * rate))
-            rl += _borderline_long_reads(small_ref[0], n, read_len, k, seed=read_len)
-            rl += [r[:rng_len] for r, rng_len in zip(rl[:50], range(100, 150))]  # ragged: short reads in the batch
-            reads = oracle.pack_seqs(rl)
-            po, pg = _params(oracle, edit_rate=rate)
-            h1, o1 = small_index.bin_reads(reads, po, threads=8)
+        for i, case in enumerate(GPU_CASES):
+            reads = long_read_batch(oracle, small_ref[0], case, ragged=True)
+            po, pg = _params(oracle, edit_rate=case[1])
+            o1, h1 = expected_hits(golden, "gpu%d" % i)
+            if have_ref:
+                _same(h1, o1, *small_index.bin_reads(reads, po, threads=8))
             h2, o2 = g.bin_reads(reads, pg)
             _same(h1, o1, h2, o2)
-            assert len(h1) > n // 4
-            if have_ref:
-                L.orc_set_ssw_kind(2)  # textbook SW: "edit <= k" would be the whole rule
-                try:
-                    h3, o3 = small_index.bin_reads(reads, po, threads=8)
-                finally:
-                    L.orc_set_ssw_kind(0)
-                n_changed += int(np.sum((o3[1:] - o3[:-1]) != (o1[1:] - o1[:-1])))
-    if have_ref:
-        assert n_changed > 0, "no read exercised the 16-bit kernel's deviation"
+            assert len(h1) > case[3] // 4
+            L.orc_set_ssw_kind(2)  # textbook SW: "edit <= k" would be the whole rule
+            try:
+                h3, o3 = small_index.bin_reads(reads, po, threads=8)
+            finally:
+                L.orc_set_ssw_kind(0)
+            n_changed += int(np.sum((o3[1:] - o3[:-1]) != (o1[1:] - o1[:-1])))
+    assert n_changed > 0, "no read exercised the 16-bit kernel's deviation"
 
 
 def test_randomized_adversarial_cases(oracle):

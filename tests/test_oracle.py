@@ -135,27 +135,17 @@ def test_index_bincode_roundtrip(oracle, tmp_path):
 
 
 def test_ssw_reference_equals_restated_sw(oracle):
-    """oracle/_ref/libssw_ref.so (the reference's ssw.c) vs the textbook restatement, reads <= 253 bp
-    (SURVEY fact 3), and the theorem ed <= k  =>  SW >= L - 2k that lets the GPU drop the SW stage."""
-    if not oracle.ssw_ref_available():
-        pytest.skip("oracle/_ref/libssw_ref.so not built (reference tree absent)")
-    rng = random.Random(4)
-    for _ in range(400):
-        L = rng.randint(15, 253)
-        read = bytes(rng.choice(b"ACGTN" if rng.random() < 0.2 else b"ACGT") for _ in range(L))
-        s = list(read)
-        for _ in range(rng.randint(0, L // 4)):
-            i = rng.randrange(len(s))
-            r = rng.random()
-            if r < 0.5:
-                s[i] = rng.choice(b"ACGTN")
-            elif r < 0.75:
-                s.insert(i, rng.choice(b"ACGT"))
-            elif len(s) > 1:
-                del s[i]
-        ref = bytes(rng.choice(b"ACGT") for _ in range(rng.randint(0, 20))) + bytes(s) + \
-            bytes(rng.choice(b"ACGT") for _ in range(rng.randint(0, 20)))
-        a = oracle.ssw_score(read, ref, 1)
+    """The reference's ssw.c (its scores stored in tests/golden/ssw_scores.npz, and oracle/_ref/libssw_ref.so itself
+    when it is built) vs the textbook restatement, reads <= 253 bp (SURVEY fact 3), and the theorem
+    ed <= k  =>  SW >= L - 2k that lets the GPU drop the SW stage."""
+    from tests.golden.make_ssw_golden import PATH, short_sw_pairs
+    scores = np.load(PATH)["short_scores"]
+    have_ref = oracle.ssw_ref_available()
+    for i, (read, ref) in enumerate(short_sw_pairs()):
+        L = len(read)
+        a = int(scores[i])
+        if have_ref:
+            assert oracle.ssw_score(read, ref, 1) == a
         b = oracle.ssw_score(read, ref, 2)
         assert a == b
         ed = oracle.min_edit_distance(read.replace(b"N", b"."), ref)
