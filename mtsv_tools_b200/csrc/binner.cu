@@ -1136,41 +1136,6 @@ __global__ void __launch_bounds__(128) ssw_full_kernel(BinnerJobs jobs, const ui
   }
 }
 
-// A/B knob for measurements: MTSV_B200_VERIFIER=legacy routes short reads through verify_kernel as well
-static bool legacy_verifier() {  // read per sub-batch so that a test can flip it in-process
-  const char* e = getenv("MTSV_B200_VERIFIER");
-  return e && strcmp(e, "legacy") == 0;
-}
-
-static int launch_verify_warp(const BinnerJobs& jobs, const DeviceIndex& ix, uint32_t max_len, bool uniform,
-                              uint32_t* out, cudaStream_t st) {
-  if (jobs.n == 0) return 0;
-  const uint32_t words = (max_len + 63) / 64;
-  const unsigned grid = (jobs.n + kVerifyThreads - 1) / kVerifyThreads;
-#define MTSV_VW_CASE(WW, UU)                                                                     \
-  {                                                                                              \
-    size_t smem = (size_t)5 * WW * kVerifyThreads * sizeof(uint64_t);                            \
-    MTSV_LAUNCH((verify_warp_kernel<WW, UU>), grid, kVerifyThreads, smem, st, jobs, ix.text4,    \
-                ix.text4_words - 1, out);                                                        \
-  }
-#define MTSV_VW_CASES(UU)                 \
-  if (words <= 1) MTSV_VW_CASE(1, UU)     \
-  else if (words == 2) MTSV_VW_CASE(2, UU) \
-  else if (words == 3) MTSV_VW_CASE(3, UU) \
-  else MTSV_VW_CASE(4, UU)
-  if (uniform) {
-    MTSV_VW_CASES(true)
-  } else {
-    MTSV_VW_CASES(false)
-  }
-#undef MTSV_VW_CASES
-#undef MTSV_VW_CASE
-  MTSV_CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
-constexpr uint32_t kMaxReadLen = 4096;
-
 // ------------------------------------------------------------------------------------------
 // select / emit
 // ------------------------------------------------------------------------------------------
@@ -1518,41 +1483,6 @@ static int validate_params(const mtsvgpu_params* in, Params* p) {
   return 0;
 }
 
-struct StageClock {
-  mtsvgpu_index* h;
-  Lane& ln;
-  StageClock(mtsvgpu_index* hh, Lane& l) : h(hh), ln(l) {}
-  cudaEvent_t next_event() {
-    if (ln.ev_next == ln.ev_pool.size()) {
-      cudaEvent_t e;
-      cudaEventCreate(&e);
-      ln.ev_pool.push_back(e);
-    }
-    return ln.ev_pool[ln.ev_next++];
-  }
-  void begin(int stage) {
-    if (!h->profiling) return;
-    cudaEvent_t a = next_event(), b = next_event();
-    cudaEventRecord(a, ln.stream);
-    ln.ev_used.push_back({stage, {a, b}});
-  }
-  void end() {
-    if (!h->profiling) return;
-    cudaEventRecord(ln.ev_used.back().second.second, ln.stream);
-  }
-  void resolve() {
-    if (!h->profiling) return;
-    cudaStreamSynchronize(ln.stream);
-    for (auto& e : ln.ev_used) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, e.second.first, e.second.second);
-      ln.stats.ms[e.first] += ms;
-    }
-    ln.ev_used.clear();
-    ln.ev_next = 0;
-  }
-};
-
 int run_segmented_sort(cudaStream_t st, DevBuf& worklist, uint64_t* keys, const uint32_t* seg_off,
                               const uint32_t* seg_cnt, uint32_t nq, uint32_t min_count, BatchCounters* d_ctr) {
   if (worklist.cap < (size_t)3 * nq * 4) {
@@ -1636,82 +1566,130 @@ static void emit_abort(mtsvgpu_index* h, int rc) {
   h->emit_cv.notify_all();
 }
 
-// One device sub-batch: reads [read0, read0 + n_reads).  Returns 1 when the seed hits exceed the
-// in-flight cap and the caller must split the range (nothing was emitted in that case).
-static int run_sub_batch(mtsvgpu_index* h, Lane& ln, const Params& p, const uint8_t* d_seqs,
-                         const uint64_t* d_seq_off, uint64_t read0, uint32_t n_reads,
-                         uint64_t slot_bound, uint64_t sub_bytes, uint64_t pack_base, uint64_t* out_total) {
-  const uint64_t batch_read0 = 0;
-  DeviceIndex& ix = h->ix;
-  BatchWorkspace& ws = *ln.ws;  // scratch of this lane
-  BatchWorkspace& res = h->ws;  // batch results (shared, appended in slice order)
-  cudaStream_t st = ln.stream;
-  StageClock clk(h, ln);
-  const uint32_t nq = n_reads * p.ns;
-  ReadsView rv{d_seqs, d_seq_off, read0, n_reads};
-  const uint64_t hit_cap = h->opts.max_batch_hits ? h->opts.max_batch_hits : (1ull << 27);
+// What stays fixed over one bin_batch_device call
+struct BatchCall {
+  mtsvgpu_index* h;
+  Params p;
+  const uint8_t* d_seqs;
+  const uint64_t* d_seq_off;
+  BatchSource* src;  // null: device-resident input
+  const char* group_verify;  // MTSV_B200_GROUP_VERIFY: unset = where it pays, "0" = never, anything else = always
+};
 
+// One device sub-batch, reads [rv.read0, rv.read0 + rv.n_reads), as it passes through the stages below.  A stage
+// reserves the workspace buffers it is the first to use; 1 from a stage: too large, the caller splits the range.
+struct SubBatch : BatchCall {
+  Lane& ln;
+  BatchWorkspace& ws;  // scratch of the lane
+  cudaStream_t st;
+  ReadsView rv;
+  EncView ev{};
+  uint32_t nq;  // strands
+  size_t qn;    // nq + 1
+  BatchCounters* d_ctr = nullptr;
+  BatchCounters hc;      // the device counters as last fetched
+  bool uniform = false;  // every read has the same length (never when a read was left out)
+  uint32_t uni_spq = 0;  // seed slots per strand when they are addressed arithmetically, else 0
+  uint32_t n_slots = 0, n_hits = 0, n_cand = 0;
+  uint64_t n_verified = 0;
+
+  SubBatch(const BatchCall& c, Lane& l, uint64_t read0, uint32_t n_reads)
+      : BatchCall(c), ln(l), ws(*l.ws), st(l.stream),
+        rv{c.d_seqs, c.d_seq_off, read0, n_reads}, nq(n_reads * c.p.ns), qn((size_t)nq + 1) {}
+  unsigned qgrid() const { return (nq + 255) / 256; }
+  int fetch() { return fetch_counters(ln, d_ctr, &hc, st); }
+  // per-stage timing (profiling only)
+  cudaEvent_t next_event() {
+    if (ln.ev_next == ln.ev_pool.size()) {
+      cudaEvent_t e;
+      cudaEventCreate(&e);
+      ln.ev_pool.push_back(e);
+    }
+    return ln.ev_pool[ln.ev_next++];
+  }
+  void begin(int stage) {
+    if (!h->profiling) return;
+    cudaEvent_t a = next_event(), b = next_event();
+    cudaEventRecord(a, ln.stream);
+    ln.ev_used.push_back({stage, {a, b}});
+  }
+  void end() {
+    if (!h->profiling) return;
+    cudaEventRecord(ln.ev_used.back().second.second, ln.stream);
+  }
+  void resolve() {
+    if (!h->profiling) return;
+    cudaStreamSynchronize(ln.stream);
+    for (auto& e : ln.ev_used) {
+      float ms = 0;
+      cudaEventElapsedTime(&ms, e.second.first, e.second.second);
+      ln.stats.ms[e.first] += ms;
+    }
+    ln.ev_used.clear();
+    ln.ev_next = 0;
+  }
+
+  int slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pack_base);
+  int search();
+  int candidates();
+  int verify();
+  int launch_verify_warp(const BinnerJobs& jobs);
+  template <int W>
+  int launch_verify_warp(const BinnerJobs& jobs);
+  int verify_ssw(const BinnerJobs& jobs);
+  int verify_grouped(const BinnerJobs& jobs, bool* done);
+  int select_append(uint64_t* out_total);
+};
+
+// ---- seed slots, then the reads' bit planes ----
+int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pack_base) {
+  const uint32_t n_reads = rv.n_reads;
   MTSV_TRY(ws.counters.reserve(sizeof(BatchCounters)));
-  BatchCounters* d_ctr = ws.counters.as<BatchCounters>();
+  d_ctr = ws.counters.as<BatchCounters>();
   MTSV_CUDA_TRY(cudaMemsetAsync(d_ctr, 0, sizeof(BatchCounters), st));
-  const size_t qn = (size_t)nq + 1;
   MTSV_TRY(ws.slot_off.reserve(qn * 4));
-  MTSV_TRY(ws.q_nseeds.reserve(qn * 4));
-  MTSV_TRY(ws.q_nhits.reserve(qn * 4));
-  MTSV_TRY(ws.hit_off.reserve(qn * 4));
-  MTSV_TRY(ws.q_ncand.reserve(qn * 4));
-  MTSV_TRY(ws.cand_off.reserve(qn * 4));
-  MTSV_TRY(ws.q_nout.reserve(qn * 4));
-  MTSV_TRY(ws.out_off.reserve(qn * 4));
-  MTSV_TRY(ws.worklist.reserve(3 * qn * 4));
-  MTSV_TRY(ws.slot_q.reserve((slot_bound + 1) * 4));
-  MTSV_TRY(ws.slot_lo.reserve((slot_bound + 1) * 4));
-  MTSV_TRY(ws.slot_cnt.reserve((slot_bound + 1) * 4));
-  MTSV_TRY(ws.slot_hoff.reserve((slot_bound + 1) * 4));
+  for (DevBuf* b : {&ws.slot_q, &ws.slot_lo, &ws.slot_cnt, &ws.slot_hoff}) MTSV_TRY(b->reserve((slot_bound + 1) * 4));
   MTSV_TRY(ws.scan_tmp.reserve(((qn + 2047) / 2048 + 1) * 8));
   const uint64_t total_words64 = (sub_bytes >> 6) + n_reads;  // words of one strand (closed-form layout)
-  if (total_words64 * p.ns > 0x7fffffffull) return 1;        // caller splits
+  if (total_words64 * p.ns > 0x7fffffffull) return 1;
   const uint32_t total_words = (uint32_t)total_words64;
   MTSV_TRY(ws.enc.reserve(((size_t)total_words * p.ns + 1) * sizeof(ReadWord)));
-  EncView ev{ws.enc.as<ReadWord>(), total_words};
+  ev = EncView{ws.enc.as<ReadWord>(), total_words};
 
-  BatchCounters hc;
-  const unsigned qgrid = (nq + 255) / 256;
-
-  // ---- seed slots ----
-  clk.begin(ST_PREP);
+  begin(ST_PREP);
   uint32_t* slot_off = ws.slot_off.as<uint32_t>();
-  MTSV_LAUNCH(count_slots_kernel, qgrid, 256, 0, st, rv, p, nq, slot_off, d_ctr);
+  MTSV_LAUNCH(count_slots_kernel, qgrid(), 256, 0, st, rv, p, nq, slot_off, d_ctr);
   MTSV_TRY(exclusive_scan_u32(slot_off, slot_off, nq, ws.scan_tmp, (uint64_t*)&d_ctr->total_slots, st));
-  clk.end();
-  MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
+  end();
+  MTSV_TRY(fetch());
   if (hc.bad_offsets) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
   ln.stats.n_reads_over_limit += hc.n_over_len;
   if (hc.total_slots > slot_bound)
     return set_error(MTSVGPU_ECUDA, "internal: seed slots %llu exceed bound %llu (reads [%llu,+%u), %llu bytes)",
-                     hc.total_slots, (unsigned long long)slot_bound, (unsigned long long)read0, n_reads,
+                     hc.total_slots, (unsigned long long)slot_bound, (unsigned long long)rv.read0, n_reads,
                      (unsigned long long)sub_bytes);
-  const uint32_t n_slots = (uint32_t)hc.total_slots;
+  n_slots = (uint32_t)hc.total_slots;
   // min_len == max_len: every read of the sub-batch has the same length (never when a read was left out)
   const uint32_t min_len = hc.n_over_len ? 0u : ~hc.inv_min_len;
+  uniform = min_len == hc.max_len;
   ln.stats.n_seed_slots += n_slots;
   // (only now that the slot count is known to fit the buffers)
-  clk.begin(ST_PREP);
+  begin(ST_PREP);
   // all reads of one length: slots are addressed arithmetically, no slot -> query map needed
-  const uint32_t uni_spq = (min_len == hc.max_len && nq && n_slots % nq == 0) ? n_slots / nq : 0;
-  if (!uni_spq) MTSV_LAUNCH(expand_slots_kernel, qgrid, 256, 0, st, slot_off, nq, ws.slot_q.as<uint32_t>());
-  if (!h->packed_input) {
+  uni_spq = (uniform && nq && n_slots % nq == 0) ? n_slots / nq : 0;
+  if (!uni_spq) MTSV_LAUNCH(expand_slots_kernel, qgrid(), 256, 0, st, slot_off, nq, ws.slot_q.as<uint32_t>());
+  if (!src || src->pack_base.empty()) {
     MTSV_LAUNCH(encode_reads_kernel, (n_reads + 127) / 128, 128, 0, st, rv, ws.enc.as<ReadWord>());
   } else {
     // d_seqs holds packed records: the sub-batch's first one at pack_base
     const uint32_t* rel = nullptr;
-    if (min_len != hc.max_len) {
+    if (!uniform) {
       MTSV_TRY(ws.pack_rel.reserve(((size_t)n_reads + 1) * 4));
       MTSV_LAUNCH(packed_sizes_kernel, (n_reads + 127) / 128, 128, 0, st, rv, ws.pack_rel.as<uint32_t>());
       MTSV_TRY(exclusive_scan_u32(ws.pack_rel.as<uint32_t>(), ws.pack_rel.as<uint32_t>(), n_reads, ws.scan_tmp, nullptr, st));
       rel = ws.pack_rel.as<uint32_t>();
     }
-    MTSV_LAUNCH(unpack_reads_kernel, (n_reads + 127) / 128, 128, 0, st, rv, d_seqs + pack_base,
+    MTSV_LAUNCH(unpack_reads_kernel, (n_reads + 127) / 128, 128, 0, st, rv, rv.seqs + pack_base,
                 packed_record_bytes(hc.max_len), rel, ws.enc.as<ReadWord>());
   }
   if (p.ns == 2) {
@@ -1720,186 +1698,213 @@ static int run_sub_batch(mtsvgpu_index* h, Lane& ln, const Params& p, const uint
     MTSV_LAUNCH(encode_rc_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, rv, ws.enc.as<ReadWord>(),
                 total_words, w_max);
   }
-  clk.end();
+  end();
+  return 0;
+}
 
-  // ---- seed search ----
-  clk.begin(ST_SEARCH);
+// ---- seed search, then the seed rule replayed and the hit offsets ----
+int SubBatch::search() {
+  for (DevBuf* b : {&ws.q_nseeds, &ws.q_nhits, &ws.hit_off}) MTSV_TRY(b->reserve(qn * 4));
+  const uint32_t* slot_off = ws.slot_off.as<uint32_t>();
+  begin(ST_SEARCH);
   if (n_slots)
-    MTSV_LAUNCH(seed_search_kernel, (n_slots + 255) / 256, 256, 0, st, ix.fm_view(), ix.ktab_view(), rv, ev, p,
+    MTSV_LAUNCH(seed_search_kernel, (n_slots + 255) / 256, 256, 0, st, h->ix.fm_view(), h->ix.ktab_view(), rv, ev, p,
                 slot_off, ws.slot_q.as<uint32_t>(), n_slots, ws.slot_lo.as<uint32_t>(),
                 ws.slot_cnt.as<uint32_t>(), d_ctr, h->profiling ? 1 : 0, hc.max_len, uni_spq);
-  clk.end();
-
-  // ---- replay the seed rule, hit offsets ----
-  clk.begin(ST_SELECT);
-  MTSV_LAUNCH(seed_select_kernel, qgrid, 256, 0, st, rv, ev, p, slot_off, nq, ws.slot_cnt.as<uint32_t>(),
+  end();
+  begin(ST_SELECT);
+  MTSV_LAUNCH(seed_select_kernel, qgrid(), 256, 0, st, rv, ev, p, slot_off, nq, ws.slot_cnt.as<uint32_t>(),
               ws.slot_hoff.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), d_ctr);
   MTSV_TRY(exclusive_scan_u32(ws.q_nhits.as<uint32_t>(), ws.hit_off.as<uint32_t>(), nq, ws.scan_tmp,
                               (uint64_t*)&d_ctr->total_hits, st));
-  clk.end();
-  MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
+  end();
+  MTSV_TRY(fetch());
   ln.stats.n_strands_over_hits += hc.overflow;
+  const uint64_t hit_cap = h->opts.max_batch_hits ? h->opts.max_batch_hits : (1ull << 27);
   if (hc.total_hits > hit_cap || hc.total_hits > 0xfffffff0ull) {
-    if (n_reads == 1)
+    if (rv.n_reads == 1)
       return set_error(MTSVGPU_ELIMIT, "one read produced %llu seed hits (cap %llu)", hc.total_hits,
                        (unsigned long long)hit_cap);
-    return 1;  // caller splits
+    return 1;
   }
-  const uint32_t n_hits = (uint32_t)hc.total_hits;
+  n_hits = (uint32_t)hc.total_hits;
   ln.stats.n_seed_hits += n_hits;
   for (int i = 0; i < 32; ++i) ln.stats.rank_queries += hc.rank_steps[i];  // sectors touched by seed search
+  return 0;
+}
 
-  uint64_t sub_out = 0;
-  uint32_t n_cand = 0;
-  if (n_hits) {
-    MTSV_TRY(ws.hit_keys.reserve((size_t)n_hits * 8));
-    MTSV_TRY(ws.cand_sparse.reserve((size_t)n_hits * sizeof(CandRec)));
-    // ---- locate ----
-    clk.begin(ST_LOCATE);
-    MTSV_LAUNCH(locate_kernel, qgrid, 256, 0, st, ix.fm_view(), ix.sa_view(), p, slot_off, nq,
-                ws.slot_lo.as<uint32_t>(), ws.slot_cnt.as<uint32_t>(), ws.slot_hoff.as<uint32_t>(),
-                ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.hit_keys.as<uint64_t>());
-    clk.end();
-    // ---- sort hits per query ----
-    clk.begin(ST_SORT);
-    MTSV_TRY(run_segmented_sort(st, ws.worklist, ws.hit_keys.as<uint64_t>(), ws.hit_off.as<uint32_t>(),
-                                ws.q_nhits.as<uint32_t>(), nq, kLightItems, d_ctr));
-    clk.end();
-    // ---- coalesce ----
-    clk.begin(ST_COALESCE);
-    MTSV_TRY(ws.cand_stage.reserve((size_t)n_hits * sizeof(CandRec)));
-    MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_heavy, 0, 3 * sizeof(unsigned int), st));
-    MTSV_LAUNCH(coalesce_kernel, (n_reads + 127) / 128, 128, 0, st, ix.bins_view(), rv, p, nq,
-                ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(),
-                ws.hit_keys.as<uint64_t>(), ws.cand_sparse.as<CandRec>(), ws.q_ncand.as<uint32_t>(),
-                ws.worklist.as<uint32_t>(), ws.worklist.as<uint32_t>() + nq, d_ctr);
-    MTSV_LAUNCH(coalesce_heavy_kernel, sm_count() * 16, 128, 0, st, ix.bins_view(), rv, p, ws.hit_off.as<uint32_t>(),
-                ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.hit_keys.as<uint64_t>(),
-                ws.cand_sparse.as<CandRec>(), ws.q_ncand.as<uint32_t>(), ws.worklist.as<uint32_t>(), d_ctr);
-    MTSV_LAUNCH(coalesce_monster_kernel, sm_count(), 1024, 0, st, ix.bins_view(), rv, p, ws.hit_off.as<uint32_t>(),
-                ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.hit_keys.as<uint64_t>(),
-                ws.cand_sparse.as<CandRec>(), ws.cand_stage.as<CandRec>(), ws.q_ncand.as<uint32_t>(),
-                ws.worklist.as<uint32_t>() + nq, d_ctr);
-    MTSV_TRY(exclusive_scan_u32(ws.q_ncand.as<uint32_t>(), ws.cand_off.as<uint32_t>(), nq, ws.scan_tmp,
-                                (uint64_t*)&d_ctr->total_cands, st));
-    clk.end();
-    MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
-    n_cand = (uint32_t)hc.total_cands;
+// ---- locate, sort per strand, coalesce into candidates, rank ----
+int SubBatch::candidates() {
+  const DeviceIndex& ix = h->ix;
+  for (DevBuf* b : {&ws.q_ncand, &ws.cand_off}) MTSV_TRY(b->reserve(qn * 4));
+  if (!n_hits) return 0;
+  MTSV_TRY(ws.worklist.reserve(3 * qn * 4));
+  MTSV_TRY(ws.hit_keys.reserve((size_t)n_hits * 8));
+  MTSV_TRY(ws.cand_sparse.reserve((size_t)n_hits * sizeof(CandRec)));
+  begin(ST_LOCATE);
+  MTSV_LAUNCH(locate_kernel, qgrid(), 256, 0, st, ix.fm_view(), ix.sa_view(), p, ws.slot_off.as<uint32_t>(), nq,
+              ws.slot_lo.as<uint32_t>(), ws.slot_cnt.as<uint32_t>(), ws.slot_hoff.as<uint32_t>(),
+              ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.hit_keys.as<uint64_t>());
+  end();
+  begin(ST_SORT);
+  MTSV_TRY(run_segmented_sort(st, ws.worklist, ws.hit_keys.as<uint64_t>(), ws.hit_off.as<uint32_t>(),
+                              ws.q_nhits.as<uint32_t>(), nq, kLightItems, d_ctr));
+  end();
+  begin(ST_COALESCE);
+  MTSV_TRY(ws.cand_stage.reserve((size_t)n_hits * sizeof(CandRec)));
+  MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_heavy, 0, 3 * sizeof(unsigned int), st));
+  MTSV_LAUNCH(coalesce_kernel, (rv.n_reads + 127) / 128, 128, 0, st, ix.bins_view(), rv, p, nq,
+              ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(),
+              ws.hit_keys.as<uint64_t>(), ws.cand_sparse.as<CandRec>(), ws.q_ncand.as<uint32_t>(),
+              ws.worklist.as<uint32_t>(), ws.worklist.as<uint32_t>() + nq, d_ctr);
+  MTSV_LAUNCH(coalesce_heavy_kernel, sm_count() * 16, 128, 0, st, ix.bins_view(), rv, p, ws.hit_off.as<uint32_t>(),
+              ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.hit_keys.as<uint64_t>(),
+              ws.cand_sparse.as<CandRec>(), ws.q_ncand.as<uint32_t>(), ws.worklist.as<uint32_t>(), d_ctr);
+  MTSV_LAUNCH(coalesce_monster_kernel, sm_count(), 1024, 0, st, ix.bins_view(), rv, p, ws.hit_off.as<uint32_t>(),
+              ws.q_nhits.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.hit_keys.as<uint64_t>(),
+              ws.cand_sparse.as<CandRec>(), ws.cand_stage.as<CandRec>(), ws.q_ncand.as<uint32_t>(),
+              ws.worklist.as<uint32_t>() + nq, d_ctr);
+  MTSV_TRY(exclusive_scan_u32(ws.q_ncand.as<uint32_t>(), ws.cand_off.as<uint32_t>(), nq, ws.scan_tmp,
+                              (uint64_t*)&d_ctr->total_cands, st));
+  end();
+  MTSV_TRY(fetch());
+  n_cand = (uint32_t)hc.total_cands;
+  if (!n_cand) return 0;
+  MTSV_TRY(ws.cand_dense.reserve((size_t)n_cand * sizeof(CandRec)));
+  MTSV_TRY(ws.cand_q.reserve((size_t)n_cand * 4));
+  begin(ST_RANK);
+  MTSV_LAUNCH(rank_emit_kernel, qgrid(), 256, 0, st, nq, ws.hit_off.as<uint32_t>(), ws.q_ncand.as<uint32_t>(),
+              ws.cand_off.as<uint32_t>(), ws.cand_sparse.as<CandRec>(), ws.cand_dense.as<CandRec>(),
+              ws.cand_q.as<uint32_t>());
+  end();
+  return 0;
+}
+
+// ---- verify (sub-batches with candidates): the route is chosen up front ----
+int SubBatch::verify() {
+  const bool ssw = hc.max_len >= 254;  // reads the SW pre-filter is not implied for
+  // several candidates per strand on average: verify TaxID group leaders first (see cand_leader_kernel).  Worth
+  // trying only where some TaxID has several sequences (otherwise two candidates of one TaxID would have to be two
+  // windows of the same sequence) and the sub-batch has more candidates than strands.
+  bool grouped = !ssw && (group_verify ? group_verify[0] != '0' : n_cand > nq && h->ix.n_bins > h->ix.n_taxids);
+  MTSV_TRY(ws.cand_edit.reserve((size_t)n_cand * 4));
+  begin(ST_VERIFY);
+  MTSV_TRY(ws.cand_flag.reserve(((size_t)n_cand + 1) * 4));
+  MTSV_TRY(ws.cand_order.reserve((size_t)n_cand * 4));
+  MTSV_LAUNCH(cand_class_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand,
+              ws.cand_flag.as<uint32_t>(), (h->profiling && !grouped) ? d_ctr : nullptr, 1);
+  MTSV_TRY(exclusive_scan_u32(ws.cand_flag.as<uint32_t>(), ws.cand_flag.as<uint32_t>(), n_cand, ws.scan_tmp,
+                              nullptr, st));
+  MTSV_LAUNCH(cand_order_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(),
+              ws.cand_flag.as<uint32_t>(), n_cand, ws.cand_order.as<uint32_t>());
+  BinnerJobs jobs{rv, ev, p, ws.cand_dense.as<CandRec>(), ws.cand_q.as<uint32_t>(),
+                  ws.cand_off.as<uint32_t>(), ws.cand_order.as<uint32_t>(), h->ix.text, n_cand};
+  n_verified = n_cand;
+  if (ssw) {
+    MTSV_TRY(verify_ssw(jobs));
+  } else {
+    if (grouped) MTSV_TRY(verify_grouped(jobs, &grouped));
+    if (!grouped) MTSV_TRY(launch_verify_warp(jobs));
   }
-  bool grouped = false;
+  end();
+  return 0;
+}
+
+// the warp verifier (reads of at most 253 bases) over a job list
+int SubBatch::launch_verify_warp(const BinnerJobs& jobs) {
+  if (jobs.n == 0) return 0;
+  const uint32_t words = (std::max(hc.max_len, 1u) + 63) / 64;
+  if (words <= 1) return launch_verify_warp<1>(jobs);
+  if (words == 2) return launch_verify_warp<2>(jobs);
+  if (words == 3) return launch_verify_warp<3>(jobs);
+  return launch_verify_warp<4>(jobs);
+}
+template <int W>
+int SubBatch::launch_verify_warp(const BinnerJobs& jobs) {
+  const unsigned grid = (jobs.n + kVerifyThreads - 1) / kVerifyThreads;
+  const size_t smem = (size_t)5 * W * kVerifyThreads * sizeof(uint64_t);
+  auto kernel = uniform ? verify_warp_kernel<W, true> : verify_warp_kernel<W, false>;
+  MTSV_LAUNCH(kernel, grid, kVerifyThreads, smem, st, jobs, h->ix.text4, h->ix.text4_words - 1, ws.cand_edit.as<uint32_t>());
+  MTSV_CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+// reads of 254 bases or more: the per-lane verifier, then the SW filter (band first, full matrices where it fails)
+int SubBatch::verify_ssw(const BinnerJobs& jobs) {
+  const uint32_t max_len = hc.max_len;
+  for (DevBuf* b : {&ws.cand_end, &ws.ssw_list}) MTSV_TRY(b->reserve((size_t)n_cand * 4));
+  uint32_t* cand_end = ws.cand_end.as<uint32_t>();
+  MTSV_TRY(launch_verify<4>(jobs, max_len, ws.cand_edit.as<uint32_t>(), cand_end, h->profiling ? d_ctr : nullptr, st));
+  // scratch of the full-matrix pass: 4 rows of max_len u16 per thread, about 64 MB in all
+  const uint32_t full_threads =
+      (uint32_t)std::min<size_t>(8192, std::max<size_t>(256, ((size_t)64 << 20) / ((size_t)max_len * 8))) / 128 * 128;
+  MTSV_TRY(ws.ssw_scratch.reserve((size_t)full_threads * 4 * max_len * sizeof(uint16_t)));
+  MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_ssw_full, 0, sizeof(unsigned int), st));
+  MTSV_LAUNCH(ssw_band_kernel, (n_cand + 127) / 128, 128, 0, st, jobs, cand_end, ws.cand_edit.as<uint32_t>(),
+              ws.ssw_list.as<uint32_t>(), &d_ctr->n_ssw_full);
+  MTSV_LAUNCH(ssw_full_kernel, full_threads / 128, 128, 0, st, jobs, ws.ssw_list.as<uint32_t>(), &d_ctr->n_ssw_full,
+              ws.cand_edit.as<uint32_t>(), ws.ssw_scratch.as<uint16_t>(), max_len);
+  return 0;
+}
+
+// Two rounds: the leaders, then the members whose leader did not pass.  The list lengths come back to the host (two
+// short synchronisations per sub-batch, only on this route): the launches are sized exactly — a grid sized for every
+// candidate costs more in empty blocks than the round saves.  *done = false (nothing verified) when more than 90 %
+// of the candidates are leaders, or when forced, all of them: the caller takes the warp route instead.
+int SubBatch::verify_grouped(const BinnerJobs& jobs, bool* done) {
+  const unsigned grid = (n_cand + 255) / 256;
+  BatchCounters* ctr = h->profiling ? d_ctr : nullptr;
+  for (DevBuf* b : {&ws.cand_lead, &ws.cand_order2}) MTSV_TRY(b->reserve((size_t)n_cand * 4));
+  uint32_t* flag = ws.cand_flag.as<uint32_t>();
+  MTSV_LAUNCH(cand_leader_kernel, (nq + 127) / 128, 128, 0, st, h->ix.bins_view(), nq, ws.cand_off.as<uint32_t>(),
+              ws.cand_dense.as<CandRec>(), ws.cand_lead.as<uint32_t>());
+  MTSV_LAUNCH(cand_round_flags_kernel, grid, 256, 0, st, ws.cand_order.as<uint32_t>(), ws.cand_lead.as<uint32_t>(),
+              ws.cand_edit.as<uint32_t>(), n_cand, 1, flag);
+  MTSV_TRY(exclusive_scan_u32(flag, flag, n_cand, ws.scan_tmp, (uint64_t*)&d_ctr->verified[0], st));
+  MTSV_TRY(fetch());
+  const uint32_t n1 = (uint32_t)hc.verified[0];
+  *done = !((uint64_t)n1 * 10 > (uint64_t)n_cand * 9 && !(group_verify && n1 < n_cand));
+  if (!*done) {
+    if (ctr)  // (the reference bytes the warp route will read)
+      MTSV_LAUNCH(cand_class_kernel, grid, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand, (uint32_t*)nullptr, ctr, 0);
+    return 0;
+  }
+  MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_edit.p, 0xff, (size_t)n_cand * 4, st));  // kNoEdit until verified
+  BinnerJobs round_jobs = jobs;
+  round_jobs.order = ws.cand_order2.as<uint32_t>();
+  MTSV_LAUNCH(cand_compact_order_kernel, grid, 256, 0, st, ws.cand_order.as<uint32_t>(), flag, n_cand,
+              ws.cand_dense.as<CandRec>(), ws.cand_order2.as<uint32_t>(), ctr);
+  round_jobs.n = n1;
+  MTSV_TRY(launch_verify_warp(round_jobs));
+  MTSV_LAUNCH(cand_round_flags_kernel, grid, 256, 0, st, ws.cand_order.as<uint32_t>(), ws.cand_lead.as<uint32_t>(),
+              ws.cand_edit.as<uint32_t>(), n_cand, 2, flag);
+  MTSV_TRY(exclusive_scan_u32(flag, flag, n_cand, ws.scan_tmp, (uint64_t*)&d_ctr->verified[1], st));
+  MTSV_TRY(fetch());
+  const uint32_t n2 = (uint32_t)hc.verified[1];
+  if (n2) {
+    MTSV_LAUNCH(cand_compact_order_kernel, grid, 256, 0, st, ws.cand_order.as<uint32_t>(), flag, n_cand,
+                ws.cand_dense.as<CandRec>(), ws.cand_order2.as<uint32_t>(), ctr);
+    round_jobs.n = n2;
+    MTSV_TRY(launch_verify_warp(round_jobs));
+  }
+  n_verified = (uint64_t)n1 + n2;
+  return 0;
+}
+
+// ---- select, then append to the batch output: in slice order, after the other lane's previous append ----
+int SubBatch::select_append(uint64_t* out_total) {
+  for (DevBuf* b : {&ws.q_nout, &ws.out_off}) MTSV_TRY(b->reserve(qn * 4));
+  uint64_t sub_out = 0;
   if (n_cand) {
-    MTSV_TRY(ws.cand_dense.reserve((size_t)n_cand * sizeof(CandRec)));
-    MTSV_TRY(ws.cand_q.reserve((size_t)n_cand * 4));
-    MTSV_TRY(ws.cand_edit.reserve((size_t)n_cand * 4));
     MTSV_TRY(ws.hit_tmp.reserve((size_t)n_cand * sizeof(HitRec)));
-    // ---- rank ----
-    clk.begin(ST_RANK);
-    MTSV_LAUNCH(rank_emit_kernel, qgrid, 256, 0, st, nq, ws.hit_off.as<uint32_t>(),
-                ws.q_ncand.as<uint32_t>(), ws.cand_off.as<uint32_t>(), ws.cand_sparse.as<CandRec>(),
-                ws.cand_dense.as<CandRec>(), ws.cand_q.as<uint32_t>());
-    clk.end();
-    // ---- verify ----
-    clk.begin(ST_VERIFY);
-    MTSV_TRY(ws.cand_flag.reserve(((size_t)n_cand + 1) * 4));
-    MTSV_TRY(ws.cand_order.reserve((size_t)n_cand * 4));
-    const bool need_ssw = hc.max_len >= 254;  // reads the SW pre-filter is not implied for
-    // several candidates per strand on average: verify TaxID group leaders first (see cand_leader_kernel)
-    {
-      const char* ge = getenv("MTSV_B200_GROUP_VERIFY");
-      // (worth trying only where some TaxID has several sequences — otherwise two candidates of one TaxID would have
-      // to be two windows of the same sequence — and the sub-batch has more candidates than strands)
-      grouped = !need_ssw && !legacy_verifier() && (ge ? ge[0] != '0' : (n_cand > nq && ix.n_bins > ix.n_taxids));
-    }
-    MTSV_LAUNCH(cand_class_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand,
-                ws.cand_flag.as<uint32_t>(), (h->profiling && !grouped) ? d_ctr : nullptr, 1);
-    MTSV_TRY(exclusive_scan_u32(ws.cand_flag.as<uint32_t>(), ws.cand_flag.as<uint32_t>(), n_cand, ws.scan_tmp,
-                                nullptr, st));
-    MTSV_LAUNCH(cand_order_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(),
-                ws.cand_flag.as<uint32_t>(), n_cand, ws.cand_order.as<uint32_t>());
-    BinnerJobs jobs{rv, ev, p, ws.cand_dense.as<CandRec>(), ws.cand_q.as<uint32_t>(),
-                    ws.cand_off.as<uint32_t>(), ws.cand_order.as<uint32_t>(), ix.text, n_cand};
-    uint64_t n_verified = n_cand;
-    if (grouped) {
-      // round 1: the leaders.  The list lengths come back to the host (two short synchronisations per sub-batch,
-      // only on this path): an all-leaders sub-batch falls through to the plain launch, and the launches are sized
-      // exactly — a grid sized for every candidate costs more in empty blocks than the round saves.
-      MTSV_TRY(ws.cand_lead.reserve((size_t)n_cand * 4));
-      MTSV_TRY(ws.cand_order2.reserve((size_t)n_cand * 4));
-      uint32_t* flag = ws.cand_flag.as<uint32_t>();
-      MTSV_LAUNCH(cand_leader_kernel, (nq + 127) / 128, 128, 0, st, ix.bins_view(), nq, ws.cand_off.as<uint32_t>(),
-                  ws.cand_dense.as<CandRec>(), ws.cand_lead.as<uint32_t>());
-      MTSV_LAUNCH(cand_round_flags_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_order.as<uint32_t>(),
-                  ws.cand_lead.as<uint32_t>(), ws.cand_edit.as<uint32_t>(), n_cand, 1, flag);
-      MTSV_TRY(exclusive_scan_u32(flag, flag, n_cand, ws.scan_tmp, (uint64_t*)&d_ctr->verified[0], st));
-      MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
-      const uint32_t n1 = (uint32_t)hc.verified[0];
-      if ((uint64_t)n1 * 10 > (uint64_t)n_cand * 9 && !(getenv("MTSV_B200_GROUP_VERIFY") && n1 < n_cand)) {
-        grouped = false;  // (nearly) one candidate per (strand, TaxID): holding the few others back does not pay
-        if (h->profiling)
-          MTSV_LAUNCH(cand_class_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand,
-                      (uint32_t*)nullptr, d_ctr, 0);
-      } else {
-        MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_edit.p, 0xff, (size_t)n_cand * 4, st));  // kNoEdit until verified
-        BinnerJobs round_jobs = jobs;
-        round_jobs.order = ws.cand_order2.as<uint32_t>();
-        MTSV_LAUNCH(cand_compact_order_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_order.as<uint32_t>(), flag,
-                    n_cand, ws.cand_dense.as<CandRec>(), ws.cand_order2.as<uint32_t>(), h->profiling ? d_ctr : nullptr);
-        round_jobs.n = n1;
-        MTSV_TRY(launch_verify_warp(round_jobs, ix, std::max(hc.max_len, 1u), min_len == hc.max_len,
-                                    ws.cand_edit.as<uint32_t>(), st));
-        // round 2: members whose leader did not pass
-        MTSV_LAUNCH(cand_round_flags_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_order.as<uint32_t>(),
-                    ws.cand_lead.as<uint32_t>(), ws.cand_edit.as<uint32_t>(), n_cand, 2, flag);
-        MTSV_TRY(exclusive_scan_u32(flag, flag, n_cand, ws.scan_tmp, (uint64_t*)&d_ctr->verified[1], st));
-        MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
-        const uint32_t n2 = (uint32_t)hc.verified[1];
-        if (n2) {
-          MTSV_LAUNCH(cand_compact_order_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_order.as<uint32_t>(), flag,
-                      n_cand, ws.cand_dense.as<CandRec>(), ws.cand_order2.as<uint32_t>(), h->profiling ? d_ctr : nullptr);
-          round_jobs.n = n2;
-          MTSV_TRY(launch_verify_warp(round_jobs, ix, std::max(hc.max_len, 1u), min_len == hc.max_len,
-                                      ws.cand_edit.as<uint32_t>(), st));
-        }
-        n_verified = (uint64_t)n1 + n2;
-      }
-    }
-    if (grouped) {
-      // (both rounds launched above)
-    } else if (!need_ssw && !legacy_verifier()) {
-      MTSV_TRY(launch_verify_warp(jobs, ix, std::max(hc.max_len, 1u), min_len == hc.max_len,
-                                  ws.cand_edit.as<uint32_t>(), st));
-    } else {
-      uint32_t* cand_end = nullptr;
-      if (need_ssw) {
-        MTSV_TRY(ws.cand_end.reserve((size_t)n_cand * 4));
-        MTSV_TRY(ws.ssw_list.reserve((size_t)n_cand * 4));
-        cand_end = ws.cand_end.as<uint32_t>();
-      }
-      MTSV_TRY(launch_verify<4>(jobs, hc.max_len, ws.cand_edit.as<uint32_t>(), cand_end,
-                                h->profiling ? d_ctr : nullptr, st));
-      if (need_ssw) {
-        // scratch of the full-matrix pass: 4 rows of max_len u16 per thread, about 64 MB in all
-        const uint32_t full_threads =
-            (uint32_t)std::min<size_t>(8192, std::max<size_t>(256, ((size_t)64 << 20) / ((size_t)hc.max_len * 8))) /
-            128 * 128;
-        MTSV_TRY(ws.ssw_scratch.reserve((size_t)full_threads * 4 * hc.max_len * sizeof(uint16_t)));
-        MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_ssw_full, 0, sizeof(unsigned int), st));
-        MTSV_LAUNCH(ssw_band_kernel, (n_cand + 127) / 128, 128, 0, st, jobs, cand_end, ws.cand_edit.as<uint32_t>(),
-                    ws.ssw_list.as<uint32_t>(), &d_ctr->n_ssw_full);
-        MTSV_LAUNCH(ssw_full_kernel, full_threads / 128, 128, 0, st, jobs, ws.ssw_list.as<uint32_t>(),
-                    &d_ctr->n_ssw_full, ws.cand_edit.as<uint32_t>(), ws.ssw_scratch.as<uint16_t>(), hc.max_len);
-      }
-    }
-    clk.end();
-    // ---- select ----
-    clk.begin(ST_EMIT);
-    MTSV_LAUNCH(select_kernel, (nq + 127) / 128, 128, 0, st, ix.bins_view(), rv, p, nq,
-                ws.cand_off.as<uint32_t>(), ws.cand_dense.as<CandRec>(), ws.cand_edit.as<uint32_t>(),
-                ws.hit_tmp.as<HitRec>(), ws.q_nout.as<uint32_t>());
+    begin(ST_EMIT);
+    MTSV_LAUNCH(select_kernel, (nq + 127) / 128, 128, 0, st, h->ix.bins_view(), rv, p, nq, ws.cand_off.as<uint32_t>(),
+                ws.cand_dense.as<CandRec>(), ws.cand_edit.as<uint32_t>(), ws.hit_tmp.as<HitRec>(),
+                ws.q_nout.as<uint32_t>());
     MTSV_TRY(exclusive_scan_u32(ws.q_nout.as<uint32_t>(), ws.out_off.as<uint32_t>(), nq, ws.scan_tmp,
                                 (uint64_t*)&d_ctr->total_out, st));
-    clk.end();
-    MTSV_TRY(fetch_counters(ln, d_ctr, &hc, st));
+    end();
+    MTSV_TRY(fetch());
     sub_out = hc.total_out;
     ln.stats.n_candidates += n_verified;
     for (int i = 0; i < 32; ++i) ln.stats.window_bytes += hc.window_bytes[i];
@@ -1907,66 +1912,69 @@ static int run_sub_batch(mtsvgpu_index* h, Lane& ln, const Params& p, const uint
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_off.p, 0, qn * 4, st));
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_off.p, 0, qn * 4, st));
   }
-  // ---- append to the batch output: in slice order, after the other lane's previous append ----
   MTSV_TRY(emit_acquire(h, ln));
   Lane& other = h->lanes[&ln == &h->lanes[0] ? 1 : 0];
   if (other.emit_event) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, other.emit_event, 0));
-  MTSV_TRY(grow_preserve(res.out_hits, *out_total * sizeof(HitRec), (*out_total + sub_out + 1) * sizeof(HitRec),
-                         st));
-  clk.begin(ST_EMIT);
+  BatchWorkspace& res = h->ws;  // batch results (shared, appended in slice order)
+  MTSV_TRY(grow_preserve(res.out_hits, *out_total * sizeof(HitRec), (*out_total + sub_out + 1) * sizeof(HitRec), st));
+  begin(ST_EMIT);
   MTSV_LAUNCH(gather_hits_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
               ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), res.out_hits.as<HitRec>(), *out_total,
-              res.out_hit_off.as<uint64_t>(), read0 - batch_read0);
-  clk.end();
+              res.out_hit_off.as<uint64_t>(), rv.read0);
+  end();
   MTSV_CUDA_TRY(cudaGetLastError());
   if (!ln.emit_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&ln.emit_event, cudaEventDisableTiming));
   MTSV_CUDA_TRY(cudaEventRecord(ln.emit_event, st));
   // host API: start copying this sub-batch's results out while the next one computes
-  if (h->results_hook) MTSV_TRY(h->results_hook(h, *out_total, sub_out, read0 - batch_read0, n_reads, st));
-  clk.resolve();
+  if (src) MTSV_TRY(src->results(*out_total, sub_out, rv.read0, rv.n_reads, st));
+  resolve();
   *out_total += sub_out;
   ln.stats.n_hits += sub_out;
   ln.stats.n_queries += nq;
   return 0;
 }
 
-// seq_off accessor: host copy when the caller has one, otherwise single 8-byte D2H reads
-struct OffsetSource {
-  const uint64_t* host;
-  const uint64_t* dev;
-  cudaStream_t st;
-  int get(uint64_t i, uint64_t* v) const {
-    if (host) {
-      *v = host[i];
-      return 0;
-    }
-    MTSV_CUDA_TRY(cudaMemcpyAsync(v, dev + i, 8, cudaMemcpyDeviceToHost, st));
-    MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-    return 0;
-  }
-};
+// One device sub-batch: reads [read0, read0 + n_reads).  Returns 1 when it exceeds the in-flight limits and the
+// caller must split the range (nothing was emitted in that case).
+static int run_sub_batch(const BatchCall& call, Lane& ln, uint64_t read0, uint32_t n_reads, uint64_t slot_bound,
+                         uint64_t sub_bytes, uint64_t pack_base, uint64_t* out_total) {
+  SubBatch s(call, ln, read0, n_reads);
+  int rc = s.slots_encode(slot_bound, sub_bytes, pack_base);
+  if (rc == 0) rc = s.search();
+  if (rc != 0) return rc;
+  MTSV_TRY(s.candidates());
+  if (s.n_cand) MTSV_TRY(s.verify());
+  return s.select_append(out_total);
+}
 
 // One uploaded slice [read0, read0 + n_reads): processed in groups of ln.chunk_reads reads.  A group whose seed
 // hits overflow the in-flight cap (run_sub_batch returns 1, nothing emitted) is retried at half the size, and
 // the smaller size is kept for what follows (repetitive references: hundreds of hits per read).
-static int run_range(mtsvgpu_index* h, Lane& ln, const Params& p, const uint8_t* d_seqs, const uint64_t* d_seq_off,
-                     const OffsetSource& offs, uint64_t read0, uint64_t n_reads, uint64_t off_lo,
+static int run_range(const BatchCall& call, Lane& ln, uint64_t read0, uint64_t n_reads, uint64_t off_lo,
                      uint64_t off_hi, uint64_t* out_total) {
   if (off_hi < off_lo) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
+  const Params& p = call.p;
+  const uint64_t* h_off = call.src ? call.src->seq_off : nullptr;  // host copy of seq_off
   uint64_t r = read0, off_r = off_lo;
   // packed input: byte offset of the record of read r (the slice's first record was placed by the uploader)
-  uint64_t pack_r = h->packed_input && ln.slice < h->pack_slice_base.size() ? h->pack_slice_base[ln.slice] : 0;
+  const bool packed = call.src && !call.src->pack_base.empty();
+  uint64_t pack_r = packed ? call.src->pack_base[ln.slice] : 0;
   const uint64_t r_end = read0 + n_reads;
   while (r < r_end) {
     uint64_t nr = std::min(r_end - r, std::max<uint64_t>(ln.chunk_reads, 1));
     uint64_t off_e = off_hi;
-    if (r + nr < r_end) MTSV_TRY(offs.get(r + nr, &off_e));
+    if (r + nr < r_end && h_off) {
+      off_e = h_off[r + nr];
+    } else if (r + nr < r_end) {
+      MTSV_CUDA_TRY(cudaMemcpyAsync(&off_e, call.d_seq_off + r + nr, 8, cudaMemcpyDeviceToHost, ln.stream));
+      MTSV_CUDA_TRY(cudaStreamSynchronize(ln.stream));
+    }
     if (off_e < off_r) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
     // bound on seed slots from the byte count: slots(L) <= L/G + 1 per strand
     const uint64_t bytes = off_e - off_r;
     const uint64_t slot_bound = (bytes / p.G + nr) * p.ns + 1;
     const bool too_big = slot_bound > 0xfffffff0ull || nr * p.ns > 0x7ffffff0ull;
-    int rc = too_big ? 1 : run_sub_batch(h, ln, p, d_seqs, d_seq_off, r, (uint32_t)nr, slot_bound, bytes, pack_r, out_total);
+    int rc = too_big ? 1 : run_sub_batch(call, ln, r, (uint32_t)nr, slot_bound, bytes, pack_r, out_total);
     if (rc == 1) {
       if (nr == 1) return set_error(MTSVGPU_ELIMIT, "a single read exceeds the device batch limits");
       ln.chunk_reads = std::max<uint64_t>(1, nr / 2);
@@ -1974,20 +1982,34 @@ static int run_range(mtsvgpu_index* h, Lane& ln, const Params& p, const uint8_t*
     }
     if (rc != 0) return rc;
     ln.stats.n_sub_batches += 1;
-    if (h->packed_input && r + nr < r_end && offs.host)  // (only after a split: a slice is normally one group)
-      for (uint64_t i = r; i < r + nr; ++i) pack_r += packed_record_bytes((uint32_t)(offs.host[i + 1] - offs.host[i]));
+    if (packed && r + nr < r_end)  // (only after a split: a slice is normally one group)
+      for (uint64_t i = r; i < r + nr; ++i) pack_r += packed_record_bytes((uint32_t)(h_off[i + 1] - h_off[i]));
     r += nr;
     off_r = off_e;
   }
   return 0;
 }
 
+static void add_stats(mtsvgpu_batch_stats& to, const mtsvgpu_batch_stats& from) {
+  for (int i = 0; i < MTSVGPU_N_STAGES; ++i) to.ms[i] += from.ms[i];  // (launches[] is not filled)
+  to.n_queries += from.n_queries;
+  to.n_seed_slots += from.n_seed_slots;
+  to.n_seed_hits += from.n_seed_hits;
+  to.n_candidates += from.n_candidates;
+  to.n_hits += from.n_hits;
+  to.window_bytes += from.window_bytes;
+  to.rank_queries += from.rank_queries;
+  to.n_sub_batches += from.n_sub_batches;
+  to.n_reads_over_limit += from.n_reads_over_limit;
+  to.n_strands_over_hits += from.n_strands_over_hits;
+}
+
 int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_seq_off, uint64_t n_reads,
-                     const uint64_t* h_seq_off_or_null, const mtsvgpu_params* params,
-                     const mtsvgpu_hit** d_hits, const uint64_t** d_hit_off, uint64_t* n_hits) {
+                     BatchSource* src, const mtsvgpu_params* params, const mtsvgpu_hit** d_hits,
+                     const uint64_t** d_hit_off, uint64_t* n_hits) {
   if (!h) return set_error(MTSVGPU_EINVAL, "index is NULL");
-  Params p;
-  MTSV_TRY(validate_params(params, &p));
+  BatchCall call{h, {}, d_seqs, d_seq_off, src, getenv("MTSV_B200_GROUP_VERIFY")};
+  MTSV_TRY(validate_params(params, &call.p));
   if (!d_seq_off) return set_error(MTSVGPU_EINVAL, "seq_off is NULL");
   MTSV_CUDA_TRY(cudaSetDevice(h->ix.device));
   cudaStream_t st = h->stream;
@@ -1995,49 +2017,29 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   BatchWorkspace& ws = h->ws;
   MTSV_TRY(ws.out_hit_off.reserve((n_reads + 1) * 8));
   uint64_t total = 0;
-  const bool host_path = h->sub_batch_hook != nullptr;
-  const uint64_t step = h->opts.batch_reads ? h->opts.batch_reads : (host_path ? kDefaultStepHost : kDefaultStepDevice);
   if (n_reads == 0) {
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_hit_off.p, 0, 8, st));
     MTSV_TRY(grow_preserve(ws.out_hits, 0, sizeof(HitRec), st));
   }
-  // sub-batch boundaries of seq_off: one strided gather instead of copying 8 B per read
-  // the host API (sub_batch_hook set) uploads slice by slice: short first slices fill the pipeline
   // ---- lanes: the slices of a batch alternate between two lanes (own stream, scratch and host thread each): the
   // synchronisation bubbles and kernel tails of one slice are filled by the other — ~10 % on the small slices of
-  // the host API, 4 % on the large ones of device-resident input.  One lane when per-stage timing is on, so that
-  // the event timers measure kernels that run alone.  MTSV_B200_LANES=1|2 overrides. ----
-  const char* lanes_env = getenv("MTSV_B200_LANES");
-  int want_lanes = (host_path || !h->profiling) ? 2 : 1;
-  if (lanes_env && (atoi(lanes_env) == 1 || atoi(lanes_env) == 2)) want_lanes = atoi(lanes_env);
-  std::vector<uint64_t> rb;
-  uint64_t stride = step;  // device-resident input: slices of equal size
-  if (host_path) {
-    rb = sub_batch_bounds(n_reads, step, true);
-  } else {
-    uint64_t k = (n_reads + step - 1) / step;
-    // an even number of slices, so that both lanes get the same share; a batch that fits one slice is still cut in
-    // two when it is large enough (MTSV_B200_SPLIT_MIN reads, default 2^21: +3 % at 2.5 M reads; at 1.25 M reads the
-    // halves gain 3 % on an idle host and lose as much with eight ranks' threads competing for it)
-    static const uint64_t split_min = getenv("MTSV_B200_SPLIT_MIN") ? strtoull(getenv("MTSV_B200_SPLIT_MIN"), nullptr, 10) : (1ull << 21);
-    if (want_lanes == 2 && ((k >= 2 && (k & 1)) || (k == 1 && n_reads >= split_min))) ++k;
-    stride = k ? (n_reads + k - 1) / k : step;
-    rb.push_back(0);
-    for (uint64_t i = 1; i <= k; ++i) rb.push_back(std::min(n_reads, i * stride));
-  }
+  // the host API, 4 % on the large ones of device-resident input.  One lane for device-resident input when per-stage
+  // timing is on, so that the event timers measure kernels that run alone. ----
+  const bool two_lanes = src || !h->profiling;
+  const std::vector<uint64_t> rb = src ? src->bounds : slice_bounds(n_reads, h->opts.batch_reads, false, two_lanes);
   const uint64_t n_sub = rb.size() - 1;
   std::vector<uint64_t> bounds(n_sub + 1, 0);
   if (n_reads) {
-    if (h_seq_off_or_null) {
-      for (uint64_t i = 0; i <= n_sub; ++i) bounds[i] = h_seq_off_or_null[rb[i]];
+    if (src) {
+      for (uint64_t i = 0; i <= n_sub; ++i) bounds[i] = src->seq_off[rb[i]];
     } else {
-      // (boundaries are multiples of the stride: one strided gather)
-      MTSV_CUDA_TRY(cudaMemcpy2DAsync(bounds.data(), 8, d_seq_off, stride * 8, 8, n_sub, cudaMemcpyDeviceToHost, st));
+      // (boundaries are multiples of the first slice's size: one strided gather instead of copying 8 B per read)
+      MTSV_CUDA_TRY(cudaMemcpy2DAsync(bounds.data(), 8, d_seq_off, rb[1] * 8, 8, n_sub, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaMemcpyAsync(&bounds[n_sub], d_seq_off + n_reads, 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     }
   }
-  const int n_lanes = n_sub >= 2 ? want_lanes : 1;
+  const int n_lanes = n_sub >= 2 && two_lanes ? 2 : 1;
   h->lanes[0].stream = st;
   h->lanes[0].ws = &h->ws;
   h->lanes[1].ws = &h->ws1;
@@ -2055,14 +2057,13 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   h->abort_msg.clear();
   for (Lane& ln : h->lanes) {
     ln.has_turn = false;
-    ln.chunk_reads = step;
+    ln.chunk_reads = UINT64_MAX;  // a whole slice
     memset(&ln.stats, 0, sizeof ln.stats);
   }
   const int device = h->ix.device;
   auto lane_main = [&](int li) {
     Lane& ln = h->lanes[li];
     if (li != 0) cudaSetDevice(device);
-    OffsetSource offs{h_seq_off_or_null, d_seq_off, ln.stream};
     for (uint64_t i = (uint64_t)li; i < n_sub; i += (uint64_t)n_lanes) {
       {
         std::lock_guard<std::mutex> lk(h->emit_mu);
@@ -2070,9 +2071,8 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
       }
       ln.slice = i;
       int rc = 0;
-      if (h->sub_batch_hook) rc = h->sub_batch_hook(h, i, ln.stream);
-      if (rc == 0)
-        rc = run_range(h, ln, p, d_seqs, d_seq_off, offs, rb[i], rb[i + 1] - rb[i], bounds[i], bounds[i + 1], &total);
+      if (src) rc = src->wait_slice(i, ln.stream);
+      if (rc == 0) rc = run_range(call, ln, rb[i], rb[i + 1] - rb[i], bounds[i], bounds[i + 1], &total);
       if (rc != 0) {
         emit_abort(h, rc);
         return;
@@ -2090,22 +2090,7 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   } else {
     lane_main(0);
   }
-  for (Lane& ln : h->lanes) {  // merge the per-lane statistics
-    for (int i = 0; i < MTSVGPU_N_STAGES; ++i) {
-      h->stats.ms[i] += ln.stats.ms[i];
-      h->stats.launches[i] += ln.stats.launches[i];
-    }
-    h->stats.n_queries += ln.stats.n_queries;
-    h->stats.n_seed_slots += ln.stats.n_seed_slots;
-    h->stats.n_seed_hits += ln.stats.n_seed_hits;
-    h->stats.n_candidates += ln.stats.n_candidates;
-    h->stats.n_hits += ln.stats.n_hits;
-    h->stats.window_bytes += ln.stats.window_bytes;
-    h->stats.rank_queries += ln.stats.rank_queries;
-    h->stats.n_sub_batches += ln.stats.n_sub_batches;
-    h->stats.n_reads_over_limit += ln.stats.n_reads_over_limit;
-    h->stats.n_strands_over_hits += ln.stats.n_strands_over_hits;
-  }
+  for (Lane& ln : h->lanes) add_stats(h->stats, ln.stats);
   if (h->abort_rc != 0) {
     cudaStreamSynchronize(st);
     if (h->lane1_stream) cudaStreamSynchronize(h->lane1_stream);
@@ -2225,7 +2210,7 @@ int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off
       return set_error(MTSVGPU_EINVAL, "offsets not monotone");
     max_len = std::max<uint64_t>(max_len, pat_off[i + 1] - pat_off[i]);
   }
-  if (max_len > kMaxReadLen) return set_error(MTSVGPU_ELIMIT, "pattern longer than %u", kMaxReadLen);
+  if (max_len > kMaxReadLenDev) return set_error(MTSVGPU_ELIMIT, "pattern longer than %u", kMaxReadLenDev);
   uint64_t pb = pat_off[n_pairs], tb = text_off[n_pairs];
   DevBuf dp, dpo, dt, dto, de, dw;
   int rc = 0;

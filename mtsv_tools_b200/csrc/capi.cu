@@ -126,11 +126,24 @@ static cudaEvent_t trace_event(std::vector<cudaEvent_t>& pool, size_t i) {
   return pool[i];
 }
 
-static int wait_for_sub_batch_input(mtsvgpu_index* ix, uint64_t i, cudaStream_t st) {
+// Per-call state of bin_batch_host, shared by the uploader thread and the compute lanes
+struct HostUpload : BatchSource {
+  mtsvgpu_index* ix;
+  std::atomic<uint64_t> slices_enqueued{0};  // slices whose upload has been enqueued (uploader thread)
+  std::atomic<int> upload_rc{0};
+  std::string upload_msg;
+  uint64_t out_copied_hits = 0, out_copied_reads = 0;  // prefix already on its way to the pinned buffers
+  bool out_overlap_ok = false;
+  explicit HostUpload(mtsvgpu_index* h) : ix(h) {}
+  int upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool trace, uint64_t* h2d_bytes);
+  int wait_slice(uint64_t i, cudaStream_t st) override;
+  int results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads, cudaStream_t st) override;
+};
+
+int HostUpload::wait_slice(uint64_t i, cudaStream_t st) {
   // the uploader thread enqueues slice after slice; wait (on the host) until slice i's event has been recorded
-  while (ix->slices_enqueued.load(std::memory_order_acquire) <= i) {
-    if (ix->upload_rc.load(std::memory_order_acquire) != 0)
-      return set_error(ix->upload_rc.load(), "%s", ix->upload_msg.c_str());
+  while (slices_enqueued.load(std::memory_order_acquire) <= i) {
+    if (upload_rc.load(std::memory_order_acquire) != 0) return set_error(upload_rc.load(), "%s", upload_msg.c_str());
     std::this_thread::yield();
   }
   if (i < ix->in_events.size()) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, ix->in_events[i], 0));
@@ -141,13 +154,12 @@ static int wait_for_sub_batch_input(mtsvgpu_index* ix, uint64_t i, cudaStream_t 
 // Results of a finished sub-batch go to the pinned result buffers on the copy-out stream while the next
 // sub-batch computes.  Only used when the pinned buffers are known to be large enough (they keep the size
 // of earlier batches); otherwise everything is copied at the end.
-static int copy_results_slice(mtsvgpu_index* ix, uint64_t first_hit, uint64_t n_hits, uint64_t first_read,
-                              uint64_t n_reads, cudaStream_t st) {
-  if (!ix->out_overlap_ok) return 0;
+int HostUpload::results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads, cudaStream_t st) {
+  if (!out_overlap_ok) return 0;
   if ((first_hit + n_hits) * sizeof(mtsvgpu_hit) > ix->pin_hits_cap ||
-      (first_read + n_reads + 1) * sizeof(uint64_t) > ix->pin_off_cap || first_hit != ix->out_copied_hits ||
-      first_read != ix->out_copied_reads) {
-    ix->out_overlap_ok = false;  // does not fit / unexpected order: the caller copies everything at the end
+      (first_read + n_reads + 1) * sizeof(uint64_t) > ix->pin_off_cap || first_hit != out_copied_hits ||
+      first_read != out_copied_reads) {
+    out_overlap_ok = false;  // does not fit / unexpected order: the caller copies everything at the end
     return 0;
   }
   MTSV_CUDA_TRY(cudaEventRecord(ix->out_event, st));
@@ -159,8 +171,8 @@ static int copy_results_slice(mtsvgpu_index* ix, uint64_t first_hit, uint64_t n_
                                   n_hits * sizeof(mtsvgpu_hit), cudaMemcpyDeviceToHost, ix->copy_out_stream));
   MTSV_CUDA_TRY(cudaMemcpyAsync((uint64_t*)ix->pin_off + first_read, d_off + first_read,
                                 (n_reads + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out_stream));
-  ix->out_copied_hits = first_hit + n_hits;
-  ix->out_copied_reads = first_read + n_reads;
+  out_copied_hits = first_hit + n_hits;
+  out_copied_reads = first_read + n_reads;
   return 0;
 }
 
@@ -180,15 +192,16 @@ static bool uniform_lengths(const uint64_t* o, uint64_t n_reads) {  // o[0 .. n_
 
 // The uploader: enqueues the slices one after the other on the copy-in stream (runs on its own host thread so
 // that checking a slice's lengths does not hold up the compute lanes; it stays far ahead of the DMA engine).
-static int upload_slices(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* offs, uint64_t base, uint64_t bytes,
-                         const std::vector<uint64_t>& rb, bool trace, bool packed, uint64_t* h2d_bytes) {
+int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool trace, uint64_t* h2d_bytes) {
   MTSV_CUDA_TRY(cudaSetDevice(ix->ix.device));
   BatchWorkspace& ws = ix->ws;
   cudaStream_t cin = ix->copy_in_stream;
-  const uint64_t n_sub = rb.size() - 1;
+  const uint64_t* offs = seq_off;
+  const bool packed = !pack_base.empty();
+  const uint64_t n_sub = bounds.size() - 1;
   uint64_t pack_at = 0;  // packed input: byte offset of the next slice's first record
   for (uint64_t i = 0; i < n_sub; ++i) {
-    uint64_t r0 = rb[i], r1 = rb[i + 1];
+    uint64_t r0 = bounds[i], r1 = bounds[i + 1];
     if (r1 < r0 || offs[r1] < offs[r0]) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
     const uint64_t b0 = offs[r0];
     uint64_t c0 = b0, cn = offs[r1] - b0;  // what is copied: the slice's bases, or its packed records
@@ -204,7 +217,7 @@ static int upload_slices(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t*
           pb += 3 * ((offs[r + 1] - offs[r] + 7) >> 3);
         }
       }
-      ix->pack_slice_base[i] = pack_at;
+      pack_base[i] = pack_at;
       c0 = pack_at;
       cn = pb;
       pack_at += pb;
@@ -226,7 +239,7 @@ static int upload_slices(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t*
     *h2d_bytes += cn;
     MTSV_CUDA_TRY(cudaEventRecord(ix->in_events[i], cin));
     if (trace) cudaEventRecord(g_trace_landed[i], cin);
-    ix->slices_enqueued.store(i + 1, std::memory_order_release);
+    slices_enqueued.store(i + 1, std::memory_order_release);
   }
   return 0;
 }
@@ -261,9 +274,11 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
     offs = rebased.data();
   }
   // ---- H2D, pipelined per device sub-batch ----
-  const uint64_t step = ix->opts.batch_reads ? ix->opts.batch_reads : kDefaultStepHost;
-  const std::vector<uint64_t> rb = sub_batch_bounds(n_reads, step, true);
-  const uint64_t n_sub = n_reads ? rb.size() - 1 : 0;
+  HostUpload up(ix);
+  up.seq_off = offs;
+  up.bounds = slice_bounds(n_reads, ix->opts.batch_reads, true, true);
+  const uint64_t n_sub = up.bounds.size() - 1;
+  if (packed) up.pack_base.assign(n_sub, 0);
   while (ix->in_events.size() < n_sub) {
     cudaEvent_t e;
     MTSV_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -275,18 +290,14 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
     if (n_sub) trace_event(g_trace_started, n_sub - 1);
   }
   if (trace && n_sub) trace_event(g_trace_landed, n_sub - 1);
-  ix->slices_enqueued.store(0);
-  ix->upload_rc.store(0);
-  ix->packed_input = packed;
-  ix->pack_slice_base.assign(n_sub + 1, 0);
   uint64_t h2d_bytes = 0;
   std::thread uploader;
   if (n_sub) {
     uploader = std::thread([&] {
-      int urc = upload_slices(ix, seqs, offs, packed ? 0 : base, bytes, rb, trace, packed, &h2d_bytes);
+      int urc = up.upload(seqs, packed ? 0 : base, bytes, trace, &h2d_bytes);
       if (urc != 0) {
-        ix->upload_msg = last_error_cstr();
-        ix->upload_rc.store(urc, std::memory_order_release);
+        up.upload_msg = last_error_cstr();
+        up.upload_rc.store(urc, std::memory_order_release);
       }
     });
   } else {
@@ -297,19 +308,13 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   const mtsvgpu_hit* d_hits = nullptr;
   const uint64_t* d_hit_off = nullptr;
   uint64_t n_hits = 0;
-  ix->sub_batch_hook = wait_for_sub_batch_input;
   // overlap the result copy when the pinned buffers from earlier batches are big enough for this one
-  ix->out_copied_hits = ix->out_copied_reads = 0;
-  ix->out_overlap_ok = pinned_result && ix->pin_hits && ix->pin_off &&
-                       (n_reads + 1) * sizeof(uint64_t) <= ix->pin_off_cap;
-  ix->results_hook = ix->out_overlap_ok ? copy_results_slice : nullptr;
+  up.out_overlap_ok = pinned_result && ix->pin_hits && ix->pin_off &&
+                      (n_reads + 1) * sizeof(uint64_t) <= ix->pin_off_cap;
   // a device-side regrowth of the output buffer would invalidate copies in flight: reserve generously
-  if (ix->out_overlap_ok) (void)ws.out_hits.reserve(ix->pin_hits_cap);
-  int rc = bin_batch_device(ix, ws.d_seqs.as<uint8_t>(), ws.d_seq_off.as<uint64_t>(), n_reads, offs, params,
+  if (up.out_overlap_ok) (void)ws.out_hits.reserve(ix->pin_hits_cap);
+  int rc = bin_batch_device(ix, ws.d_seqs.as<uint8_t>(), ws.d_seq_off.as<uint64_t>(), n_reads, &up, params,
                             &d_hits, &d_hit_off, &n_hits);
-  ix->sub_batch_hook = nullptr;
-  ix->results_hook = nullptr;
-  ix->packed_input = false;
   if (uploader.joinable()) uploader.join();
   ix->stats.h2d_bytes = h2d_bytes;
   if (rc != 0) {
@@ -339,11 +344,9 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
       return set_error(MTSVGPU_ENOMEM, "host allocation of the result failed");
     }
   }
-  cudaError_t e = cudaSuccess;
-  if (pinned_result && ix->out_overlap_ok && ix->out_copied_hits == n_hits && ix->out_copied_reads == n_reads) {
-    e = cudaStreamSynchronize(ix->copy_out_stream);  // everything was copied slice by slice
-  } else {
-    e = cudaStreamSynchronize(ix->copy_out_stream);
+  cudaError_t e = cudaStreamSynchronize(ix->copy_out_stream);
+  // (nothing more to copy when everything was copied slice by slice)
+  if (!(pinned_result && up.out_overlap_ok && up.out_copied_hits == n_hits && up.out_copied_reads == n_reads)) {
     if (e == cudaSuccess && n_hits)
       e = cudaMemcpyAsync(h_hits, d_hits, n_hits * sizeof(mtsvgpu_hit), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_off, d_hit_off, ob, cudaMemcpyDeviceToHost, st);
@@ -367,13 +370,13 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
       cudaEventElapsedTime(&a, g_trace_t0, g_trace_landed[i]);
       cudaEventElapsedTime(&b, g_trace_t0, g_trace_started[i]);
       fprintf(stderr, "[mtsv_b200 trace]   %2llu: %8llu  %7.2f  %7.2f\n", (unsigned long long)i,
-              (unsigned long long)(rb[i + 1] - rb[i]), a, b);
+              (unsigned long long)(up.bounds[i + 1] - up.bounds[i]), a, b);
     }
   }
   if (trace)
     fprintf(stderr, "[mtsv_b200 trace] bin_batch_host: enqueue H2D %.2f ms, compute %.2f ms, tail (D2H rest) %.2f ms, "
                     "overlapped D2H %s\n", t_enq - t_begin, t_comp - t_enq, now() - t_comp,
-            ix->out_overlap_ok ? "yes" : "no");
+            up.out_overlap_ok ? "yes" : "no");
   return 0;
 }
 

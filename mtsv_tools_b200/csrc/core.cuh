@@ -1193,12 +1193,10 @@ MTSV_HD uint32_t select_item(const BinsView& bv, const Params& p, const CandRec*
 // ---------------------------------------------------------------------------------------------
 // host-side schedule (no device code; here so that tests/emul can check it)
 // ---------------------------------------------------------------------------------------------
-// Read boundaries of the device sub-batches of one batch call.  Device-resident input: equal slices of `step`
-// reads.  Host input (ramp): the slices are uploaded one by one while earlier ones compute, so the call lasts
-// about (upload of everything) + (upload of the first slice) + (compute of the last slice): the first slices
-// grow geometrically from step/16 and the last ones shrink to step/8.  Shared by capi.cu (uploads) and
-// binner.cu (compute) so that they agree.
-constexpr uint64_t kDefaultStepDevice = 1ull << 22, kDefaultStepHost = 1ull << 20;
+// Read boundaries of slices of at most `step` reads.  Without the ramp: equal slices of `step` reads.  With the
+// ramp (host input): the slices are uploaded one by one while earlier ones compute, so the call lasts about
+// (upload of everything) + (upload of the first slice) + (compute of the last slice): the first slices grow
+// geometrically from step/16 and the last ones shrink to step/8.
 inline std::vector<uint64_t> sub_batch_bounds(uint64_t n_reads, uint64_t step, bool ramp) {
   std::vector<uint64_t> b{0};
   if (step == 0) step = 1;
@@ -1224,6 +1222,24 @@ inline std::vector<uint64_t> sub_batch_bounds(uint64_t n_reads, uint64_t step, b
     }
     while (r < n_reads) b.push_back(r = std::min(n_reads, r + step));
   }
+  return b;
+}
+
+// The slices of one batch call, for the uploader of host input and the compute lanes alike.  step = reads per slice,
+// 0 for the default of the input's kind.  Host input: the ramped slices above.  Device-resident input: k = ceil(n /
+// step) slices of equal size; with two lanes an even number, so that both lanes get the same share, and a batch that
+// fits one slice is still cut in two when it is large enough (kSplitMinReads: +3 % at 2.5 M reads; at 1.25 M reads
+// the halves gain 3 % on an idle host and lose as much with eight ranks' threads competing for it).  Bound i is
+// min(n, i * ceil(n / k)), so the last slice can be empty.
+constexpr uint64_t kDefaultStepDevice = 1ull << 22, kDefaultStepHost = 1ull << 20, kSplitMinReads = 1ull << 21;
+inline std::vector<uint64_t> slice_bounds(uint64_t n_reads, uint64_t step, bool host_input, bool two_lanes) {
+  if (step == 0) step = host_input ? kDefaultStepHost : kDefaultStepDevice;
+  if (host_input) return sub_batch_bounds(n_reads, step, true);
+  uint64_t k = (n_reads + step - 1) / step;
+  if (two_lanes && ((k >= 2 && (k & 1)) || (k == 1 && n_reads >= kSplitMinReads))) ++k;
+  const uint64_t stride = k ? (n_reads + k - 1) / k : step;
+  std::vector<uint64_t> b{0};
+  for (uint64_t i = 1; i <= k; ++i) b.push_back(std::min(n_reads, i * stride));
   return b;
 }
 

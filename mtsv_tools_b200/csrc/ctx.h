@@ -140,8 +140,6 @@ struct BatchWorkspace {
   DevBuf enc;
   // scan scratch, counters, worklists
   DevBuf scan_tmp, counters, worklist;
-  // per sub-batch results before concatenation
-  DevBuf sub_hits, sub_hit_off;
   // whole-batch results (device-resident API)
   DevBuf out_hits, out_hit_off;
   // staged inputs for the host API
@@ -168,6 +166,19 @@ struct Lane {
   size_t ev_next = 0;
 };
 
+// What the host API knows about a batch that bin_batch_device computes from device buffers it is still filling (none
+// for device-resident input: a null source).  The uploader writes pack_base[i] before it lets wait_slice(i) return.
+struct BatchSource {
+  const uint64_t* seq_off = nullptr;  // host copy of the device seq_off
+  std::vector<uint64_t> bounds;       // read boundaries of the slices (slice_bounds)
+  std::vector<uint64_t> pack_base;    // packed records: byte offset of each slice's first record; empty: raw bytes
+  // before slice i is computed: wait until it has landed, ordering `stream` after its upload
+  virtual int wait_slice(uint64_t i, cudaStream_t stream) = 0;
+  // after a sub-batch's results are enqueued on `stream`
+  virtual int results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads,
+                      cudaStream_t stream) = 0;
+};
+
 }  // namespace mtsv
 
 struct mtsvgpu_index {
@@ -190,22 +201,9 @@ struct mtsvgpu_index {
   mtsvgpu_batch_stats stats{};
   // host API: copy streams, per-sub-batch "input landed" events, pinned result buffers
   cudaStream_t copy_in_stream = nullptr;
-  std::atomic<uint64_t> slices_enqueued{0};  // host API: slices whose upload has been enqueued (uploader thread)
-  std::atomic<int> upload_rc{0};
-  std::string upload_msg;
   std::vector<cudaEvent_t> in_events;
-  // host API, packed input (mtsvgpu_bin_batch_packed): d_seqs holds packed records; byte offset of each slice's
-  // first record (filled by the uploader before the slice is announced)
-  bool packed_input = false;
-  std::vector<uint64_t> pack_slice_base;
-  // called before each slice on the stream that will compute it
-  int (*sub_batch_hook)(mtsvgpu_index*, uint64_t, cudaStream_t) = nullptr;
-  // called after each sub-batch's results are enqueued on `stream`: (first hit, #hits, first read, #reads, stream)
-  int (*results_hook)(mtsvgpu_index*, uint64_t, uint64_t, uint64_t, uint64_t, cudaStream_t) = nullptr;
   cudaStream_t copy_out_stream = nullptr;
   cudaEvent_t out_event = nullptr;
-  uint64_t out_copied_hits = 0, out_copied_reads = 0;  // prefix already on its way to the pinned buffers
-  bool out_overlap_ok = false;
   void* pin_hits = nullptr;
   size_t pin_hits_cap = 0;
   void* pin_off = nullptr;
@@ -244,7 +242,7 @@ int index_export(mtsvgpu_index* h, uint8_t* text_out, uint8_t* bwt_out, uint64_t
 int suffix_array_host(int device, const uint8_t* text, uint64_t n, uint32_t* sa_out, uint8_t* bwt_out);
 // binner.cu
 int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_seq_off,
-                     uint64_t n_reads, const uint64_t* h_seq_off_or_null,
+                     uint64_t n_reads, BatchSource* src,
                      const mtsvgpu_params* params, const mtsvgpu_hit** d_hits,
                      const uint64_t** d_hit_off, uint64_t* n_hits);
 int backward_search_batch(mtsvgpu_index* h, const uint8_t* pats, uint32_t pat_len, uint64_t n_pats,

@@ -361,10 +361,6 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   }
   if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
   MTSV_CUDA_TRY(cudaSetDevice(device));
-  if (const char* g = getenv("MTSV_B200_L2_FETCH")) {  // experiment knob: L2 fetch granularity hint
-    cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(g));
-    (void)cudaGetLastError();
-  }
 
   mtsvgpu_index* h = new mtsvgpu_index;
   if (opts) h->opts = *opts;

@@ -69,7 +69,7 @@ void BatchWorkspace::release_all() {
   DevBuf* all[] = {&slot_off, &q_nseeds, &q_nhits, &hit_off,  &q_ncand,    &cand_off,   &q_nout,
                    &out_off,  &slot_q,   &slot_lo, &slot_cnt, &slot_hoff,  &hit_keys,   &cand_sparse,
                    &cand_stage, &cand_dense, &cand_q, &cand_edit, &hit_tmp, &scan_tmp,   &counters,
-                   &worklist, &sub_hits, &sub_hit_off, &out_hits, &out_hit_off, &d_seqs, &d_seq_off,
+                   &worklist, &out_hits, &out_hit_off, &d_seqs, &d_seq_off,
                    &cand_flag, &cand_order, &enc, &cand_end, &ssw_list, &ssw_scratch, &pack_rel, &cand_lead, &cand_order2};
   for (DevBuf* b : all) b->release();
 }

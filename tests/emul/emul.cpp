@@ -449,6 +449,14 @@ uint32_t emul_sub_batch_bounds(uint64_t n_reads, uint64_t step, int ramp, uint64
   return (uint32_t)b.size();
 }
 
+// the slices one batch call computes (core.cuh::slice_bounds); returns the number of boundaries
+uint32_t emul_slice_bounds(uint64_t n_reads, uint64_t step, int host_input, int two_lanes, uint64_t* out,
+                           uint32_t cap) {
+  std::vector<uint64_t> b = slice_bounds(n_reads, step, host_input != 0, two_lanes != 0);
+  for (size_t i = 0; i < b.size() && i < cap; ++i) out[i] = b[i];
+  return (uint32_t)b.size();
+}
+
 // packed reads: the device's unpacker (core.cuh::unpack_word) applied to a record, next to the planes the device
 // computes from the raw bytes (encode_fwd_word).  out: W words of {lo, hi, nn} for each of the two routes.
 // `from_record`: a record made elsewhere (the product's AVX2 / SWAR packer); NULL = core.cuh::pack_read.

@@ -67,6 +67,8 @@ def lib():
                                          C.POINTER(C.c_uint32)]
     L.emul_sub_batch_bounds.restype = C.c_uint32
     L.emul_sub_batch_bounds.argtypes = [C.c_uint64, C.c_uint64, C.c_int, C.POINTER(C.c_uint64), C.c_uint32]
+    L.emul_slice_bounds.restype = C.c_uint32
+    L.emul_slice_bounds.argtypes = [C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_uint64), C.c_uint32]
     L.emul_ssw_accepts.restype = C.c_uint32
     L.emul_ssw_accepts.argtypes = [C.c_char_p, C.c_uint32, C.c_char_p, C.c_uint32, C.c_uint32, C.c_uint32,
                                    C.c_uint32, C.c_int]
@@ -172,6 +174,13 @@ def sub_batch_bounds(n_reads, step, ramp):
     """Read boundaries of the device slices of one batch call (core.cuh::sub_batch_bounds)."""
     buf = (C.c_uint64 * 4096)()
     n = lib().emul_sub_batch_bounds(n_reads, step, int(ramp), buf, 4096)
+    return [int(buf[i]) for i in range(min(n, 4096))]
+
+
+def slice_bounds(n_reads, step, host_input, two_lanes):
+    """Read boundaries of the slices one batch call computes (core.cuh::slice_bounds); step 0 = the default."""
+    buf = (C.c_uint64 * 4096)()
+    n = lib().emul_slice_bounds(n_reads, step, int(host_input), int(two_lanes), buf, 4096)
     return [int(buf[i]) for i in range(min(n, 4096))]
 
 

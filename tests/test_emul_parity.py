@@ -292,7 +292,9 @@ def test_pipeline_reads_of_254_bases_and_more(oracle, emul, small_ref, small_ind
 
 def test_slice_schedule(emul):
     """The slices of one batch call: cover the reads exactly once, in order, never longer than the step;
-    with host input short first and last slices (the call lasts upload + first upload + last compute)."""
+    with host input short first and last slices (the call lasts upload + first upload + last compute).
+    Device-resident input: ceil(n / step) slices of equal size; with two lanes an even number of them, and a
+    batch of 2^21 reads or more that fits one slice is cut in two."""
     rng = random.Random(3)
     for _ in range(2000):
         n = rng.choice([0, 1, 2, rng.randint(0, 5000), rng.randint(0, 3 << 20), rng.randint(0, 40 << 20)])
@@ -306,9 +308,29 @@ def test_slice_schedule(emul):
             assert all(0 < s <= step for s in sizes), (n, step, ramp, sizes[:8])
             if not ramp:
                 assert all(s == step for s in sizes[:-1])
+        assert emul.slice_bounds(n, step, True, True) == emul.sub_batch_bounds(n, step, True)
+        for two_lanes in (False, True):
+            b = emul.slice_bounds(n, step, False, two_lanes)
+            assert b[0] == 0 and b[-1] == n and all(x <= y for x, y in zip(b, b[1:]))
+            k = -(-n // step)
+            if two_lanes and ((k >= 2 and k % 2) or (k == 1 and n >= 1 << 21)):
+                k += 1
+            assert len(b) == k + 1, (n, step, two_lanes, len(b))
+            stride = -(-n // k) if k else 0
+            assert b == [min(n, i * stride) for i in range(k + 1)], (n, step, two_lanes)
     b = emul.sub_batch_bounds(10_000_000, 1 << 20, True)
     sizes = [y - x for x, y in zip(b, b[1:])]
     assert sizes[0] == 1 << 16 and sizes[-1] == 1 << 17 and max(sizes) <= 1 << 20
+    # an odd slice count is made even, the last slice can then be empty
+    assert emul.slice_bounds(5, 2, False, True) == [0, 2, 4, 5, 5]
+    assert emul.slice_bounds(5, 2, False, False) == [0, 2, 4, 5]
+    assert emul.slice_bounds((1 << 21) - 1, 1 << 22, False, True) == [0, (1 << 21) - 1]
+    assert emul.slice_bounds(1 << 21, 1 << 22, False, True) == [0, 1 << 20, 1 << 21]
+    # step 0: 2^22 reads per slice for device-resident input, 2^20 (ramped) for host input
+    for n in (0, 5, 3 << 20, 9 << 22):
+        for two_lanes in (False, True):
+            assert emul.slice_bounds(n, 0, False, two_lanes) == emul.slice_bounds(n, 1 << 22, False, two_lanes)
+        assert emul.slice_bounds(n, 0, True, True) == emul.sub_batch_bounds(n, 1 << 20, True)
 
 
 CASES = [

@@ -315,11 +315,11 @@ def test_pipeline_n_rich_reference(oracle):
             assert len(h1) > 500
 
 
-def test_verifier_fast_and_legacy_paths_agree(oracle, small_ref, small_index):
+def test_warp_and_per_lane_verifiers_match_the_oracle(oracle, small_ref, small_index):
     """Batches whose reads all have at most 253 bases go through verify_warp_kernel (warp-uniform block range, 4-bit
-    text); the per-lane verify_kernel (+ SW re-check) takes the others.  Both must give the oracle's hits on
-    uniform batches (1, 3 and 4 words; 256 bases = the per-lane path either way) and on a ragged one (mutated
-    reads of 1..253 bases so that the edit budget is actually used)."""
+    text); the per-lane verify_kernel (+ SW re-check) takes the others.  Both must give the oracle's hits: the warp
+    verifier on uniform batches (1, 3 and 4 words) and on a ragged one (mutated reads of 1..253 bases so that the
+    edit budget is actually used), the per-lane one on a uniform batch of 256 bases."""
     rng = np.random.default_rng(21)
     ref = small_ref[0]
     batches = {"uniform_150": synth.make_reads(small_ref[0], small_ref[1], 4000, 150, seed=31, sub=0.05),
@@ -335,23 +335,14 @@ def test_verifier_fast_and_legacy_paths_agree(oracle, small_ref, small_index):
             s[int(rng.integers(0, L))] = b"ACGTN"[int(rng.integers(0, 5))]
         rl.append(bytes(s))
     batches["ragged"] = oracle.pack_seqs(rl)
-    old = os.environ.get("MTSV_B200_VERIFIER")
-    try:
-        with _gpu_index(small_index) as g:
-            for name, reads in batches.items():
-                for flags in ({}, dict(edit_rate=0.2, seed_gap=5), dict(edit_rate=0.05)):
-                    po, pg = _params(oracle, **flags)
-                    h1, o1 = small_index.bin_reads(reads, po, threads=8)
-                    assert len(h1) > 100, name
-                    for mode in ("warp", "legacy"):
-                        os.environ["MTSV_B200_VERIFIER"] = mode
-                        h2, o2 = g.bin_reads(reads, pg)
-                        _same(h1, o1, h2, o2)
-    finally:
-        if old is None:
-            os.environ.pop("MTSV_B200_VERIFIER", None)
-        else:
-            os.environ["MTSV_B200_VERIFIER"] = old
+    with _gpu_index(small_index) as g:
+        for name, reads in batches.items():
+            for flags in ({}, dict(edit_rate=0.2, seed_gap=5), dict(edit_rate=0.05)):
+                po, pg = _params(oracle, **flags)
+                h1, o1 = small_index.bin_reads(reads, po, threads=8)
+                assert len(h1) > 100, name
+                h2, o2 = g.bin_reads(reads, pg)
+                _same(h1, o1, h2, o2)
 
 
 def test_pipeline_reads_longer_than_253(oracle, small_ref, small_index):
