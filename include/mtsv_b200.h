@@ -61,6 +61,13 @@ typedef struct {
   uint32_t reserved;
 } mtsvgpu_hit;
 
+/* One read's assignment to a TaxID with the minimum edit of its hits there: what the default results format
+ * prints as `TaxID=edit` (write_assignments, src/binner.rs:330-352) and what mtsv-collapse mode TaxId keeps. */
+typedef struct {
+  uint32_t tax_id;
+  uint32_t edit;
+} mtsvgpu_taxhit;
+
 /* `Bin` — src/index.rs:44-54 (same field order as the bincode record). */
 typedef struct {
   uint32_t gi;
@@ -108,7 +115,7 @@ typedef struct {
   double build_seconds;    /* mtsvgpu_index_build only: text assembly + suffix array + BWT */
 } mtsvgpu_index_info;
 
-/* Per-stage device time of the last mtsvgpu_bin_batch*(), CUDA events on the launch stream (ms). */
+/* Per-stage device time of the last mtsvgpu_bin_batch*() or mtsvgpu_assign_batch*(), CUDA events on the launch stream (ms). */
 #define MTSVGPU_N_STAGES 12
 typedef struct {
   float ms[MTSVGPU_N_STAGES];
@@ -186,6 +193,25 @@ MTSVGPU_API int mtsvgpu_bin_batch_device(mtsvgpu_index* ix, const uint8_t* d_seq
 MTSVGPU_API int mtsvgpu_bin_batch_packed(mtsvgpu_index* ix, const uint8_t* packed, uint64_t packed_bytes,
                              const uint64_t* seq_off, uint64_t n_reads, const mtsvgpu_params* params,
                              const mtsvgpu_hit** hits, const uint64_t** hit_off, uint64_t* n_hits);
+/* ---- the default results format computed on the device ----
+ * The same batches as the three calls above with a smaller output: per read each TaxID that the matching
+ * mtsvgpu_bin_batch_* call returns a hit for (on either strand) appears once, with the minimum edit of those hits,
+ * by ascending TaxID — exactly the `TaxID=edit` list write_assignments prints (src/binner.rs:330-352); a read
+ * without hits gets an empty range.  8 bytes per record instead of 24 per hit, and fewer records where both
+ * strands hit a TaxID.  Output is CSR by read: records of read i are (*out)[(*out_off)[i] .. (*out_off)[i+1]),
+ * *n_out records in all.  Inputs, ownership and lifetimes are those of the matching mtsvgpu_bin_batch_* call: the
+ * pinned and packed results live in the handle's page-locked buffers and the device results in its device
+ * buffers, until the next batch call of either kind on the handle.  mtsvgpu_last_batch_stats reports the call as
+ * for a bin call (n_hits counts the Hit records before the merge). */
+MTSVGPU_API int mtsvgpu_assign_batch_device(mtsvgpu_index* ix, const uint8_t* d_seqs, const uint64_t* d_seq_off,
+                                uint64_t n_reads, const mtsvgpu_params* params,
+                                const mtsvgpu_taxhit** d_out, const uint64_t** d_out_off, uint64_t* n_out);
+MTSVGPU_API int mtsvgpu_assign_batch_pinned(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off,
+                                uint64_t n_reads, const mtsvgpu_params* params,
+                                const mtsvgpu_taxhit** out, const uint64_t** out_off, uint64_t* n_out);
+MTSVGPU_API int mtsvgpu_assign_batch_packed(mtsvgpu_index* ix, const uint8_t* packed, uint64_t packed_bytes,
+                                const uint64_t* seq_off, uint64_t n_reads, const mtsvgpu_params* params,
+                                const mtsvgpu_taxhit** out, const uint64_t** out_off, uint64_t* n_out);
 /* Host helpers of the packed format (no GPU involved).  mtsvgpu_packed_size: bytes of the records of n_reads reads.
  * mtsvgpu_pack_reads: raw read bytes -> records, on `threads` host threads (0 = all); *packed_bytes gets the size. */
 MTSVGPU_API uint64_t mtsvgpu_packed_size(const uint64_t* seq_off, uint64_t n_reads);
@@ -227,10 +253,6 @@ MTSVGPU_API int mtsvgpu_edit_distance(int device, const uint8_t* pats, const uin
  * of per-read counts (u32); the result lists, per read, each TaxID once with its minimum edit, by
  * ascending TaxID (write_collapsed_taxid, src/collapse.rs:278-279).  *d_out / *d_out_off are device
  * allocations released with mtsvgpu_device_free().  stream: a cudaStream_t or NULL. */
-typedef struct {
-  uint32_t tax_id;
-  uint32_t edit;
-} mtsvgpu_taxhit;
 MTSVGPU_API int mtsvgpu_collapse_device(int device, void* stream, uint32_t n_parts,
                             const mtsvgpu_hit* const* d_hits, const uint32_t* const* d_counts,
                             uint64_t n_reads, mtsvgpu_taxhit** d_out, uint64_t** d_out_off, uint64_t* n_out);

@@ -26,6 +26,10 @@ class HitStruct(C.Structure):
                 ("edit", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+class TaxHitStruct(C.Structure):
+    _fields_ = [("tax_id", C.c_uint32), ("edit", C.c_uint32)]
+
+
 class BinStruct(C.Structure):
     _fields_ = [("gi", C.c_uint32), ("tax_id", C.c_uint32), ("start", C.c_uint64), ("end", C.c_uint64)]
 
@@ -60,7 +64,7 @@ class StatsStruct(C.Structure):
 # every symbol include/mtsv_b200.h declares
 EXPORTS = [
     "mtsvgpu_index_open", "mtsvgpu_index_from_parts", "mtsvgpu_index_build", "mtsvgpu_index_write", "mtsvgpu_index_export", "mtsvgpu_suffix_array", "mtsvgpu_index_close", "mtsvgpu_index_get_info",
-    "mtsvgpu_bin_batch", "mtsvgpu_bin_batch_pinned", "mtsvgpu_bin_batch_device", "mtsvgpu_bin_batch_packed", "mtsvgpu_packed_size", "mtsvgpu_pack_reads", "mtsvgpu_pack_read", "mtsvgpu_host_alloc", "mtsvgpu_host_free", "mtsvgpu_last_batch_stats", "mtsvgpu_set_stream",
+    "mtsvgpu_bin_batch", "mtsvgpu_bin_batch_pinned", "mtsvgpu_bin_batch_device", "mtsvgpu_bin_batch_packed", "mtsvgpu_assign_batch_device", "mtsvgpu_assign_batch_pinned", "mtsvgpu_assign_batch_packed", "mtsvgpu_packed_size", "mtsvgpu_pack_reads", "mtsvgpu_pack_read", "mtsvgpu_host_alloc", "mtsvgpu_host_free", "mtsvgpu_last_batch_stats", "mtsvgpu_set_stream",
     "mtsvgpu_set_profiling", "mtsvgpu_backward_search", "mtsvgpu_locate", "mtsvgpu_edit_distance",
     "mtsvgpu_collapse_device", "mtsvgpu_collapse_device_taxid_gi", "mtsvgpu_device_free", "mtsvgpu_comm_create", "mtsvgpu_comm_connect", "mtsvgpu_comm_destroy", "mtsvgpu_bin_batch_chunked", "mtsvgpu_free", "mtsvgpu_last_error", "mtsvgpu_launch_count", "mtsvgpu_version",
 ]
@@ -107,6 +111,9 @@ def load_library():
                                            C.POINTER(vp), C.POINTER(vp), u64p]
     L.mtsvgpu_bin_batch_packed.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(ParamsStruct),
                                            C.POINTER(vp), C.POINTER(vp), u64p]
+    L.mtsvgpu_assign_batch_device.argtypes = L.mtsvgpu_bin_batch_device.argtypes
+    L.mtsvgpu_assign_batch_pinned.argtypes = L.mtsvgpu_bin_batch_pinned.argtypes
+    L.mtsvgpu_assign_batch_packed.argtypes = L.mtsvgpu_bin_batch_packed.argtypes
     L.mtsvgpu_packed_size.restype = C.c_uint64
     L.mtsvgpu_packed_size.argtypes = [vp, C.c_uint64]
     L.mtsvgpu_pack_reads.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, u64p, C.c_int]

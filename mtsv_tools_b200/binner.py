@@ -34,3 +34,16 @@ def results_lines(names, hits, hit_off, long_info_output=False):
         if b > a:
             out.append(format_assignments(name, hits[a:b], long_info_output))
     return out
+
+
+def assignment_lines(names, taxhits, off):
+    """Default-format lines of a whole batch from the merged records of MGIndex.assign_reads* (each TaxID of a read
+    once with its minimum edit, by ascending TaxID): the lines that results_lines(..., long_info_output=False) gives
+    for the hits of the matching bin_reads* call."""
+    out = []
+    for i, name in enumerate(names):
+        a, b = int(off[i]), int(off[i + 1])
+        if b > a:
+            body = ",".join("%d=%d" % (int(t["tax_id"]), int(t["edit"])) for t in taxhits[a:b])
+            out.append("%s:%s\n" % (name, body))
+    return out

@@ -1327,6 +1327,63 @@ __global__ void __launch_bounds__(256) gather_hits_kernel(uint32_t nq, uint32_t 
   }
 }
 
+// ---- assignments output: each read's selected hits of both strands merged into (TaxID, edit) records ----
+// The selected hits of strand q (hit_tmp at cand_off[q], compacted to out_off[q]) become keys tax << 32 | edit; the
+// strands of read r are queries r*ns .. r*ns+ns-1, so read r's keys are the segment [seg_off[r], seg_off[r + 1]).
+__global__ void __launch_bounds__(256) taxid_keys_kernel(uint32_t nq, uint32_t ns,
+                                                         const uint32_t* __restrict__ cand_off,
+                                                         const uint32_t* __restrict__ out_off,
+                                                         const HitRec* __restrict__ hit_tmp,
+                                                         uint64_t* __restrict__ keys, uint32_t* __restrict__ seg_off,
+                                                         uint32_t* __restrict__ seg_cnt) {
+  uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+  const unsigned lane = threadIdx.x & 31;
+  if (q <= nq && q % ns == 0) {
+    seg_off[q / ns] = out_off[q];  // q == nq: the end
+    if (q < nq) seg_cnt[q / ns] = out_off[q + ns] - out_off[q];
+  }
+  uint32_t n = 0, src = 0, dst = 0;
+  if (q < nq) {
+    n = out_off[q + 1] - out_off[q];
+    src = cand_off[q];
+    dst = out_off[q];
+    if (n <= kLightItems)
+      for (uint32_t i = 0; i < n; ++i)
+        keys[dst + i] = ((uint64_t)hit_tmp[src + i].tax_id << 32) | hit_tmp[src + i].edit;
+  }
+  unsigned heavy = __ballot_sync(0xffffffffu, n > kLightItems);
+  while (heavy) {
+    int sl = __ffs(heavy) - 1;
+    heavy &= heavy - 1;
+    uint32_t n_s = __shfl_sync(0xffffffffu, n, sl), src_s = __shfl_sync(0xffffffffu, src, sl);
+    uint32_t dst_s = __shfl_sync(0xffffffffu, dst, sl);
+    for (uint32_t i = lane; i < n_s; i += 32)
+      keys[dst_s + i] = ((uint64_t)hit_tmp[src_s + i].tax_id << 32) | hit_tmp[src_s + i].edit;
+  }
+}
+
+// records per read, after the segments have been sorted
+__global__ void __launch_bounds__(256) taxid_count_kernel(const uint64_t* __restrict__ keys,
+                                                          const uint32_t* __restrict__ seg_off, uint32_t n_reads,
+                                                          uint32_t* __restrict__ n_out) {
+  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_reads) return;
+  n_out[r] = taxid_count(keys, seg_off[r], seg_off[r + 1]);
+}
+
+// appends the sub-batch's records to the batch output at out_base; read offsets go to out_off from read_base on
+__global__ void __launch_bounds__(256) taxid_write_kernel(const uint64_t* __restrict__ keys,
+                                                          const uint32_t* __restrict__ seg_off,
+                                                          const uint32_t* __restrict__ tax_off, uint32_t n_reads,
+                                                          mtsvgpu_taxhit* __restrict__ out, uint64_t out_base,
+                                                          uint64_t* __restrict__ out_off, uint64_t read_base) {
+  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r > n_reads) return;
+  out_off[read_base + r] = out_base + tax_off[r];  // r == n_reads: the end
+  if (r == n_reads) return;
+  taxid_write(keys, seg_off[r], seg_off[r + 1], out + out_base, tax_off[r]);
+}
+
 // verification order: multi-seed candidates first, single-seed ones after (stable within each class)
 __global__ void cand_class_kernel(const CandRec* __restrict__ cand, uint32_t n, uint32_t* __restrict__ flag,
                                   BatchCounters* __restrict__ ctr, int write_flags) {
@@ -1574,6 +1631,7 @@ struct BatchCall {
   const uint64_t* d_seq_off;
   BatchSource* src;  // null: device-resident input
   const char* group_verify;  // MTSV_B200_GROUP_VERIFY: unset = where it pays, "0" = never, anything else = always
+  BatchOutput kind;
 };
 
 // One device sub-batch, reads [rv.read0, rv.read0 + rv.n_reads), as it passes through the stages below.  A stage
@@ -1638,7 +1696,14 @@ struct SubBatch : BatchCall {
   int launch_verify_warp(const BinnerJobs& jobs);
   int verify_ssw(const BinnerJobs& jobs);
   int verify_grouped(const BinnerJobs& jobs, bool* done);
+  int merge_taxids();
   int select_append(uint64_t* out_total);
+  // assignments output, per read: the segment of its keys, its record count and record offset.  These reuse
+  // per-strand buffers that are dead once the candidates are ranked (each holds nq + 1 >= n_reads + 1 entries).
+  uint32_t* seg_off() const { return ws.hit_off.as<uint32_t>(); }
+  uint32_t* seg_cnt() const { return ws.q_nhits.as<uint32_t>(); }
+  uint32_t* tax_cnt() const { return ws.q_nseeds.as<uint32_t>(); }
+  uint32_t* tax_off() const { return ws.q_ncand.as<uint32_t>(); }
 };
 
 // ---- seed slots, then the reads' bit planes ----
@@ -1891,10 +1956,25 @@ int SubBatch::verify_grouped(const BinnerJobs& jobs, bool* done) {
   return 0;
 }
 
+// ---- assignments output: sort each read's keys and count its TaxIDs (before the sub-batch's scalars are fetched,
+// so that the host learns the record total from the synchronisation the selection already makes).  The keys go to
+// hit_keys, dead since coalesce: n_out <= n_cand <= n_hits keys. ----
+int SubBatch::merge_taxids() {
+  const uint32_t nr = rv.n_reads;
+  uint64_t* keys = ws.hit_keys.as<uint64_t>();
+  MTSV_LAUNCH(taxid_keys_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
+              ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), keys, seg_off(), seg_cnt());
+  MTSV_TRY(run_segmented_sort(st, ws.worklist, keys, seg_off(), seg_cnt(), nr, 1, d_ctr));
+  MTSV_LAUNCH(taxid_count_kernel, (nr + 255) / 256, 256, 0, st, keys, seg_off(), nr, tax_cnt());
+  MTSV_TRY(exclusive_scan_u32(tax_cnt(), tax_off(), nr, ws.scan_tmp, (uint64_t*)&d_ctr->total_taxhits, st));
+  return 0;
+}
+
 // ---- select, then append to the batch output: in slice order, after the other lane's previous append ----
 int SubBatch::select_append(uint64_t* out_total) {
   for (DevBuf* b : {&ws.q_nout, &ws.out_off}) MTSV_TRY(b->reserve(qn * 4));
-  uint64_t sub_out = 0;
+  const bool taxhits = kind == BatchOutput::TaxHits;
+  uint64_t sub_out = 0, sub_tax = 0;
   if (n_cand) {
     MTSV_TRY(ws.hit_tmp.reserve((size_t)n_cand * sizeof(HitRec)));
     begin(ST_EMIT);
@@ -1903,11 +1983,16 @@ int SubBatch::select_append(uint64_t* out_total) {
                 ws.q_nout.as<uint32_t>());
     MTSV_TRY(exclusive_scan_u32(ws.q_nout.as<uint32_t>(), ws.out_off.as<uint32_t>(), nq, ws.scan_tmp,
                                 (uint64_t*)&d_ctr->total_out, st));
+    if (taxhits) MTSV_TRY(merge_taxids());
     end();
     MTSV_TRY(fetch());
     sub_out = hc.total_out;
+    sub_tax = hc.total_taxhits;
     ln.stats.n_candidates += n_verified;
     for (int i = 0; i < 32; ++i) ln.stats.window_bytes += hc.window_bytes[i];
+  } else if (taxhits) {  // no keys: every read gets an empty range
+    MTSV_CUDA_TRY(cudaMemsetAsync(seg_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
+    MTSV_CUDA_TRY(cudaMemsetAsync(tax_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
   } else {
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_off.p, 0, qn * 4, st));
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_off.p, 0, qn * 4, st));
@@ -1916,19 +2001,27 @@ int SubBatch::select_append(uint64_t* out_total) {
   Lane& other = h->lanes[&ln == &h->lanes[0] ? 1 : 0];
   if (other.emit_event) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, other.emit_event, 0));
   BatchWorkspace& res = h->ws;  // batch results (shared, appended in slice order)
-  MTSV_TRY(grow_preserve(res.out_hits, *out_total * sizeof(HitRec), (*out_total + sub_out + 1) * sizeof(HitRec), st));
+  const size_t rec = taxhits ? sizeof(mtsvgpu_taxhit) : sizeof(HitRec);
+  const uint64_t sub_rec = taxhits ? sub_tax : sub_out;
+  MTSV_TRY(grow_preserve(res.out_hits, *out_total * rec, (*out_total + sub_rec + 1) * rec, st));
   begin(ST_EMIT);
-  MTSV_LAUNCH(gather_hits_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
-              ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), res.out_hits.as<HitRec>(), *out_total,
-              res.out_hit_off.as<uint64_t>(), rv.read0);
+  if (taxhits) {
+    MTSV_LAUNCH(taxid_write_kernel, (rv.n_reads + 1 + 255) / 256, 256, 0, st, ws.hit_keys.as<uint64_t>(), seg_off(),
+                tax_off(), rv.n_reads, res.out_hits.as<mtsvgpu_taxhit>(), *out_total, res.out_hit_off.as<uint64_t>(),
+                rv.read0);
+  } else {
+    MTSV_LAUNCH(gather_hits_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
+                ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), res.out_hits.as<HitRec>(), *out_total,
+                res.out_hit_off.as<uint64_t>(), rv.read0);
+  }
   end();
   MTSV_CUDA_TRY(cudaGetLastError());
   if (!ln.emit_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&ln.emit_event, cudaEventDisableTiming));
   MTSV_CUDA_TRY(cudaEventRecord(ln.emit_event, st));
   // host API: start copying this sub-batch's results out while the next one computes
-  if (src) MTSV_TRY(src->results(*out_total, sub_out, rv.read0, rv.n_reads, st));
+  if (src) MTSV_TRY(src->results(*out_total, sub_rec, rv.read0, rv.n_reads, st));
   resolve();
-  *out_total += sub_out;
+  *out_total += sub_rec;
   ln.stats.n_hits += sub_out;
   ln.stats.n_queries += nq;
   return 0;
@@ -2005,10 +2098,10 @@ static void add_stats(mtsvgpu_batch_stats& to, const mtsvgpu_batch_stats& from) 
 }
 
 int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_seq_off, uint64_t n_reads,
-                     BatchSource* src, const mtsvgpu_params* params, const mtsvgpu_hit** d_hits,
-                     const uint64_t** d_hit_off, uint64_t* n_hits) {
+                     BatchSource* src, BatchOutput kind, const mtsvgpu_params* params, const void** d_out,
+                     const uint64_t** d_out_off, uint64_t* n_out) {
   if (!h) return set_error(MTSVGPU_EINVAL, "index is NULL");
-  BatchCall call{h, {}, d_seqs, d_seq_off, src, getenv("MTSV_B200_GROUP_VERIFY")};
+  BatchCall call{h, {}, d_seqs, d_seq_off, src, getenv("MTSV_B200_GROUP_VERIFY"), kind};
   MTSV_TRY(validate_params(params, &call.p));
   if (!d_seq_off) return set_error(MTSVGPU_EINVAL, "seq_off is NULL");
   MTSV_CUDA_TRY(cudaSetDevice(h->ix.device));
@@ -2097,9 +2190,9 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
     return set_error(h->abort_rc, "%s", h->abort_msg.c_str());
   }
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  if (d_hits) *d_hits = reinterpret_cast<const mtsvgpu_hit*>(ws.out_hits.p);
-  if (d_hit_off) *d_hit_off = ws.out_hit_off.as<uint64_t>();
-  if (n_hits) *n_hits = total;
+  if (d_out) *d_out = ws.out_hits.p;
+  if (d_out_off) *d_out_off = ws.out_hit_off.as<uint64_t>();
+  if (n_out) *n_out = total;
   return 0;
 }
 

@@ -91,7 +91,15 @@ int mtsvgpu_last_batch_stats(const mtsvgpu_index* ix, mtsvgpu_batch_stats* stats
 int mtsvgpu_bin_batch_device(mtsvgpu_index* ix, const uint8_t* d_seqs, const uint64_t* d_seq_off,
                              uint64_t n_reads, const mtsvgpu_params* params, const mtsvgpu_hit** d_hits,
                              const uint64_t** d_hit_off, uint64_t* n_hits) {
-  return bin_batch_device(ix, d_seqs, d_seq_off, n_reads, nullptr, params, d_hits, d_hit_off, n_hits);
+  return bin_batch_device(ix, d_seqs, d_seq_off, n_reads, nullptr, BatchOutput::Hits, params, (const void**)d_hits,
+                          d_hit_off, n_hits);
+}
+
+int mtsvgpu_assign_batch_device(mtsvgpu_index* ix, const uint8_t* d_seqs, const uint64_t* d_seq_off, uint64_t n_reads,
+                                const mtsvgpu_params* params, const mtsvgpu_taxhit** d_out, const uint64_t** d_out_off,
+                                uint64_t* n_out) {
+  return bin_batch_device(ix, d_seqs, d_seq_off, n_reads, nullptr, BatchOutput::TaxHits, params, (const void**)d_out,
+                          d_out_off, n_out);
 }
 
 static int ensure_pinned(void** p, size_t* cap, size_t bytes) {
@@ -134,7 +142,8 @@ struct HostUpload : BatchSource {
   std::string upload_msg;
   uint64_t out_copied_hits = 0, out_copied_reads = 0;  // prefix already on its way to the pinned buffers
   bool out_overlap_ok = false;
-  explicit HostUpload(mtsvgpu_index* h) : ix(h) {}
+  size_t rec_bytes;  // result records: mtsvgpu_hit or mtsvgpu_taxhit
+  HostUpload(mtsvgpu_index* h, size_t rec) : ix(h), rec_bytes(rec) {}
   int upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool trace, uint64_t* h2d_bytes);
   int wait_slice(uint64_t i, cudaStream_t st) override;
   int results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads, cudaStream_t st) override;
@@ -156,7 +165,7 @@ int HostUpload::wait_slice(uint64_t i, cudaStream_t st) {
 // of earlier batches); otherwise everything is copied at the end.
 int HostUpload::results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads, cudaStream_t st) {
   if (!out_overlap_ok) return 0;
-  if ((first_hit + n_hits) * sizeof(mtsvgpu_hit) > ix->pin_hits_cap ||
+  if ((first_hit + n_hits) * rec_bytes > ix->pin_hits_cap ||
       (first_read + n_reads + 1) * sizeof(uint64_t) > ix->pin_off_cap || first_hit != out_copied_hits ||
       first_read != out_copied_reads) {
     out_overlap_ok = false;  // does not fit / unexpected order: the caller copies everything at the end
@@ -164,11 +173,11 @@ int HostUpload::results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read
   }
   MTSV_CUDA_TRY(cudaEventRecord(ix->out_event, st));
   MTSV_CUDA_TRY(cudaStreamWaitEvent(ix->copy_out_stream, ix->out_event, 0));
-  const mtsvgpu_hit* d_hits = ix->ws.out_hits.as<mtsvgpu_hit>();
+  const uint8_t* d_recs = ix->ws.out_hits.as<uint8_t>();
   const uint64_t* d_off = ix->ws.out_hit_off.as<uint64_t>();
   if (n_hits)
-    MTSV_CUDA_TRY(cudaMemcpyAsync((mtsvgpu_hit*)ix->pin_hits + first_hit, d_hits + first_hit,
-                                  n_hits * sizeof(mtsvgpu_hit), cudaMemcpyDeviceToHost, ix->copy_out_stream));
+    MTSV_CUDA_TRY(cudaMemcpyAsync((uint8_t*)ix->pin_hits + first_hit * rec_bytes, d_recs + first_hit * rec_bytes,
+                                  n_hits * rec_bytes, cudaMemcpyDeviceToHost, ix->copy_out_stream));
   MTSV_CUDA_TRY(cudaMemcpyAsync((uint64_t*)ix->pin_off + first_read, d_off + first_read,
                                 (n_reads + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out_stream));
   out_copied_hits = first_hit + n_hits;
@@ -247,9 +256,9 @@ int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool 
 // Host-buffer batch: the reads are uploaded sub-batch by sub-batch on a copy stream while earlier
 // sub-batches compute (pass page-locked buffers to get the overlap; pageable ones work, serially).
 // pinned_result: 0 = results in malloc'ed memory (mtsvgpu_free), 1 = in the handle's page-locked
-// buffers, valid until the next batch call on this handle.
+// buffers, valid until the next batch call on this handle.  kind: Hit records or merged (TaxID, edit) records.
 static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off, uint64_t n_reads,
-                          const mtsvgpu_params* params, int pinned_result, mtsvgpu_hit** hits,
+                          const mtsvgpu_params* params, BatchOutput kind, int pinned_result, void** hits,
                           uint64_t** hit_off, uint64_t* n_hits_out, bool packed = false, uint64_t packed_bytes = 0) {
   if (!ix || !seq_off || !hits || !hit_off) return set_error(MTSVGPU_EINVAL, "null argument");
   *hits = nullptr;
@@ -274,7 +283,8 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
     offs = rebased.data();
   }
   // ---- H2D, pipelined per device sub-batch ----
-  HostUpload up(ix);
+  const size_t rec = kind == BatchOutput::TaxHits ? sizeof(mtsvgpu_taxhit) : sizeof(mtsvgpu_hit);
+  HostUpload up(ix, rec);
   up.seq_off = offs;
   up.bounds = slice_bounds(n_reads, ix->opts.batch_reads, true, true);
   const uint64_t n_sub = up.bounds.size() - 1;
@@ -305,7 +315,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   }
   const double t_enq = trace ? now() : 0;
   // ---- compute (each sub-batch waits for its slice) ----
-  const mtsvgpu_hit* d_hits = nullptr;
+  const void* d_hits = nullptr;
   const uint64_t* d_hit_off = nullptr;
   uint64_t n_hits = 0;
   // overlap the result copy when the pinned buffers from earlier batches are big enough for this one
@@ -313,7 +323,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
                       (n_reads + 1) * sizeof(uint64_t) <= ix->pin_off_cap;
   // a device-side regrowth of the output buffer would invalidate copies in flight: reserve generously
   if (up.out_overlap_ok) (void)ws.out_hits.reserve(ix->pin_hits_cap);
-  int rc = bin_batch_device(ix, ws.d_seqs.as<uint8_t>(), ws.d_seq_off.as<uint64_t>(), n_reads, &up, params,
+  int rc = bin_batch_device(ix, ws.d_seqs.as<uint8_t>(), ws.d_seq_off.as<uint64_t>(), n_reads, &up, kind, params,
                             &d_hits, &d_hit_off, &n_hits);
   if (uploader.joinable()) uploader.join();
   ix->stats.h2d_bytes = h2d_bytes;
@@ -325,18 +335,18 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   const double t_comp = trace ? now() : 0;
   MTSV_CUDA_TRY(cudaStreamSynchronize(cin));
   // ---- D2H ----
-  mtsvgpu_hit* h_hits = nullptr;
+  void* h_hits = nullptr;
   uint64_t* h_off = nullptr;
-  const size_t hb = (n_hits ? n_hits : 1) * sizeof(mtsvgpu_hit), ob = (n_reads + 1) * sizeof(uint64_t);
+  const size_t hb = (n_hits ? n_hits : 1) * rec, ob = (n_reads + 1) * sizeof(uint64_t);
   if (pinned_result) {
     // slices may still be on their way into the buffers ensure_pinned is about to replace
     MTSV_CUDA_TRY(cudaStreamSynchronize(ix->copy_out_stream));
     MTSV_TRY(ensure_pinned(&ix->pin_hits, &ix->pin_hits_cap, hb));
     MTSV_TRY(ensure_pinned(&ix->pin_off, &ix->pin_off_cap, ob));
-    h_hits = (mtsvgpu_hit*)ix->pin_hits;
+    h_hits = ix->pin_hits;
     h_off = (uint64_t*)ix->pin_off;
   } else {
-    h_hits = (mtsvgpu_hit*)malloc(hb);
+    h_hits = malloc(hb);
     h_off = (uint64_t*)malloc(ob);
     if (!h_hits || !h_off) {
       free(h_hits);
@@ -348,7 +358,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   // (nothing more to copy when everything was copied slice by slice)
   if (!(pinned_result && up.out_overlap_ok && up.out_copied_hits == n_hits && up.out_copied_reads == n_reads)) {
     if (e == cudaSuccess && n_hits)
-      e = cudaMemcpyAsync(h_hits, d_hits, n_hits * sizeof(mtsvgpu_hit), cudaMemcpyDeviceToHost, st);
+      e = cudaMemcpyAsync(h_hits, d_hits, n_hits * rec, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(h_off, d_hit_off, ob, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
   }
@@ -382,29 +392,47 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
 
 int mtsvgpu_bin_batch(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off, uint64_t n_reads,
                       const mtsvgpu_params* params, mtsvgpu_hit** hits, uint64_t** hit_off) {
-  return bin_batch_host(ix, seqs, seq_off, n_reads, params, 0, hits, hit_off, nullptr);
+  return bin_batch_host(ix, seqs, seq_off, n_reads, params, BatchOutput::Hits, 0, (void**)hits, hit_off, nullptr);
+}
+
+// the pinned-result entry points: results in the handle's page-locked buffers
+static int batch_pinned(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off, uint64_t n_reads,
+                        const mtsvgpu_params* params, BatchOutput kind, const void** out, const uint64_t** out_off,
+                        uint64_t* n_out, bool packed, uint64_t packed_bytes) {
+  void* h = nullptr;
+  uint64_t* o = nullptr;
+  int rc = bin_batch_host(ix, seqs, seq_off, n_reads, params, kind, 1, &h, &o, n_out, packed, packed_bytes);
+  if (out) *out = h;
+  if (out_off) *out_off = o;
+  return rc;
 }
 
 int mtsvgpu_bin_batch_pinned(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off, uint64_t n_reads,
                              const mtsvgpu_params* params, const mtsvgpu_hit** hits,
                              const uint64_t** hit_off, uint64_t* n_hits) {
-  mtsvgpu_hit* h = nullptr;
-  uint64_t* o = nullptr;
-  int rc = bin_batch_host(ix, seqs, seq_off, n_reads, params, 1, &h, &o, n_hits);
-  if (hits) *hits = h;
-  if (hit_off) *hit_off = o;
-  return rc;
+  return batch_pinned(ix, seqs, seq_off, n_reads, params, BatchOutput::Hits, (const void**)hits, hit_off, n_hits,
+                      false, 0);
 }
 
 int mtsvgpu_bin_batch_packed(mtsvgpu_index* ix, const uint8_t* packed, uint64_t packed_bytes, const uint64_t* seq_off,
                              uint64_t n_reads, const mtsvgpu_params* params, const mtsvgpu_hit** hits,
                              const uint64_t** hit_off, uint64_t* n_hits) {
-  mtsvgpu_hit* h = nullptr;
-  uint64_t* o = nullptr;
-  int rc = bin_batch_host(ix, packed, seq_off, n_reads, params, 1, &h, &o, n_hits, true, packed_bytes);
-  if (hits) *hits = h;
-  if (hit_off) *hit_off = o;
-  return rc;
+  return batch_pinned(ix, packed, seq_off, n_reads, params, BatchOutput::Hits, (const void**)hits, hit_off, n_hits,
+                      true, packed_bytes);
+}
+
+int mtsvgpu_assign_batch_pinned(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t* seq_off, uint64_t n_reads,
+                                const mtsvgpu_params* params, const mtsvgpu_taxhit** out, const uint64_t** out_off,
+                                uint64_t* n_out) {
+  return batch_pinned(ix, seqs, seq_off, n_reads, params, BatchOutput::TaxHits, (const void**)out, out_off, n_out,
+                      false, 0);
+}
+
+int mtsvgpu_assign_batch_packed(mtsvgpu_index* ix, const uint8_t* packed, uint64_t packed_bytes,
+                                const uint64_t* seq_off, uint64_t n_reads, const mtsvgpu_params* params,
+                                const mtsvgpu_taxhit** out, const uint64_t** out_off, uint64_t* n_out) {
+  return batch_pinned(ix, packed, seq_off, n_reads, params, BatchOutput::TaxHits, (const void**)out, out_off, n_out,
+                      true, packed_bytes);
 }
 
 int mtsvgpu_collapse_device(int device, void* stream, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,

@@ -306,10 +306,12 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
     return set_error(MTSVGPU_ELIMIT, "%llu reads per rank exceed the communicator's max_local_reads %llu",
                      (unsigned long long)step, (unsigned long long)c->lay.max_local_reads);
   // ---- this chunk's hits for all reads (a plain single-index run) ----
-  const mtsvgpu_hit* d_hits = nullptr;
+  const void* d_recs = nullptr;
   const uint64_t* d_hit_off = nullptr;
   uint64_t n_hits = 0;
-  MTSV_TRY(bin_batch_device(h, d_seqs, d_seq_off, n_reads, nullptr, params, &d_hits, &d_hit_off, &n_hits));
+  MTSV_TRY(bin_batch_device(h, d_seqs, d_seq_off, n_reads, nullptr, BatchOutput::Hits, params, &d_recs, &d_hit_off,
+                            &n_hits));
+  const mtsvgpu_hit* d_hits = static_cast<const mtsvgpu_hit*>(d_recs);
   cudaStream_t st = h->stream;
   static const bool trace = getenv("MTSV_B200_TRACE") != nullptr;  // phase times on stderr
   cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};

@@ -44,9 +44,7 @@ __global__ void collapse_count_kernel(const uint64_t* __restrict__ keys, const u
                                       uint32_t n_reads, uint32_t* __restrict__ n_out) {
   uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n_reads) return;
-  uint32_t b = comb_off[r], e = comb_off[r + 1], c = 0;
-  for (uint32_t i = b; i < e; ++i) c += (i == b) || (keys[i] >> 32) != (keys[i - 1] >> 32);
-  n_out[r] = c;
+  n_out[r] = taxid_count(keys, comb_off[r], comb_off[r + 1]);
 }
 
 __global__ void collapse_write_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ comb_off,
@@ -56,13 +54,7 @@ __global__ void collapse_write_kernel(const uint64_t* __restrict__ keys, const u
   if (r > n_reads) return;
   out_off[r] = out_off32[r];
   if (r == n_reads) return;
-  uint32_t b = comb_off[r], e = comb_off[r + 1], w = out_off32[r];
-  for (uint32_t i = b; i < e; ++i)
-    if (i == b || (keys[i] >> 32) != (keys[i - 1] >> 32)) {
-      out[w].tax_id = (uint32_t)(keys[i] >> 32);
-      out[w].edit = (uint32_t)(keys[i] & 0xffffffffu);
-      ++w;
-    }
+  taxid_write(keys, comb_off[r], comb_off[r + 1], out, out_off32[r]);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -1191,6 +1191,27 @@ MTSV_HD uint32_t select_item(const BinsView& bv, const Params& p, const CandRec*
 }
 
 // ---------------------------------------------------------------------------------------------
+// merge of one read's hits into (TaxID, edit) records: each TaxID once with its smallest edit, by ascending TaxID —
+// mtsv-collapse mode TaxId (src/collapse.rs:597-602, :278-279) and the default results format of write_assignments
+// (src/binner.rs:330-352).  keys[b, e): tax << 32 | edit, sorted ascending, so a TaxID's smallest edit comes first.
+// ---------------------------------------------------------------------------------------------
+MTSV_HD uint32_t taxid_count(const uint64_t* keys, uint32_t b, uint32_t e) {
+  uint32_t c = 0;
+  for (uint32_t i = b; i < e; ++i) c += (i == b) || (keys[i] >> 32) != (keys[i - 1] >> 32);
+  return c;
+}
+// writes the records to out[w, w + taxid_count(keys, b, e))
+template <typename TaxHit>
+MTSV_HD void taxid_write(const uint64_t* keys, uint32_t b, uint32_t e, TaxHit* out, uint32_t w) {
+  for (uint32_t i = b; i < e; ++i)
+    if (i == b || (keys[i] >> 32) != (keys[i - 1] >> 32)) {
+      out[w].tax_id = (uint32_t)(keys[i] >> 32);
+      out[w].edit = (uint32_t)(keys[i] & 0xffffffffu);
+      ++w;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // host-side schedule (no device code; here so that tests/emul can check it)
 // ---------------------------------------------------------------------------------------------
 // Read boundaries of slices of at most `step` reads.  Without the ramp: equal slices of `step` reads.  With the

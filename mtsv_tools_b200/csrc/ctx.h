@@ -61,6 +61,7 @@ struct BatchCounters {  // device-side scalars of one sub-batch
   unsigned int n_ssw_full, n_over_len;  // candidates of reads >= 254 bases that needed the full SW matrices; reads over the length limit
   unsigned long long verified[2];  // two-round verification: candidates verified in round 1 / round 2
   unsigned long long rank_steps[32], window_bytes[32];  // profiling only; spread to avoid one hot address
+  unsigned long long total_taxhits;  // assignments output: merged (TaxID, edit) records of the sub-batch
 };
 
 
@@ -140,7 +141,7 @@ struct BatchWorkspace {
   DevBuf enc;
   // scan scratch, counters, worklists
   DevBuf scan_tmp, counters, worklist;
-  // whole-batch results (device-resident API)
+  // whole-batch results (device-resident API): mtsvgpu_hit or mtsvgpu_taxhit records
   DevBuf out_hits, out_hit_off;
   // staged inputs for the host API
   DevBuf d_seqs, d_seq_off;
@@ -166,6 +167,10 @@ struct Lane {
   size_t ev_next = 0;
 };
 
+// What a batch call returns, CSR by read: the Hit records of every strand (mtsvgpu_hit), or per read each TaxID once
+// with its minimum edit over both strands, by ascending TaxID (mtsvgpu_taxhit: the default results format)
+enum class BatchOutput { Hits, TaxHits };
+
 // What the host API knows about a batch that bin_batch_device computes from device buffers it is still filling (none
 // for device-resident input: a null source).  The uploader writes pack_base[i] before it lets wait_slice(i) return.
 struct BatchSource {
@@ -174,7 +179,7 @@ struct BatchSource {
   std::vector<uint64_t> pack_base;    // packed records: byte offset of each slice's first record; empty: raw bytes
   // before slice i is computed: wait until it has landed, ordering `stream` after its upload
   virtual int wait_slice(uint64_t i, cudaStream_t stream) = 0;
-  // after a sub-batch's results are enqueued on `stream`
+  // after a sub-batch's results are enqueued on `stream` (records of the call's BatchOutput)
   virtual int results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads,
                       cudaStream_t stream) = 0;
 };
@@ -242,9 +247,9 @@ int index_export(mtsvgpu_index* h, uint8_t* text_out, uint8_t* bwt_out, uint64_t
 int suffix_array_host(int device, const uint8_t* text, uint64_t n, uint32_t* sa_out, uint8_t* bwt_out);
 // binner.cu
 int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_seq_off,
-                     uint64_t n_reads, BatchSource* src,
-                     const mtsvgpu_params* params, const mtsvgpu_hit** d_hits,
-                     const uint64_t** d_hit_off, uint64_t* n_hits);
+                     uint64_t n_reads, BatchSource* src, BatchOutput kind,
+                     const mtsvgpu_params* params, const void** d_out,
+                     const uint64_t** d_out_off, uint64_t* n_out);
 int backward_search_batch(mtsvgpu_index* h, const uint8_t* pats, uint32_t pat_len, uint64_t n_pats,
                           uint64_t* lower, uint64_t* upper);
 int locate_batch(mtsvgpu_index* h, const uint64_t* rows, uint64_t n_rows, uint64_t* pos);

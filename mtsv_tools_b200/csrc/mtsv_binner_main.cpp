@@ -3,8 +3,9 @@
 // Mirrors src/bin/mtsv-binner.rs:21-331 (flags, defaults, validation, exit codes, resume-by-results
 // :347-411) and the host part of src/binner.rs (gz sniffing :21-33, FASTA/FASTQ records via their
 // id = header up to the first whitespace, --read-offset skipping :169-199, write_assignments :310-379).
-// The per-read work (normalisation, both strands, matching_tax_ids) is one mtsvgpu_bin_batch_packed call
-// per batch of reads.  The reference's host is Rust; no Rust toolchain exists in this image, so the
+// The per-read work (normalisation, both strands, matching_tax_ids, and for the default results format the
+// per-TaxID minimum edit) is one mtsvgpu_assign_batch_packed call per batch of reads (mtsvgpu_bin_batch_packed
+// for --output-format long).  The reference's host is Rust; no Rust toolchain exists in this image, so the
 // driver is C++ over the same C ABI a Rust build.rs would link (INTEGRATION.md).
 //
 // Host pipeline (the reference: cue's reader -> N workers -> single writer, src/binner.rs:149-217):
@@ -152,10 +153,23 @@ inline void put_u64(std::string* out, uint64_t v) {
   while (n) out->push_back(tmp[--n]);
 }
 
-// one result line, or nothing when the read has no hit (:316-318).  Default format: minimum edit per TaxID, by
-// TaxID (:330-352, BTreeMap order); long: minimum edit per (TaxID, GI, offset), in that order (:354-376)
-void format_assignments(const char* id, size_t id_len, const mtsvgpu_hit* hits, uint64_t n, bool long_fmt,
-                        std::string* out) {
+// one result line, or nothing when the read has no assignment (:316-318).  Default format (:330-352): the
+// library's merged records are already one per TaxID with its minimum edit, by TaxID (BTreeMap order).
+void format_taxhits(const char* id, size_t id_len, const mtsvgpu_taxhit* recs, uint64_t n, std::string* out) {
+  if (n == 0) return;
+  out->append(id, id_len);
+  out->push_back(':');
+  for (uint64_t i = 0; i < n; ++i) {
+    if (i) out->push_back(',');
+    put_u64(out, recs[i].tax_id);
+    out->push_back('=');
+    put_u64(out, recs[i].edit);
+  }
+  out->push_back('\n');
+}
+
+// long format (:354-376): minimum edit per (TaxID, GI, offset), in that order
+void format_hits_long(const char* id, size_t id_len, const mtsvgpu_hit* hits, uint64_t n, std::string* out) {
   if (n == 0) return;
   out->append(id, id_len);
   out->push_back(':');
@@ -168,12 +182,10 @@ void format_assignments(const char* id, size_t id_len, const mtsvgpu_hit* hits, 
     v = big.data();
   }
   for (uint64_t i = 0; i < n; ++i) v[i] = hits + i;
-  auto less = [long_fmt](const mtsvgpu_hit* a, const mtsvgpu_hit* b) {
+  auto less = [](const mtsvgpu_hit* a, const mtsvgpu_hit* b) {
     if (a->tax_id != b->tax_id) return a->tax_id < b->tax_id;
-    if (long_fmt) {
-      if (a->gi != b->gi) return a->gi < b->gi;
-      if (a->offset != b->offset) return a->offset < b->offset;
-    }
+    if (a->gi != b->gi) return a->gi < b->gi;
+    if (a->offset != b->offset) return a->offset < b->offset;
     return a->edit < b->edit;
   };
   if (n > 1) std::sort(v, v + n, less);
@@ -181,18 +193,16 @@ void format_assignments(const char* id, size_t id_len, const mtsvgpu_hit* hits, 
   for (uint64_t i = 0; i < n; ++i) {
     if (i) {
       const mtsvgpu_hit *a = v[i - 1], *b = v[i];
-      const bool same = a->tax_id == b->tax_id && (!long_fmt || (a->gi == b->gi && a->offset == b->offset));
+      const bool same = a->tax_id == b->tax_id && a->gi == b->gi && a->offset == b->offset;
       if (same) continue;  // the smaller edit of the key came first
     }
     if (!first) out->push_back(',');
     first = false;
     put_u64(out, v[i]->tax_id);
-    if (long_fmt) {
-      out->push_back('-');
-      put_u64(out, v[i]->gi);
-      out->push_back('-');
-      put_u64(out, v[i]->offset);
-    }
+    out->push_back('-');
+    put_u64(out, v[i]->gi);
+    out->push_back('-');
+    put_u64(out, v[i]->offset);
     out->push_back('=');
     put_u64(out, v[i]->edit);
   }
@@ -309,7 +319,8 @@ struct Batch {
   uint64_t seq = 0;
   std::vector<std::unique_ptr<ParsedBlock>> parts;
   uint64_t n_reads = 0;
-  std::vector<mtsvgpu_hit> hits;
+  std::vector<mtsvgpu_hit> hits;        // long format: the Hit records
+  std::vector<mtsvgpu_taxhit> taxhits;  // default format: merged (TaxID, edit) records
   std::vector<uint64_t> hit_off;
   std::vector<std::string> text;  // one per part, filled by the formatter tasks
   std::atomic<uint32_t> pending{0};
@@ -656,11 +667,14 @@ int main(int argc, char** argv) {
         uint32_t x = 12345u + (uint32_t)g;
         for (auto& c : wseq) c = (uint8_t)"ACGT"[(x = x * 1664525u + 1013904223u) >> 30];
         for (size_t i = 0; i <= 256; ++i) woff[i] = i * 150;
-        mtsvgpu_hit* wh = nullptr;
-        uint64_t* wo = nullptr;
-        if (mtsvgpu_bin_batch(handles[(size_t)g], wseq.data(), woff.data(), 256, &p, &wh, &wo) == 0) {
-          mtsvgpu_free(wh);
-          mtsvgpu_free(wo);
+        const uint64_t* wo = nullptr;
+        uint64_t wn = 0;
+        if (long_fmt) {
+          const mtsvgpu_hit* wh = nullptr;
+          (void)mtsvgpu_bin_batch_pinned(handles[(size_t)g], wseq.data(), woff.data(), 256, &p, &wh, &wo, &wn);
+        } else {
+          const mtsvgpu_taxhit* wt = nullptr;
+          (void)mtsvgpu_assign_batch_pinned(handles[(size_t)g], wseq.data(), woff.data(), 256, &p, &wt, &wo, &wn);
         }
       });
     for (auto& t : openers) t.join();
@@ -843,12 +857,18 @@ int main(int argc, char** argv) {
           for (uint32_t i = 0; i < part->n; ++i) pin_off[++r] = (bases += part->len[i]);
           std::vector<uint8_t>().swap(part->packed);
         }
+        // default format: the library merges each read's hits into its TaxID=edit list; long: the Hit records
         const mtsvgpu_hit* hits = nullptr;
+        const mtsvgpu_taxhit* taxhits = nullptr;
         const uint64_t* hit_off = nullptr;
         uint64_t n_hits = 0;
         ms_gather = since(tb0);
         const auto tc0 = std::chrono::steady_clock::now();
-        if (mtsvgpu_bin_batch_packed(ix, pin_packed, pbytes, pin_off, b->n_reads, &p, &hits, &hit_off, &n_hits) != 0) {
+        const int rc = long_fmt ? mtsvgpu_bin_batch_packed(ix, pin_packed, pbytes, pin_off, b->n_reads, &p, &hits,
+                                                           &hit_off, &n_hits)
+                                : mtsvgpu_assign_batch_packed(ix, pin_packed, pbytes, pin_off, b->n_reads, &p, &taxhits,
+                                                              &hit_off, &n_hits);
+        if (rc != 0) {
           sh.fail(2, std::string("Error running query: ") + mtsvgpu_last_error());
           break;
         }
@@ -858,10 +878,14 @@ int main(int argc, char** argv) {
           over_len += bst.n_reads_over_limit;
           over_hits += bst.n_strands_over_hits;
         }
-        b->hits.assign(hits, hits + n_hits);  // the handle's buffers are reused by its next batch
+        if (long_fmt)  // (the handle's buffers are reused by its next batch)
+          b->hits.assign(hits, hits + n_hits);
+        else
+          b->taxhits.assign(taxhits, taxhits + n_hits);
         b->hit_off.assign(hit_off, hit_off + b->n_reads + 1);
-        logf("DEBUG", "gpu %d batch %llu: %llu reads, %llu hits; waited+gathered %.1f ms, library call %.1f ms, results copied %.1f ms",
-             g, (unsigned long long)b->seq, (unsigned long long)b->n_reads, (unsigned long long)n_hits, ms_gather, ms_call,
+        logf("DEBUG", "gpu %d batch %llu: %llu reads, %llu %s; waited+gathered %.1f ms, library call %.1f ms, results copied %.1f ms",
+             g, (unsigned long long)b->seq, (unsigned long long)b->n_reads, (unsigned long long)n_hits,
+             long_fmt ? "hits" : "assignments", ms_gather, ms_call,
              since(tc0) - ms_call);
       }
       // format: one pool task per parsed block of the batch
@@ -886,7 +910,10 @@ int main(int argc, char** argv) {
             } else {
               const uint64_t h0 = b->hit_off[r0 + i], h1 = b->hit_off[r0 + i + 1];
               const size_t before = text.size();
-              format_assignments(part.ids.data() + id0, id1 - id0, b->hits.data() + h0, h1 - h0, long_fmt, &text);
+              if (long_fmt)
+                format_hits_long(part.ids.data() + id0, id1 - id0, b->hits.data() + h0, h1 - h0, &text);
+              else
+                format_taxhits(part.ids.data() + id0, id1 - id0, b->taxhits.data() + h0, h1 - h0, &text);
               lines += text.size() != before;
             }
             id0 = id1;

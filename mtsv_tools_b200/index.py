@@ -6,13 +6,16 @@ from collections import namedtuple
 import numpy as np
 
 from . import _lib
-from ._lib import HitStruct, BinStruct, InfoStruct, OptsStruct, ParamsStruct, StatsStruct, check
+from ._lib import HitStruct, BinStruct, InfoStruct, OptsStruct, ParamsStruct, StatsStruct, TaxHitStruct, check
 
 #: `Hit` — src/index.rs:30-40
 Hit = namedtuple("Hit", ["tax_id", "gi", "offset", "edit"])
 
 HIT_DTYPE = np.dtype([("tax_id", "<u4"), ("gi", "<u4"), ("offset", "<u8"), ("edit", "<u4"),
                       ("reserved", "<u4")])
+
+#: mtsvgpu_taxhit: one `TaxID=edit` entry of the default results format (src/binner.rs:330-352)
+TAXHIT_DTYPE = np.dtype([("tax_id", "<u4"), ("edit", "<u4")])
 
 
 class Params:
@@ -255,6 +258,55 @@ class MGIndex:
         check(L.mtsvgpu_bin_batch_device(self._h, C.c_void_p(d_seqs_ptr), C.c_void_p(d_seq_off_ptr), n_reads,
                                          C.byref(ps), C.byref(dh), C.byref(do), C.byref(nh)))
         return dh.value, do.value, nh.value
+
+    @staticmethod
+    def _pinned_taxhits(tp, op, n_out, n):
+        offs = np.frombuffer((C.c_uint8 * ((n + 1) * 8)).from_address(op.value), dtype=np.uint64)
+        size = C.sizeof(TaxHitStruct)
+        recs = np.frombuffer((C.c_uint8 * (max(n_out, 1) * size)).from_address(tp.value), dtype=TAXHIT_DTYPE)[:n_out]
+        return recs, offs
+
+    def assign_reads(self, reads, params=None, strands=2):
+        """mtsvgpu_assign_batch_pinned: the default results format computed on the device.  reads as for bin_reads.
+        Returns (taxhits, off): a structured array (TAXHIT_DTYPE) and CSR offsets per read.  Read i's records are
+        each TaxID it hits on either strand, once, with the minimum edit of those hits, by ascending TaxID.  Copies."""
+        L = _lib.load_library()
+        params = params or Params()
+        cat, off = reads if isinstance(reads, tuple) else pack_reads(reads)
+        cat = np.ascontiguousarray(cat, dtype=np.uint8)
+        off = np.ascontiguousarray(off, dtype=np.uint64)
+        n = len(off) - 1
+        ps = params.c_struct(strands)
+        tp, op, nt = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        check(L.mtsvgpu_assign_batch_pinned(self._h, _ptr(cat), _ptr(off), n, C.byref(ps), C.byref(tp), C.byref(op),
+                                            C.byref(nt)))
+        recs, offs = self._pinned_taxhits(tp, op, int(nt.value), n)
+        return recs.copy(), offs.copy()
+
+    def assign_reads_packed(self, packed, off, params=None, strands=2):
+        """mtsvgpu_assign_batch_packed: packed records (pack_reads_planes) + their base offsets in; results as
+        assign_reads, but views of the handle's page-locked buffers, valid until the next batch call on this index."""
+        L = _lib.load_library()
+        params = params or Params()
+        assert packed.dtype == np.uint8 and off.dtype == np.uint64 and packed.flags.c_contiguous
+        n = len(off) - 1
+        ps = params.c_struct(strands)
+        tp, op, nt = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        check(L.mtsvgpu_assign_batch_packed(self._h, _ptr(packed) if len(packed) else None, len(packed), _ptr(off), n,
+                                            C.byref(ps), C.byref(tp), C.byref(op), C.byref(nt)))
+        return self._pinned_taxhits(tp, op, int(nt.value), n)
+
+    def assign_reads_device(self, d_seqs_ptr, d_seq_off_ptr, n_reads, params=None, strands=2):
+        """mtsvgpu_assign_batch_device: device pointers in, as for bin_reads_device.  Returns (d_taxhits_ptr,
+        d_off_ptr, n_taxhits): 8-byte (tax_id, edit) records and n_reads + 1 uint64 offsets, valid until the next
+        batch call."""
+        L = _lib.load_library()
+        params = params or Params()
+        ps = params.c_struct(strands)
+        dt, do, nt = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        check(L.mtsvgpu_assign_batch_device(self._h, C.c_void_p(d_seqs_ptr), C.c_void_p(d_seq_off_ptr), n_reads,
+                                            C.byref(ps), C.byref(dt), C.byref(do), C.byref(nt)))
+        return dt.value, do.value, nt.value
 
     def matching_tax_ids(self, sequence, edit_freq=0.13, seed_length=18, seed_gap=15,
                          min_seeds_percent=0.015, max_hits=2000, tune_max_hits=200,
