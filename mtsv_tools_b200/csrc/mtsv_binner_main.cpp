@@ -9,7 +9,7 @@
 // driver is C++ over the same C ABI a Rust build.rs would link (INTEGRATION.md).
 //
 // Host pipeline (the reference: cue's reader -> N workers -> single writer, src/binner.rs:149-217):
-//   reader thread     inflates / reads the file in large blocks and cuts them at record boundaries
+//   reader thread     inflates / reads the file in large blocks of whole records (fastx.h)
 //   --threads workers parse the records of a block (id, sequence) and pack each sequence straight into the
 //                     bit planes the device consumes (mtsvgpu_pack_read: no intermediate copy of the bases);
 //                     the same pool later formats result lines
@@ -27,10 +27,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
-#include <fcntl.h>
 #include <sys/stat.h>
-#include <unistd.h>
-#include <zlib.h>
 
 #include <algorithm>
 #include <atomic>
@@ -48,6 +45,7 @@
 #include <vector>
 
 #include "../../include/mtsv_b200.h"
+#include "fastx.h"
 
 namespace {
 
@@ -61,86 +59,6 @@ void logf(const char* level, const char* fmt, ...) {
   fputc('\n', stderr);
   va_end(ap);
 }
-
-// ---- FASTA / FASTQ records (bio::io::{fasta,fastq}); gz or plain via zlib (src/binner.rs:21-33) ----
-struct Record {
-  std::string id, seq;
-};
-
-class FastxReader {
- public:
-  FastxReader(const char* path, bool fastq) : fastq_(fastq) {
-    gz_ = gzopen(path, "rb");  // transparently reads uncompressed files too (magic 1f 8b sniffing)
-    if (gz_) gzbuffer(gz_, 1 << 20);
-  }
-  ~FastxReader() {
-    if (gz_) gzclose(gz_);
-  }
-  bool ok() const { return gz_ != nullptr; }
-  // returns 1 = record, 0 = EOF, -1 = parse error
-  int next(Record* r) {
-    r->id.clear();
-    r->seq.clear();
-    if (!have_line_ && !read_line()) return 0;
-    while (line_.empty()) {
-      if (!read_line()) return 0;
-    }
-    const char lead = fastq_ ? '@' : '>';
-    if (line_[0] != lead) return -1;
-    size_t e = 1;
-    while (e < line_.size() && !isspace((unsigned char)line_[e])) ++e;
-    r->id.assign(line_, 1, e - 1);
-    have_line_ = false;
-    if (!fastq_) {
-      while (read_line()) {
-        if (!line_.empty() && line_[0] == '>') break;
-        r->seq += line_;
-      }
-      return 1;
-    }
-    // FASTQ: sequence lines up to '+', then as many quality characters as bases
-    bool plus = false;
-    while (read_line()) {
-      if (!line_.empty() && line_[0] == '+') {
-        plus = true;
-        have_line_ = false;
-        break;
-      }
-      r->seq += line_;
-    }
-    if (!plus) return -1;
-    size_t q = 0;
-    while (q < r->seq.size()) {
-      if (!read_line()) return -1;
-      q += line_.size();
-      have_line_ = false;
-    }
-    if (q != r->seq.size()) return -1;
-    return 1;  // (the empty quality line of an empty record is skipped as a blank line by the next call)
-  }
-
- private:
-  bool read_line() {
-    line_.clear();
-    char buf[1 << 16];
-    bool got = false;
-    while (gzgets(gz_, buf, sizeof buf)) {
-      got = true;
-      size_t n = strlen(buf);
-      bool eol = n && buf[n - 1] == '\n';
-      if (eol) --n;
-      if (n && buf[n - 1] == '\r') --n;
-      line_.append(buf, n);
-      if (eol) break;
-    }
-    have_line_ = got;
-    return got;
-  }
-  gzFile gz_ = nullptr;
-  bool fastq_;
-  std::string line_;
-  bool have_line_ = false;
-};
 
 // ---- write_assignments (src/binner.rs:310-379) ----
 inline void put_u64(std::string* out, uint64_t v) {
@@ -247,24 +165,28 @@ bool resume_offset(const char* results, const char* input, bool fastq, uint64_t*
   }
   std::unordered_set<std::string> ids;
   if (!read_ids_from_results(results, &ids, err)) return false;
-  FastxReader rd(input, fastq);
-  if (!rd.ok()) {
+  FastxBlocks in(input, fastq);
+  if (!in.ok()) {
     *err = "cannot open input";
     return false;
   }
-  Record r;
-  uint64_t idx = 0, last = 0;
+  std::string text, id;
+  uint64_t n, idx = 0, last = 0;
   bool any = false;
   int rc;
-  while ((rc = rd.next(&r)) == 1) {
-    if (ids.count(r.id)) {
-      last = idx;
-      any = true;
+  while ((rc = in.next(&text, &n)) == 1) {
+    Lines ln{text.data(), text.data() + text.size()};
+    FastxRecord r;
+    while (next_record(ln, fastq, true, &r) == 1) {
+      if (ids.count(id.assign(r.id, r.id_end))) {
+        last = idx;
+        any = true;
+      }
+      ++idx;
     }
-    ++idx;
   }
   if (rc < 0) {
-    *err = "parse error while scanning input";
+    *err = rc == -1 ? "parse error while scanning input" : "cannot read input";
     return false;
   }
   *offset = any ? last + 1 : 0;
@@ -303,7 +225,7 @@ void usage() {
 struct TextBlock {  // whole records, as they stand in the file
   uint64_t seq = 0;
   std::string text;
-  uint32_t n_records = 0;
+  uint64_t n_records = 0;
 };
 
 struct ParsedBlock {
@@ -369,77 +291,6 @@ class Pool {  // fixed set of workers running queued tasks
   bool stop_ = false;
 };
 
-// lines of a text span; '\r' before '\n' is dropped; `terminated` tells whether the line ended in a newline
-// (the last line of a span may be cut by the span's end)
-struct Lines {
-  const char *p, *end;
-  bool terminated = true;
-  bool next(const char** b, const char** e) {
-    if (p >= end) return false;
-    const char* nl = (const char*)memchr(p, '\n', (size_t)(end - p));
-    terminated = nl != nullptr;
-    *b = p;
-    *e = nl ? nl : end;
-    p = nl ? nl + 1 : end;
-    if (*e > *b && (*e)[-1] == '\r') --*e;
-    return true;
-  }
-};
-
-// Counts the complete records at the start of [p, end) and returns where the last one ends (*cut); -1 on a
-// malformed record.  `eof`: the span is the rest of the file, so a last line without newline is whole and a FASTA
-// record needs no following header to be complete.  Same record grammar as FastxReader::next
-// (bio::io::{fasta,fastq}: multi-line sequences, quality read by length).
-int64_t scan_records(const char* p, const char* end, bool fastq, bool eof, const char** cut) {
-  int64_t n = 0;
-  *cut = p;
-  Lines ln{p, end};
-  const char *b, *e;
-  for (;;) {
-    for (;;) {  // blank lines between records
-      if (!ln.next(&b, &e)) {
-        *cut = end;
-        return n;
-      }
-      if (!ln.terminated && !eof) return n;
-      if (e > b) break;
-      *cut = ln.p;
-    }
-    if (*b != (fastq ? '@' : '>')) return -1;
-    if (!fastq) {
-      for (;;) {  // sequence lines, up to the next header
-        if (ln.p >= end) {
-          if (!eof) return n;
-          *cut = end;
-          return n + 1;
-        }
-        if (*ln.p == '>') break;
-        ln.next(&b, &e);
-        if (!ln.terminated && !eof) return n;
-      }
-      ++n;
-      *cut = ln.p;
-      continue;
-    }
-    uint64_t seq_len = 0;
-    for (;;) {  // sequence lines, up to the '+' line
-      if (!ln.next(&b, &e)) return eof ? -1 : n;
-      if (!ln.terminated && !eof) return n;
-      if (e > b && *b == '+') break;
-      seq_len += (uint64_t)(e - b);
-    }
-    uint64_t q = 0;
-    while (q < seq_len) {  // as many quality characters as bases
-      if (!ln.next(&b, &e)) return eof ? -1 : n;
-      if (!ln.terminated && !eof) return n;
-      q += (uint64_t)(e - b);
-    }
-    if (q != seq_len) return -1;
-    ++n;
-    *cut = ln.p;
-  }
-}
-
 struct Shared {
   std::mutex mu;
   std::condition_variable cv;
@@ -459,74 +310,36 @@ struct Shared {
   }
 };
 
-// parse + pack one block of whole records (a pool task)
-void parse_block(const TextBlock& tb, bool fastq, ParsedBlock* out) {
+// parse + pack one block of whole records, all but the first `skip` (a pool task)
+void parse_block(const TextBlock& tb, bool fastq, uint64_t skip, ParsedBlock* out) {
   out->n = 0;
-  out->len.reserve(tb.n_records);
-  out->id_end.reserve(tb.n_records);
+  out->len.reserve(tb.n_records - skip);
+  out->id_end.reserve(tb.n_records - skip);
   out->packed.reserve(tb.text.size() / 4);
   Lines ln{tb.text.data(), tb.text.data() + tb.text.size()};
-  const char *b, *e;
+  FastxRecord r;
   std::string multi;
-  bool have = ln.next(&b, &e);
-  while (have) {
-    if (e == b) {
-      have = ln.next(&b, &e);
-      continue;
-    }
-    if (*b != (fastq ? '@' : '>')) {
+  for (uint64_t i = 0; next_record(ln, fastq, true, &r) == 1; ++i) {
+    if (i < skip) continue;
+    if (r.len > 0xfffffff0ull) {
       out->bad = true;
       return;
     }
-    const char* ie = b + 1;
-    while (ie < e && !isspace((unsigned char)*ie)) ++ie;  // record.id(): up to the first whitespace
-    out->ids.append(b + 1, (size_t)(ie - b - 1));
+    out->ids.append(r.id, r.id_end);
     out->id_end.push_back((uint32_t)out->ids.size());
-    const char *sb = nullptr, *se = nullptr;
-    int seq_lines = 0;
-    multi.clear();
-    bool plus = false;
-    while ((have = ln.next(&b, &e))) {
-      if (e > b && *b == (fastq ? '+' : '>')) {
-        plus = true;
-        break;
-      }
-      if (seq_lines == 0) {
-        sb = b;
-        se = e;
-      } else {
-        if (seq_lines == 1) multi.assign(sb, (size_t)(se - sb));
-        multi.append(b, (size_t)(e - b));
-      }
-      ++seq_lines;
-    }
-    const uint8_t* seq = seq_lines > 1 ? (const uint8_t*)multi.data() : (const uint8_t*)sb;
-    const uint64_t L = seq_lines > 1 ? multi.size() : (seq_lines == 1 ? (uint64_t)(se - sb) : 0);
-    if (L > 0xfffffff0ull) {
-      out->bad = true;
-      return;
+    const char* seq = r.seq;
+    if (r.seq_lines > 1) {  // only a multi-line sequence is copied
+      multi.clear();
+      Lines sl{r.seq, r.seq_end};
+      const char *b, *e;
+      while (sl.next(&b, &e)) multi.append(b, e);
+      seq = multi.data();
     }
     const size_t at = out->packed.size();
-    out->packed.resize(at + 3 * ((L + 7) >> 3));
-    if (L) mtsvgpu_pack_read(seq, (uint32_t)L, out->packed.data() + at);
-    out->len.push_back((uint32_t)L);
+    out->packed.resize(at + 3 * ((r.len + 7) >> 3));
+    if (r.len) mtsvgpu_pack_read((const uint8_t*)seq, (uint32_t)r.len, out->packed.data() + at);
+    out->len.push_back((uint32_t)r.len);
     ++out->n;
-    if (fastq) {
-      if (!plus) {
-        out->bad = true;
-        return;
-      }
-      uint64_t q = 0;
-      while (q < L) {
-        if (!(have = ln.next(&b, &e))) {
-          out->bad = true;
-          return;
-        }
-        q += (uint64_t)(e - b);
-      }
-      have = ln.next(&b, &e);
-    }
-    // (FASTA: b..e is the next header, or have == false)
   }
 }
 
@@ -581,13 +394,24 @@ int main(int argc, char** argv) {
   }
   const bool dump_mt = dump_reads && n_threads != 0;
   if (dump_reads && !dump_mt && (fasta || fastq)) {
-    FastxReader rd(fasta ? fasta : fastq, fastq != nullptr);
-    if (!rd.ok()) return 2;
-    Record r;
+    FastxBlocks in(fasta ? fasta : fastq, fastq != nullptr);
+    if (!in.ok()) return 2;
+    std::string text;
+    uint64_t n, idx = 0;
     int rc;
-    uint64_t idx = 0;
-    while ((rc = rd.next(&r)) == 1)
-      if (idx++ >= read_offset) printf("%s\t%s\n", r.id.c_str(), r.seq.c_str());
+    while ((rc = in.next(&text, &n)) == 1) {
+      Lines ln{text.data(), text.data() + text.size()};
+      FastxRecord r;
+      while (next_record(ln, fastq != nullptr, true, &r) == 1) {
+        if (idx++ < read_offset) continue;
+        fwrite(r.id, 1, (size_t)(r.id_end - r.id), stdout);
+        putchar('\t');
+        Lines sl{r.seq, r.seq_end};
+        const char *b, *e;
+        while (sl.next(&b, &e)) fwrite(b, 1, (size_t)(e - b), stdout);
+        putchar('\n');
+      }
+    }
     return rc < 0 ? 12 : 0;
   }
   if ((!fasta && !fastq) || (fasta && fastq) || (!index && !dump_mt)) {
@@ -633,21 +457,11 @@ int main(int argc, char** argv) {
     logf("ERROR", "Error running query: cannot open %s: %s", results, strerror(errno));
     return 2;
   }
-  gzFile gz = gzopen(input, "rb");  // reads uncompressed files too (magic 1f 8b sniffing, src/binner.rs:21-33)
-  if (!gz) {
+  FastxBlocks blocks(input, is_fastq);  // src/binner.rs:21-33
+  if (!blocks.ok()) {
     logf("ERROR", "Error running query: cannot open %s", input);
     if (!dump_mt) fclose(out);
     return 2;
-  }
-  gzbuffer(gz, 1 << 20);
-  // an uncompressed file is read with plain read(2): no pass through zlib's copy-through mode
-  int plain_fd = -1;
-  struct stat ist;
-  if (stat(input, &ist) == 0 && S_ISREG(ist.st_mode) && gzdirect(gz)) {
-    plain_fd = open(input, O_RDONLY);
-#ifdef POSIX_FADV_SEQUENTIAL
-    if (plain_fd >= 0) posix_fadvise(plain_fd, 0, 0, POSIX_FADV_SEQUENTIAL);
-#endif
   }
   std::vector<mtsvgpu_index*> handles((size_t)n_gpus, nullptr);
   if (!dump_mt) {
@@ -683,7 +497,6 @@ int main(int argc, char** argv) {
         logf("ERROR", "Error running query: %s", errs[(size_t)g].c_str());
         for (auto h : handles) mtsvgpu_index_close(h);
         fclose(out);
-        gzclose(gz);
         return 2;
       }
   }
@@ -703,58 +516,25 @@ int main(int argc, char** argv) {
   std::map<uint64_t, std::unique_ptr<ParsedBlock>> parsed;  // finished blocks waiting for their turn
   uint64_t blocks_issued = 0, blocks_taken = 0;
   bool reader_done = false;
-  const size_t kBlockBytes = 4u << 20;
   const uint64_t max_blocks_in_flight = (uint64_t)std::max(8, 4 * n_threads) + batch_reads / 8192;
   std::thread reader([&] {
-    // Each block is read straight into the string that becomes the parser's input; only the cut-off tail (the
-    // beginning of the record the block edge fell into) is copied over to the next block.
-    std::string carry;
-    uint64_t records_seen = 0;  // complete records cut so far (including skipped ones)
-    bool eof = false;
-    while (!eof && !sh.failed()) {
-      const size_t have = carry.size();
-      carry.resize(have + kBlockBytes);
-      size_t filled = 0;
-      while (filled < kBlockBytes) {  // (short reads happen on pipes and at gzip member boundaries)
-        long got = plain_fd >= 0 ? (long)read(plain_fd, &carry[have + filled], kBlockBytes - filled)
-                                 : (long)gzread(gz, &carry[have + filled], (unsigned)(kBlockBytes - filled));
-        if (got < 0) {
-          sh.fail(12, "Unable to read from input file");
-          break;
-        }
-        if (got == 0) {
-          eof = true;
-          break;
-        }
-        filled += (size_t)got;
-      }
-      if (sh.failed()) break;
-      carry.resize(have + filled);
-      const char* cut = nullptr;
-      const int64_t n = scan_records(carry.data(), carry.data() + carry.size(), is_fastq, eof, &cut);
-      if (n < 0) {
-        char msg[128];
-        snprintf(msg, sizeof msg, "Unable to read from input file: malformed record after %llu reads",
-                 (unsigned long long)records_seen);
+    uint64_t records_seen = 0;  // complete records read so far (including skipped ones)
+    while (!sh.failed()) {
+      auto tb = std::make_shared<TextBlock>();
+      const int rc = blocks.next(&tb->text, &tb->n_records);
+      if (rc == 0) break;
+      if (rc < 0 || blocks.malformed_next()) {  // (the records of a block that ends at a malformed one are not binned)
+        std::string msg = "Unable to read from input file";
+        if (rc != -2) msg += ": malformed record after " + std::to_string(records_seen) + " reads";
         sh.fail(12, msg);  // src/binner.rs:81-84
         break;
       }
-      if (n == 0) {
-        if (eof) break;
-        continue;
-      }
-      auto tb = std::make_shared<TextBlock>();
-      tb->n_records = (uint32_t)n;
-      const size_t used = (size_t)(cut - carry.data());
-      std::string tail(carry, used);
-      carry.resize(used);
-      tb->text.swap(carry);
-      carry.swap(tail);
-      // .skip(read_offset) (src/binner.rs:176,199): whole blocks are dropped, a straddling block is trimmed by the parser
+      // .skip(read_offset) (src/binner.rs:176,199): whole blocks are dropped, the parser skips the first records of
+      // a straddling block
       const uint64_t first = records_seen;
-      records_seen += (uint64_t)n;
+      records_seen += tb->n_records;
       if (records_seen <= read_offset) continue;
-      const uint64_t skip_in_block = read_offset > first ? read_offset - first : 0;
+      const uint64_t skip = read_offset > first ? read_offset - first : 0;
       uint64_t seq;
       {
         std::unique_lock<std::mutex> lk(pmu);
@@ -762,22 +542,10 @@ int main(int argc, char** argv) {
         seq = blocks_issued++;
       }
       tb->seq = seq;
-      pool.submit([&, tb, skip_in_block] {
+      pool.submit([&, tb, skip] {
         auto pb = std::make_unique<ParsedBlock>();
-        if (!sh.failed()) parse_block(*tb, is_fastq, pb.get());
+        if (!sh.failed()) parse_block(*tb, is_fastq, skip, pb.get());
         if (pb->bad) sh.fail(12, "Unable to read from input file: malformed record");
-        if (skip_in_block && !pb->bad) {  // drop the first records of the block
-          ParsedBlock& b = *pb;
-          uint64_t k = std::min<uint64_t>(skip_in_block, b.n), pbytes = 0;
-          for (uint64_t i = 0; i < k; ++i) pbytes += 3 * (((uint64_t)b.len[i] + 7) >> 3);
-          const uint32_t idb = k ? b.id_end[k - 1] : 0;
-          b.packed.erase(b.packed.begin(), b.packed.begin() + (long)pbytes);
-          b.len.erase(b.len.begin(), b.len.begin() + (long)k);
-          b.ids.erase(0, idb);
-          b.id_end.erase(b.id_end.begin(), b.id_end.begin() + (long)k);
-          for (auto& x : b.id_end) x -= idb;
-          b.n -= (uint32_t)k;
-        }
         std::lock_guard<std::mutex> lk(pmu);
         parsed[tb->seq] = std::move(pb);
         pcv.notify_all();
@@ -962,8 +730,6 @@ int main(int argc, char** argv) {
     wcv.notify_all();
   }
   writer.join();
-  gzclose(gz);
-  if (plain_fd >= 0) close(plain_fd);
   for (auto h : handles) mtsvgpu_index_close(h);
   int code = 0;
   {

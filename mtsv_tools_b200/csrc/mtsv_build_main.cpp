@@ -13,7 +13,6 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
-#include <zlib.h>
 
 #include <chrono>
 #include <string>
@@ -22,6 +21,7 @@
 #include <vector>
 
 #include "../../include/mtsv_b200.h"
+#include "fastx.h"
 
 namespace {
 
@@ -236,85 +236,57 @@ int main(int argc, char** argv) {
   }
   const auto t0 = std::chrono::steady_clock::now();
   logf("DEBUG", "Opening FASTA database file...");
-  gzFile gz = gzopen(fasta, "rb");
-  if (!gz) {
+  FastxBlocks in(fasta, false);
+  if (!in.ok()) {
     logf("ERROR", "Unable to open FASTA database for parsing.");
     return 1;
   }
-  gzbuffer(gz, 1 << 20);
   std::vector<uint8_t> seqs;
   std::vector<uint64_t> off(1, 0);
   std::vector<uint32_t> gis, taxs;
-  {
-    std::string line, id;
-    std::vector<char> buf(1 << 20);
-    bool in_record = false, keep = false, partial = false;
-    auto end_record = [&]() {
-      if (in_record && keep) off.push_back(seqs.size());
-      in_record = false;
-    };
-    auto handle_line = [&](const std::string& l) -> bool {
-      if (!l.empty() && l[0] == '>') {
-        end_record();
-        size_t e = 1;
-        while (e < l.size() && !isspace((unsigned char)l[e])) ++e;
-        id.assign(l, 1, e - 1);  // record.id(): header up to the first whitespace
-        uint32_t gi = 0, tax = 0;
-        keep = true;
-        if (mapping) {
-          auto it = map.find(id);
-          if (it == map.end()) {
-            if (skip_missing) {
-              logf("WARN", "Missing mapping for header %s, skipping.", id.c_str());
-              keep = false;
-            } else {
-              logf("ERROR", "Error building index: Missing mapping for header %s", id.c_str());
-              return false;
-            }
-          } else {
-            gi = it->second.first;
-            tax = it->second.second;
+  std::string text;
+  uint64_t n;
+  int rc;
+  while ((rc = in.next(&text, &n)) == 1) {
+    if (seqs.size() + text.size() > seqs.capacity())  // (one reallocation for a block of one long record)
+      seqs.reserve(std::max(2 * seqs.capacity(), seqs.size() + text.size()));
+    Lines ln{text.data(), text.data() + text.size()};
+    FastxRecord r;
+    while (next_record(ln, false, true, &r) == 1) {
+      const std::string id(r.id, r.id_end);
+      uint32_t gi = 0, tax = 0;
+      if (mapping) {
+        auto it = map.find(id);
+        if (it == map.end()) {
+          if (!skip_missing) {
+            logf("ERROR", "Error building index: Missing mapping for header %s", id.c_str());
+            return 1;
           }
-        } else {
-          std::string err;
-          if (!parse_read_header(id, &gi, &tax, &err)) {
-            logf("ERROR", "Error building index: %s", err.c_str());
-            return false;
-          }
+          logf("WARN", "Missing mapping for header %s, skipping.", id.c_str());
+          continue;
         }
-        if (keep) {
-          gis.push_back(gi);
-          taxs.push_back(tax);
+        gi = it->second.first;
+        tax = it->second.second;
+      } else {
+        std::string err;
+        if (!parse_read_header(id, &gi, &tax, &err)) {
+          logf("ERROR", "Error building index: %s", err.c_str());
+          return 1;
         }
-        in_record = true;
-      } else if (in_record) {
-        if (keep) seqs.insert(seqs.end(), l.begin(), l.end());
-      } else if (!l.empty()) {
-        logf("ERROR", "Error building index: FASTA record does not start with '>'");
-        return false;
       }
-      return true;
-    };
-    while (gzgets(gz, buf.data(), (int)buf.size())) {
-      size_t n = strlen(buf.data());
-      const bool eol = n && buf[n - 1] == '\n';
-      if (eol) --n;
-      if (n && buf[n - 1] == '\r') --n;
-      if (partial) line.append(buf.data(), n);
-      else line.assign(buf.data(), n);
-      partial = !eol;
-      if (eol && !handle_line(line)) {
-        gzclose(gz);
-        return 1;
-      }
+      gis.push_back(gi);
+      taxs.push_back(tax);
+      Lines sl{r.seq, r.seq_end};
+      const char *b, *e;
+      while (sl.next(&b, &e)) seqs.insert(seqs.end(), b, e);
+      off.push_back(seqs.size());
     }
-    if (partial && !handle_line(line)) {
-      gzclose(gz);
-      return 1;
-    }
-    end_record();
   }
-  gzclose(gz);
+  if (rc < 0) {  // (a FASTA record can only be malformed by not starting with '>')
+    logf("ERROR", rc == -1 ? "Error building index: FASTA record does not start with '>'"
+                           : "Unable to read FASTA database.");
+    return 1;
+  }
   if (gis.empty()) {
     logf("ERROR", "Error building index: no sequences to index");
     return 1;

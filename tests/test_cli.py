@@ -40,24 +40,23 @@ def test_fastx_parsing(tmp_path):
     assert _run("--dump-reads", "--fastq", str(bad)).returncode == 12  # src/binner.rs:81-84
 
 
-def _lens(dump_stdout):
-    return "".join("%s\t%d\n" % (l.split("\t")[0], len(l.rstrip("\n").split("\t")[1]))
-                   for l in dump_stdout.splitlines(True))
-
-
-def test_pipeline_scanner_and_parser_match_the_sequential_reader(tmp_path):
-    """--dump-reads-mt drives the production path (block reader, record scanner, parser pool, ordered writer)
-    without a GPU and prints id<TAB>length; it must agree with the line-by-line reader on awkward files, in
-    particular where 4 MiB block edges cut lines and records."""
+def test_dump_reads_give_the_records_written(tmp_path):
+    """--dump-reads prints id<TAB>sequence of every record; --dump-reads-mt drives the production path (block reader,
+    parser pool, ordered writer) without a GPU and prints id<TAB>length.  Both must give the records the generators
+    wrote, on awkward files and in particular where 4 MiB block edges cut lines and records."""
     rng = np.random.default_rng(3)
+
+    def bases(alphabet, L):
+        return rng.choice(np.frombuffer(alphabet, np.uint8), size=L).tobytes().decode()
 
     def fastq(n, multi=False, crlf=False, final_newline=True):
         nl = "\r\n" if crlf else "\n"
-        parts = []
+        parts, recs = [], []
         for i in range(n):
             L = int(rng.integers(0, 400))
-            s = "".join(rng.choice(list("ACGTN"), size=L))
-            q = "".join(rng.choice(list("@+I#>"), size=L))  # quality lines that look like headers / separators
+            s = bases(b"ACGTN", L)
+            q = bases(b"@+I#>", L)  # quality lines that look like headers / separators
+            recs.append(("r%d" % i, s))
             if multi and L > 10:
                 k = int(rng.integers(1, L))
                 s, q = s[:k] + nl + s[k:], q[:k // 2] + nl + q[k // 2:]
@@ -65,42 +64,55 @@ def test_pipeline_scanner_and_parser_match_the_sequential_reader(tmp_path):
             if i % 97 == 0:
                 parts.append(nl)  # blank line between records
         t = "".join(parts)
-        return t if final_newline else t.rstrip("\r\n")
+        return (t if final_newline else t.rstrip("\r\n")), recs
 
-    def fasta(n, crlf=False, final_newline=True):
+    def fasta(n, crlf=False, final_newline=True, long_record=None):
         nl = "\r\n" if crlf else "\n"
-        parts = []
+        parts, recs = [], []
         for i in range(n):
-            L = int(rng.integers(0, 900))
-            s = "".join(rng.choice(list("ACGTNacgtn"), size=L))
+            L = 9 << 20 if i == long_record else int(rng.integers(0, 900))  # (9 MiB: more than two blocks)
+            s = bases(b"ACGTNacgtn", L)
+            recs.append(("s%d-%d" % (i, i % 7), s))
             lines = [s[j:j + 70] for j in range(0, L, 70)] or [""]
-            parts.append(">s%d-%d desc%s%s%s" % (i, i % 7, nl, nl.join(lines), nl))
+            head = ">s%d-%d desc%s" % (i, i % 7, nl)
+            if i == long_record:  # pad the header so that the first 4 MiB block ends right after a sequence line
+                start = sum(map(len, parts)) + len(head)
+                head = head.replace(" desc", " desc" + " " * (((4 << 20) - start) % (70 + len(nl))))
+            parts.append(head + nl.join(lines) + nl)
         t = "".join(parts)
-        return t if final_newline else t.rstrip("\r\n")
+        return (t if final_newline else t.rstrip("\r\n")), recs
+
+    def dump(recs):
+        return "".join("%s\t%s\n" % r for r in recs)
+
+    def lens(recs):
+        return "".join("%s\t%d\n" % (i, len(s)) for i, s in recs)
 
     cases = [("a.fq", fastq(30000), "--fastq"), ("b.fq", fastq(3000, multi=True, crlf=True), "--fastq"),
              ("c.fq", fastq(2000, final_newline=False), "--fastq"), ("d.fa", fasta(20000), "--fasta"),
-             ("e.fa", fasta(1500, crlf=True, final_newline=False), "--fasta")]
-    for name, text, flag in cases:
+             ("e.fa", fasta(1500, crlf=True, final_newline=False), "--fasta"),
+             ("f.fa", fasta(3000, long_record=2000), "--fasta")]
+    for name, (text, recs), flag in cases:
         f = tmp_path / name
         f.write_text(text, newline="")
-        want = _run("--dump-reads", flag, str(f))
-        assert want.returncode == 0
+        got = _run("--dump-reads", flag, str(f))
+        assert got.returncode == 0 and got.stdout == dump(recs), name
         for extra in ([], ["--threads", "3", "--batch-reads", "1000"], ["--read-offset", "1234"]):
             got = _run("--dump-reads-mt", flag, str(f), *extra)
             assert got.returncode == 0, (name, extra, got.stderr)
-            w = _lens(want.stdout)
-            if "--read-offset" in extra:
-                w = "".join(w.splitlines(True)[1234:])
-            assert got.stdout == w, (name, extra)
+            assert got.stdout == lens(recs[1234:] if "--read-offset" in extra else recs), (name, extra)
     gzf = tmp_path / "a.fq.gz"
     with gzip.open(gzf, "wt", newline="") as f:
-        f.write(cases[0][1])
-    assert _run("--dump-reads-mt", "--fastq", str(gzf)).stdout == _lens(_run("--dump-reads", "--fastq", str(tmp_path / "a.fq")).stdout)
+        f.write(cases[0][1][0])
+    assert _run("--dump-reads-mt", "--fastq", str(gzf)).stdout == lens(cases[0][1][1])
     # malformed input: quality shorter than the sequence, in the middle of a large file
     bad = tmp_path / "bad.fq"
-    bad.write_text(cases[0][1][:5_000_000].rsplit("@r", 1)[0] + "@x\nACGT\n+\nII\n" + "@y\nAC\n+\nII\n")
+    good = cases[0][1][0][:5_000_000].rsplit("@r", 1)[0]
+    bad.write_text(good + "@x\nACGT\n+\nII\n" + "@y\nAC\n+\nII\n")
     assert _run("--dump-reads-mt", "--fastq", str(bad)).returncode == 12
+    got = _run("--dump-reads", "--fastq", str(bad))  # the records before the malformed one, then the error
+    want = cases[0][1][1][:good.count("@r")] + [("x", "ACGT")]  # (x's quality ends in the "@y" line; "AC" is bad)
+    assert got.returncode == 12 and got.stdout == dump(want)
 
 
 def test_exit_codes_without_gpu(tmp_path):
