@@ -1561,18 +1561,13 @@ int run_segmented_sort(cudaStream_t st, DevBuf& worklist, uint64_t* keys, const 
 static int grow_preserve(DevBuf& buf, size_t used_bytes, size_t need_bytes, cudaStream_t st) {
   if (need_bytes <= buf.cap && buf.p) return 0;
   size_t want = std::max(need_bytes + need_bytes / 2, (size_t)1 << 20);
-  void* np = nullptr;
-  cudaError_t e = cudaMalloc(&np, want);
-  if (e != cudaSuccess) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-  }
+  DevPtr<uint8_t> np;
+  MTSV_TRY(dev_alloc(np, want));
   if (buf.p && used_bytes) {
-    MTSV_CUDA_TRY(cudaMemcpyAsync(np, buf.p, used_bytes, cudaMemcpyDeviceToDevice, st));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(np.get(), buf.p.get(), used_bytes, cudaMemcpyDeviceToDevice, st));
     MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   }
-  if (buf.p) cudaFree(buf.p);
-  buf.p = np;
+  buf.p = std::move(np);
   buf.cap = want;
   return 0;
 }
@@ -1588,13 +1583,17 @@ __global__ void publish_counters_kernel(const BatchCounters* __restrict__ d, Bat
 }
 
 static int fetch_counters(Lane& ln, const BatchCounters* d_ctr, BatchCounters* out, cudaStream_t st) {
-  if (!ln.h_ctr) {
-    MTSV_CUDA_TRY(cudaHostAlloc((void**)&ln.h_ctr, sizeof(BatchCounters), cudaHostAllocMapped));
-    MTSV_CUDA_TRY(cudaHostGetDevicePointer((void**)&ln.h_ctr_dev, ln.h_ctr, 0));
+  if (!ln.h_ctr) {  // the lane keeps the buffer only with its device address
+    PinnedPtr<BatchCounters> h;
+    BatchCounters* h_dev = nullptr;
+    MTSV_TRY(pinned_alloc(h, 1, cudaHostAllocMapped));
+    MTSV_CUDA_TRY(cudaHostGetDevicePointer((void**)&h_dev, h.get(), 0));
+    ln.h_ctr = std::move(h);
+    ln.h_ctr_dev = h_dev;
   }
   MTSV_LAUNCH(publish_counters_kernel, 1, 160, 0, st, d_ctr, ln.h_ctr_dev);
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  memcpy(out, ln.h_ctr, sizeof(BatchCounters));
+  memcpy(out, ln.h_ctr.get(), sizeof(BatchCounters));
   return 0;
 }
 
@@ -1863,7 +1862,7 @@ int SubBatch::verify() {
   MTSV_LAUNCH(cand_order_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(),
               ws.cand_flag.as<uint32_t>(), n_cand, ws.cand_order.as<uint32_t>());
   BinnerJobs jobs{rv, ev, p, ws.cand_dense.as<CandRec>(), ws.cand_q.as<uint32_t>(),
-                  ws.cand_off.as<uint32_t>(), ws.cand_order.as<uint32_t>(), h->ix.text, n_cand};
+                  ws.cand_off.as<uint32_t>(), ws.cand_order.as<uint32_t>(), h->ix.text.get(), n_cand};
   n_verified = n_cand;
   if (ssw) {
     MTSV_TRY(verify_ssw(jobs));
@@ -1889,7 +1888,7 @@ int SubBatch::launch_verify_warp(const BinnerJobs& jobs) {
   const unsigned grid = (jobs.n + kVerifyThreads - 1) / kVerifyThreads;
   const size_t smem = (size_t)5 * W * kVerifyThreads * sizeof(uint64_t);
   auto kernel = uniform ? verify_warp_kernel<W, true> : verify_warp_kernel<W, false>;
-  MTSV_LAUNCH(kernel, grid, kVerifyThreads, smem, st, jobs, h->ix.text4, h->ix.text4_words - 1, ws.cand_edit.as<uint32_t>());
+  MTSV_LAUNCH(kernel, grid, kVerifyThreads, smem, st, jobs, h->ix.text4.get(), h->ix.text4_words - 1, ws.cand_edit.as<uint32_t>());
   MTSV_CUDA_TRY(cudaGetLastError());
   return 0;
 }
@@ -1934,7 +1933,7 @@ int SubBatch::verify_grouped(const BinnerJobs& jobs, bool* done) {
       MTSV_LAUNCH(cand_class_kernel, grid, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand, (uint32_t*)nullptr, ctr, 0);
     return 0;
   }
-  MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_edit.p, 0xff, (size_t)n_cand * 4, st));  // kNoEdit until verified
+  MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_edit.p.get(), 0xff, (size_t)n_cand * 4, st));  // kNoEdit until verified
   BinnerJobs round_jobs = jobs;
   round_jobs.order = ws.cand_order2.as<uint32_t>();
   MTSV_LAUNCH(cand_compact_order_kernel, grid, 256, 0, st, ws.cand_order.as<uint32_t>(), flag, n_cand,
@@ -1994,8 +1993,8 @@ int SubBatch::select_append(uint64_t* out_total) {
     MTSV_CUDA_TRY(cudaMemsetAsync(seg_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
     MTSV_CUDA_TRY(cudaMemsetAsync(tax_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
   } else {
-    MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_off.p, 0, qn * 4, st));
-    MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_off.p, 0, qn * 4, st));
+    MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_off.p.get(), 0, qn * 4, st));
+    MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_off.p.get(), 0, qn * 4, st));
   }
   MTSV_TRY(emit_acquire(h, ln));
   Lane& other = h->lanes[&ln == &h->lanes[0] ? 1 : 0];
@@ -2111,7 +2110,7 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   MTSV_TRY(ws.out_hit_off.reserve((n_reads + 1) * 8));
   uint64_t total = 0;
   if (n_reads == 0) {
-    MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_hit_off.p, 0, 8, st));
+    MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_hit_off.p.get(), 0, 8, st));
     MTSV_TRY(grow_preserve(ws.out_hits, 0, sizeof(HitRec), st));
   }
   // ---- lanes: the slices of a batch alternate between two lanes (own stream, scratch and host thread each): the
@@ -2190,7 +2189,7 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
     return set_error(h->abort_rc, "%s", h->abort_msg.c_str());
   }
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  if (d_out) *d_out = ws.out_hits.p;
+  if (d_out) *d_out = ws.out_hits.p.get();
   if (d_out_off) *d_out_off = ws.out_hit_off.as<uint64_t>();
   if (n_out) *n_out = total;
   return 0;
@@ -2223,37 +2222,29 @@ int backward_search_batch(mtsvgpu_index* h, const uint8_t* pats, uint32_t pat_le
   if (n_pats > 0x0fffffffull || n_pats * pat_len > 0x7fffffffull) return set_error(MTSVGPU_ELIMIT, "too many patterns");
   MTSV_CUDA_TRY(cudaSetDevice(h->ix.device));
   cudaStream_t st = h->stream;
+  std::vector<uint64_t> off(n_pats + 1);
+  for (uint64_t i = 0; i <= n_pats; ++i) off[i] = i * pat_len;
+  const uint32_t w_max = (pat_len + 63) / 64;
+  const uint32_t total_words = (uint32_t)((n_pats * pat_len) >> 6) + (uint32_t)n_pats;
   DevBuf dp, doff, dw, dl, du;
-  int rc = 0;
-  do {
-    std::vector<uint64_t> off(n_pats + 1);
-    for (uint64_t i = 0; i <= n_pats; ++i) off[i] = i * pat_len;
-    const uint32_t w_max = (pat_len + 63) / 64;
-    const uint32_t total_words = (uint32_t)((n_pats * pat_len) >> 6) + (uint32_t)n_pats;
-    if ((rc = dp.reserve(n_pats * pat_len + 16))) break;
-    if ((rc = doff.reserve((n_pats + 1) * 8))) break;
-    if ((rc = dw.reserve(((size_t)total_words + 1) * sizeof(ReadWord)))) break;
-    if ((rc = dl.reserve(n_pats * 8))) break;
-    if ((rc = du.reserve(n_pats * 8))) break;
-    cudaMemcpyAsync(dp.p, pats, n_pats * pat_len, cudaMemcpyHostToDevice, st);
-    cudaMemcpyAsync(doff.p, off.data(), (n_pats + 1) * 8, cudaMemcpyHostToDevice, st);
-    ReadsView pv{dp.as<uint8_t>(), doff.as<uint64_t>(), 0, (uint32_t)n_pats};
-    EncView ev{dw.as<ReadWord>(), total_words};
-    const uint64_t threads = n_pats * w_max;
-    MTSV_LAUNCH(encode_fwd_kernel, (unsigned)((threads * 32 + 255) / 256), 256, 0, st, pv, dw.as<ReadWord>(), w_max, 0);
-    MTSV_LAUNCH(bs_patterns_kernel, (unsigned)((n_pats + 127) / 128), 128, 0, st, h->ix.fm_view(),
-                h->ix.ktab_view(), pv, ev, pat_len, n_pats, dl.as<uint64_t>(), du.as<uint64_t>());
-    cudaMemcpyAsync(lower, dl.p, n_pats * 8, cudaMemcpyDeviceToHost, st);
-    cudaMemcpyAsync(upper, du.p, n_pats * 8, cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) rc = set_error(MTSVGPU_ECUDA, "backward_search: %s", cudaGetErrorString(e));
-  } while (0);
-  dp.release();
-  doff.release();
-  dw.release();
-  dl.release();
-  du.release();
-  return rc;
+  MTSV_TRY(dp.reserve(n_pats * pat_len + 16));
+  MTSV_TRY(doff.reserve((n_pats + 1) * 8));
+  MTSV_TRY(dw.reserve(((size_t)total_words + 1) * sizeof(ReadWord)));
+  MTSV_TRY(dl.reserve(n_pats * 8));
+  MTSV_TRY(du.reserve(n_pats * 8));
+  cudaMemcpyAsync(dp.p.get(), pats, n_pats * pat_len, cudaMemcpyHostToDevice, st);
+  cudaMemcpyAsync(doff.p.get(), off.data(), (n_pats + 1) * 8, cudaMemcpyHostToDevice, st);
+  ReadsView pv{dp.as<uint8_t>(), doff.as<uint64_t>(), 0, (uint32_t)n_pats};
+  EncView ev{dw.as<ReadWord>(), total_words};
+  const uint64_t threads = n_pats * w_max;
+  MTSV_LAUNCH(encode_fwd_kernel, (unsigned)((threads * 32 + 255) / 256), 256, 0, st, pv, dw.as<ReadWord>(), w_max, 0);
+  MTSV_LAUNCH(bs_patterns_kernel, (unsigned)((n_pats + 127) / 128), 128, 0, st, h->ix.fm_view(), h->ix.ktab_view(), pv,
+              ev, pat_len, n_pats, dl.as<uint64_t>(), du.as<uint64_t>());
+  cudaMemcpyAsync(lower, dl.p.get(), n_pats * 8, cudaMemcpyDeviceToHost, st);
+  cudaMemcpyAsync(upper, du.p.get(), n_pats * 8, cudaMemcpyDeviceToHost, st);
+  cudaError_t e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "backward_search: %s", cudaGetErrorString(e));
+  return 0;
 }
 
 __global__ void locate_rows_kernel(FmView fm, SaView sv, const uint64_t* __restrict__ rows, uint64_t n,
@@ -2270,20 +2261,15 @@ int locate_batch(mtsvgpu_index* h, const uint64_t* rows, uint64_t n_rows, uint64
   MTSV_CUDA_TRY(cudaSetDevice(h->ix.device));
   cudaStream_t st = h->stream;
   DevBuf dr, dp;
-  int rc = 0;
-  do {
-    if ((rc = dr.reserve(n_rows * 8))) break;
-    if ((rc = dp.reserve(n_rows * 8))) break;
-    cudaMemcpyAsync(dr.p, rows, n_rows * 8, cudaMemcpyHostToDevice, st);
-    MTSV_LAUNCH(locate_rows_kernel, (unsigned)((n_rows + 127) / 128), 128, 0, st, h->ix.fm_view(),
-                h->ix.sa_view(), dr.as<uint64_t>(), n_rows, dp.as<uint64_t>());
-    cudaMemcpyAsync(pos, dp.p, n_rows * 8, cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) rc = set_error(MTSVGPU_ECUDA, "locate: %s", cudaGetErrorString(e));
-  } while (0);
-  dr.release();
-  dp.release();
-  return rc;
+  MTSV_TRY(dr.reserve(n_rows * 8));
+  MTSV_TRY(dp.reserve(n_rows * 8));
+  cudaMemcpyAsync(dr.p.get(), rows, n_rows * 8, cudaMemcpyHostToDevice, st);
+  MTSV_LAUNCH(locate_rows_kernel, (unsigned)((n_rows + 127) / 128), 128, 0, st, h->ix.fm_view(), h->ix.sa_view(),
+              dr.as<uint64_t>(), n_rows, dp.as<uint64_t>());
+  cudaMemcpyAsync(pos, dp.p.get(), n_rows * 8, cudaMemcpyDeviceToHost, st);
+  cudaError_t e = cudaStreamSynchronize(st);
+  if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "locate: %s", cudaGetErrorString(e));
+  return 0;
 }
 
 int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off, const uint8_t* texts,
@@ -2291,12 +2277,7 @@ int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off
   if (!pat_off || !text_off || !edits) return set_error(MTSVGPU_EINVAL, "null argument");
   if (n_pairs == 0) return 0;
   if (n_pairs > 0x7fffffffull) return set_error(MTSVGPU_ELIMIT, "too many pairs");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  MTSV_CUDA_TRY(cudaSetDevice(device));
+  MTSV_TRY(use_device(device));
   uint32_t max_len = 0;
   for (uint64_t i = 0; i < n_pairs; ++i) {
     if (pat_off[i + 1] < pat_off[i] || text_off[i + 1] < text_off[i])
@@ -2306,37 +2287,28 @@ int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off
   if (max_len > kMaxReadLenDev) return set_error(MTSVGPU_ELIMIT, "pattern longer than %u", kMaxReadLenDev);
   uint64_t pb = pat_off[n_pairs], tb = text_off[n_pairs];
   DevBuf dp, dpo, dt, dto, de, dw;
-  int rc = 0;
-  do {
-    if ((rc = dp.reserve(pb + 16))) break;
-    if ((rc = dt.reserve(tb + 16))) break;
-    if ((rc = dpo.reserve((n_pairs + 1) * 8))) break;
-    if ((rc = dto.reserve((n_pairs + 1) * 8))) break;
-    if ((rc = de.reserve(n_pairs * 4))) break;
-    if (pb) cudaMemcpy(dp.p, pats, pb, cudaMemcpyHostToDevice);
-    if (tb) cudaMemcpy(dt.p, texts, tb, cudaMemcpyHostToDevice);
-    cudaMemcpy(dpo.p, pat_off, (n_pairs + 1) * 8, cudaMemcpyHostToDevice);
-    cudaMemcpy(dto.p, text_off, (n_pairs + 1) * 8, cudaMemcpyHostToDevice);
-    // encode the patterns (raw bytes: N is its own class) like a one-strand read batch
-    const uint32_t w_max = std::max(1u, (max_len + 63) / 64);
-    const uint32_t total_words = (uint32_t)(pb >> 6) + (uint32_t)n_pairs;
-    if ((rc = dw.reserve(((size_t)total_words + 1) * sizeof(ReadWord)))) break;
-    ReadsView pv{dp.as<uint8_t>(), dpo.as<uint64_t>(), 0, (uint32_t)n_pairs};
-    EncView ev{dw.as<ReadWord>(), total_words};
-    const uint64_t threads = n_pairs * w_max;
-    MTSV_LAUNCH(encode_fwd_kernel, (unsigned)((threads * 32 + 255) / 256), 256, 0, 0, pv, dw.as<ReadWord>(), w_max, 1);
-    PairJobs jobs{pv, ev, dt.as<uint8_t>(), dto.as<uint64_t>(), (uint32_t)n_pairs};
-    if ((rc = launch_verify<5>(jobs, std::max(max_len, 1u), de.as<uint32_t>(), nullptr, nullptr, 0))) break;
-    cudaError_t e = cudaMemcpy(edits, de.p, n_pairs * 4, cudaMemcpyDeviceToHost);
-    if (e != cudaSuccess) rc = set_error(MTSVGPU_ECUDA, "edit_distance: %s", cudaGetErrorString(e));
-  } while (0);
-  dp.release();
-  dpo.release();
-  dt.release();
-  dto.release();
-  de.release();
-  dw.release();
-  return rc;
+  MTSV_TRY(dp.reserve(pb + 16));
+  MTSV_TRY(dt.reserve(tb + 16));
+  MTSV_TRY(dpo.reserve((n_pairs + 1) * 8));
+  MTSV_TRY(dto.reserve((n_pairs + 1) * 8));
+  MTSV_TRY(de.reserve(n_pairs * 4));
+  if (pb) cudaMemcpy(dp.p.get(), pats, pb, cudaMemcpyHostToDevice);
+  if (tb) cudaMemcpy(dt.p.get(), texts, tb, cudaMemcpyHostToDevice);
+  cudaMemcpy(dpo.p.get(), pat_off, (n_pairs + 1) * 8, cudaMemcpyHostToDevice);
+  cudaMemcpy(dto.p.get(), text_off, (n_pairs + 1) * 8, cudaMemcpyHostToDevice);
+  // encode the patterns (raw bytes: N is its own class) like a one-strand read batch
+  const uint32_t w_max = std::max(1u, (max_len + 63) / 64);
+  const uint32_t total_words = (uint32_t)(pb >> 6) + (uint32_t)n_pairs;
+  MTSV_TRY(dw.reserve(((size_t)total_words + 1) * sizeof(ReadWord)));
+  ReadsView pv{dp.as<uint8_t>(), dpo.as<uint64_t>(), 0, (uint32_t)n_pairs};
+  EncView ev{dw.as<ReadWord>(), total_words};
+  const uint64_t threads = n_pairs * w_max;
+  MTSV_LAUNCH(encode_fwd_kernel, (unsigned)((threads * 32 + 255) / 256), 256, 0, 0, pv, dw.as<ReadWord>(), w_max, 1);
+  PairJobs jobs{pv, ev, dt.as<uint8_t>(), dto.as<uint64_t>(), (uint32_t)n_pairs};
+  MTSV_TRY(launch_verify<5>(jobs, std::max(max_len, 1u), de.as<uint32_t>(), nullptr, nullptr, 0));
+  cudaError_t e = cudaMemcpy(edits, de.p.get(), n_pairs * 4, cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "edit_distance: %s", cudaGetErrorString(e));
+  return 0;
 }
 
 }  // namespace mtsv

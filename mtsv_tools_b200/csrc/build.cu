@@ -18,7 +18,7 @@
 
 namespace mtsv {
 
-int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, uint32_t** d_sa_out, int verbose);
+int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, DevPtr<uint32_t>& sa_out, int verbose);
 int bwt_from_sa_device(const uint8_t* d_text, const uint32_t* d_sa, uint64_t n, cudaStream_t st, uint8_t* d_bwt);
 
 namespace {
@@ -92,19 +92,6 @@ struct FileWriter {
   void u8(uint8_t v) { raw(&v, 1); }
 };
 
-struct DevFree {
-  void* p = nullptr;
-  ~DevFree() {
-    if (p) cudaFree(p);
-  }
-};
-struct HostFree {
-  void* p = nullptr;
-  ~HostFree() {
-    if (p) cudaFreeHost(p);
-  }
-};
-
 }  // namespace
 
 int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi, const uint32_t* tax_id, uint64_t n_seqs,
@@ -120,13 +107,7 @@ int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi
     return set_error(MTSVGPU_ELIMIT, "reference has %llu symbols; this build keeps 32-bit rows (limit 2^32-64)",
                      (unsigned long long)n);
   if (total && !seqs) return set_error(MTSVGPU_EINVAL, "seqs is NULL");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
-  MTSV_CUDA_TRY(cudaSetDevice(device));
+  MTSV_TRY(use_device(device));
   const double t0 = now_s();
   const int verbose = getenv("MTSV_B200_VERBOSE") != nullptr;
 
@@ -153,15 +134,9 @@ int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi
     cudaStream_t s;
     ~StreamGuard() { cudaStreamDestroy(s); }
   } sg{st};
-  DevFree text_g, bwt_g;
-  {
-    cudaError_t e = cudaMalloc(&text_g.p, n + 16);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%llu) for the text failed: %s", (unsigned long long)(n + 16), cudaGetErrorString(e));
-    }
-  }
-  uint8_t* d_text = (uint8_t*)text_g.p;
+  DevPtr<uint8_t> text_g, bwt_g;
+  MTSV_TRY(dev_alloc(text_g, n + 16));
+  uint8_t* d_text = text_g.get();
   if (in_place) {
     if (total) MTSV_CUDA_TRY(cudaMemcpyAsync(d_text, seqs + seq_off[0], total, cudaMemcpyDefault, st));
   } else {
@@ -175,25 +150,15 @@ int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi
   MTSV_CUDA_TRY(cudaMemsetAsync(d_text + n, 0, 16, st));
   MTSV_CUDA_TRY(cudaGetLastError());
 
-  uint32_t* d_sa = nullptr;
-  MTSV_TRY(suffix_array_device(d_text, n, st, &d_sa, verbose));
+  DevPtr<uint32_t> d_sa;
+  MTSV_TRY(suffix_array_device(d_text, n, st, d_sa, verbose));
   const double t_sa = now_s();
-  {
-    cudaError_t e = cudaMalloc(&bwt_g.p, n + 64);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      cudaFree(d_sa);
-      return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%llu) for the BWT failed: %s", (unsigned long long)(n + 64), cudaGetErrorString(e));
-    }
-  }
-  uint8_t* d_bwt = (uint8_t*)bwt_g.p;
+  MTSV_TRY(dev_alloc(bwt_g, n + 64));
+  uint8_t* d_bwt = bwt_g.get();
   MTSV_CUDA_TRY(cudaMemsetAsync(d_bwt + n, 0, 64, st));
-  int rc = bwt_from_sa_device(d_text, d_sa, n, st, d_bwt);
-  if (rc == 0 && cudaStreamSynchronize(st) != cudaSuccess) rc = set_error(MTSVGPU_ECUDA, "BWT construction failed: %s", cudaGetErrorString(cudaGetLastError()));
-  if (rc != 0) {
-    cudaFree(d_sa);
-    return rc;
-  }
+  MTSV_TRY(bwt_from_sa_device(d_text, d_sa.get(), n, st, d_bwt));
+  if (cudaStreamSynchronize(st) != cudaSuccess)
+    return set_error(MTSVGPU_ECUDA, "BWT construction failed: %s", cudaGetErrorString(cudaGetLastError()));
   const double t_bwt = now_s();
   if (verbose)
     fprintf(stderr, "[mtsv_b200 build] %llu symbols, %llu bins: suffix array %.2f s, BWT %.3f s\n", (unsigned long long)n,
@@ -208,8 +173,8 @@ int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi
   parts.bwt = d_bwt;
   parts.bwt_on_device = true;
   parts.sa_rate = 32;  // what mtsv-build samples by default (src/bin/mtsv-build.rs); only recorded
-  parts.d_sa_full = d_sa;  // consumed by index_assemble
-  MTSV_TRY(index_assemble(parts, device, opts, out));
+  parts.d_sa_full = std::move(d_sa);
+  MTSV_TRY(index_assemble(std::move(parts), device, opts, out));
   (*out)->ix.build_seconds = t_bwt - t0;
   return 0;
 }
@@ -225,30 +190,30 @@ int index_write(mtsvgpu_index* h, const char* path, uint32_t sample_interval, ui
   w.f = fopen(path, "wb");
   if (!w.f) return set_error(MTSVGPU_EIO, "cannot create %s: %s", path, strerror(errno));
   const uint64_t chunk = 1ull << 25;  // 32 Mi items per step
-  DevFree dev;
-  HostFree host;
-  MTSV_CUDA_TRY(cudaMalloc(&dev.p, chunk * 8));
-  MTSV_CUDA_TRY(cudaMallocHost(&host.p, chunk * 8));
-  uint8_t* d8 = (uint8_t*)dev.p;
-  uint64_t* d64 = (uint64_t*)dev.p;
+  DevPtr<uint64_t> dev;
+  PinnedPtr<uint64_t> host;
+  MTSV_TRY(dev_alloc(dev, chunk));
+  MTSV_TRY(pinned_alloc(host, chunk));
+  uint8_t* d8 = (uint8_t*)dev.get();
+  uint64_t* d64 = dev.get();
   const FmView fm = d.fm_view();
 
   // sequences: Vec<u8>
   w.u64(n);
   for (uint64_t o = 0; o < n && w.ok; o += chunk * 8) {
     const uint64_t c = std::min<uint64_t>(chunk * 8, n - o);
-    MTSV_CUDA_TRY(cudaMemcpyAsync(host.p, d.text + o, c, cudaMemcpyDeviceToHost, st));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(host.get(), d.text.get() + o, c, cudaMemcpyDeviceToHost, st));
     MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-    w.raw(host.p, c);
+    w.raw(host.get(), c);
   }
   // bins: Vec<Bin{gi, tax_id, start, end}>
   {
     const uint64_t nb = d.n_bins;
     std::vector<uint32_t> bs(nb), be(nb), bt(nb), bg(nb);
-    MTSV_CUDA_TRY(cudaMemcpy(bs.data(), d.bin_start, nb * 4, cudaMemcpyDeviceToHost));
-    MTSV_CUDA_TRY(cudaMemcpy(be.data(), d.bin_end, nb * 4, cudaMemcpyDeviceToHost));
-    MTSV_CUDA_TRY(cudaMemcpy(bt.data(), d.bin_tax, nb * 4, cudaMemcpyDeviceToHost));
-    MTSV_CUDA_TRY(cudaMemcpy(bg.data(), d.bin_gi, nb * 4, cudaMemcpyDeviceToHost));
+    MTSV_CUDA_TRY(cudaMemcpy(bs.data(), d.bin_start.get(), nb * 4, cudaMemcpyDeviceToHost));
+    MTSV_CUDA_TRY(cudaMemcpy(be.data(), d.bin_end.get(), nb * 4, cudaMemcpyDeviceToHost));
+    MTSV_CUDA_TRY(cudaMemcpy(bt.data(), d.bin_tax.get(), nb * 4, cudaMemcpyDeviceToHost));
+    MTSV_CUDA_TRY(cudaMemcpy(bg.data(), d.bin_gi.get(), nb * 4, cudaMemcpyDeviceToHost));
     w.u64(nb);
     for (uint64_t i = 0; i < nb; ++i) {
       w.u32(bg[i]);
@@ -262,9 +227,9 @@ int index_write(mtsvgpu_index* h, const char* path, uint32_t sample_interval, ui
   for (uint64_t o = 0; o < n && w.ok; o += chunk * 8) {
     const uint64_t c = std::min<uint64_t>(chunk * 8, n - o);
     MTSV_LAUNCH(bwt_unpack_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, o, c, d8);
-    MTSV_CUDA_TRY(cudaMemcpyAsync(host.p, d8, c, cudaMemcpyDeviceToHost, st));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(host.get(), d8, c, cudaMemcpyDeviceToHost, st));
     MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-    w.raw(host.p, c);
+    w.raw(host.get(), c);
   }
   // less: counts of smaller bytes, over the symbols 0 ..= 't'+1 of n_alphabet() "ACGTNacgtn" (bio::bwt::less)
   {
@@ -308,13 +273,13 @@ int index_write(mtsvgpu_index* h, const char* path, uint32_t sample_interval, ui
       for (uint64_t o = 0; o < len && w.ok; o += chunk) {
         const uint64_t c = std::min<uint64_t>(chunk, len - o);
         if (zero_row) {
-          memset(host.p, 0, c * 8);
+          memset(host.get(), 0, c * 8);
         } else {
           MTSV_LAUNCH(occ_checkpoint_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, sym, K, o, c, d64);
-          MTSV_CUDA_TRY(cudaMemcpyAsync(host.p, d64, c * 8, cudaMemcpyDeviceToHost, st));
+          MTSV_CUDA_TRY(cudaMemcpyAsync(host.get(), d64, c * 8, cudaMemcpyDeviceToHost, st));
           MTSV_CUDA_TRY(cudaStreamSynchronize(st));
         }
-        w.raw(host.p, c * 8);
+        w.raw(host.get(), c * 8);
       }
     }
     w.u32(sample_interval);
@@ -326,9 +291,9 @@ int index_write(mtsvgpu_index* h, const char* path, uint32_t sample_interval, ui
     for (uint64_t o = 0; o < len && w.ok; o += chunk) {
       const uint64_t c = std::min<uint64_t>(chunk, len - o);
       MTSV_LAUNCH(sa_sample_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, d.sa_view(), s, o, c, d64);
-      MTSV_CUDA_TRY(cudaMemcpyAsync(host.p, d64, c * 8, cudaMemcpyDeviceToHost, st));
+      MTSV_CUDA_TRY(cudaMemcpyAsync(host.get(), d64, c * 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-      w.raw(host.p, c * 8);
+      w.raw(host.get(), c * 8);
     }
     w.u64(s);
     if (d.dollar_row % s != 0) {  // the row holding the sentinel is kept when it is not sampled (bio SuffixArray::sample)
@@ -358,15 +323,15 @@ int index_export(mtsvgpu_index* h, uint8_t* text_out, uint8_t* bwt_out, uint64_t
   cudaStream_t st = h->stream;
   const uint64_t n = d.n;
   const FmView fm = d.fm_view();
-  if (text_out) MTSV_CUDA_TRY(cudaMemcpyAsync(text_out, d.text, n, cudaMemcpyDeviceToHost, st));
+  if (text_out) MTSV_CUDA_TRY(cudaMemcpyAsync(text_out, d.text.get(), n, cudaMemcpyDeviceToHost, st));
   const uint64_t chunk = 1ull << 28;
-  DevFree dev;
-  if (bwt_out || sample_out) MTSV_CUDA_TRY(cudaMalloc(&dev.p, chunk));
+  DevPtr<uint8_t> dev;
+  if (bwt_out || sample_out) MTSV_TRY(dev_alloc(dev, chunk));
   if (bwt_out) {
     for (uint64_t o = 0; o < n; o += chunk) {
       const uint64_t c = std::min<uint64_t>(chunk, n - o);
-      MTSV_LAUNCH(bwt_unpack_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, o, c, (uint8_t*)dev.p);
-      MTSV_CUDA_TRY(cudaMemcpyAsync(bwt_out + o, dev.p, c, cudaMemcpyDeviceToHost, st));
+      MTSV_LAUNCH(bwt_unpack_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, o, c, dev.get());
+      MTSV_CUDA_TRY(cudaMemcpyAsync(bwt_out + o, dev.get(), c, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     }
   }
@@ -375,8 +340,8 @@ int index_export(mtsvgpu_index* h, uint8_t* text_out, uint8_t* bwt_out, uint64_t
     for (uint64_t o = 0; o < len; o += step) {
       const uint64_t c = std::min<uint64_t>(step, len - o);
       MTSV_LAUNCH(sa_sample_kernel, (unsigned)((c + 255) / 256), 256, 0, st, fm, d.sa_view(), (uint64_t)sa_sample, o, c,
-                  (uint64_t*)dev.p);
-      MTSV_CUDA_TRY(cudaMemcpyAsync(sample_out + o, dev.p, c * 8, cudaMemcpyDeviceToHost, st));
+                  (uint64_t*)dev.get());
+      MTSV_CUDA_TRY(cudaMemcpyAsync(sample_out + o, dev.get(), c * 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     }
   }
@@ -389,26 +354,19 @@ int index_export(mtsvgpu_index* h, uint8_t* text_out, uint8_t* bwt_out, uint64_t
 int suffix_array_host(int device, const uint8_t* text, uint64_t n, uint32_t* sa_out, uint8_t* bwt_out) {
   if (!text || !sa_out || n == 0) return set_error(MTSVGPU_EINVAL, "null argument");
   if (text[n - 1] != '$') return set_error(MTSVGPU_EINVAL, "the text must end with '$'");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
-  MTSV_CUDA_TRY(cudaSetDevice(device));
-  DevFree t, b, sa_g;
-  MTSV_CUDA_TRY(cudaMalloc(&t.p, n + 16));
-  MTSV_CUDA_TRY(cudaMemcpy(t.p, text, n, cudaMemcpyHostToDevice));
-  uint32_t* d_sa = nullptr;
-  MTSV_TRY(suffix_array_device((const uint8_t*)t.p, n, cudaStreamPerThread, &d_sa, getenv("MTSV_B200_VERBOSE") != nullptr));
-  sa_g.p = d_sa;
+  MTSV_TRY(use_device(device));
+  DevPtr<uint8_t> t, b;
+  DevPtr<uint32_t> sa;
+  MTSV_TRY(dev_alloc(t, n + 16));
+  MTSV_CUDA_TRY(cudaMemcpy(t.get(), text, n, cudaMemcpyHostToDevice));
+  MTSV_TRY(suffix_array_device(t.get(), n, cudaStreamPerThread, sa, getenv("MTSV_B200_VERBOSE") != nullptr));
   MTSV_CUDA_TRY(cudaStreamSynchronize(cudaStreamPerThread));
-  MTSV_CUDA_TRY(cudaMemcpy(sa_out, d_sa, n * 4, cudaMemcpyDeviceToHost));
+  MTSV_CUDA_TRY(cudaMemcpy(sa_out, sa.get(), n * 4, cudaMemcpyDeviceToHost));
   if (bwt_out) {
-    MTSV_CUDA_TRY(cudaMalloc(&b.p, n));
-    MTSV_TRY(bwt_from_sa_device((const uint8_t*)t.p, d_sa, n, cudaStreamPerThread, (uint8_t*)b.p));
+    MTSV_TRY(dev_alloc(b, n));
+    MTSV_TRY(bwt_from_sa_device(t.get(), sa.get(), n, cudaStreamPerThread, b.get()));
     MTSV_CUDA_TRY(cudaStreamSynchronize(cudaStreamPerThread));
-    MTSV_CUDA_TRY(cudaMemcpy(bwt_out, b.p, n, cudaMemcpyDeviceToHost));
+    MTSV_CUDA_TRY(cudaMemcpy(bwt_out, b.get(), n, cudaMemcpyDeviceToHost));
   }
   return 0;
 }

@@ -102,19 +102,13 @@ int mtsvgpu_assign_batch_device(mtsvgpu_index* ix, const uint8_t* d_seqs, const 
                           d_out_off, n_out);
 }
 
-static int ensure_pinned(void** p, size_t* cap, size_t bytes) {
-  if (bytes <= *cap && *p) return 0;
-  if (*p) cudaFreeHost(*p);
-  *p = nullptr;
-  *cap = 0;
-  size_t want = bytes + bytes / 2 + 4096;
-  cudaError_t e = cudaMallocHost(p, want);
-  if (e != cudaSuccess) {
-    (void)cudaGetLastError();
-    *p = nullptr;
-    return set_error(MTSVGPU_ENOMEM, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
-  }
-  *cap = want;
+static int ensure_pinned(PinnedPtr<uint8_t>& p, size_t& cap, size_t bytes) {
+  if (bytes <= cap && p) return 0;
+  p.reset();
+  cap = 0;
+  const size_t want = bytes + bytes / 2 + 4096;
+  MTSV_TRY(pinned_alloc(p, want));
+  cap = want;
   return 0;
 }
 
@@ -176,9 +170,9 @@ int HostUpload::results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read
   const uint8_t* d_recs = ix->ws.out_hits.as<uint8_t>();
   const uint64_t* d_off = ix->ws.out_hit_off.as<uint64_t>();
   if (n_hits)
-    MTSV_CUDA_TRY(cudaMemcpyAsync((uint8_t*)ix->pin_hits + first_hit * rec_bytes, d_recs + first_hit * rec_bytes,
+    MTSV_CUDA_TRY(cudaMemcpyAsync(ix->pin_hits.get() + first_hit * rec_bytes, d_recs + first_hit * rec_bytes,
                                   n_hits * rec_bytes, cudaMemcpyDeviceToHost, ix->copy_out_stream));
-  MTSV_CUDA_TRY(cudaMemcpyAsync((uint64_t*)ix->pin_off + first_read, d_off + first_read,
+  MTSV_CUDA_TRY(cudaMemcpyAsync((uint64_t*)ix->pin_off.get() + first_read, d_off + first_read,
                                 (n_reads + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out_stream));
   out_copied_hits = first_hit + n_hits;
   out_copied_reads = first_read + n_reads;
@@ -311,7 +305,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
       }
     });
   } else {
-    MTSV_CUDA_TRY(cudaMemcpyAsync(ws.d_seq_off.p, offs, 8, cudaMemcpyHostToDevice, cin));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(ws.d_seq_off.p.get(), offs, 8, cudaMemcpyHostToDevice, cin));
   }
   const double t_enq = trace ? now() : 0;
   // ---- compute (each sub-batch waits for its slice) ----
@@ -341,10 +335,10 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   if (pinned_result) {
     // slices may still be on their way into the buffers ensure_pinned is about to replace
     MTSV_CUDA_TRY(cudaStreamSynchronize(ix->copy_out_stream));
-    MTSV_TRY(ensure_pinned(&ix->pin_hits, &ix->pin_hits_cap, hb));
-    MTSV_TRY(ensure_pinned(&ix->pin_off, &ix->pin_off_cap, ob));
-    h_hits = ix->pin_hits;
-    h_off = (uint64_t*)ix->pin_off;
+    MTSV_TRY(ensure_pinned(ix->pin_hits, ix->pin_hits_cap, hb));
+    MTSV_TRY(ensure_pinned(ix->pin_off, ix->pin_off_cap, ob));
+    h_hits = ix->pin_hits.get();
+    h_off = (uint64_t*)ix->pin_off.get();
   } else {
     h_hits = malloc(hb);
     h_off = (uint64_t*)malloc(ob);

@@ -167,17 +167,17 @@ struct mtsvgpu_comm {
   int device = 0;
   uint32_t rank = 0, world = 0;
   CommLayout lay{};
-  uint8_t* base = nullptr;  // my buffer
+  DevPtr<uint8_t> base;     // my buffer
   PeerTable peers{};        // peers' buffers as mapped into this process (base[rank] = base)
   bool connected = false;
   uint32_t epoch = 0;
   long long timeout_cycles = 60000000000ll;  // set from the SM clock at creation (the attribute query is a slow driver call)
-  uint32_t* d_status = nullptr;    // [0] wait status, [1] overflow flag
-  uint32_t* h_status = nullptr;    // mapped page-locked copy of the wait status
+  DevPtr<uint32_t> d_status;        // [0] wait status, [1] overflow flag
+  PinnedPtr<uint32_t> h_status;     // mapped copy of the wait status
   uint32_t* h_status_dev = nullptr;
-  uint64_t* d_n_out = nullptr;
-  mtsvgpu_taxhit* out = nullptr;   // merged result of the last batch (capacity world * cap_hits)
-  uint64_t* out_off = nullptr;
+  DevPtr<uint64_t> d_n_out;
+  DevPtr<mtsvgpu_taxhit> out;       // merged result of the last batch (capacity world * cap_hits)
+  DevPtr<uint64_t> out_off;
   CollapseScratch scratch;
 };
 
@@ -189,13 +189,6 @@ void comm_destroy(mtsvgpu_comm* c) {
   cudaDeviceSynchronize();
   for (uint32_t p = 0; p < c->world; ++p)
     if (p != c->rank && c->peers.base[p]) cudaIpcCloseMemHandle(c->peers.base[p]);
-  cudaFree(c->base);
-  cudaFree(c->d_status);
-  cudaFree(c->d_n_out);
-  cudaFree(c->out);
-  cudaFree(c->out_off);
-  if (c->h_status) cudaFreeHost(c->h_status);
-  c->scratch.release_all();
   delete c;
 }
 
@@ -208,45 +201,25 @@ int comm_create(int device, uint32_t rank, uint32_t world, uint64_t max_local_re
   if (max_local_reads == 0 || max_hits_per_source == 0) return set_error(MTSVGPU_EINVAL, "capacities must be > 0");
   if (max_local_reads > 0x7ffffff0ull || max_hits_per_source * world > 0xfffffff0ull)
     return set_error(MTSVGPU_ELIMIT, "comm capacities exceed 32-bit merge offsets");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
-  MTSV_CUDA_TRY(cudaSetDevice(device));
-  mtsvgpu_comm* c = new mtsvgpu_comm;
+  MTSV_TRY(use_device(device));
+  std::unique_ptr<mtsvgpu_comm, void (*)(mtsvgpu_comm*)> guard(new mtsvgpu_comm, comm_destroy);
+  mtsvgpu_comm* c = guard.get();
   c->device = device;
   c->rank = rank;
   c->world = world;
   c->lay.world = world;
   c->lay.max_local_reads = max_local_reads;
   c->lay.cap_hits = max_hits_per_source;
-  struct Guard {
-    mtsvgpu_comm* c;
-    ~Guard() {
-      if (c) comm_destroy(c);
-    }
-  } g{c};
-  const uint64_t bytes = c->lay.total_bytes();
-  {
-    cudaError_t e = cudaMalloc((void**)&c->base, bytes);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      c->base = nullptr;
-      return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%llu) of the exchange buffer failed: %s", (unsigned long long)bytes,
-                       cudaGetErrorString(e));
-    }
-  }
+  MTSV_TRY(dev_alloc(c->base, c->lay.total_bytes()));
   // header and per-read counts start at zero: a slot that was never (or not this batch) written reads as "no hits"
-  MTSV_CUDA_TRY(cudaMemset(c->base, 0, c->lay.hits_base()));
-  MTSV_CUDA_TRY(cudaMalloc((void**)&c->d_status, 16));
-  MTSV_CUDA_TRY(cudaMemset(c->d_status, 0, 16));
-  MTSV_CUDA_TRY(cudaMalloc((void**)&c->d_n_out, 8));
-  MTSV_CUDA_TRY(cudaHostAlloc((void**)&c->h_status, 16, cudaHostAllocMapped));
-  MTSV_CUDA_TRY(cudaHostGetDevicePointer((void**)&c->h_status_dev, c->h_status, 0));
-  MTSV_CUDA_TRY(cudaMalloc((void**)&c->out, ((uint64_t)world * max_hits_per_source + 1) * sizeof(mtsvgpu_taxhit)));
-  MTSV_CUDA_TRY(cudaMalloc((void**)&c->out_off, (max_local_reads + 1) * 8));
+  MTSV_CUDA_TRY(cudaMemset(c->base.get(), 0, c->lay.hits_base()));
+  MTSV_TRY(dev_alloc(c->d_status, 4));
+  MTSV_CUDA_TRY(cudaMemset(c->d_status.get(), 0, 16));
+  MTSV_TRY(dev_alloc(c->d_n_out, 1));
+  MTSV_TRY(pinned_alloc(c->h_status, 4, cudaHostAllocMapped));
+  MTSV_CUDA_TRY(cudaHostGetDevicePointer((void**)&c->h_status_dev, c->h_status.get(), 0));
+  MTSV_TRY(dev_alloc(c->out, (uint64_t)world * max_hits_per_source + 1));
+  MTSV_TRY(dev_alloc(c->out_off, max_local_reads + 1));
   MTSV_CUDA_TRY(cudaDeviceSynchronize());
   {
     int clock_khz = 2000000;
@@ -260,11 +233,10 @@ int comm_create(int device, uint32_t rank, uint32_t world, uint64_t max_local_re
   blob.world = world;
   blob.max_local_reads = max_local_reads;
   blob.cap_hits = max_hits_per_source;
-  MTSV_CUDA_TRY(cudaIpcGetMemHandle(&blob.mem, c->base));
+  MTSV_CUDA_TRY(cudaIpcGetMemHandle(&blob.mem, c->base.get()));
   memcpy(handle_out, &blob, sizeof blob);
-  c->peers.base[rank] = c->base;
-  g.c = nullptr;
-  *out = c;
+  c->peers.base[rank] = c->base.get();
+  *out = guard.release();
   return 0;
 }
 
@@ -321,7 +293,7 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
   }
   // ---- exchange: my hits of range d into rank d's buffer, flag, wait for everybody's flags here ----
   const uint32_t epoch = ++c->epoch, parity = epoch & 1u;
-  uint32_t* d_overflow = c->d_status + 1;
+  uint32_t* d_overflow = c->d_status.get() + 1;
   MTSV_CUDA_TRY(cudaMemsetAsync(d_overflow, 0, 4, st));
   MTSV_LAUNCH(chunk_check_kernel, 1, 32, 0, st, c->peers, c->lay, d_hit_off, n_reads, step, c->rank, epoch, d_overflow);
   {
@@ -335,22 +307,23 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
   MTSV_LAUNCH(chunk_signal_kernel, 1, 32, 0, st, c->peers, c->world, c->rank, epoch);
   const long long timeout_cycles = c->timeout_cycles;  // 30 s: a peer that never arrives is an error
   if (trace) cudaEventRecord(ev[4], st);
-  MTSV_LAUNCH(chunk_wait_kernel, 1, 32, 0, st, c->base, c->world, epoch, timeout_cycles, c->d_status, c->h_status_dev);
+  MTSV_LAUNCH(chunk_wait_kernel, 1, 32, 0, st, c->base.get(), c->world, epoch, timeout_cycles, c->d_status.get(),
+              c->h_status_dev);
   if (trace) cudaEventRecord(ev[2], st);
   // ---- merge epilogue over the world slots of my range (src/collapse.rs:597-602) ----
   const mtsvgpu_hit* part_hits[kMaxRanks];
   const uint32_t* part_counts[kMaxRanks];
   for (uint32_t s = 0; s < c->world; ++s) {
-    part_hits[s] = reinterpret_cast<const mtsvgpu_hit*>(c->base + c->lay.hits_off(parity, s));
-    part_counts[s] = reinterpret_cast<const uint32_t*>(c->base + c->lay.counts_off(parity, s));
+    part_hits[s] = reinterpret_cast<const mtsvgpu_hit*>(c->base.get() + c->lay.hits_off(parity, s));
+    part_counts[s] = reinterpret_cast<const uint32_t*>(c->base.get() + c->lay.counts_off(parity, s));
   }
   // (a failed exchange leaves slots untouched: they hold the whole, in-range lists of an earlier batch or the
   // zeros they were created with, so the merge below stays in bounds; its result is discarded)
   MTSV_TRY(collapse_taxid_async(c->scratch, st, c->world, part_hits, part_counts, (uint32_t)(hi - lo),
-                                (uint64_t)c->world * c->lay.cap_hits, c->out, c->out_off, c->d_n_out));
+                                (uint64_t)c->world * c->lay.cap_hits, c->out.get(), c->out_off.get(), c->d_n_out.get()));
   if (trace) cudaEventRecord(ev[3], st);
   uint64_t total = 0;
-  MTSV_CUDA_TRY(cudaMemcpyAsync(&total, c->d_n_out, 8, cudaMemcpyDeviceToHost, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(&total, c->d_n_out.get(), 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));  // the batch's one host synchronisation after the local binning
   if (trace) {
     float a = 0, b = 0, d = 0, sg = 0;
@@ -362,15 +335,15 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
             c->rank, (unsigned long long)n_hits, a, sg, b, d);
     for (auto& e : ev) cudaEventDestroy(e);
   }
-  const uint32_t status = c->h_status[0];
+  const uint32_t status = *c->h_status;
   if (status == 1)
     return set_error(MTSVGPU_ELIMIT, "chunk exchange: a rank produced more hits for one read range than max_hits_per_source "
                                      "(%llu); recreate the communicator with a larger capacity", (unsigned long long)c->lay.cap_hits);
   if (status == 2) return set_error(MTSVGPU_ECUDA, "chunk exchange: timed out waiting for a peer rank's data");
   if (first_read) *first_read = lo;
   if (n_local_reads) *n_local_reads = hi - lo;
-  if (d_out) *d_out = c->out;
-  if (d_out_off) *d_out_off = c->out_off;
+  if (d_out) *d_out = c->out.get();
+  if (d_out_off) *d_out_off = c->out_off.get();
   if (n_out) *n_out = total;
   return 0;
 }

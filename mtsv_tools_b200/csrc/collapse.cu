@@ -138,22 +138,15 @@ int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu
   if (!d_hits || !d_counts || !d_out || !d_out_off || !n_out) return set_error(MTSVGPU_EINVAL, "null argument");
   if (n_parts == 0 || n_parts > 16) return set_error(MTSVGPU_EINVAL, "n_parts must be in [1,16]");
   if (n_reads > 0x7ffffff0ull) return set_error(MTSVGPU_ELIMIT, "too many reads in one collapse call");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  MTSV_CUDA_TRY(cudaSetDevice(device));
+  MTSV_TRY(use_device(device));
+  if (device >= 16) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
   const uint32_t nr = (uint32_t)n_reads;
-  // grow-only workspace per device (cudaMalloc / cudaFree per call would cost more than the kernels)
-  struct Workspace {
-    DevBuf offs[16], total, comb_off, keys, scan_tmp, counters, worklist, cnt_out, off_out32;
-  };
-  static Workspace g_ws[16];
+  // grow-only workspace per device (cudaMalloc / cudaFree per call would cost more than the kernels); never
+  // destroyed: freeing at process exit would run after the CUDA runtime has been torn down
+  static CollapseScratch* const g_ws = new CollapseScratch[16];
   static std::mutex g_mu;
   std::lock_guard<std::mutex> lock(g_mu);
-  if (device < 0 || device >= 16) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
-  Workspace& w = g_ws[device];
+  CollapseScratch& w = g_ws[device];
   DevBuf* offs = w.offs;
   DevBuf &total = w.total, &comb_off = w.comb_off, &keys = w.keys, &scan_tmp = w.scan_tmp,
          &counters = w.counters, &worklist = w.worklist, &cnt_out = w.cnt_out, &off_out32 = w.off_out32;
@@ -161,7 +154,7 @@ int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu
   PartsView pv{};
   pv.n_parts = n_parts;
   MTSV_TRY(counters.reserve(sizeof(BatchCounters) + 16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p, 0, sizeof(BatchCounters) + 16, st));
+  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
   uint64_t* d_tot = reinterpret_cast<uint64_t*>(counters.as<uint8_t>() + sizeof(BatchCounters));
   for (uint32_t p = 0; p < n_parts; ++p) {
     pv.hits[p] = d_hits[p];
@@ -194,24 +187,17 @@ int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu
   MTSV_TRY(exclusive_scan_u32(cnt_out.as<uint32_t>(), off_out32.as<uint32_t>(), nr, scan_tmp, d_tot, st));
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  mtsvgpu_taxhit* out = nullptr;
-  uint64_t* out_off = nullptr;
-  if (cudaMalloc((void**)&out, (size_t)(h_tot + 1) * sizeof(mtsvgpu_taxhit)) != cudaSuccess ||
-      cudaMalloc((void**)&out_off, ((size_t)nr + 1) * 8) != cudaSuccess) {
-    (void)cudaGetLastError();
-    if (out) cudaFree(out);
-    return set_error(MTSVGPU_ENOMEM, "cudaMalloc of the collapsed result failed");
-  }
+  DevPtr<mtsvgpu_taxhit> out;
+  DevPtr<uint64_t> out_off;
+  MTSV_TRY(dev_alloc(out, h_tot + 1));
+  MTSV_TRY(dev_alloc(out_off, (uint64_t)nr + 1));
   MTSV_LAUNCH(collapse_write_kernel, rgrid, 256, 0, st, keys.as<uint64_t>(), comb_off.as<uint32_t>(),
-              off_out32.as<uint32_t>(), nr, out, out_off);
+              off_out32.as<uint32_t>(), nr, out.get(), out_off.get());
   cudaError_t e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) {
-    cudaFree(out);
-    cudaFree(out_off);
-    return set_error(MTSVGPU_ECUDA, "collapse: %s", cudaGetErrorString(e));
-  }
-  *d_out = out;
-  *d_out_off = out_off;
+  if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "collapse: %s", cudaGetErrorString(e));
+  // the caller frees the results with mtsvgpu_device_free
+  *d_out = out.release();
+  *d_out_off = out_off.release();
   *n_out = h_tot;
   return 0;
 }
@@ -227,7 +213,7 @@ int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, 
   PartsView pv{};
   pv.n_parts = n_parts;
   MTSV_TRY(w.counters.reserve(sizeof(BatchCounters) + 16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(w.counters.p, 0, sizeof(BatchCounters) + 16, st));
+  MTSV_CUDA_TRY(cudaMemsetAsync(w.counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
   uint64_t* d_tot = reinterpret_cast<uint64_t*>(w.counters.as<uint8_t>() + sizeof(BatchCounters));
   MTSV_TRY(w.scan_tmp.reserve((((size_t)nr + 1 + 2047) / 2048 + 1) * 8));
   MTSV_TRY(w.worklist.reserve((size_t)3 * (nr + 1) * 4));
@@ -262,38 +248,19 @@ int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, 
   return 0;
 }
 
-void CollapseScratch::release_all() {
-  for (auto& o : offs) o.release();
-  for (DevBuf* b : {&total, &comb_off, &keys, &scan_tmp, &counters, &worklist, &cnt_out, &off_out32}) b->release();
-}
-
 int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
                          const uint32_t* const* d_counts, uint64_t n_reads, mtsvgpu_hit** d_out,
                          uint64_t** d_out_off, uint64_t* n_out) {
   if (!d_hits || !d_counts || !d_out || !d_out_off || !n_out) return set_error(MTSVGPU_EINVAL, "null argument");
   if (n_parts == 0 || n_parts > 16) return set_error(MTSVGPU_EINVAL, "n_parts must be in [1,16]");
   if (n_reads > 0x07fffff0ull) return set_error(MTSVGPU_ELIMIT, "too many reads in one collapse call");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  MTSV_CUDA_TRY(cudaSetDevice(device));
+  MTSV_TRY(use_device(device));
   const uint32_t nr = (uint32_t)n_reads;
   DevBuf offs[16], total, comb_off, comb, flag, scan_tmp, counters, cnt_out, off_out32;
-  struct Release {
-    DevBuf* a[16 + 8];
-    int n = 0;
-    ~Release() {
-      for (int i = 0; i < n; ++i) a[i]->release();
-    }
-  } rel;
-  for (auto& o : offs) rel.a[rel.n++] = &o;
-  for (DevBuf* b : {&total, &comb_off, &comb, &flag, &scan_tmp, &counters, &cnt_out, &off_out32}) rel.a[rel.n++] = b;
   PartsView pv{};
   pv.n_parts = n_parts;
   MTSV_TRY(counters.reserve(16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p, 0, 16, st));
+  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p.get(), 0, 16, st));
   uint64_t* d_tot = counters.as<uint64_t>();
   for (uint32_t p = 0; p < n_parts; ++p) {
     pv.hits[p] = d_hits[p];
@@ -328,24 +295,16 @@ int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mt
   MTSV_TRY(exclusive_scan_u32(cnt_out.as<uint32_t>(), off_out32.as<uint32_t>(), nr, scan_tmp, d_tot, st));
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  mtsvgpu_hit* out = nullptr;
-  uint64_t* out_off = nullptr;
-  if (cudaMalloc((void**)&out, (size_t)(h_tot + 1) * sizeof(mtsvgpu_hit)) != cudaSuccess ||
-      cudaMalloc((void**)&out_off, ((size_t)nr + 1) * 8) != cudaSuccess) {
-    (void)cudaGetLastError();
-    if (out) cudaFree(out);
-    return set_error(MTSVGPU_ENOMEM, "cudaMalloc of the collapsed result failed");
-  }
+  DevPtr<mtsvgpu_hit> out;
+  DevPtr<uint64_t> out_off;
+  MTSV_TRY(dev_alloc(out, h_tot + 1));
+  MTSV_TRY(dev_alloc(out_off, (uint64_t)nr + 1));
   MTSV_LAUNCH(collapse_long_write_kernel, wgrid, 128, 0, st, comb.as<mtsvgpu_hit>(), comb_off.as<uint32_t>(),
-              flag.as<uint8_t>(), off_out32.as<uint32_t>(), nr, out, out_off);
+              flag.as<uint8_t>(), off_out32.as<uint32_t>(), nr, out.get(), out_off.get());
   cudaError_t e = cudaStreamSynchronize(st);
-  if (e != cudaSuccess) {
-    cudaFree(out);
-    cudaFree(out_off);
-    return set_error(MTSVGPU_ECUDA, "collapse (taxid-gi): %s", cudaGetErrorString(e));
-  }
-  *d_out = out;
-  *d_out_off = out_off;
+  if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "collapse (taxid-gi): %s", cudaGetErrorString(e));
+  *d_out = out.release();
+  *d_out_off = out_off.release();
   *n_out = h_tot;
   return 0;
 }

@@ -8,6 +8,7 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -42,15 +43,52 @@ extern std::atomic<uint64_t> g_launches;
     ::mtsv::g_launches.fetch_add(1, std::memory_order_relaxed);   \
   } while (0)
 
+// owners of device and page-locked memory
+struct CudaFree {
+  void operator()(void* p) const;
+};
+struct CudaFreeHost {
+  void operator()(void* p) const;
+};
+template <typename T>
+using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T>
+using PinnedPtr = std::unique_ptr<T, CudaFreeHost>;
+
+// The library's only allocators (cudaMalloc, cudaHostAlloc).  A failure clears the runtime's last error, so that it
+// cannot fail a later, unrelated call, and returns MTSVGPU_ENOMEM.
+int device_alloc(void** p, size_t bytes);
+int pinned_alloc(void** p, size_t bytes, unsigned flags);
+
+// `count ? count : 1` elements of T; the bytes are added to *acc
+template <typename T>
+int dev_alloc(DevPtr<T>& p, uint64_t count, uint64_t* acc = nullptr) {
+  const size_t bytes = (size_t)(count ? count : 1) * sizeof(T);
+  void* q = nullptr;
+  MTSV_TRY(device_alloc(&q, bytes));
+  p.reset(static_cast<T*>(q));
+  if (acc) *acc += bytes;
+  return 0;
+}
+template <typename T>
+int pinned_alloc(PinnedPtr<T>& p, uint64_t count, unsigned flags = cudaHostAllocDefault) {
+  void* q = nullptr;
+  MTSV_TRY(pinned_alloc(&q, (size_t)(count ? count : 1) * sizeof(T), flags));
+  p.reset(static_cast<T*>(q));
+  return 0;
+}
+
+// MTSVGPU_ENODEVICE without a device, MTSVGPU_EINVAL for a number outside [0, count), else cudaSetDevice
+int use_device(int device);
+
 // growable device allocation
 struct DevBuf {
-  void* p = nullptr;
+  DevPtr<uint8_t> p;
   size_t cap = 0;
   int reserve(size_t bytes);  // contents are NOT preserved
-  void release();
   template <typename T>
   T* as() const {
-    return reinterpret_cast<T*>(p);
+    return reinterpret_cast<T*>(p.get());
   }
 };
 
@@ -70,27 +108,27 @@ struct DeviceIndex {
   int device = 0;
   uint64_t n = 0;  // rows / text length incl. '$'
   // FM-index
-  FmBlock* blocks = nullptr;
-  SuperCounts* super = nullptr;
-  uint32_t* n_before = nullptr;
+  DevPtr<FmBlock> blocks;
+  DevPtr<SuperCounts> super;
+  DevPtr<uint32_t> n_before;
   uint64_t n_blocks = 0, n_super = 0;
   uint32_t C[5] = {0, 0, 0, 0, 0};
-  uint32_t* d_C = nullptr;  // device copy of C
+  DevPtr<uint32_t> d_C;  // device copy of C
   uint32_t dollar_row = 0;
   // suffix array at the device rate
-  uint32_t* sa = nullptr;
+  DevPtr<uint32_t> sa;
   uint32_t sa_rate = 1;
   uint64_t sa_len = 0;
   uint64_t file_sa_rate = 0;
   // k-mer interval table
-  uint2* ktab = nullptr;
+  DevPtr<uint2> ktab;
   uint32_t ktab_k = 0;
   uint32_t ktab_direct = 0;  // unique k-mers hold (text position, preceding symbols) instead of their SA interval
   // reference text (bytes, as in the file) and bins (SoA)
-  uint8_t* text = nullptr;
-  uint64_t* text4 = nullptr;  // the same text as 4-bit match classes (0..3 = A,C,G,T, 4 = anything else), 16 per word
+  DevPtr<uint8_t> text;
+  DevPtr<uint64_t> text4;  // the same text as 4-bit match classes (0..3 = A,C,G,T, 4 = anything else), 16 per word
   uint64_t text4_words = 0;
-  uint32_t *bin_start = nullptr, *bin_end = nullptr, *bin_tax = nullptr, *bin_gi = nullptr;
+  DevPtr<uint32_t> bin_start, bin_end, bin_tax, bin_gi;
   uint64_t n_bins = 0;
   uint64_t n_taxids = 0;  // distinct TaxIDs among the bins (== n_bins: no TaxID has a second sequence)
   uint64_t device_bytes = 0;
@@ -98,17 +136,19 @@ struct DeviceIndex {
 
   FmView fm_view() const {
     FmView v;
-    v.blocks = blocks;
-    v.super = super;
-    v.n_before = n_before;
-    v.C = d_C;
+    v.blocks = blocks.get();
+    v.super = super.get();
+    v.n_before = n_before.get();
+    v.C = d_C.get();
     v.n = (uint32_t)n;
     v.dollar_row = dollar_row;
     return v;
   }
-  SaView sa_view() const { return SaView{sa, sa_rate}; }
-  KtabView ktab_view() const { return KtabView{ktab, ktab_k, ktab_direct, text}; }
-  BinsView bins_view() const { return BinsView{bin_start, bin_end, bin_tax, bin_gi, (uint32_t)n_bins}; }
+  SaView sa_view() const { return SaView{sa.get(), sa_rate}; }
+  KtabView ktab_view() const { return KtabView{ktab.get(), ktab_k, ktab_direct, text.get()}; }
+  BinsView bins_view() const {
+    return BinsView{bin_start.get(), bin_end.get(), bin_tax.get(), bin_gi.get(), (uint32_t)n_bins};
+  }
 };
 
 enum Stage {
@@ -145,7 +185,6 @@ struct BatchWorkspace {
   DevBuf out_hits, out_hit_off;
   // staged inputs for the host API
   DevBuf d_seqs, d_seq_off;
-  void release_all();
 };
 
 // One in-flight device sub-batch.  A batch call alternates its slices between two lanes (own stream, own
@@ -154,7 +193,7 @@ struct BatchWorkspace {
 struct Lane {
   cudaStream_t stream = nullptr;     // lane 0: the handle's stream; lane 1: a private non-blocking stream
   BatchWorkspace* ws = nullptr;      // scratch of the lane (results and staged inputs live in the handle's ws)
-  BatchCounters* h_ctr = nullptr;    // page-locked, mapped: sub-batch scalars published by the device
+  PinnedPtr<BatchCounters> h_ctr;    // mapped: sub-batch scalars published by the device
   BatchCounters* h_ctr_dev = nullptr;
   cudaEvent_t emit_event = nullptr;  // recorded after each append to the batch output
   bool has_turn = false;             // holds the output turnstile for its current slice
@@ -209,9 +248,9 @@ struct mtsvgpu_index {
   std::vector<cudaEvent_t> in_events;
   cudaStream_t copy_out_stream = nullptr;
   cudaEvent_t out_event = nullptr;
-  void* pin_hits = nullptr;
+  mtsv::PinnedPtr<uint8_t> pin_hits;
   size_t pin_hits_cap = 0;
-  void* pin_off = nullptr;
+  mtsv::PinnedPtr<uint8_t> pin_off;
   size_t pin_off_cap = 0;
 };
 
@@ -228,10 +267,10 @@ struct IndexParts {
   const uint64_t* sa_sample = nullptr;  // host: suffix array rows 0, s, 2s, ... (the file's sample)
   uint64_t sa_sample_len = 0;
   uint64_t sa_rate = 0;  // s
-  uint32_t* d_sa_full = nullptr;  // instead of sa_sample: the complete suffix array on the device (adopted)
+  DevPtr<uint32_t> d_sa_full;  // instead of sa_sample: the complete suffix array on the device (adopted)
 };
 // index.cu
-int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out);
+int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out);
 int index_from_host_parts(const uint8_t* text, uint64_t n, const mtsvgpu_bin* bins, uint64_t n_bins,
                           const uint8_t* bwt, const uint64_t* sa_sample, uint64_t sa_sample_len,
                           uint64_t sa_rate, int device, const mtsvgpu_index_opts* opts,
@@ -266,7 +305,6 @@ int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mt
                          uint64_t** d_out_off, uint64_t* n_out);
 struct CollapseScratch {
   DevBuf offs[16], total, comb_off, keys, scan_tmp, counters, worklist, cnt_out, off_out32;
-  void release_all();
 };
 int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
                          const uint32_t* const* d_counts, uint32_t nr, uint64_t hit_cap, mtsvgpu_taxhit* out,

@@ -228,19 +228,6 @@ static double now_s() {
   return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
-template <typename T>
-static int dev_alloc(T** p, uint64_t count, uint64_t* acc) {
-  size_t bytes = (size_t)(count ? count : 1) * sizeof(T);
-  cudaError_t e = cudaMalloc((void**)p, bytes);
-  if (e != cudaSuccess) {
-    (void)cudaGetLastError();
-    *p = nullptr;
-    return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
-  }
-  if (acc) *acc += bytes;
-  return 0;
-}
-
 // reference text -> 4-bit match classes, 16 symbols per 64-bit word (symbol i of a word in bits 4i..4i+3)
 __global__ void text_pack4_kernel(const uint8_t* __restrict__ text, uint64_t n, uint64_t* __restrict__ text4,
                                   uint64_t n_words) {
@@ -261,32 +248,14 @@ __global__ void text_pack4_kernel(const uint8_t* __restrict__ text, uint64_t n, 
 
 void index_destroy(mtsvgpu_index* h) {
   if (!h) return;
-  cudaSetDevice(h->ix.device);
-  DeviceIndex& d = h->ix;
-  cudaFree(d.blocks);
-  cudaFree(d.super);
-  cudaFree(d.n_before);
-  cudaFree(d.d_C);
-  cudaFree(d.sa);
-  cudaFree(d.ktab);
-  cudaFree(d.text);
-  cudaFree(d.text4);
-  cudaFree(d.bin_start);
-  cudaFree(d.bin_end);
-  cudaFree(d.bin_tax);
-  cudaFree(d.bin_gi);
-  h->ws.release_all();
-  h->ws1.release_all();
+  cudaSetDevice(h->ix.device);  // the members' memory is freed by `delete h`, on this device
   for (Lane& ln : h->lanes) {
-    if (ln.h_ctr) cudaFreeHost(ln.h_ctr);
     if (ln.emit_event) cudaEventDestroy(ln.emit_event);
     for (cudaEvent_t e : ln.ev_pool) cudaEventDestroy(e);
   }
   if (h->lane1_stream) cudaStreamDestroy(h->lane1_stream);
   if (h->fork_event) cudaEventDestroy(h->fork_event);
   if (h->join_event) cudaEventDestroy(h->join_event);
-  if (h->pin_hits) cudaFreeHost(h->pin_hits);
-  if (h->pin_off) cudaFreeHost(h->pin_off);
   for (cudaEvent_t e : h->in_events) cudaEventDestroy(e);
   if (h->copy_in_stream) cudaStreamDestroy(h->copy_in_stream);
   if (h->copy_out_stream) cudaStreamDestroy(h->copy_out_stream);
@@ -307,7 +276,7 @@ static uint32_t auto_ktab_k(uint64_t n) {
   return k;
 }
 
-int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out) {
+int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out) {
   double t0 = now_s();
   const uint8_t* text = parts.text;
   const uint64_t n = parts.n;
@@ -317,12 +286,6 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   const uint64_t* sa_sample = parts.sa_sample;
   const uint64_t sa_sample_len = parts.sa_sample_len;
   const uint64_t sa_rate = parts.sa_rate;
-  struct SaGuard {  // a device suffix array handed in is consumed whatever happens
-    uint32_t* p;
-    ~SaGuard() {
-      if (p) cudaFree(p);
-    }
-  } sag{parts.d_sa_full};
   if (!text || !bins || !bwt || (!sa_sample && !parts.d_sa_full) || !out)
     return set_error(MTSVGPU_EINVAL, "null argument");
   *out = nullptr;
@@ -354,27 +317,16 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
                        (unsigned long long)prev_end, (unsigned long long)(n - 1));
   }
 
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    (void)cudaGetLastError();
-    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
-  }
-  if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
-  MTSV_CUDA_TRY(cudaSetDevice(device));
+  MTSV_TRY(use_device(device));
 
-  mtsvgpu_index* h = new mtsvgpu_index;
+  std::unique_ptr<mtsvgpu_index, void (*)(mtsvgpu_index*)> guard(new mtsvgpu_index, index_destroy);
+  mtsvgpu_index* h = guard.get();
   if (opts) h->opts = *opts;
   DeviceIndex& d = h->ix;
   d.device = device;
   d.n = n;
   d.n_bins = n_bins;
   d.file_sa_rate = sa_rate;
-  struct Guard {
-    mtsvgpu_index* h;
-    ~Guard() {
-      if (h) index_destroy(h);
-    }
-  } guard{h};
 
   MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   h->stream = h->own_stream;
@@ -384,19 +336,19 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   cudaStream_t st = h->stream;
 
   // ---- text and bins ----
-  MTSV_TRY(dev_alloc(&d.text, n + 16, &d.device_bytes));
-  MTSV_CUDA_TRY(cudaMemcpyAsync(d.text, text, n, cudaMemcpyDefault, st));
-  MTSV_CUDA_TRY(cudaMemsetAsync(d.text + n, 0, 16, st));
+  MTSV_TRY(dev_alloc(d.text, n + 16, &d.device_bytes));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(d.text.get(), text, n, cudaMemcpyDefault, st));
+  MTSV_CUDA_TRY(cudaMemsetAsync(d.text.get() + n, 0, 16, st));
   if (parts.text_on_device) {
     uint8_t last = 0;
-    MTSV_CUDA_TRY(cudaMemcpyAsync(&last, d.text + n - 1, 1, cudaMemcpyDeviceToHost, st));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(&last, d.text.get() + n - 1, 1, cudaMemcpyDeviceToHost, st));
     MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     if (last != '$') return set_error(MTSVGPU_EFORMAT, "sequences do not end with '$'");
   }
   // 4-bit match classes for the verifier's fast path (+ 2 words of slack: it reads one word ahead)
   d.text4_words = (n + 15) / 16 + 2;
-  MTSV_TRY(dev_alloc(&d.text4, d.text4_words, &d.device_bytes));
-  MTSV_LAUNCH(text_pack4_kernel, (unsigned)((d.text4_words + 255) / 256), 256, 0, st, d.text, n, d.text4,
+  MTSV_TRY(dev_alloc(d.text4, d.text4_words, &d.device_bytes));
+  MTSV_LAUNCH(text_pack4_kernel, (unsigned)((d.text4_words + 255) / 256), 256, 0, st, d.text.get(), n, d.text4.get(),
               d.text4_words);
   {
     std::vector<uint32_t> bs(n_bins), be(n_bins), bt(n_bins), bg(n_bins);
@@ -411,63 +363,53 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
       std::sort(t.begin(), t.end());
       d.n_taxids = (uint64_t)(std::unique(t.begin(), t.end()) - t.begin());
     }
-    MTSV_TRY(dev_alloc(&d.bin_start, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(&d.bin_end, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(&d.bin_tax, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(&d.bin_gi, n_bins, &d.device_bytes));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_start, bs.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_end, be.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_tax, bt.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_gi, bg.data(), n_bins * 4, cudaMemcpyHostToDevice));
+    MTSV_TRY(dev_alloc(d.bin_start, n_bins, &d.device_bytes));
+    MTSV_TRY(dev_alloc(d.bin_end, n_bins, &d.device_bytes));
+    MTSV_TRY(dev_alloc(d.bin_tax, n_bins, &d.device_bytes));
+    MTSV_TRY(dev_alloc(d.bin_gi, n_bins, &d.device_bytes));
+    MTSV_CUDA_TRY(cudaMemcpy(d.bin_start.get(), bs.data(), n_bins * 4, cudaMemcpyHostToDevice));
+    MTSV_CUDA_TRY(cudaMemcpy(d.bin_end.get(), be.data(), n_bins * 4, cudaMemcpyHostToDevice));
+    MTSV_CUDA_TRY(cudaMemcpy(d.bin_tax.get(), bt.data(), n_bins * 4, cudaMemcpyHostToDevice));
+    MTSV_CUDA_TRY(cudaMemcpy(d.bin_gi.get(), bg.data(), n_bins * 4, cudaMemcpyHostToDevice));
   }
 
   // ---- BWT re-layout ----
   d.n_blocks = n / kRowsPerBlock + 1;
   d.n_super = (d.n_blocks + kBlocksPerSuper - 1) / kBlocksPerSuper;
-  MTSV_TRY(dev_alloc(&d.blocks, d.n_super * kBlocksPerSuper, &d.device_bytes));
-  MTSV_TRY(dev_alloc(&d.super, d.n_super, &d.device_bytes));
-  MTSV_TRY(dev_alloc(&d.n_before, d.n_super * kBlocksPerSuper, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.blocks, d.n_super * kBlocksPerSuper, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.super, d.n_super, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.n_before, d.n_super * kBlocksPerSuper, &d.device_bytes));
 
-  uint8_t* d_bwt = nullptr;
-  uint32_t *d_super_tot = nullptr, *d_super_n = nullptr;
-  unsigned long long* d_totals = nullptr;
-  PackDiag* d_diag = nullptr;
-  uint64_t* d_sample = nullptr;
-  uint2* d_ktmp = nullptr;
-  struct TmpGuard {
-    void** p[7];
-    ~TmpGuard() {
-      for (auto q : p)
-        if (q && *q) cudaFree(*q);
-    }
-  } tg{{(void**)&d_bwt, (void**)&d_super_tot, (void**)&d_super_n, (void**)&d_totals,
-        (void**)&d_diag, (void**)&d_sample, (void**)&d_ktmp}};
+  DevPtr<uint8_t> d_bwt;
+  DevPtr<uint32_t> d_super_tot, d_super_n;
+  DevPtr<unsigned long long> d_totals;
+  DevPtr<PackDiag> d_diag;
   // (a BWT that is already on the device is used where it lies: the caller pads it by 64 bytes)
   const uint8_t* bwt_dev = bwt;
   if (!parts.bwt_on_device) {
-    MTSV_TRY(dev_alloc(&d_bwt, n + 64, nullptr));
-    bwt_dev = d_bwt;
+    MTSV_TRY(dev_alloc(d_bwt, n + 64));
+    bwt_dev = d_bwt.get();
   }
-  MTSV_TRY(dev_alloc(&d_super_tot, d.n_super * 5, nullptr));
-  MTSV_TRY(dev_alloc(&d_super_n, d.n_super, nullptr));
-  MTSV_TRY(dev_alloc(&d_totals, 5, nullptr));
-  MTSV_TRY(dev_alloc(&d_diag, 1, nullptr));
-  MTSV_CUDA_TRY(cudaMemsetAsync(d_diag, 0, sizeof(PackDiag), st));
-  if (!parts.bwt_on_device) MTSV_CUDA_TRY(cudaMemcpyAsync(d_bwt, bwt, n, cudaMemcpyHostToDevice, st));
+  MTSV_TRY(dev_alloc(d_super_tot, d.n_super * 5));
+  MTSV_TRY(dev_alloc(d_super_n, d.n_super));
+  MTSV_TRY(dev_alloc(d_totals, 5));
+  MTSV_TRY(dev_alloc(d_diag, 1));
+  MTSV_CUDA_TRY(cudaMemsetAsync(d_diag.get(), 0, sizeof(PackDiag), st));
+  if (!parts.bwt_on_device) MTSV_CUDA_TRY(cudaMemcpyAsync(d_bwt.get(), bwt, n, cudaMemcpyHostToDevice, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   double t_relayout0 = now_s();
 
   MTSV_LAUNCH(fm_pack_kernel, (unsigned)d.n_super, kBlocksPerSuper, 0, st, bwt_dev, n, d.n_blocks,
-              d.blocks, d.n_before, d_super_tot, d_diag);
-  MTSV_LAUNCH(fm_super_scan_kernel, 1, 32, 0, st, d_super_tot, d.n_super, d.super, d_super_n,
-              d_totals);
-  MTSV_LAUNCH(fm_finish_kernel, (unsigned)((d.n_blocks + 255) / 256), 256, 0, st, d.n_before,
-              d.n_blocks, d_super_n);
+              d.blocks.get(), d.n_before.get(), d_super_tot.get(), d_diag.get());
+  MTSV_LAUNCH(fm_super_scan_kernel, 1, 32, 0, st, d_super_tot.get(), d.n_super, d.super.get(), d_super_n.get(),
+              d_totals.get());
+  MTSV_LAUNCH(fm_finish_kernel, (unsigned)((d.n_blocks + 255) / 256), 256, 0, st, d.n_before.get(),
+              d.n_blocks, d_super_n.get());
   MTSV_CUDA_TRY(cudaGetLastError());
   unsigned long long totals[5];
   PackDiag diag;
-  MTSV_CUDA_TRY(cudaMemcpyAsync(totals, d_totals, sizeof totals, cudaMemcpyDeviceToHost, st));
-  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag, sizeof diag, cudaMemcpyDeviceToHost, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(totals, d_totals.get(), sizeof totals, cudaMemcpyDeviceToHost, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag.get(), sizeof diag, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   if (diag.n_dollar != 1)
     return set_error(MTSVGPU_EFORMAT, "BWT holds %llu '$' symbols, expected exactly 1", diag.n_dollar);
@@ -482,10 +424,9 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   d.C[SYM_G] = (uint32_t)(1 + totals[0] + totals[1]);
   d.C[SYM_N] = (uint32_t)(1 + totals[0] + totals[1] + totals[2]);
   d.C[SYM_T] = (uint32_t)(1 + totals[0] + totals[1] + totals[2] + totals[4]);
-  MTSV_TRY(dev_alloc(&d.d_C, 8, &d.device_bytes));
-  MTSV_CUDA_TRY(cudaMemcpy(d.d_C, d.C, 5 * sizeof(uint32_t), cudaMemcpyHostToDevice));
-  if (d_bwt) cudaFree(d_bwt);
-  d_bwt = nullptr;
+  MTSV_TRY(dev_alloc(d.d_C, 8, &d.device_bytes));
+  MTSV_CUDA_TRY(cudaMemcpy(d.d_C.get(), d.C, 5 * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  d_bwt.reset();
 
   // ---- suffix array at the device rate ----
   size_t free_b = 0, total_b = 0;
@@ -494,19 +435,18 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   if (parts.d_sa_full) {
     // built on this device (sufsort.cu): the complete array is adopted as it is, or thinned to the requested rate
     if (rate <= 1) {
-      d.sa = parts.d_sa_full;
-      sag.p = nullptr;
+      d.sa = std::move(parts.d_sa_full);
       d.sa_rate = 1;
       d.sa_len = n;
       d.device_bytes += n * 4;
     } else {
       d.sa_rate = rate;
       d.sa_len = (n + rate - 1) / rate;
-      MTSV_TRY(dev_alloc(&d.sa, d.sa_len, &d.device_bytes));
-      MTSV_LAUNCH(sa_thin_kernel, (unsigned)((d.sa_len + 255) / 256), 256, 0, st, parts.d_sa_full, d.sa_len, rate, d.sa);
+      MTSV_TRY(dev_alloc(d.sa, d.sa_len, &d.device_bytes));
+      MTSV_LAUNCH(sa_thin_kernel, (unsigned)((d.sa_len + 255) / 256), 256, 0, st, parts.d_sa_full.get(), d.sa_len, rate,
+                  d.sa.get());
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-      cudaFree(sag.p);
-      sag.p = nullptr;
+      parts.d_sa_full.reset();
     }
   } else {
   if (rate == 0) {
@@ -518,22 +458,21 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   if (rate > sa_rate) rate = (uint32_t)sa_rate;
   d.sa_rate = rate;
   d.sa_len = (n + rate - 1) / rate;
-  MTSV_TRY(dev_alloc(&d.sa, d.sa_len, &d.device_bytes));
-  MTSV_TRY(dev_alloc(&d_sample, sa_sample_len, nullptr));
-  MTSV_CUDA_TRY(cudaMemcpyAsync(d_sample, sa_sample, sa_sample_len * 8, cudaMemcpyHostToDevice, st));
-  MTSV_CUDA_TRY(cudaMemsetAsync(d.sa, 0xff, d.sa_len * 4, st));
+  MTSV_TRY(dev_alloc(d.sa, d.sa_len, &d.device_bytes));
+  DevPtr<uint64_t> d_sample;
+  MTSV_TRY(dev_alloc(d_sample, sa_sample_len));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(d_sample.get(), sa_sample, sa_sample_len * 8, cudaMemcpyHostToDevice, st));
+  MTSV_CUDA_TRY(cudaMemsetAsync(d.sa.get(), 0xff, d.sa_len * 4, st));
   MTSV_LAUNCH(sa_densify_kernel, (unsigned)((sa_sample_len + 127) / 128), 128, 0, st, d.fm_view(),
-              d_sample, sa_sample_len, (uint32_t)sa_rate, rate, d.sa, d_diag);
+              d_sample.get(), sa_sample_len, (uint32_t)sa_rate, rate, d.sa.get(), d_diag.get());
   MTSV_CUDA_TRY(cudaGetLastError());
-  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag, sizeof diag, cudaMemcpyDeviceToHost, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag.get(), sizeof diag, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   if (diag.sa_mismatch != 0 || diag.rows_seen != n)
     return set_error(MTSVGPU_EFORMAT,
                      "suffix-array samples are inconsistent with the BWT (%llu LF walks disagree, "
                      "%llu of %llu rows reached)",
                      diag.sa_mismatch, diag.rows_seen, (unsigned long long)n);
-  cudaFree(d_sample);
-  d_sample = nullptr;
   }
 
   // ---- k-mer interval table ----
@@ -545,13 +484,12 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
     MTSV_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
     while (kk > 1 && (1ull << (2 * kk)) * 8ull * 5 / 4 > free_b / 3) --kk;
     uint64_t size = 1ull << (2 * kk);
-    MTSV_TRY(dev_alloc(&d.ktab, size, &d.device_bytes));
+    MTSV_TRY(dev_alloc(d.ktab, size, &d.device_bytes));
     if (kk >= 1) {
-      uint64_t tmp_size = kk >= 2 ? (1ull << (2 * (kk - 1))) : 1;
-      cudaError_t e = cudaMalloc((void**)&d_ktmp, tmp_size * sizeof(uint2));
-      if (e != cudaSuccess) return set_error(MTSVGPU_ENOMEM, "k-mer table scratch: %s", cudaGetErrorString(e));
+      DevPtr<uint2> d_ktmp;
+      MTSV_TRY(dev_alloc(d_ktmp, kk >= 2 ? (1ull << (2 * (kk - 1))) : 1));
       // levels alternate between the two buffers so that level kk lands in d.ktab
-      uint2* bufs[2] = {d.ktab, d_ktmp};
+      uint2* bufs[2] = {d.ktab.get(), d_ktmp.get()};
       int cur = (kk % 2 == 0) ? 0 : 1;  // level 0 buffer
       MTSV_LAUNCH(ktab_init_kernel, 1, 1, 0, st, bufs[cur], (uint32_t)n);
       uint64_t cur_size = 1;
@@ -565,14 +503,12 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
       // row indexes of ordinary entries must stay below the direct tag; MTSV_B200_KTAB_DIRECT=0 is an A/B knob
       const char* de = getenv("MTSV_B200_KTAB_DIRECT");
       if (n < ((uint64_t)kKtabDirectTag << 24) && !(de && de[0] == '0')) {
-        MTSV_LAUNCH(ktab_direct_kernel, (unsigned)((size + 255) / 256), 256, 0, st, d.fm_view(), d.sa_view(), d.text,
-                    d.ktab, size);
+        MTSV_LAUNCH(ktab_direct_kernel, (unsigned)((size + 255) / 256), 256, 0, st, d.fm_view(), d.sa_view(),
+                    d.text.get(), d.ktab.get(), size);
         d.ktab_direct = 1;
       }
       MTSV_CUDA_TRY(cudaGetLastError());
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-      cudaFree(d_ktmp);
-      d_ktmp = nullptr;
     }
   }
   d.ktab_k = kk;
@@ -580,8 +516,7 @@ int index_assemble(const IndexParts& parts, int device, const mtsvgpu_index_opts
   double t1 = now_s();
   d.relayout_seconds = t1 - t_relayout0;
   d.load_seconds = t1 - t0;
-  guard.h = nullptr;
-  *out = h;
+  *out = guard.release();
   return 0;
 }
 
@@ -599,7 +534,7 @@ int index_from_host_parts(const uint8_t* text, uint64_t n, const mtsvgpu_bin* bi
   parts.sa_sample = sa_sample;
   parts.sa_sample_len = sa_sample_len;
   parts.sa_rate = sa_rate;
-  return index_assemble(parts, device, opts, out);
+  return index_assemble(std::move(parts), device, opts, out);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -395,33 +395,6 @@ __global__ void __launch_bounds__(256) sfx_bwt_kernel(const uint8_t* __restrict_
   bwt[r] = text[p ? p - 1 : n - 1];  // bwt[r] = text[SA[r] - 1], the sentinel for SA[r] == 0 (bio::bwt)
 }
 
-template <typename T>
-struct Scoped {  // cudaFree on scope exit
-  T* p = nullptr;
-  ~Scoped() {
-    if (p) cudaFree(p);
-  }
-  int alloc(uint64_t count) {
-    const size_t bytes = (size_t)(count ? count : 1) * sizeof(T);
-    cudaError_t e = cudaMalloc((void**)&p, bytes);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      p = nullptr;
-      return set_error(MTSVGPU_ENOMEM, "suffix sort: cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
-    }
-    return 0;
-  }
-  void reset() {
-    if (p) cudaFree(p);
-    p = nullptr;
-  }
-  T* release() {
-    T* q = p;
-    p = nullptr;
-    return q;
-  }
-};
-
 uint32_t bits_of(uint64_t v) {  // bits needed to hold values 0..v
   uint32_t b = 1;
   while (b < 64 && (v >> b)) ++b;
@@ -432,12 +405,11 @@ unsigned grid_for(uint64_t items, unsigned threads) { return (unsigned)((items +
 
 }  // namespace
 
-// Suffix array (u32, n entries, cudaMalloc'ed: the caller owns *d_sa_out) of the n symbols at d_text, the last of
-// which must be the only '$'.  `verbose` prints one line per round on stderr.
-int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, uint32_t** d_sa_out, int verbose) {
-  if (!d_text || !d_sa_out || n < 1) return set_error(MTSVGPU_EINVAL, "suffix sort: bad argument");
+// Suffix array (u32, n entries) of the n symbols at d_text, the last of which must be the only '$'.  `verbose` prints
+// one line per round on stderr.
+int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, DevPtr<uint32_t>& sa_out, int verbose) {
+  if (!d_text || n < 1) return set_error(MTSVGPU_EINVAL, "suffix sort: bad argument");
   if (n >= (1ull << 32) - 64) return set_error(MTSVGPU_ELIMIT, "suffix sort: %llu symbols (limit 2^32-64)", (unsigned long long)n);
-  *d_sa_out = nullptr;
   // test knobs: symbols in the round-0 key, pairs per slab
   uint32_t K = 21;
   uint64_t slab = 1ull << 29;
@@ -446,50 +418,40 @@ int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, uint
 
   SortScratch sc;
   DevBuf ms_tmp, sum_tmp;
-  struct Rel {
-    SortScratch& s;
-    DevBuf &a, &b;
-    ~Rel() {
-      s.hist.release();
-      s.scan_tmp.release();
-      a.release();
-      b.release();
-    }
-  } rel{sc, ms_tmp, sum_tmp};
-  Scoped<uint32_t> sa, rank, apos, apos_next;
-  Scoped<unsigned long long> d_scalar;
-  MTSV_TRY(sa.alloc(n + 1));  // (+1: may trade places with the scan buffer of round 0)
-  MTSV_TRY(rank.alloc(n));
-  MTSV_TRY(d_scalar.alloc(2));
+  DevPtr<uint32_t> sa, rank, apos, apos_next;
+  DevPtr<unsigned long long> d_scalar;
+  MTSV_TRY(dev_alloc(sa, n + 1));  // (+1: may trade places with the scan buffer of round 0)
+  MTSV_TRY(dev_alloc(rank, n));
+  MTSV_TRY(dev_alloc(d_scalar, 2));
   uint64_t m = 0;  // active pairs
 
   // ---- round 0 ----
   {
-    Scoped<uint64_t> k0, k1;
-    Scoped<uint32_t> v1;
-    MTSV_TRY(k0.alloc(n));
-    MTSV_TRY(k1.alloc(n));
-    MTSV_TRY(v1.alloc(n + 1));
-    MTSV_LAUNCH(sfx_init_kernel, grid_for((n + 7) / 8, 256), 256, 0, st, d_text, n, K, k0.p, sa.p);
+    DevPtr<uint64_t> k0, k1;
+    DevPtr<uint32_t> v1;
+    MTSV_TRY(dev_alloc(k0, n));
+    MTSV_TRY(dev_alloc(k1, n));
+    MTSV_TRY(dev_alloc(v1, n + 1));
+    MTSV_LAUNCH(sfx_init_kernel, grid_for((n + 7) / 8, 256), 256, 0, st, d_text, n, K, k0.get(), sa.get());
     std::vector<uint32_t> shifts;
     for (uint32_t s = 0; s < 3 * K; s += 8) shifts.push_back(s);
     int where = 0;
-    MTSV_TRY(radix_sort_pairs(st, k0.p, k1.p, sa.p, v1.p, n, shifts, sc, &where));
-    uint64_t* ks = where ? k1.p : k0.p;
-    uint64_t* kfree = where ? k0.p : k1.p;
-    if (where) std::swap(sa.p, v1.p);  // the sorted suffix starts are the suffix array so far
+    MTSV_TRY(radix_sort_pairs(st, k0.get(), k1.get(), sa.get(), v1.get(), n, shifts, sc, &where));
+    uint64_t* ks = where ? k1.get() : k0.get();
+    uint64_t* kfree = where ? k0.get() : k1.get();
+    if (where) std::swap(sa, v1);  // the sorted suffix starts are the suffix array so far
     uint32_t* headv = reinterpret_cast<uint32_t*>(kfree);  // n u32 fit in the idle key buffer
-    uint32_t* idx = v1.p;
+    uint32_t* idx = v1.get();
     MTSV_LAUNCH(sfx_heads_kernel, grid_for(n, 256), 256, 0, st, ks, (const uint32_t*)nullptr, n, headv);
     MTSV_TRY(inclusive_max_scan_u32(headv, n, ms_tmp, st));
-    MTSV_LAUNCH(sfx_publish_kernel, grid_for(n, 256), 256, 0, st, sa.p, (const uint32_t*)nullptr, headv, n, sa.p, rank.p);
+    MTSV_LAUNCH(sfx_publish_kernel, grid_for(n, 256), 256, 0, st, sa.get(), (const uint32_t*)nullptr, headv, n, sa.get(), rank.get());
     MTSV_LAUNCH(sfx_stays_kernel, grid_for(n, 256), 256, 0, st, headv, (const uint32_t*)nullptr, n, idx);
-    MTSV_TRY(exclusive_scan_u32(idx, idx, n, sum_tmp, (uint64_t*)d_scalar.p, st));
-    MTSV_CUDA_TRY(cudaMemcpyAsync(&m, d_scalar.p, 8, cudaMemcpyDeviceToHost, st));
+    MTSV_TRY(exclusive_scan_u32(idx, idx, n, sum_tmp, (uint64_t*)d_scalar.get(), st));
+    MTSV_CUDA_TRY(cudaMemcpyAsync(&m, d_scalar.get(), 8, cudaMemcpyDeviceToHost, st));
     MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     if (m) {
-      MTSV_TRY(apos.alloc(m));
-      MTSV_LAUNCH(sfx_compact_kernel, grid_for(n, 256), 256, 0, st, idx, (const uint32_t*)nullptr, n, apos.p);
+      MTSV_TRY(dev_alloc(apos, m));
+      MTSV_LAUNCH(sfx_compact_kernel, grid_for(n, 256), 256, 0, st, idx, (const uint32_t*)nullptr, n, apos.get());
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
     }
     MTSV_CUDA_TRY(cudaGetLastError());
@@ -503,46 +465,46 @@ int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, uint
   for (uint32_t i = 0; i < lo_passes; ++i) shifts.push_back(8 * i);
   for (uint32_t i = 0; i < hi_passes; ++i) shifts.push_back(32 + 8 * i);
   uint64_t ws_cap = 0;
-  Scoped<uint64_t> k0, k1;
-  Scoped<uint32_t> v0, v1, headv, idx;
+  DevPtr<uint64_t> k0, k1;
+  DevPtr<uint32_t> v0, v1, headv, idx;
   auto reserve_ws = [&](uint64_t need) -> int {
     if (need <= ws_cap) return 0;
     k0.reset(); k1.reset(); v0.reset(); v1.reset(); headv.reset(); idx.reset();
-    MTSV_TRY(k0.alloc(need));
-    MTSV_TRY(k1.alloc(need));
-    MTSV_TRY(v0.alloc(need));
-    MTSV_TRY(v1.alloc(need));
-    MTSV_TRY(headv.alloc(need));
-    MTSV_TRY(idx.alloc(need + 1));
+    MTSV_TRY(dev_alloc(k0, need));
+    MTSV_TRY(dev_alloc(k1, need));
+    MTSV_TRY(dev_alloc(v0, need));
+    MTSV_TRY(dev_alloc(v1, need));
+    MTSV_TRY(dev_alloc(headv, need));
+    MTSV_TRY(dev_alloc(idx, need + 1));
     ws_cap = need;
     return 0;
   };
   for (uint32_t round = 1; m > 0; ++round) {
     if (round > 40) return set_error(MTSVGPU_ECUDA, "suffix sort: internal error, no convergence");
-    MTSV_TRY(apos_next.alloc(m));
+    MTSV_TRY(dev_alloc(apos_next, m));
     uint64_t m_next = 0, a = 0, n_slabs = 0;
     while (a < m) {
       unsigned long long b = 0;
-      MTSV_LAUNCH(sfx_slab_cut_kernel, 1, 1, 0, st, apos.p, m, a, slab, sa.p, rank.p, d_scalar.p);
-      MTSV_CUDA_TRY(cudaMemcpyAsync(&b, d_scalar.p, 8, cudaMemcpyDeviceToHost, st));
+      MTSV_LAUNCH(sfx_slab_cut_kernel, 1, 1, 0, st, apos.get(), m, a, slab, sa.get(), rank.get(), d_scalar.get());
+      MTSV_CUDA_TRY(cudaMemcpyAsync(&b, d_scalar.get(), 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
       if (b <= a || b > m) return set_error(MTSVGPU_ECUDA, "suffix sort: internal error, bad slab [%llu,%llu)", (unsigned long long)a, b);
       const uint64_t ms = b - a;
       MTSV_TRY(reserve_ws(std::max<uint64_t>(ms, std::min(slab, m))));
-      const uint32_t* pos = apos.p + a;
-      MTSV_LAUNCH(sfx_slab_keys_kernel, grid_for(ms, 256), 256, 0, st, pos, ms, sa.p, rank.p, n, h, k0.p, v0.p);
+      const uint32_t* pos = apos.get() + a;
+      MTSV_LAUNCH(sfx_slab_keys_kernel, grid_for(ms, 256), 256, 0, st, pos, ms, sa.get(), rank.get(), n, h, k0.get(), v0.get());
       int where = 0;
-      MTSV_TRY(radix_sort_pairs(st, k0.p, k1.p, v0.p, v1.p, ms, shifts, sc, &where));
-      const uint64_t* ks = where ? k1.p : k0.p;
-      const uint32_t* vs = where ? v1.p : v0.p;
-      MTSV_LAUNCH(sfx_heads_kernel, grid_for(ms, 256), 256, 0, st, ks, pos, ms, headv.p);
-      MTSV_TRY(inclusive_max_scan_u32(headv.p, ms, ms_tmp, st));
-      MTSV_LAUNCH(sfx_publish_kernel, grid_for(ms, 256), 256, 0, st, vs, pos, headv.p, ms, sa.p, rank.p);
-      MTSV_LAUNCH(sfx_stays_kernel, grid_for(ms, 256), 256, 0, st, headv.p, pos, ms, idx.p);
-      MTSV_TRY(exclusive_scan_u32(idx.p, idx.p, ms, sum_tmp, (uint64_t*)d_scalar.p + 1, st));
-      MTSV_LAUNCH(sfx_compact_kernel, grid_for(ms, 256), 256, 0, st, idx.p, pos, ms, apos_next.p + m_next);
+      MTSV_TRY(radix_sort_pairs(st, k0.get(), k1.get(), v0.get(), v1.get(), ms, shifts, sc, &where));
+      const uint64_t* ks = where ? k1.get() : k0.get();
+      const uint32_t* vs = where ? v1.get() : v0.get();
+      MTSV_LAUNCH(sfx_heads_kernel, grid_for(ms, 256), 256, 0, st, ks, pos, ms, headv.get());
+      MTSV_TRY(inclusive_max_scan_u32(headv.get(), ms, ms_tmp, st));
+      MTSV_LAUNCH(sfx_publish_kernel, grid_for(ms, 256), 256, 0, st, vs, pos, headv.get(), ms, sa.get(), rank.get());
+      MTSV_LAUNCH(sfx_stays_kernel, grid_for(ms, 256), 256, 0, st, headv.get(), pos, ms, idx.get());
+      MTSV_TRY(exclusive_scan_u32(idx.get(), idx.get(), ms, sum_tmp, (uint64_t*)d_scalar.get() + 1, st));
+      MTSV_LAUNCH(sfx_compact_kernel, grid_for(ms, 256), 256, 0, st, idx.get(), pos, ms, apos_next.get() + m_next);
       unsigned long long kept = 0;
-      MTSV_CUDA_TRY(cudaMemcpyAsync(&kept, d_scalar.p + 1, 8, cudaMemcpyDeviceToHost, st));
+      MTSV_CUDA_TRY(cudaMemcpyAsync(&kept, d_scalar.get() + 1, 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
       MTSV_CUDA_TRY(cudaGetLastError());
       m_next += kept;
@@ -552,12 +514,12 @@ int suffix_array_device(const uint8_t* d_text, uint64_t n, cudaStream_t st, uint
     if (verbose)
       fprintf(stderr, "[mtsv_b200 sufsort] round %u: h=%llu, %llu pairs in %llu slab(s), %llu still tied\n", round,
               (unsigned long long)h, (unsigned long long)m, (unsigned long long)n_slabs, (unsigned long long)m_next);
-    std::swap(apos.p, apos_next.p);
+    std::swap(apos, apos_next);
     apos_next.reset();
     m = m_next;
     h *= 2;
   }
-  *d_sa_out = sa.release();
+  sa_out = std::move(sa);
   return 0;
 }
 

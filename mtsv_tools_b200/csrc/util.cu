@@ -1,4 +1,4 @@
-// util.cu — error plumbing, device buffers and the exclusive-scan primitive used between stages.
+// util.cu — error plumbing, device selection, memory allocation and the exclusive-scan primitive used between stages.
 #include <stdio.h>
 
 #include "ctx.h"
@@ -37,41 +37,47 @@ unsigned sm_count() {
   return (unsigned)n;
 }
 
-int DevBuf::reserve(size_t bytes) {
-  if (bytes <= cap && p) return 0;
-  if (p) {
-    cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
-  size_t want = bytes + bytes / 4 + 256;  // headroom so slowly growing batches do not realloc
-  cudaError_t e = cudaMalloc(&p, want);
-  if (e != cudaSuccess) {
+void CudaFree::operator()(void* p) const { cudaFree(p); }
+void CudaFreeHost::operator()(void* p) const { cudaFreeHost(p); }
+
+int device_alloc(void** p, size_t bytes) {
+  const cudaError_t e = cudaMalloc(p, bytes);
+  if (e == cudaSuccess) return 0;
+  (void)cudaGetLastError();
+  *p = nullptr;
+  return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
+}
+
+int pinned_alloc(void** p, size_t bytes, unsigned flags) {
+  const cudaError_t e = cudaHostAlloc(p, bytes, flags);
+  if (e == cudaSuccess) return 0;
+  (void)cudaGetLastError();
+  *p = nullptr;
+  return set_error(MTSVGPU_ENOMEM, "cudaHostAlloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
+}
+
+int use_device(int device) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     (void)cudaGetLastError();
-    e = cudaMalloc(&p, bytes ? bytes : 256);
-    if (e != cudaSuccess) {
-      p = nullptr;
-      return set_error(MTSVGPU_ENOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-    }
-    want = bytes ? bytes : 256;
+    return set_error(MTSVGPU_ENODEVICE, "no CUDA device available (this library has no CPU path)");
   }
-  cap = want;
+  if (device < 0 || device >= ndev) return set_error(MTSVGPU_EINVAL, "device %d out of range", device);
+  MTSV_CUDA_TRY(cudaSetDevice(device));
   return 0;
 }
 
-void DevBuf::release() {
-  if (p) cudaFree(p);
-  p = nullptr;
+int DevBuf::reserve(size_t bytes) {
+  if (bytes <= cap && p) return 0;
+  p.reset();
   cap = 0;
-}
-
-void BatchWorkspace::release_all() {
-  DevBuf* all[] = {&slot_off, &q_nseeds, &q_nhits, &hit_off,  &q_ncand,    &cand_off,   &q_nout,
-                   &out_off,  &slot_q,   &slot_lo, &slot_cnt, &slot_hoff,  &hit_keys,   &cand_sparse,
-                   &cand_stage, &cand_dense, &cand_q, &cand_edit, &hit_tmp, &scan_tmp,   &counters,
-                   &worklist, &out_hits, &out_hit_off, &d_seqs, &d_seq_off,
-                   &cand_flag, &cand_order, &enc, &cand_end, &ssw_list, &ssw_scratch, &pack_rel, &cand_lead, &cand_order2};
-  for (DevBuf* b : all) b->release();
+  size_t want = bytes + bytes / 4 + 256;  // headroom so slowly growing batches do not realloc
+  if (dev_alloc(p, want) != 0) {
+    want = bytes ? bytes : 256;
+    MTSV_TRY(dev_alloc(p, want));
+  }
+  cap = want;
+  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------
