@@ -2,16 +2,12 @@
 visits every chunk, and the per-read hit lists are merged the way ``mtsv-collapse`` merges the per-chunk
 results files (src/collapse.rs:543-654, mode TaxId: minimum edit per TaxID, :597-602).
 
-Product path: ``ChunkComm`` = mtsvgpu_comm_* / mtsvgpu_bin_batch_chunked — the exchange and the merge run
-inside the library (csrc/chunked.cu: hits stored straight into the owning rank's buffer over NVLink peer
-memory, one flag barrier, collapse as the epilogue); the host only moves `world` 128-byte handles once.
-``exchange_hits`` / ``bin_reads_chunk_sharded`` below are the earlier formulation on torch.distributed
-collectives (all_to_all_single x3): kept as the A/B baseline the fused path is checked and timed against,
-and because it runs on gloo without a GPU.
+``ChunkComm`` = mtsvgpu_comm_* / mtsvgpu_bin_batch_chunked — the exchange and the merge run inside the library
+(csrc/chunked.cu: hits stored straight into the owning rank's buffer over NVLink peer memory, one flag barrier,
+collapse as the epilogue); the host only moves `world` 128-byte handles once.  ``collapse_parts_device`` and
+``collapse_parts_device_taxid_gi`` run the library's merge on hit lists the caller already holds on the device.
 """
 import ctypes as C
-
-import numpy as np
 
 from . import _lib
 from ._lib import check
@@ -105,98 +101,37 @@ def read_ranges(n_reads, world):
     return [min(n_reads, i * step) for i in range(world + 1)]
 
 
-def collapse_parts_device(device, stream, parts_hits, parts_counts, n_reads):
-    """parts_hits / parts_counts: lists of torch CUDA tensors (uint8 bytes of mtsvgpu_hit[], int32 counts).
-    Returns (taxhits [n,2] int64-free uint32 numpy via D2H?, ...) — device pointers wrapped as torch tensors:
-    (pairs uint32 tensor of shape [n_out, 2], offsets int64 tensor [n_reads+1])."""
+def _collapse_parts(fn, rec_bytes, device, stream, parts_hits, parts_counts, n_reads):
+    """Runs the C collapse entry point `fn` (records of `rec_bytes` bytes).  Returns (uint8 tensor of the merged
+    records, offsets int64 tensor [n_reads+1]), copies that own their memory."""
     import torch
     L = _lib.load_library()
     n = len(parts_hits)
     hp = (C.c_void_p * n)(*[C.c_void_p(t.data_ptr()) for t in parts_hits])
     cp = (C.c_void_p * n)(*[C.c_void_p(t.data_ptr()) for t in parts_counts])
     d_out, d_off, n_out = C.c_void_p(), C.c_void_p(), C.c_uint64()
-    check(L.mtsvgpu_collapse_device(device, C.c_void_p(stream or 0), n, hp, cp, n_reads, C.byref(d_out),
-                                    C.byref(d_off), C.byref(n_out)))
+    check(getattr(L, fn)(device, C.c_void_p(stream or 0), n, hp, cp, n_reads, C.byref(d_out), C.byref(d_off),
+                         C.byref(n_out)))
     dev = torch.device("cuda", device)
-    pairs = torch.as_tensor(_DevArray(d_out.value, max(1, n_out.value) * 8), device=dev).clone()
+    recs = torch.as_tensor(_DevArray(d_out.value, max(1, n_out.value) * rec_bytes), device=dev).clone()
     offs = torch.as_tensor(_DevArray(d_off.value, (n_reads + 1) * 8), device=dev).clone()
     L.mtsvgpu_device_free(d_out)
     L.mtsvgpu_device_free(d_off)
-    pairs = pairs.view(torch.int32).reshape(-1, 2)[: n_out.value]
-    return pairs, offs.view(torch.int64)
+    return recs[: n_out.value * rec_bytes], offs.view(torch.int64)
+
+
+def collapse_parts_device(device, stream, parts_hits, parts_counts, n_reads):
+    """mtsv-collapse's mode TaxId on the device (src/collapse.rs:597-602): per read each TaxID once with its smallest
+    edit, by ascending TaxID.  parts_hits / parts_counts: lists of torch CUDA tensors (uint8 bytes of mtsvgpu_hit[],
+    int32 hits per read) for the same n_reads reads; stream: a CUDA stream handle or None.  Returns (pairs int32
+    tensor [n_out, 2] = (tax_id, edit), offsets int64 tensor [n_reads+1])."""
+    import torch
+    pairs, offs = _collapse_parts("mtsvgpu_collapse_device", 8, device, stream, parts_hits, parts_counts, n_reads)
+    return pairs.view(torch.int32).reshape(-1, 2), offs
 
 
 def collapse_parts_device_taxid_gi(device, stream, parts_hits, parts_counts, n_reads):
     """mtsv-collapse's mode TaxIdGi on the device (src/collapse.rs:603-625): per read and (TaxID, GI) the hit with
     the smallest edit, ties to the smallest offset, listed by (TaxID, GI).  Same inputs as collapse_parts_device;
     returns (hits uint8 tensor of 24-byte mtsvgpu_hit records, offsets int64 tensor [n_reads+1])."""
-    import torch
-    L = _lib.load_library()
-    n = len(parts_hits)
-    hp = (C.c_void_p * n)(*[C.c_void_p(t.data_ptr()) for t in parts_hits])
-    cp = (C.c_void_p * n)(*[C.c_void_p(t.data_ptr()) for t in parts_counts])
-    d_out, d_off, n_out = C.c_void_p(), C.c_void_p(), C.c_uint64()
-    check(L.mtsvgpu_collapse_device_taxid_gi(device, C.c_void_p(stream or 0), n, hp, cp, n_reads, C.byref(d_out),
-                                             C.byref(d_off), C.byref(n_out)))
-    dev = torch.device("cuda", device)
-    hits = torch.as_tensor(_DevArray(d_out.value, max(1, n_out.value) * 24), device=dev).clone()[: n_out.value * 24]
-    offs = torch.as_tensor(_DevArray(d_off.value, (n_reads + 1) * 8), device=dev).clone()
-    L.mtsvgpu_device_free(d_out)
-    L.mtsvgpu_device_free(d_off)
-    return hits, offs.view(torch.int64)
-
-
-def exchange_hits(hits_bytes, counts, bounds, group=None):
-    """The communication step.  hits_bytes: uint8 tensor (24 B per hit, CSR by read over ALL reads of the
-    batch); counts: int32 tensor [n_reads] (hits per read).  bounds: read_ranges().  Returns, for this
-    rank's range, the list over source ranks of (hits_bytes, counts).  Works on CUDA tensors with NCCL and
-    on CPU tensors with gloo (the unit tests)."""
-    import torch
-    import torch.distributed as dist
-    world = dist.get_world_size(group)
-    rank = dist.get_rank(group)
-    n_local = bounds[rank + 1] - bounds[rank]
-    # hits each destination receives from me = sum of my counts over its range
-    csum = torch.zeros(len(counts) + 1, dtype=torch.int64, device=counts.device)
-    csum[1:] = torch.cumsum(counts.to(torch.int64), 0)
-    b = torch.tensor(bounds, dtype=torch.int64, device=counts.device)
-    send_hits = (csum[b[1:]] - csum[b[:-1]])  # [world]
-    recv_hits = torch.empty_like(send_hits)
-    dist.all_to_all_single(recv_hits, send_hits, group=group)
-    send_hits_l = [int(x) for x in send_hits.tolist()]
-    recv_hits_l = [int(x) for x in recv_hits.tolist()]
-    # counts: every rank sends me its counts for my range (n_local each)
-    cnt_send_split = [bounds[j + 1] - bounds[j] for j in range(world)]
-    cnt_recv = torch.empty(n_local * world, dtype=counts.dtype, device=counts.device)
-    dist.all_to_all_single(cnt_recv, counts.contiguous(), output_split_sizes=[n_local] * world,
-                           input_split_sizes=cnt_send_split, group=group)
-    # hits
-    hit_recv = torch.empty(sum(recv_hits_l) * 24, dtype=torch.uint8, device=hits_bytes.device)
-    dist.all_to_all_single(hit_recv, hits_bytes.contiguous()[: sum(send_hits_l) * 24],
-                           output_split_sizes=[x * 24 for x in recv_hits_l],
-                           input_split_sizes=[x * 24 for x in send_hits_l], group=group)
-    parts, o = [], 0
-    for j in range(world):
-        parts.append((hit_recv[o * 24:(o + recv_hits_l[j]) * 24], cnt_recv[j * n_local:(j + 1) * n_local]))
-        o += recv_hits_l[j]
-    return parts
-
-
-def bin_reads_chunk_sharded(index, d_reads, d_off, n_reads, params, device, group=None, collapse_fn=None):
-    """One batch in chunk-sharded mode.  Every rank calls this with the SAME reads (device tensors) and its
-    own chunk's index.  Returns (pairs, offsets) for this rank's range of reads: pairs[k] = (tax_id, edit)."""
-    import torch
-    import torch.distributed as dist
-    world = dist.get_world_size(group)
-    d_hits, d_hit_off, n_hits = index.bin_reads_device(d_reads.data_ptr(), d_off.data_ptr(), n_reads, params)
-    dev = torch.device("cuda", device)
-    hits_bytes = torch.as_tensor(_DevArray(d_hits, max(1, n_hits) * 24), device=dev)[: n_hits * 24]
-    off = torch.as_tensor(_DevArray(d_hit_off, (n_reads + 1) * 8), device=dev).view(torch.int64)
-    counts = (off[1:] - off[:-1]).to(torch.int32)
-    bounds = read_ranges(n_reads, world)
-    parts = exchange_hits(hits_bytes, counts, bounds, group)
-    rank = dist.get_rank(group)
-    fn = collapse_fn or (lambda ph, pc, n: collapse_parts_device(device, torch.cuda.current_stream().cuda_stream,
-                                                                 ph, pc, n))
-    torch.cuda.current_stream().synchronize()
-    return fn([p[0] for p in parts], [p[1] for p in parts], bounds[rank + 1] - bounds[rank])
+    return _collapse_parts("mtsvgpu_collapse_device_taxid_gi", 24, device, stream, parts_hits, parts_counts, n_reads)

@@ -1330,6 +1330,7 @@ __global__ void __launch_bounds__(256) gather_hits_kernel(uint32_t nq, uint32_t 
 // ---- assignments output: each read's selected hits of both strands merged into (TaxID, edit) records ----
 // The selected hits of strand q (hit_tmp at cand_off[q], compacted to out_off[q]) become keys tax << 32 | edit; the
 // strands of read r are queries r*ns .. r*ns+ns-1, so read r's keys are the segment [seg_off[r], seg_off[r + 1]).
+// collapse.cu's taxid_merge_count / taxid_merge_write merge the segments.
 __global__ void __launch_bounds__(256) taxid_keys_kernel(uint32_t nq, uint32_t ns,
                                                          const uint32_t* __restrict__ cand_off,
                                                          const uint32_t* __restrict__ out_off,
@@ -1360,28 +1361,6 @@ __global__ void __launch_bounds__(256) taxid_keys_kernel(uint32_t nq, uint32_t n
     for (uint32_t i = lane; i < n_s; i += 32)
       keys[dst_s + i] = ((uint64_t)hit_tmp[src_s + i].tax_id << 32) | hit_tmp[src_s + i].edit;
   }
-}
-
-// records per read, after the segments have been sorted
-__global__ void __launch_bounds__(256) taxid_count_kernel(const uint64_t* __restrict__ keys,
-                                                          const uint32_t* __restrict__ seg_off, uint32_t n_reads,
-                                                          uint32_t* __restrict__ n_out) {
-  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= n_reads) return;
-  n_out[r] = taxid_count(keys, seg_off[r], seg_off[r + 1]);
-}
-
-// appends the sub-batch's records to the batch output at out_base; read offsets go to out_off from read_base on
-__global__ void __launch_bounds__(256) taxid_write_kernel(const uint64_t* __restrict__ keys,
-                                                          const uint32_t* __restrict__ seg_off,
-                                                          const uint32_t* __restrict__ tax_off, uint32_t n_reads,
-                                                          mtsvgpu_taxhit* __restrict__ out, uint64_t out_base,
-                                                          uint64_t* __restrict__ out_off, uint64_t read_base) {
-  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r > n_reads) return;
-  out_off[read_base + r] = out_base + tax_off[r];  // r == n_reads: the end
-  if (r == n_reads) return;
-  taxid_write(keys, seg_off[r], seg_off[r + 1], out + out_base, tax_off[r]);
 }
 
 // verification order: multi-seed candidates first, single-seed ones after (stable within each class)
@@ -1963,10 +1942,8 @@ int SubBatch::merge_taxids() {
   uint64_t* keys = ws.hit_keys.as<uint64_t>();
   MTSV_LAUNCH(taxid_keys_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
               ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), keys, seg_off(), seg_cnt());
-  MTSV_TRY(run_segmented_sort(st, ws.worklist, keys, seg_off(), seg_cnt(), nr, 1, d_ctr));
-  MTSV_LAUNCH(taxid_count_kernel, (nr + 255) / 256, 256, 0, st, keys, seg_off(), nr, tax_cnt());
-  MTSV_TRY(exclusive_scan_u32(tax_cnt(), tax_off(), nr, ws.scan_tmp, (uint64_t*)&d_ctr->total_taxhits, st));
-  return 0;
+  return taxid_merge_count(st, ws.worklist, ws.scan_tmp, keys, seg_off(), seg_cnt(), nr, n_cand, d_ctr, tax_cnt(),
+                           tax_off(), (uint64_t*)&d_ctr->total_taxhits);
 }
 
 // ---- select, then append to the batch output: in slice order, after the other lane's previous append ----
@@ -2005,9 +1982,8 @@ int SubBatch::select_append(uint64_t* out_total) {
   MTSV_TRY(grow_preserve(res.out_hits, *out_total * rec, (*out_total + sub_rec + 1) * rec, st));
   begin(ST_EMIT);
   if (taxhits) {
-    MTSV_LAUNCH(taxid_write_kernel, (rv.n_reads + 1 + 255) / 256, 256, 0, st, ws.hit_keys.as<uint64_t>(), seg_off(),
-                tax_off(), rv.n_reads, res.out_hits.as<mtsvgpu_taxhit>(), *out_total, res.out_hit_off.as<uint64_t>(),
-                rv.read0);
+    taxid_merge_write(st, ws.hit_keys.as<uint64_t>(), seg_off(), tax_off(), rv.n_reads, res.out_hits.as<mtsvgpu_taxhit>(),
+                      *out_total, res.out_hit_off.as<uint64_t>(), rv.read0);
   } else {
     MTSV_LAUNCH(gather_hits_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
                 ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), res.out_hits.as<HitRec>(), *out_total,

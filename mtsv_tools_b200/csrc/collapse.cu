@@ -1,16 +1,58 @@
-// collapse.cu — chunk-sharded operation (SURVEY §8e): merge the hit lists that several MG-index
-// chunks produced for the SAME reads.  This is the reduction mtsv-collapse performs on results files
-// (src/collapse.rs:543-654); mode TaxId: for equal read ids keep the minimum edit per TaxID
-// (:597-602), hits listed by ascending TaxID (write_collapsed_taxid, :278-279); mode TaxIdGi further down.
+// collapse.cu — the library's (TaxID, edit) merge, and the device collapse of chunk-sharded operation.
 //
-// Inputs: n_parts device arrays of mtsvgpu_hit, each with a per-read u32 count array for the same
-// n_reads reads (after the NCCL exchange every rank holds all parts for its own range of reads).
+// The merge (taxid_merge_count / taxid_merge_write): per read, a segment of keys tax << 32 | edit becomes each TaxID
+// once with its minimum edit, by ascending TaxID (core.cuh::taxid_count / taxid_write).  The binner's assignments
+// output (binner.cu) and the TaxId collapse below both go through it.
+//
+// The collapse (SURVEY §8e): merge the hit lists that several MG-index chunks produced for the SAME reads.  This is
+// the reduction mtsv-collapse performs on results files (src/collapse.rs:543-654); mode TaxId: for equal read ids
+// keep the minimum edit per TaxID (:597-602), hits listed by ascending TaxID (write_collapsed_taxid, :278-279); mode
+// TaxIdGi further down.  Inputs: n_parts device arrays of mtsvgpu_hit, each with a per-read u32 count array for the
+// same n_reads reads (after the chunk exchange every rank holds all parts for its own range of reads).
 // All kernels are flat over reads / hits; the per-read sort reuses the binner's segmented sorts.
 #include <mutex>
 
 #include "ctx.h"
 
 namespace mtsv {
+
+// records per read, after the segments have been sorted
+__global__ void __launch_bounds__(256) taxid_count_kernel(const uint64_t* __restrict__ keys,
+                                                          const uint32_t* __restrict__ seg_off, uint32_t n_reads,
+                                                          uint32_t* __restrict__ n_out) {
+  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_reads) return;
+  n_out[r] = taxid_count(keys, seg_off[r], seg_off[r + 1]);
+}
+
+// appends the sub-batch's records to the batch output at out_base; read offsets go to out_off from read_base on
+__global__ void __launch_bounds__(256) taxid_write_kernel(const uint64_t* __restrict__ keys,
+                                                          const uint32_t* __restrict__ seg_off,
+                                                          const uint32_t* __restrict__ tax_off, uint32_t n_reads,
+                                                          mtsvgpu_taxhit* __restrict__ out, uint64_t out_base,
+                                                          uint64_t* __restrict__ out_off, uint64_t read_base) {
+  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r > n_reads) return;
+  out_off[read_base + r] = out_base + tax_off[r];  // r == n_reads: the end
+  if (r == n_reads) return;
+  taxid_write(keys, seg_off[r], seg_off[r + 1], out + out_base, tax_off[r]);
+}
+
+int taxid_merge_count(cudaStream_t st, DevBuf& worklist, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
+                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, BatchCounters* d_ctr,
+                      uint32_t* tax_cnt, uint32_t* tax_off, uint64_t* d_total) {
+  if (n_reads) {
+    if (key_bound) MTSV_TRY(run_segmented_sort(st, worklist, keys, seg_off, seg_cnt, n_reads, 1, d_ctr));
+    MTSV_LAUNCH(taxid_count_kernel, (n_reads + 255) / 256, 256, 0, st, keys, seg_off, n_reads, tax_cnt);
+  }
+  return exclusive_scan_u32(tax_cnt, tax_off, n_reads, scan_tmp, d_total, st);
+}
+
+void taxid_merge_write(cudaStream_t st, const uint64_t* keys, const uint32_t* seg_off, const uint32_t* tax_off,
+                       uint32_t n_reads, mtsvgpu_taxhit* out, uint64_t out_base, uint64_t* out_off, uint64_t read_base) {
+  MTSV_LAUNCH(taxid_write_kernel, (n_reads + 1 + 255) / 256, 256, 0, st, keys, seg_off, tax_off, n_reads, out, out_base,
+              out_off, read_base);
+}
 
 struct PartsView {
   const mtsvgpu_hit* hits[16];
@@ -38,23 +80,6 @@ __global__ void collapse_scatter_kernel(PartsView pv, uint32_t n_reads, const ui
   const mtsvgpu_hit* src = pv.hits[p] + pv.offs[p][r];
   uint32_t n = pv.counts[p][r];
   for (uint32_t i = 0; i < n; ++i) keys[dst + i] = ((uint64_t)src[i].tax_id << 32) | src[i].edit;
-}
-
-__global__ void collapse_count_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ comb_off,
-                                      uint32_t n_reads, uint32_t* __restrict__ n_out) {
-  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= n_reads) return;
-  n_out[r] = taxid_count(keys, comb_off[r], comb_off[r + 1]);
-}
-
-__global__ void collapse_write_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ comb_off,
-                                      const uint32_t* __restrict__ out_off32, uint32_t n_reads,
-                                      mtsvgpu_taxhit* __restrict__ out, uint64_t* __restrict__ out_off) {
-  uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r > n_reads) return;
-  out_off[r] = out_off32[r];
-  if (r == n_reads) return;
-  taxid_write(keys, comb_off[r], comb_off[r + 1], out, out_off32[r]);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -132,6 +157,42 @@ __global__ void __launch_bounds__(128) collapse_long_write_kernel(const mtsvgpu_
   }
 }
 
+// The parts of one collapse call: pv, their per-read offsets, and per read the combined count (w.total) and offset
+// (w.comb_off); the combined total goes to *d_tot.
+static int prepare_parts(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
+                         const uint32_t* const* d_counts, uint32_t nr, PartsView* pv, uint64_t** d_tot) {
+  *pv = PartsView{};
+  pv->n_parts = n_parts;
+  MTSV_TRY(w.counters.reserve(sizeof(BatchCounters) + 16));
+  MTSV_CUDA_TRY(cudaMemsetAsync(w.counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
+  *d_tot = reinterpret_cast<uint64_t*>(w.counters.as<uint8_t>() + sizeof(BatchCounters));
+  for (uint32_t p = 0; p < n_parts; ++p) {
+    pv->hits[p] = d_hits[p];
+    pv->counts[p] = d_counts[p];
+    MTSV_TRY(w.offs[p].reserve(((size_t)nr + 1) * 4));
+    MTSV_TRY(exclusive_scan_u32(d_counts[p], w.offs[p].as<uint32_t>(), nr, w.scan_tmp, nullptr, st));
+    pv->offs[p] = w.offs[p].as<uint32_t>();
+  }
+  for (DevBuf* b : {&w.total, &w.comb_off, &w.cnt_out, &w.off_out32}) MTSV_TRY(b->reserve(((size_t)nr + 1) * 4));
+  if (nr) MTSV_LAUNCH(collapse_total_kernel, (nr + 255) / 256 + 1, 256, 0, st, *pv, nr, w.total.as<uint32_t>());
+  return exclusive_scan_u32(w.total.as<uint32_t>(), w.comb_off.as<uint32_t>(), nr, w.scan_tmp, *d_tot, st);
+}
+
+// Mode TaxId after prepare_parts: the parts' hits as keys in read order (at most hit_cap of them), merged; per read
+// the record count (w.cnt_out) and offset (w.off_out32), the record total to *d_n_out.
+static int merge_parts_count(CollapseScratch& w, cudaStream_t st, const PartsView& pv, uint32_t nr, uint64_t hit_cap,
+                             uint64_t* d_n_out) {
+  MTSV_TRY(w.keys.reserve((size_t)(hit_cap + 1) * 8));
+  if (nr && hit_cap) {
+    const uint64_t threads = (uint64_t)nr * pv.n_parts;
+    MTSV_LAUNCH(collapse_scatter_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, pv, nr,
+                w.comb_off.as<uint32_t>(), w.keys.as<uint64_t>());
+  }
+  return taxid_merge_count(st, w.worklist, w.scan_tmp, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(),
+                           w.total.as<uint32_t>(), nr, hit_cap, w.counters.as<BatchCounters>(), w.cnt_out.as<uint32_t>(),
+                           w.off_out32.as<uint32_t>(), d_n_out);
+}
+
 int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
                     const uint32_t* const* d_counts, uint64_t n_reads, mtsvgpu_taxhit** d_out,
                     uint64_t** d_out_off, uint64_t* n_out) {
@@ -147,52 +208,22 @@ int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu
   static std::mutex g_mu;
   std::lock_guard<std::mutex> lock(g_mu);
   CollapseScratch& w = g_ws[device];
-  DevBuf* offs = w.offs;
-  DevBuf &total = w.total, &comb_off = w.comb_off, &keys = w.keys, &scan_tmp = w.scan_tmp,
-         &counters = w.counters, &worklist = w.worklist, &cnt_out = w.cnt_out, &off_out32 = w.off_out32;
-
-  PartsView pv{};
-  pv.n_parts = n_parts;
-  MTSV_TRY(counters.reserve(sizeof(BatchCounters) + 16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
-  uint64_t* d_tot = reinterpret_cast<uint64_t*>(counters.as<uint8_t>() + sizeof(BatchCounters));
-  for (uint32_t p = 0; p < n_parts; ++p) {
-    pv.hits[p] = d_hits[p];
-    pv.counts[p] = d_counts[p];
-    MTSV_TRY(offs[p].reserve(((size_t)nr + 1) * 4));
-    MTSV_TRY(exclusive_scan_u32(d_counts[p], offs[p].as<uint32_t>(), nr, scan_tmp, nullptr, st));
-    pv.offs[p] = offs[p].as<uint32_t>();
-  }
-  MTSV_TRY(total.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(comb_off.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(cnt_out.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(off_out32.reserve(((size_t)nr + 1) * 4));
-  const unsigned rgrid = (nr + 255) / 256 + 1;
-  if (nr) MTSV_LAUNCH(collapse_total_kernel, rgrid, 256, 0, st, pv, nr, total.as<uint32_t>());
-  MTSV_TRY(exclusive_scan_u32(total.as<uint32_t>(), comb_off.as<uint32_t>(), nr, scan_tmp, d_tot, st));
+  PartsView pv;
+  uint64_t* d_tot = nullptr;
+  MTSV_TRY(prepare_parts(w, st, n_parts, d_hits, d_counts, nr, &pv, &d_tot));
   uint64_t h_tot = 0;
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   if (h_tot > 0xfffffff0ull) return set_error(MTSVGPU_ELIMIT, "more than 2^32 hits in one collapse call");
-  MTSV_TRY(keys.reserve((size_t)(h_tot + 1) * 8));
-  if (nr && h_tot) {
-    const uint64_t threads = (uint64_t)nr * n_parts;
-    MTSV_LAUNCH(collapse_scatter_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, pv, nr,
-                comb_off.as<uint32_t>(), keys.as<uint64_t>());
-    MTSV_TRY(run_segmented_sort(st, worklist, keys.as<uint64_t>(), comb_off.as<uint32_t>(), total.as<uint32_t>(), nr,
-                                1, counters.as<BatchCounters>()));
-  }
-  if (nr) MTSV_LAUNCH(collapse_count_kernel, rgrid, 256, 0, st, keys.as<uint64_t>(), comb_off.as<uint32_t>(), nr,
-                      cnt_out.as<uint32_t>());
-  MTSV_TRY(exclusive_scan_u32(cnt_out.as<uint32_t>(), off_out32.as<uint32_t>(), nr, scan_tmp, d_tot, st));
+  MTSV_TRY(merge_parts_count(w, st, pv, nr, h_tot, d_tot));
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   DevPtr<mtsvgpu_taxhit> out;
   DevPtr<uint64_t> out_off;
   MTSV_TRY(dev_alloc(out, h_tot + 1));
   MTSV_TRY(dev_alloc(out_off, (uint64_t)nr + 1));
-  MTSV_LAUNCH(collapse_write_kernel, rgrid, 256, 0, st, keys.as<uint64_t>(), comb_off.as<uint32_t>(),
-              off_out32.as<uint32_t>(), nr, out.get(), out_off.get());
+  taxid_merge_write(st, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(), w.off_out32.as<uint32_t>(), nr, out.get(), 0,
+                    out_off.get(), 0);
   cudaError_t e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "collapse: %s", cudaGetErrorString(e));
   // the caller frees the results with mtsvgpu_device_free
@@ -210,40 +241,15 @@ int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, 
                          uint64_t* out_off, uint64_t* d_n_out) {
   if (n_parts == 0 || n_parts > 16) return set_error(MTSVGPU_EINVAL, "n_parts must be in [1,16]");
   if (hit_cap > 0xfffffff0ull) return set_error(MTSVGPU_ELIMIT, "more than 2^32 hits in one collapse call");
-  PartsView pv{};
-  pv.n_parts = n_parts;
-  MTSV_TRY(w.counters.reserve(sizeof(BatchCounters) + 16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(w.counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
-  uint64_t* d_tot = reinterpret_cast<uint64_t*>(w.counters.as<uint8_t>() + sizeof(BatchCounters));
+  // (the scans and the sort synchronise the stream when they have to grow these)
   MTSV_TRY(w.scan_tmp.reserve((((size_t)nr + 1 + 2047) / 2048 + 1) * 8));
   MTSV_TRY(w.worklist.reserve((size_t)3 * (nr + 1) * 4));
-  for (uint32_t p = 0; p < n_parts; ++p) {
-    pv.hits[p] = d_hits[p];
-    pv.counts[p] = d_counts[p];
-    MTSV_TRY(w.offs[p].reserve(((size_t)nr + 1) * 4));
-    MTSV_TRY(exclusive_scan_u32(d_counts[p], w.offs[p].as<uint32_t>(), nr, w.scan_tmp, nullptr, st));
-    pv.offs[p] = w.offs[p].as<uint32_t>();
-  }
-  MTSV_TRY(w.total.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(w.comb_off.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(w.cnt_out.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(w.off_out32.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(w.keys.reserve((size_t)(hit_cap + 1) * 8));
-  const unsigned rgrid = (nr + 255) / 256 + 1;
-  if (nr) MTSV_LAUNCH(collapse_total_kernel, rgrid, 256, 0, st, pv, nr, w.total.as<uint32_t>());
-  MTSV_TRY(exclusive_scan_u32(w.total.as<uint32_t>(), w.comb_off.as<uint32_t>(), nr, w.scan_tmp, d_tot, st));
-  if (nr) {
-    const uint64_t threads = (uint64_t)nr * n_parts;
-    MTSV_LAUNCH(collapse_scatter_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, pv, nr,
-                w.comb_off.as<uint32_t>(), w.keys.as<uint64_t>());
-    MTSV_TRY(run_segmented_sort(st, w.worklist, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(), w.total.as<uint32_t>(),
-                                nr, 1, w.counters.as<BatchCounters>()));
-    MTSV_LAUNCH(collapse_count_kernel, rgrid, 256, 0, st, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(), nr,
-                w.cnt_out.as<uint32_t>());
-  }
-  MTSV_TRY(exclusive_scan_u32(w.cnt_out.as<uint32_t>(), w.off_out32.as<uint32_t>(), nr, w.scan_tmp, d_n_out, st));
-  MTSV_LAUNCH(collapse_write_kernel, rgrid, 256, 0, st, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(),
-              w.off_out32.as<uint32_t>(), nr, out, out_off);
+  PartsView pv;
+  uint64_t* d_tot = nullptr;
+  MTSV_TRY(prepare_parts(w, st, n_parts, d_hits, d_counts, nr, &pv, &d_tot));
+  MTSV_TRY(merge_parts_count(w, st, pv, nr, hit_cap, d_n_out));
+  taxid_merge_write(st, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(), w.off_out32.as<uint32_t>(), nr, out, 0,
+                    out_off, 0);
   MTSV_CUDA_TRY(cudaGetLastError());
   return 0;
 }
@@ -256,26 +262,11 @@ int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mt
   if (n_reads > 0x07fffff0ull) return set_error(MTSVGPU_ELIMIT, "too many reads in one collapse call");
   MTSV_TRY(use_device(device));
   const uint32_t nr = (uint32_t)n_reads;
-  DevBuf offs[16], total, comb_off, comb, flag, scan_tmp, counters, cnt_out, off_out32;
-  PartsView pv{};
-  pv.n_parts = n_parts;
-  MTSV_TRY(counters.reserve(16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(counters.p.get(), 0, 16, st));
-  uint64_t* d_tot = counters.as<uint64_t>();
-  for (uint32_t p = 0; p < n_parts; ++p) {
-    pv.hits[p] = d_hits[p];
-    pv.counts[p] = d_counts[p];
-    MTSV_TRY(offs[p].reserve(((size_t)nr + 1) * 4));
-    MTSV_TRY(exclusive_scan_u32(d_counts[p], offs[p].as<uint32_t>(), nr, scan_tmp, nullptr, st));
-    pv.offs[p] = offs[p].as<uint32_t>();
-  }
-  MTSV_TRY(total.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(comb_off.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(cnt_out.reserve(((size_t)nr + 1) * 4));
-  MTSV_TRY(off_out32.reserve(((size_t)nr + 1) * 4));
-  const unsigned rgrid = (nr + 255) / 256 + 1;
-  if (nr) MTSV_LAUNCH(collapse_total_kernel, rgrid, 256, 0, st, pv, nr, total.as<uint32_t>());
-  MTSV_TRY(exclusive_scan_u32(total.as<uint32_t>(), comb_off.as<uint32_t>(), nr, scan_tmp, d_tot, st));
+  CollapseScratch w;
+  DevBuf comb, flag;
+  PartsView pv;
+  uint64_t* d_tot = nullptr;
+  MTSV_TRY(prepare_parts(w, st, n_parts, d_hits, d_counts, nr, &pv, &d_tot));
   uint64_t h_tot = 0;
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
@@ -287,20 +278,20 @@ int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mt
     if (h_tot) {
       const uint64_t threads = (uint64_t)nr * n_parts;
       MTSV_LAUNCH(collapse_gather_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, pv, nr,
-                  comb_off.as<uint32_t>(), comb.as<mtsvgpu_hit>());
+                  w.comb_off.as<uint32_t>(), comb.as<mtsvgpu_hit>());
     }
-    MTSV_LAUNCH(collapse_long_flag_kernel, wgrid, 128, 0, st, comb.as<mtsvgpu_hit>(), comb_off.as<uint32_t>(), nr,
-                flag.as<uint8_t>(), cnt_out.as<uint32_t>());
+    MTSV_LAUNCH(collapse_long_flag_kernel, wgrid, 128, 0, st, comb.as<mtsvgpu_hit>(), w.comb_off.as<uint32_t>(), nr,
+                flag.as<uint8_t>(), w.cnt_out.as<uint32_t>());
   }
-  MTSV_TRY(exclusive_scan_u32(cnt_out.as<uint32_t>(), off_out32.as<uint32_t>(), nr, scan_tmp, d_tot, st));
+  MTSV_TRY(exclusive_scan_u32(w.cnt_out.as<uint32_t>(), w.off_out32.as<uint32_t>(), nr, w.scan_tmp, d_tot, st));
   MTSV_CUDA_TRY(cudaMemcpyAsync(&h_tot, d_tot, 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   DevPtr<mtsvgpu_hit> out;
   DevPtr<uint64_t> out_off;
   MTSV_TRY(dev_alloc(out, h_tot + 1));
   MTSV_TRY(dev_alloc(out_off, (uint64_t)nr + 1));
-  MTSV_LAUNCH(collapse_long_write_kernel, wgrid, 128, 0, st, comb.as<mtsvgpu_hit>(), comb_off.as<uint32_t>(),
-              flag.as<uint8_t>(), off_out32.as<uint32_t>(), nr, out.get(), out_off.get());
+  MTSV_LAUNCH(collapse_long_write_kernel, wgrid, 128, 0, st, comb.as<mtsvgpu_hit>(), w.comb_off.as<uint32_t>(),
+              flag.as<uint8_t>(), w.off_out32.as<uint32_t>(), nr, out.get(), out_off.get());
   cudaError_t e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return set_error(MTSVGPU_ECUDA, "collapse (taxid-gi): %s", cudaGetErrorString(e));
   *d_out = out.release();

@@ -297,6 +297,17 @@ int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off
                         uint32_t* edits);
 int run_segmented_sort(cudaStream_t st, DevBuf& worklist, uint64_t* keys, const uint32_t* seg_off,
                        const uint32_t* seg_cnt, uint32_t nq, uint32_t min_count, BatchCounters* d_ctr);
+// collapse.cu
+// The (TaxID, edit) merge of keys tax << 32 | edit, read r's keys at [seg_off[r], seg_off[r] + seg_cnt[r])
+// (seg_off[n_reads] = the end).  taxid_merge_count sorts each segment (none when key_bound, a bound on the keys, is
+// 0), counts its records into tax_cnt and scans them into tax_off; the record total goes to *d_total.
+// taxid_merge_write then writes read r's records to out[out_base + tax_off[r]] on and out_off[read_base + r] =
+// out_base + tax_off[r] for r = 0 .. n_reads.
+int taxid_merge_count(cudaStream_t st, DevBuf& worklist, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
+                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, BatchCounters* d_ctr,
+                      uint32_t* tax_cnt, uint32_t* tax_off, uint64_t* d_total);
+void taxid_merge_write(cudaStream_t st, const uint64_t* keys, const uint32_t* seg_off, const uint32_t* tax_off,
+                       uint32_t n_reads, mtsvgpu_taxhit* out, uint64_t out_base, uint64_t* out_off, uint64_t read_base);
 int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
                     const uint32_t* const* d_counts, uint64_t n_reads, mtsvgpu_taxhit** d_out,
                     uint64_t** d_out_off, uint64_t* n_out);

@@ -1,5 +1,5 @@
-"""Chunk-sharded operation (SURVEY §8e): the NCCL exchange logic on CPU with gloo (world_size 2) and the
-device collapse kernel against the oracle's restatement of mtsv-collapse's merge rule."""
+"""Chunk-sharded operation (SURVEY §8e): the collapse rule's KATs, the device collapse against the oracle's
+restatement of mtsv-collapse's merge rule, and the fused exchange (mtsvgpu_bin_batch_chunked) against the oracle."""
 import os
 import socket
 
@@ -12,76 +12,6 @@ import torch.multiprocessing as mp
 from mtsv_tools_b200 import chunked
 
 HIT_DTYPE = np.dtype([("tax_id", "<u4"), ("gi", "<u4"), ("offset", "<u8"), ("edit", "<u4"), ("reserved", "<u4")])
-
-
-def _fake_hits(rank, n_reads, seed=0):
-    """Deterministic per-rank hit lists (as a chunk would produce) for the same reads."""
-    rng = np.random.default_rng(seed * 100 + rank)
-    counts = rng.integers(0, 5, size=n_reads).astype(np.int32)
-    counts[rng.random(n_reads) < 0.3] = 0
-    hits = np.zeros(int(counts.sum()), dtype=HIT_DTYPE)
-    hits["tax_id"] = rng.integers(1, 8, size=len(hits)) + 10 * (rng.random(len(hits)) < 0.5) * rank
-    hits["gi"] = rng.integers(1, 100, size=len(hits))
-    hits["offset"] = rng.integers(0, 1000, size=len(hits))
-    hits["edit"] = rng.integers(0, 20, size=len(hits))
-    offs = np.zeros(n_reads + 1, dtype=np.uint64)
-    offs[1:] = np.cumsum(counts)
-    return hits, offs, counts
-
-
-def _collapse_numpy(parts_hits, parts_counts, n):
-    from oracle import pyoracle
-    parts = []
-    for hb, c in zip(parts_hits, parts_counts):
-        hits = np.frombuffer(hb.numpy().tobytes(), dtype=HIT_DTYPE)
-        offs = np.zeros(n + 1, dtype=np.uint64)
-        offs[1:] = np.cumsum(c.numpy())
-        parts.append((hits, offs))
-    return pyoracle.collapse_taxid(parts)
-
-
-def _worker(rank, world, port, n_reads, out):
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    try:
-        hits, offs, counts = _fake_hits(rank, n_reads)
-        hb = torch.from_numpy(np.frombuffer(hits.tobytes(), dtype=np.uint8).copy())
-        bounds = chunked.read_ranges(n_reads, world)
-        parts = chunked.exchange_hits(hb, torch.from_numpy(counts), bounds)
-        pairs, po = _collapse_numpy([p[0] for p in parts], [p[1] for p in parts], bounds[rank + 1] - bounds[rank])
-        out.put((rank, pairs, po))
-    finally:
-        dist.destroy_process_group()
-
-
-def test_exchange_gloo_world2():
-    from oracle import pyoracle
-    world, n_reads = 2, 1001
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    procs = [ctx.Process(target=_worker, args=(r, world, port, n_reads, q)) for r in range(world)]
-    for p in procs:
-        p.start()
-    got = {}
-    for _ in range(world):
-        r, pairs, po = q.get(timeout=120)
-        got[r] = (pairs, po)
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    # expected: collapse of both ranks' full lists, then cut into the two ranges
-    full = [(_fake_hits(r, n_reads)[0], _fake_hits(r, n_reads)[1]) for r in range(world)]
-    want_pairs, want_off = pyoracle.collapse_taxid(full)
-    bounds = chunked.read_ranges(n_reads, world)
-    for r in range(world):
-        a, b = int(want_off[bounds[r]]), int(want_off[bounds[r + 1]])
-        assert np.array_equal(got[r][0], want_pairs[a:b])
-        assert np.array_equal(got[r][1], want_off[bounds[r]:bounds[r + 1] + 1] - want_off[bounds[r]])
 
 
 def test_collapse_rule_kats():
