@@ -2101,10 +2101,15 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
     if (src) {
       for (uint64_t i = 0; i <= n_sub; ++i) bounds[i] = src->seq_off[rb[i]];
     } else {
-      // (boundaries are multiples of the first slice's size: one strided gather instead of copying 8 B per read)
-      MTSV_CUDA_TRY(cudaMemcpy2DAsync(bounds.data(), 8, d_seq_off, rb[1] * 8, 8, n_sub, cudaMemcpyDeviceToHost, st));
+      // (boundaries are multiples of the first slice's size: one strided gather instead of copying 8 B per read).
+      // Only the slices that start inside the batch are gathered: an even slice count can leave the last slice
+      // empty, and its row i * rb[1] lies past seq_off[n_reads], which is where it starts and ends.
+      uint64_t n_inside = 0;
+      while (n_inside < n_sub && rb[n_inside] < n_reads) ++n_inside;
+      MTSV_CUDA_TRY(cudaMemcpy2DAsync(bounds.data(), 8, d_seq_off, rb[1] * 8, 8, n_inside, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaMemcpyAsync(&bounds[n_sub], d_seq_off + n_reads, 8, cudaMemcpyDeviceToHost, st));
       MTSV_CUDA_TRY(cudaStreamSynchronize(st));
+      for (uint64_t i = n_inside; i < n_sub; ++i) bounds[i] = bounds[n_sub];
     }
   }
   const int n_lanes = n_sub >= 2 && two_lanes ? 2 : 1;

@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
 
 from mtsv_tools_b200 import assignment_lines, results_lines, synth  # noqa: E402
 from mtsv_tools_b200.chunked import _DevArray  # noqa: E402
-from mtsv_tools_b200.index import TAXHIT_DTYPE, pack_reads, pack_reads_planes  # noqa: E402
+from mtsv_tools_b200.index import HIT_DTYPE, TAXHIT_DTYPE, pack_reads, pack_reads_planes  # noqa: E402
 from tests.test_gpu_parity import CASES, _gpu_index, _params  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -52,17 +52,58 @@ def _device_assign(g, reads, pg, strands=2):
     return recs.view(TAXHIT_DTYPE)[:nt].copy(), offs.view(np.uint64).copy()
 
 
-def _assert_device_shape(n_reads, batch_reads):
-    """Device-resident input whose even slice count leaves the last slice empty fails in the strided gather of the
-    slice bounds (a known bug of its own).  The shapes of these tests are chosen to avoid it; this checks that they
-    still do, with the library's own slicing code (core.cuh::slice_bounds, compiled for the CPU)."""
-    from tests import emul_api
-    b = emul_api.slice_bounds(n_reads, batch_reads, False, True)
-    assert len(b) < 2 or b[-2] < b[-1], "device-resident shape %d reads / batch_reads %d leaves an empty slice: %s" % (
-        n_reads, batch_reads, b[-3:])
+def _from_device(ptr, n, dtype):
+    """n records of `dtype` at a device pointer the library returned, copied to the host."""
+    raw = torch.as_tensor(_DevArray(ptr, max(n, 1) * dtype.itemsize), device="cuda").cpu().numpy()
+    return raw.view(dtype)[:n].copy()
 
 
-def _check(g, reads, names, pg, want_lines, strands=2, entries=("pinned", "packed", "device"), batch_reads=0):
+def _seq_off_with_tail(off, tail):
+    """seq_off at the start of a longer device tensor whose `tail` further entries hold 1 << 62: a slice bound
+    fetched from past seq_off[n] is then far beyond the batch (and the batch fails) instead of reading whatever
+    follows the array."""
+    t = np.full(len(off) + tail, 1 << 62, np.int64)
+    t[:len(off)] = np.asarray(off, np.uint64).astype(np.int64)
+    return torch.from_numpy(t).cuda()
+
+
+# (reads, batch_reads) of device-resident batches whose slice count is raised to an even number, which leaves the
+# last slice empty: 5 reads in steps of 2 are sliced 0 2 4 5 5
+EMPTY_LAST_SLICE = [(5, 2), (3, 1), (9, 4), (1000, 16), (4097, 16), (20000, 97)]
+
+
+def test_device_input_whose_last_slice_is_empty(oracle, emul, small_ref, small_index):
+    """mtsvgpu_bin_batch_device and mtsvgpu_assign_batch_device on batches whose last slice is empty, against the
+    oracle; with per-stage timing on (one lane: no empty slice) as the control.  Every slice bound, the empty slice's
+    too, is seq_off[n] or an entry before it."""
+    cat, off = small_ref[0], small_ref[1]
+    po, pg = _params(oracle)
+    for n, step in EMPTY_LAST_SLICE:
+        b = emul.slice_bounds(n, step, False, True)
+        assert b[-3] < b[-2] == b[-1] == n, (n, step, b[-3:])
+        assert emul.slice_bounds(n, step, False, False)[-2] < n
+        reads = synth.make_reads(cat, off, n, 150, seed=n)
+        h1, o1 = small_index.bin_reads(reads, po, threads=8)
+        want = _reduce(h1, o1)
+        d_seqs = torch.from_numpy(np.concatenate([reads[0], np.zeros(1, np.uint8)])).cuda()
+        d_off = _seq_off_with_tail(reads[1], b[1] + 1)
+        with _gpu_index(small_index, batch_reads=step) as g:
+            for profiling in (False, True):
+                g.set_profiling(profiling)
+                what = "%d reads, batch_reads %d, profiling %d" % (n, step, profiling)
+                dh, do, nh = g.bin_reads_device(d_seqs.data_ptr(), d_off.data_ptr(), n, pg)
+                hits, offs = _from_device(dh, nh, HIT_DTYPE), _from_device(do, n + 1, np.dtype(np.uint64))
+                assert np.array_equal(offs, o1), what
+                for f in ("tax_id", "gi", "offset", "edit"):
+                    assert np.array_equal(hits[f], h1[f]), (what, f)
+                dt, do, nt = g.assign_reads_device(d_seqs.data_ptr(), d_off.data_ptr(), n, pg)
+                _same((_from_device(dt, nt, TAXHIT_DTYPE), _from_device(do, n + 1, np.dtype(np.uint64))), want, what)
+                st = g.last_batch_stats()
+                assert st["n_queries"] == 2 * n and st["n_hits"] == len(h1), what
+                assert st["n_sub_batches"] >= (len(b) - 2 if not profiling else 1), what
+
+
+def _check(g, reads, names, pg, want_lines, strands=2, entries=("pinned", "packed", "device")):
     """Each entry point against the oracle's lines and against the host reduction of this handle's bin output."""
     h, o = g.bin_reads(reads, pg, strands)
     want = _reduce(h, o)
@@ -74,7 +115,6 @@ def _check(g, reads, names, pg, want_lines, strands=2, entries=("pinned", "packe
             pk, poff = pack_reads_planes(reads)
             got = tuple(x.copy() for x in g.assign_reads_packed(pk, poff, pg, strands))
         else:
-            _assert_device_shape(len(names), batch_reads)
             got = _device_assign(g, reads, pg, strands)
         _same(got, want, entry)
         assert assignment_lines(names, *got) == want_lines, entry
@@ -105,7 +145,7 @@ def test_assign_pipeline_small(oracle, small_ref, small_index, name, flags, opts
     po, pg = _params(oracle, **flags)
     h1, o1 = small_index.bin_reads(reads, po, threads=8)
     with _gpu_index(small_index, **opts) as g:
-        _check(g, reads, names, pg, oracle.results_lines(names, h1, o1, False), batch_reads=opts.get("batch_reads", 0))
+        _check(g, reads, names, pg, oracle.results_lines(names, h1, o1, False))
 
 
 def test_assign_packed_ragged(oracle, small_ref, small_index):
@@ -187,8 +227,7 @@ def test_assign_merges_a_taxid_hit_on_both_strands(oracle):
             for flags in flag_sets:
                 po, pg = _params(oracle, **flags)
                 h1, o1 = ix.bin_reads(reads, po, threads=8)
-                t, to = _check(g, reads, names, pg, oracle.results_lines(names, h1, o1, False),
-                               batch_reads=opts.get("batch_reads", 0))
+                t, to = _check(g, reads, names, pg, oracle.results_lines(names, h1, o1, False))
                 if len(t) < len(h1):
                     merged_sets += 1
                     n_rep, n_diff = _repeated_taxids(h1, o1)
@@ -287,7 +326,7 @@ def test_assign_reads_over_the_length_limit(oracle, small_ref, small_index):
     want_lines = oracle.results_lines([names[i] for i in keep], h1, o1, False)
     for opts in ({}, {"batch_reads": 300}):
         with _gpu_index(small_index, **opts) as g:
-            _check(g, lst, names, pg, want_lines, batch_reads=opts.get("batch_reads", 0))
+            _check(g, lst, names, pg, want_lines)
             assert g.last_batch_stats()["n_reads_over_limit"] == 2
 
 
@@ -306,7 +345,7 @@ def test_assign_slices_splits_regrowth_and_interleaving(oracle, small_ref, small
     for opts in ({"batch_reads": 97}, {"batch_reads": 1024}, {"max_batch_hits": 5000}, {}):
         with _gpu_index(small_index, **opts) as g:
             for reads, (names, lines) in zip(batches, want):
-                _check(g, reads, names, pg, lines, batch_reads=opts.get("batch_reads", 0))
+                _check(g, reads, names, pg, lines)
             # the same batches again: the pinned buffers now fit, the copy-out overlaps the compute
             for reads, (names, lines) in zip(batches, want):
                 t, to = g.assign_reads(reads, pg)
