@@ -15,6 +15,8 @@
 //
 // All per-item arithmetic lives in core.cuh (shared with the CPU emulation tests).
 #include <algorithm>
+#include <condition_variable>
+#include <mutex>
 #include <thread>
 
 #include "ctx.h"
@@ -305,165 +307,8 @@ __global__ void __launch_bounds__(256) locate_kernel(FmView fm, SaView sv, Param
   }
 }
 
-// ------------------------------------------------------------------------------------------
-// segmented sort of u64 keys: bitonic network in its "all ascending" form (first step of each
-// merge compares i with its mirror i ^ (k-1)), which tolerates virtual +inf padding, so segment
-// lengths need not be powers of two.  Segment q = keys[seg_off[q] .. + seg_cnt[q]).
-//   <= 32 keys : one warp, registers + shuffles
-//   <= 4096    : one CTA, shared memory
-//   larger     : one CTA, in place in global memory (rare: > 4096 seed hits for one read-strand)
-// ------------------------------------------------------------------------------------------
-constexpr uint32_t kSortMedium = 4096;
 constexpr uint32_t kLightItems = 16;  // segments this small are ordered by their consumer's own lane
 constexpr uint32_t kMonsterHits = 1024;  // strands with more seed hits than this get a whole CTA in coalesce
-
-__device__ __forceinline__ uint64_t warp_sort_u64(uint64_t v, unsigned lane) {
-#pragma unroll
-  for (int k = 2; k <= 32; k <<= 1) {
-    {
-      uint64_t o = __shfl_xor_sync(0xffffffffu, v, k - 1);
-      bool low = (lane & (k - 1)) < ((lane ^ (k - 1)) & (k - 1));
-      v = low ? (v < o ? v : o) : (v > o ? v : o);
-    }
-#pragma unroll
-    for (int j = k >> 2; j > 0; j >>= 1) {
-      uint64_t o = __shfl_xor_sync(0xffffffffu, v, j);
-      bool low = (lane & j) == 0;
-      v = low ? (v < o ? v : o) : (v > o ? v : o);
-    }
-  }
-  return v;
-}
-
-// Segments are classified once (warp-aggregated appends to three work lists); segments of at most
-// `min_count` keys are left to their consumer (the per-lane paths of coalesce / rank_emit order a
-// handful of keys themselves, which beats launching a warp per query).
-__global__ void __launch_bounds__(256) sort_classify_kernel(const uint32_t* __restrict__ seg_cnt, uint32_t nq,
-                                                            uint32_t min_count, uint32_t* __restrict__ warp_list,
-                                                            uint32_t* __restrict__ medium_list,
-                                                            uint32_t* __restrict__ large_list,
-                                                            BatchCounters* __restrict__ ctr) {
-  uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
-  const unsigned lane = threadIdx.x & 31;
-  uint32_t n = q < nq ? seg_cnt[q] : 0;
-  int cls = n <= min_count || n < 2 ? -1 : (n <= 32 ? 0 : (n <= kSortMedium ? 1 : 2));
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    unsigned m = __ballot_sync(0xffffffffu, cls == c);
-    if (!m) continue;
-    unsigned int* counter = c == 0 ? &ctr->n_warp : (c == 1 ? &ctr->n_medium : &ctr->n_large);
-    uint32_t* list = c == 0 ? warp_list : (c == 1 ? medium_list : large_list);
-    uint32_t base = 0;
-    if (lane == (unsigned)(__ffs(m) - 1)) base = atomicAdd(counter, (unsigned)__popc(m));
-    base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-    if (cls == c) list[base + __popc(m & ((1u << lane) - 1))] = q;
-  }
-}
-
-__global__ void __launch_bounds__(256) sort_warp_kernel(uint64_t* __restrict__ keys,
-                                                        const uint32_t* __restrict__ seg_off,
-                                                        const uint32_t* __restrict__ seg_cnt,
-                                                        const uint32_t* __restrict__ list,
-                                                        const BatchCounters* __restrict__ ctr) {
-  const unsigned lane = threadIdx.x & 31;
-  const uint32_t n_list = ctr->n_warp;
-  const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t it = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; it < n_list; it += warps) {
-    uint32_t q = list[it];
-    uint32_t n = seg_cnt[q];
-    uint64_t* base = keys + seg_off[q];
-    uint64_t v = lane < n ? base[lane] : ~0ull;
-    v = warp_sort_u64(v, lane);
-    if (lane < n) base[lane] = v;
-  }
-}
-
-__global__ void __launch_bounds__(512) sort_medium_kernel(uint64_t* __restrict__ keys,
-                                                          const uint32_t* __restrict__ seg_off,
-                                                          const uint32_t* __restrict__ seg_cnt,
-                                                          const uint32_t* __restrict__ list,
-                                                          const BatchCounters* __restrict__ ctr) {
-  __shared__ uint64_t sk[kSortMedium];
-  const uint32_t n_list = ctr->n_medium;
-  for (uint32_t it = blockIdx.x; it < n_list; it += gridDim.x) {
-    uint32_t q = list[it];
-    uint32_t n = seg_cnt[q];
-    uint64_t* base = keys + seg_off[q];
-    uint32_t N = 64;
-    while (N < n) N <<= 1;
-    for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) sk[i] = i < n ? base[i] : ~0ull;
-    __syncthreads();
-    for (uint32_t k = 2; k <= N; k <<= 1) {
-      for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) {
-        uint32_t l = i ^ (k - 1);
-        if (l > i) {
-          uint64_t a = sk[i], b = sk[l];
-          if (a > b) {
-            sk[i] = b;
-            sk[l] = a;
-          }
-        }
-      }
-      __syncthreads();
-      for (uint32_t j = k >> 2; j > 0; j >>= 1) {
-        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) {
-          uint32_t l = i ^ j;
-          if (l > i) {
-            uint64_t a = sk[i], b = sk[l];
-            if (a > b) {
-              sk[i] = b;
-              sk[l] = a;
-            }
-          }
-        }
-        __syncthreads();
-      }
-    }
-    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) base[i] = sk[i];
-    __syncthreads();
-  }
-}
-
-__global__ void __launch_bounds__(1024) sort_large_kernel(uint64_t* __restrict__ keys,
-                                                          const uint32_t* __restrict__ seg_off,
-                                                          const uint32_t* __restrict__ seg_cnt,
-                                                          const uint32_t* __restrict__ list,
-                                                          const BatchCounters* __restrict__ ctr) {
-  const uint32_t n_list = ctr->n_large;
-  for (uint32_t it = blockIdx.x; it < n_list; it += gridDim.x) {
-    uint32_t q = list[it];
-    uint32_t n = seg_cnt[q];
-    uint64_t* base = keys + seg_off[q];
-    uint64_t N = 64;
-    while (N < n) N <<= 1;
-    for (uint64_t k = 2; k <= N; k <<= 1) {
-      for (uint64_t i = threadIdx.x; i < n; i += blockDim.x) {
-        uint64_t l = i ^ (k - 1);
-        if (l > i && l < n) {
-          uint64_t a = base[i], b = base[l];
-          if (a > b) {
-            base[i] = b;
-            base[l] = a;
-          }
-        }
-      }
-      __syncthreads();
-      for (uint64_t j = k >> 2; j > 0; j >>= 1) {
-        for (uint64_t i = threadIdx.x; i < n; i += blockDim.x) {
-          uint64_t l = i ^ j;
-          if (l > i && l < n) {
-            uint64_t a = base[i], b = base[l];
-            if (a > b) {
-              base[i] = b;
-              base[l] = a;
-            }
-          }
-        }
-        __syncthreads();
-      }
-    }
-  }
-}
 
 // ------------------------------------------------------------------------------------------
 // coalesce / rank
@@ -1519,23 +1364,6 @@ static int validate_params(const mtsvgpu_params* in, Params* p) {
   return 0;
 }
 
-int run_segmented_sort(cudaStream_t st, DevBuf& worklist, uint64_t* keys, const uint32_t* seg_off,
-                              const uint32_t* seg_cnt, uint32_t nq, uint32_t min_count, BatchCounters* d_ctr) {
-  if (worklist.cap < (size_t)3 * nq * 4) {
-    MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-    MTSV_TRY(worklist.reserve((size_t)3 * nq * 4));
-  }
-  uint32_t* lists = worklist.as<uint32_t>();
-  MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_warp, 0, 3 * sizeof(unsigned int), st));
-  MTSV_LAUNCH(sort_classify_kernel, (nq + 255) / 256, 256, 0, st, seg_cnt, nq, min_count, lists, lists + nq,
-              lists + 2 * (size_t)nq, d_ctr);
-  MTSV_LAUNCH(sort_warp_kernel, sm_count() * 8, 256, 0, st, keys, seg_off, seg_cnt, lists, d_ctr);
-  MTSV_LAUNCH(sort_medium_kernel, sm_count() * 4, 512, 0, st, keys, seg_off, seg_cnt, lists + nq, d_ctr);
-  MTSV_LAUNCH(sort_large_kernel, sm_count(), 1024, 0, st, keys, seg_off, seg_cnt, lists + 2 * (size_t)nq, d_ctr);
-  MTSV_CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
 // grow-with-preserve for the whole-batch output
 static int grow_preserve(DevBuf& buf, size_t used_bytes, size_t need_bytes, cudaStream_t st) {
   if (need_bytes <= buf.cap && buf.p) return 0;
@@ -1576,30 +1404,54 @@ static int fetch_counters(Lane& ln, const BatchCounters* d_ctr, BatchCounters* o
   return 0;
 }
 
-// ---- ordered output: slices append to the batch result in slice order ----
-static int emit_acquire(mtsvgpu_index* h, Lane& ln) {
-  if (ln.has_turn) return 0;
-  std::unique_lock<std::mutex> lk(h->emit_mu);
-  h->emit_cv.wait(lk, [&] { return h->abort_rc != 0 || h->emit_turn == ln.slice; });
-  if (h->abort_rc != 0) return set_error(h->abort_rc, "%s", h->abort_msg.c_str());
-  ln.has_turn = true;
-  return 0;
-}
-static void emit_release(mtsvgpu_index* h, Lane& ln) {  // the slice is complete
-  std::lock_guard<std::mutex> lk(h->emit_mu);
-  if (ln.has_turn) h->emit_turn = ln.slice + 1;
-  ln.has_turn = false;
-  h->emit_cv.notify_all();
-}
+// ---- the state of one bin_batch_device call ----
+struct LaneRun {  // what one lane does in the call
+  uint64_t slice = 0;                 // index of the slice being processed
+  bool has_turn = false;              // holds the output turnstile for that slice
+  uint64_t chunk_reads = UINT64_MAX;  // reads per launch group (a whole slice); halves when a group overflows the seed-hit cap
+  mtsvgpu_batch_stats stats{};
+  std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> ev_used;  // per-stage timing: (stage, event pair)
+  size_t ev_next = 0;                                                        // next unused event of the lane's pool
+};
+
 const char* last_error_cstr();
-static void emit_abort(mtsvgpu_index* h, int rc) {
-  std::lock_guard<std::mutex> lk(h->emit_mu);
-  if (h->abort_rc == 0) {
-    h->abort_rc = rc;
-    h->abort_msg = last_error_cstr();
+// Ordered output: slices append to the batch result in slice order, a turnstile over the slice index.  The first
+// failure aborts the call; a lane waiting for its turn then returns that error.
+struct BatchRun {
+  std::mutex mu;
+  std::condition_variable cv;
+  uint64_t turn = 0;
+  int abort_rc = 0;
+  std::string abort_msg;
+  LaneRun lanes[2];
+
+  int emit_acquire(LaneRun& lr) {
+    if (lr.has_turn) return 0;
+    std::unique_lock<std::mutex> lk(mu);
+    cv.wait(lk, [&] { return abort_rc != 0 || turn == lr.slice; });
+    if (abort_rc != 0) return set_error(abort_rc, "%s", abort_msg.c_str());
+    lr.has_turn = true;
+    return 0;
   }
-  h->emit_cv.notify_all();
-}
+  void emit_release(LaneRun& lr) {  // the slice is complete
+    std::lock_guard<std::mutex> lk(mu);
+    if (lr.has_turn) turn = lr.slice + 1;
+    lr.has_turn = false;
+    cv.notify_all();
+  }
+  void emit_abort(int rc) {
+    std::lock_guard<std::mutex> lk(mu);
+    if (abort_rc == 0) {
+      abort_rc = rc;
+      abort_msg = last_error_cstr();
+    }
+    cv.notify_all();
+  }
+  bool aborted() {
+    std::lock_guard<std::mutex> lk(mu);
+    return abort_rc != 0;
+  }
+};
 
 // What stays fixed over one bin_batch_device call
 struct BatchCall {
@@ -1615,7 +1467,9 @@ struct BatchCall {
 // One device sub-batch, reads [rv.read0, rv.read0 + rv.n_reads), as it passes through the stages below.  A stage
 // reserves the workspace buffers it is the first to use; 1 from a stage: too large, the caller splits the range.
 struct SubBatch : BatchCall {
+  BatchRun& run;
   Lane& ln;
+  LaneRun& lr;  // the lane's state in this call
   BatchWorkspace& ws;  // scratch of the lane
   cudaStream_t st;
   ReadsView rv;
@@ -1629,40 +1483,40 @@ struct SubBatch : BatchCall {
   uint32_t n_slots = 0, n_hits = 0, n_cand = 0;
   uint64_t n_verified = 0;
 
-  SubBatch(const BatchCall& c, Lane& l, uint64_t read0, uint32_t n_reads)
-      : BatchCall(c), ln(l), ws(*l.ws), st(l.stream),
+  SubBatch(const BatchCall& c, BatchRun& r, int li, uint64_t read0, uint32_t n_reads)
+      : BatchCall(c), run(r), ln(c.h->lanes[li]), lr(r.lanes[li]), ws(*ln.ws), st(ln.stream),
         rv{c.d_seqs, c.d_seq_off, read0, n_reads}, nq(n_reads * c.p.ns), qn((size_t)nq + 1) {}
   unsigned qgrid() const { return (nq + 255) / 256; }
   int fetch() { return fetch_counters(ln, d_ctr, &hc, st); }
   // per-stage timing (profiling only)
   cudaEvent_t next_event() {
-    if (ln.ev_next == ln.ev_pool.size()) {
+    if (lr.ev_next == ln.ev_pool.size()) {
       cudaEvent_t e;
       cudaEventCreate(&e);
       ln.ev_pool.push_back(e);
     }
-    return ln.ev_pool[ln.ev_next++];
+    return ln.ev_pool[lr.ev_next++];
   }
   void begin(int stage) {
     if (!h->profiling) return;
     cudaEvent_t a = next_event(), b = next_event();
     cudaEventRecord(a, ln.stream);
-    ln.ev_used.push_back({stage, {a, b}});
+    lr.ev_used.push_back({stage, {a, b}});
   }
   void end() {
     if (!h->profiling) return;
-    cudaEventRecord(ln.ev_used.back().second.second, ln.stream);
+    cudaEventRecord(lr.ev_used.back().second.second, ln.stream);
   }
   void resolve() {
     if (!h->profiling) return;
     cudaStreamSynchronize(ln.stream);
-    for (auto& e : ln.ev_used) {
+    for (auto& e : lr.ev_used) {
       float ms = 0;
       cudaEventElapsedTime(&ms, e.second.first, e.second.second);
-      ln.stats.ms[e.first] += ms;
+      lr.stats.ms[e.first] += ms;
     }
-    ln.ev_used.clear();
-    ln.ev_next = 0;
+    lr.ev_used.clear();
+    lr.ev_next = 0;
   }
 
   int slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pack_base);
@@ -1706,7 +1560,7 @@ int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pac
   end();
   MTSV_TRY(fetch());
   if (hc.bad_offsets) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
-  ln.stats.n_reads_over_limit += hc.n_over_len;
+  lr.stats.n_reads_over_limit += hc.n_over_len;
   if (hc.total_slots > slot_bound)
     return set_error(MTSVGPU_ECUDA, "internal: seed slots %llu exceed bound %llu (reads [%llu,+%u), %llu bytes)",
                      hc.total_slots, (unsigned long long)slot_bound, (unsigned long long)rv.read0, n_reads,
@@ -1715,7 +1569,7 @@ int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pac
   // min_len == max_len: every read of the sub-batch has the same length (never when a read was left out)
   const uint32_t min_len = hc.n_over_len ? 0u : ~hc.inv_min_len;
   uniform = min_len == hc.max_len;
-  ln.stats.n_seed_slots += n_slots;
+  lr.stats.n_seed_slots += n_slots;
   // (only now that the slot count is known to fit the buffers)
   begin(ST_PREP);
   // all reads of one length: slots are addressed arithmetically, no slot -> query map needed
@@ -1762,7 +1616,7 @@ int SubBatch::search() {
                               (uint64_t*)&d_ctr->total_hits, st));
   end();
   MTSV_TRY(fetch());
-  ln.stats.n_strands_over_hits += hc.overflow;
+  lr.stats.n_strands_over_hits += hc.overflow;
   const uint64_t hit_cap = h->opts.max_batch_hits ? h->opts.max_batch_hits : (1ull << 27);
   if (hc.total_hits > hit_cap || hc.total_hits > 0xfffffff0ull) {
     if (rv.n_reads == 1)
@@ -1771,8 +1625,8 @@ int SubBatch::search() {
     return 1;
   }
   n_hits = (uint32_t)hc.total_hits;
-  ln.stats.n_seed_hits += n_hits;
-  for (int i = 0; i < 32; ++i) ln.stats.rank_queries += hc.rank_steps[i];  // sectors touched by seed search
+  lr.stats.n_seed_hits += n_hits;
+  for (int i = 0; i < 32; ++i) lr.stats.rank_queries += hc.rank_steps[i];  // sectors touched by seed search
   return 0;
 }
 
@@ -1781,7 +1635,8 @@ int SubBatch::candidates() {
   const DeviceIndex& ix = h->ix;
   for (DevBuf* b : {&ws.q_ncand, &ws.cand_off}) MTSV_TRY(b->reserve(qn * 4));
   if (!n_hits) return 0;
-  MTSV_TRY(ws.worklist.reserve(3 * qn * 4));
+  MTSV_TRY(ws.worklist.reserve((size_t)2 * nq * 4));
+  MTSV_TRY(ws.sort.reserve(nq));
   MTSV_TRY(ws.hit_keys.reserve((size_t)n_hits * 8));
   MTSV_TRY(ws.cand_sparse.reserve((size_t)n_hits * sizeof(CandRec)));
   begin(ST_LOCATE);
@@ -1790,8 +1645,8 @@ int SubBatch::candidates() {
               ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.hit_keys.as<uint64_t>());
   end();
   begin(ST_SORT);
-  MTSV_TRY(run_segmented_sort(st, ws.worklist, ws.hit_keys.as<uint64_t>(), ws.hit_off.as<uint32_t>(),
-                              ws.q_nhits.as<uint32_t>(), nq, kLightItems, d_ctr));
+  MTSV_TRY(run_segmented_sort(st, ws.sort, ws.hit_keys.as<uint64_t>(), ws.hit_off.as<uint32_t>(),
+                              ws.q_nhits.as<uint32_t>(), nq, kLightItems));
   end();
   begin(ST_COALESCE);
   MTSV_TRY(ws.cand_stage.reserve((size_t)n_hits * sizeof(CandRec)));
@@ -1942,8 +1797,8 @@ int SubBatch::merge_taxids() {
   uint64_t* keys = ws.hit_keys.as<uint64_t>();
   MTSV_LAUNCH(taxid_keys_kernel, (nq + 1 + 255) / 256, 256, 0, st, nq, p.ns, ws.cand_off.as<uint32_t>(),
               ws.out_off.as<uint32_t>(), ws.hit_tmp.as<HitRec>(), keys, seg_off(), seg_cnt());
-  return taxid_merge_count(st, ws.worklist, ws.scan_tmp, keys, seg_off(), seg_cnt(), nr, n_cand, d_ctr, tax_cnt(),
-                           tax_off(), (uint64_t*)&d_ctr->total_taxhits);
+  return taxid_merge_count(st, ws.sort, ws.scan_tmp, keys, seg_off(), seg_cnt(), nr, n_cand, tax_cnt(), tax_off(),
+                           (uint64_t*)&d_ctr->total_taxhits);
 }
 
 // ---- select, then append to the batch output: in slice order, after the other lane's previous append ----
@@ -1964,8 +1819,8 @@ int SubBatch::select_append(uint64_t* out_total) {
     MTSV_TRY(fetch());
     sub_out = hc.total_out;
     sub_tax = hc.total_taxhits;
-    ln.stats.n_candidates += n_verified;
-    for (int i = 0; i < 32; ++i) ln.stats.window_bytes += hc.window_bytes[i];
+    lr.stats.n_candidates += n_verified;
+    for (int i = 0; i < 32; ++i) lr.stats.window_bytes += hc.window_bytes[i];
   } else if (taxhits) {  // no keys: every read gets an empty range
     MTSV_CUDA_TRY(cudaMemsetAsync(seg_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
     MTSV_CUDA_TRY(cudaMemsetAsync(tax_off(), 0, ((size_t)rv.n_reads + 1) * 4, st));
@@ -1973,7 +1828,7 @@ int SubBatch::select_append(uint64_t* out_total) {
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.out_off.p.get(), 0, qn * 4, st));
     MTSV_CUDA_TRY(cudaMemsetAsync(ws.cand_off.p.get(), 0, qn * 4, st));
   }
-  MTSV_TRY(emit_acquire(h, ln));
+  MTSV_TRY(run.emit_acquire(lr));
   Lane& other = h->lanes[&ln == &h->lanes[0] ? 1 : 0];
   if (other.emit_event) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, other.emit_event, 0));
   BatchWorkspace& res = h->ws;  // batch results (shared, appended in slice order)
@@ -1997,16 +1852,16 @@ int SubBatch::select_append(uint64_t* out_total) {
   if (src) MTSV_TRY(src->results(*out_total, sub_rec, rv.read0, rv.n_reads, st));
   resolve();
   *out_total += sub_rec;
-  ln.stats.n_hits += sub_out;
-  ln.stats.n_queries += nq;
+  lr.stats.n_hits += sub_out;
+  lr.stats.n_queries += nq;
   return 0;
 }
 
 // One device sub-batch: reads [read0, read0 + n_reads).  Returns 1 when it exceeds the in-flight limits and the
 // caller must split the range (nothing was emitted in that case).
-static int run_sub_batch(const BatchCall& call, Lane& ln, uint64_t read0, uint32_t n_reads, uint64_t slot_bound,
-                         uint64_t sub_bytes, uint64_t pack_base, uint64_t* out_total) {
-  SubBatch s(call, ln, read0, n_reads);
+static int run_sub_batch(const BatchCall& call, BatchRun& run, int li, uint64_t read0, uint32_t n_reads,
+                         uint64_t slot_bound, uint64_t sub_bytes, uint64_t pack_base, uint64_t* out_total) {
+  SubBatch s(call, run, li, read0, n_reads);
   int rc = s.slots_encode(slot_bound, sub_bytes, pack_base);
   if (rc == 0) rc = s.search();
   if (rc != 0) return rc;
@@ -2015,21 +1870,23 @@ static int run_sub_batch(const BatchCall& call, Lane& ln, uint64_t read0, uint32
   return s.select_append(out_total);
 }
 
-// One uploaded slice [read0, read0 + n_reads): processed in groups of ln.chunk_reads reads.  A group whose seed
+// One uploaded slice [read0, read0 + n_reads): processed in groups of lr.chunk_reads reads.  A group whose seed
 // hits overflow the in-flight cap (run_sub_batch returns 1, nothing emitted) is retried at half the size, and
 // the smaller size is kept for what follows (repetitive references: hundreds of hits per read).
-static int run_range(const BatchCall& call, Lane& ln, uint64_t read0, uint64_t n_reads, uint64_t off_lo,
+static int run_range(const BatchCall& call, BatchRun& run, int li, uint64_t read0, uint64_t n_reads, uint64_t off_lo,
                      uint64_t off_hi, uint64_t* out_total) {
   if (off_hi < off_lo) return set_error(MTSVGPU_EINVAL, "seq_off is not monotone");
   const Params& p = call.p;
+  const Lane& ln = call.h->lanes[li];
+  LaneRun& lr = run.lanes[li];
   const uint64_t* h_off = call.src ? call.src->seq_off : nullptr;  // host copy of seq_off
   uint64_t r = read0, off_r = off_lo;
   // packed input: byte offset of the record of read r (the slice's first record was placed by the uploader)
   const bool packed = call.src && !call.src->pack_base.empty();
-  uint64_t pack_r = packed ? call.src->pack_base[ln.slice] : 0;
+  uint64_t pack_r = packed ? call.src->pack_base[lr.slice] : 0;
   const uint64_t r_end = read0 + n_reads;
   while (r < r_end) {
-    uint64_t nr = std::min(r_end - r, std::max<uint64_t>(ln.chunk_reads, 1));
+    uint64_t nr = std::min(r_end - r, std::max<uint64_t>(lr.chunk_reads, 1));
     uint64_t off_e = off_hi;
     if (r + nr < r_end && h_off) {
       off_e = h_off[r + nr];
@@ -2042,14 +1899,14 @@ static int run_range(const BatchCall& call, Lane& ln, uint64_t read0, uint64_t n
     const uint64_t bytes = off_e - off_r;
     const uint64_t slot_bound = (bytes / p.G + nr) * p.ns + 1;
     const bool too_big = slot_bound > 0xfffffff0ull || nr * p.ns > 0x7ffffff0ull;
-    int rc = too_big ? 1 : run_sub_batch(call, ln, r, (uint32_t)nr, slot_bound, bytes, pack_r, out_total);
+    int rc = too_big ? 1 : run_sub_batch(call, run, li, r, (uint32_t)nr, slot_bound, bytes, pack_r, out_total);
     if (rc == 1) {
       if (nr == 1) return set_error(MTSVGPU_ELIMIT, "a single read exceeds the device batch limits");
-      ln.chunk_reads = std::max<uint64_t>(1, nr / 2);
+      lr.chunk_reads = std::max<uint64_t>(1, nr / 2);
       continue;
     }
     if (rc != 0) return rc;
-    ln.stats.n_sub_batches += 1;
+    lr.stats.n_sub_batches += 1;
     if (packed && r + nr < r_end)  // (only after a split: a slice is normally one group)
       for (uint64_t i = r; i < r + nr; ++i) pack_r += packed_record_bytes((uint32_t)(h_off[i + 1] - h_off[i]));
     r += nr;
@@ -2114,8 +1971,6 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   }
   const int n_lanes = n_sub >= 2 && two_lanes ? 2 : 1;
   h->lanes[0].stream = st;
-  h->lanes[0].ws = &h->ws;
-  h->lanes[1].ws = &h->ws1;
   if (n_lanes == 2) {
     if (!h->lane1_stream) MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->lane1_stream, cudaStreamNonBlocking));
     if (!h->fork_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&h->fork_event, cudaEventDisableTiming));
@@ -2125,32 +1980,22 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
     MTSV_CUDA_TRY(cudaEventRecord(h->fork_event, st));
     MTSV_CUDA_TRY(cudaStreamWaitEvent(h->lane1_stream, h->fork_event, 0));
   }
-  h->emit_turn = 0;
-  h->abort_rc = 0;
-  h->abort_msg.clear();
-  for (Lane& ln : h->lanes) {
-    ln.has_turn = false;
-    ln.chunk_reads = UINT64_MAX;  // a whole slice
-    memset(&ln.stats, 0, sizeof ln.stats);
-  }
+  BatchRun run;
   const int device = h->ix.device;
   auto lane_main = [&](int li) {
-    Lane& ln = h->lanes[li];
+    LaneRun& lr = run.lanes[li];
     if (li != 0) cudaSetDevice(device);
     for (uint64_t i = (uint64_t)li; i < n_sub; i += (uint64_t)n_lanes) {
-      {
-        std::lock_guard<std::mutex> lk(h->emit_mu);
-        if (h->abort_rc != 0) return;
-      }
-      ln.slice = i;
+      if (run.aborted()) return;
+      lr.slice = i;
       int rc = 0;
-      if (src) rc = src->wait_slice(i, ln.stream);
-      if (rc == 0) rc = run_range(call, ln, rb[i], rb[i + 1] - rb[i], bounds[i], bounds[i + 1], &total);
+      if (src) rc = src->wait_slice(i, h->lanes[li].stream);
+      if (rc == 0) rc = run_range(call, run, li, rb[i], rb[i + 1] - rb[i], bounds[i], bounds[i + 1], &total);
       if (rc != 0) {
-        emit_abort(h, rc);
+        run.emit_abort(rc);
         return;
       }
-      emit_release(h, ln);
+      run.emit_release(lr);
     }
   };
   if (n_lanes == 2) {
@@ -2163,11 +2008,11 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   } else {
     lane_main(0);
   }
-  for (Lane& ln : h->lanes) add_stats(h->stats, ln.stats);
-  if (h->abort_rc != 0) {
+  for (const LaneRun& lr : run.lanes) add_stats(h->stats, lr.stats);
+  if (run.abort_rc != 0) {
     cudaStreamSynchronize(st);
     if (h->lane1_stream) cudaStreamSynchronize(h->lane1_stream);
-    return set_error(h->abort_rc, "%s", h->abort_msg.c_str());
+    return set_error(run.abort_rc, "%s", run.abort_msg.c_str());
   }
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   if (d_out) *d_out = ws.out_hits.p.get();

@@ -112,22 +112,6 @@ static int ensure_pinned(PinnedPtr<uint8_t>& p, size_t& cap, size_t bytes) {
   return 0;
 }
 
-// MTSV_B200_TRACE=1: per-slice timeline of the host API (when each slice landed, when its compute started)
-static std::vector<cudaEvent_t> g_trace_landed, g_trace_started;
-static cudaEvent_t g_trace_t0 = nullptr;
-static bool trace_on() {
-  static const bool t = getenv("MTSV_B200_TRACE") != nullptr;
-  return t;
-}
-static cudaEvent_t trace_event(std::vector<cudaEvent_t>& pool, size_t i) {
-  while (pool.size() <= i) {
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    pool.push_back(e);
-  }
-  return pool[i];
-}
-
 // Per-call state of bin_batch_host, shared by the uploader thread and the compute lanes
 struct HostUpload : BatchSource {
   mtsvgpu_index* ix;
@@ -137,8 +121,12 @@ struct HostUpload : BatchSource {
   uint64_t out_copied_hits = 0, out_copied_reads = 0;  // prefix already on its way to the pinned buffers
   bool out_overlap_ok = false;
   size_t rec_bytes;  // result records: mtsvgpu_hit or mtsvgpu_taxhit
+  // MTSV_B200_TRACE: per-slice timeline (when each slice landed, when its compute started), from the handle's pool
+  cudaEvent_t trace_t0 = nullptr;
+  const cudaEvent_t* trace_landed = nullptr;
+  const cudaEvent_t* trace_started = nullptr;
   HostUpload(mtsvgpu_index* h, size_t rec) : ix(h), rec_bytes(rec) {}
-  int upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool trace, uint64_t* h2d_bytes);
+  int upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, uint64_t* h2d_bytes);
   int wait_slice(uint64_t i, cudaStream_t st) override;
   int results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read, uint64_t n_reads, cudaStream_t st) override;
 };
@@ -150,7 +138,7 @@ int HostUpload::wait_slice(uint64_t i, cudaStream_t st) {
     std::this_thread::yield();
   }
   if (i < ix->in_events.size()) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, ix->in_events[i], 0));
-  if (trace_on()) cudaEventRecord(g_trace_started[i], st);  // (pre-created by the caller: two lanes call this)
+  if (trace_started) MTSV_CUDA_TRY(cudaEventRecord(trace_started[i], st));
   return 0;
 }
 
@@ -195,7 +183,7 @@ static bool uniform_lengths(const uint64_t* o, uint64_t n_reads) {  // o[0 .. n_
 
 // The uploader: enqueues the slices one after the other on the copy-in stream (runs on its own host thread so
 // that checking a slice's lengths does not hold up the compute lanes; it stays far ahead of the DMA engine).
-int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool trace, uint64_t* h2d_bytes) {
+int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, uint64_t* h2d_bytes) {
   MTSV_CUDA_TRY(cudaSetDevice(ix->ix.device));
   BatchWorkspace& ws = ix->ws;
   cudaStream_t cin = ix->copy_in_stream;
@@ -241,7 +229,7 @@ int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, bool 
       MTSV_CUDA_TRY(cudaMemcpyAsync(ws.d_seqs.as<uint8_t>() + c0, seqs + base + c0, cn, cudaMemcpyHostToDevice, cin));
     *h2d_bytes += cn;
     MTSV_CUDA_TRY(cudaEventRecord(ix->in_events[i], cin));
-    if (trace) cudaEventRecord(g_trace_landed[i], cin);
+    if (trace_landed) MTSV_CUDA_TRY(cudaEventRecord(trace_landed[i], cin));
     slices_enqueued.store(i + 1, std::memory_order_release);
   }
   return 0;
@@ -289,16 +277,21 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
     ix->in_events.push_back(e);
   }
   if (trace) {
-    if (!g_trace_t0) cudaEventCreate(&g_trace_t0);
-    cudaEventRecord(g_trace_t0, cin);
-    if (n_sub) trace_event(g_trace_started, n_sub - 1);
+    while (ix->trace_events.size() < 2 * n_sub + 1) {
+      cudaEvent_t e;
+      MTSV_CUDA_TRY(cudaEventCreate(&e));
+      ix->trace_events.push_back(e);
+    }
+    up.trace_t0 = ix->trace_events[0];
+    up.trace_landed = ix->trace_events.data() + 1;
+    up.trace_started = ix->trace_events.data() + 1 + n_sub;
+    MTSV_CUDA_TRY(cudaEventRecord(up.trace_t0, cin));
   }
-  if (trace && n_sub) trace_event(g_trace_landed, n_sub - 1);
   uint64_t h2d_bytes = 0;
   std::thread uploader;
   if (n_sub) {
     uploader = std::thread([&] {
-      int urc = up.upload(seqs, packed ? 0 : base, bytes, trace, &h2d_bytes);
+      int urc = up.upload(seqs, packed ? 0 : base, bytes, &h2d_bytes);
       if (urc != 0) {
         up.upload_msg = last_error_cstr();
         up.upload_rc.store(urc, std::memory_order_release);
@@ -367,20 +360,22 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   *hit_off = h_off;
   if (n_hits_out) *n_hits_out = n_hits;
   if (trace) {
-    cudaDeviceSynchronize();
-    fprintf(stderr, "[mtsv_b200 trace] slice: reads, landed at ms, compute started at ms\n");
-    for (uint64_t i = 0; i < n_sub && i < g_trace_started.size(); ++i) {
+    // one write per call, so that the tables of calls on other threads do not interleave with it
+    std::string out = "[mtsv_b200 trace] slice: reads, landed at ms, compute started at ms\n";
+    char line[256];
+    for (uint64_t i = 0; i < n_sub; ++i) {
       float a = 0, b = 0;
-      cudaEventElapsedTime(&a, g_trace_t0, g_trace_landed[i]);
-      cudaEventElapsedTime(&b, g_trace_t0, g_trace_started[i]);
-      fprintf(stderr, "[mtsv_b200 trace]   %2llu: %8llu  %7.2f  %7.2f\n", (unsigned long long)i,
-              (unsigned long long)(up.bounds[i + 1] - up.bounds[i]), a, b);
+      cudaEventElapsedTime(&a, up.trace_t0, up.trace_landed[i]);  // (every slice's events have completed)
+      cudaEventElapsedTime(&b, up.trace_t0, up.trace_started[i]);
+      snprintf(line, sizeof line, "[mtsv_b200 trace]   %2llu: %8llu  %7.2f  %7.2f\n", (unsigned long long)i,
+               (unsigned long long)(up.bounds[i + 1] - up.bounds[i]), a, b);
+      out += line;
     }
+    snprintf(line, sizeof line, "[mtsv_b200 trace] bin_batch_host: enqueue H2D %.2f ms, compute %.2f ms, tail (D2H "
+             "rest) %.2f ms, overlapped D2H %s\n", t_enq - t_begin, t_comp - t_enq, now() - t_comp,
+             up.out_overlap_ok ? "yes" : "no");
+    fputs((out + line).c_str(), stderr);
   }
-  if (trace)
-    fprintf(stderr, "[mtsv_b200 trace] bin_batch_host: enqueue H2D %.2f ms, compute %.2f ms, tail (D2H rest) %.2f ms, "
-                    "overlapped D2H %s\n", t_enq - t_begin, t_comp - t_enq, now() - t_comp,
-            up.out_overlap_ok ? "yes" : "no");
   return 0;
 }
 

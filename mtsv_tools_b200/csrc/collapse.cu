@@ -9,7 +9,7 @@
 // keep the minimum edit per TaxID (:597-602), hits listed by ascending TaxID (write_collapsed_taxid, :278-279); mode
 // TaxIdGi further down.  Inputs: n_parts device arrays of mtsvgpu_hit, each with a per-read u32 count array for the
 // same n_reads reads (after the chunk exchange every rank holds all parts for its own range of reads).
-// All kernels are flat over reads / hits; the per-read sort reuses the binner's segmented sorts.
+// All kernels are flat over reads / hits; the per-read sort is segsort.cu's.
 #include <mutex>
 
 #include "ctx.h"
@@ -38,11 +38,11 @@ __global__ void __launch_bounds__(256) taxid_write_kernel(const uint64_t* __rest
   taxid_write(keys, seg_off[r], seg_off[r + 1], out + out_base, tax_off[r]);
 }
 
-int taxid_merge_count(cudaStream_t st, DevBuf& worklist, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
-                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, BatchCounters* d_ctr,
-                      uint32_t* tax_cnt, uint32_t* tax_off, uint64_t* d_total) {
+int taxid_merge_count(cudaStream_t st, SegSortScratch& sort, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
+                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, uint32_t* tax_cnt,
+                      uint32_t* tax_off, uint64_t* d_total) {
   if (n_reads) {
-    if (key_bound) MTSV_TRY(run_segmented_sort(st, worklist, keys, seg_off, seg_cnt, n_reads, 1, d_ctr));
+    if (key_bound) MTSV_TRY(run_segmented_sort(st, sort, keys, seg_off, seg_cnt, n_reads, 1));
     MTSV_LAUNCH(taxid_count_kernel, (n_reads + 255) / 256, 256, 0, st, keys, seg_off, n_reads, tax_cnt);
   }
   return exclusive_scan_u32(tax_cnt, tax_off, n_reads, scan_tmp, d_total, st);
@@ -163,9 +163,8 @@ static int prepare_parts(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, 
                          const uint32_t* const* d_counts, uint32_t nr, PartsView* pv, uint64_t** d_tot) {
   *pv = PartsView{};
   pv->n_parts = n_parts;
-  MTSV_TRY(w.counters.reserve(sizeof(BatchCounters) + 16));
-  MTSV_CUDA_TRY(cudaMemsetAsync(w.counters.p.get(), 0, sizeof(BatchCounters) + 16, st));
-  *d_tot = reinterpret_cast<uint64_t*>(w.counters.as<uint8_t>() + sizeof(BatchCounters));
+  MTSV_TRY(w.comb_total.reserve(8));
+  *d_tot = w.comb_total.as<uint64_t>();
   for (uint32_t p = 0; p < n_parts; ++p) {
     pv->hits[p] = d_hits[p];
     pv->counts[p] = d_counts[p];
@@ -188,9 +187,9 @@ static int merge_parts_count(CollapseScratch& w, cudaStream_t st, const PartsVie
     MTSV_LAUNCH(collapse_scatter_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, pv, nr,
                 w.comb_off.as<uint32_t>(), w.keys.as<uint64_t>());
   }
-  return taxid_merge_count(st, w.worklist, w.scan_tmp, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(),
-                           w.total.as<uint32_t>(), nr, hit_cap, w.counters.as<BatchCounters>(), w.cnt_out.as<uint32_t>(),
-                           w.off_out32.as<uint32_t>(), d_n_out);
+  return taxid_merge_count(st, w.sort, w.scan_tmp, w.keys.as<uint64_t>(), w.comb_off.as<uint32_t>(),
+                           w.total.as<uint32_t>(), nr, hit_cap, w.cnt_out.as<uint32_t>(), w.off_out32.as<uint32_t>(),
+                           d_n_out);
 }
 
 int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
@@ -243,7 +242,7 @@ int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, 
   if (hit_cap > 0xfffffff0ull) return set_error(MTSVGPU_ELIMIT, "more than 2^32 hits in one collapse call");
   // (the scans and the sort synchronise the stream when they have to grow these)
   MTSV_TRY(w.scan_tmp.reserve((((size_t)nr + 1 + 2047) / 2048 + 1) * 8));
-  MTSV_TRY(w.worklist.reserve((size_t)3 * (nr + 1) * 4));
+  MTSV_TRY(w.sort.reserve(nr + 1));
   PartsView pv;
   uint64_t* d_tot = nullptr;
   MTSV_TRY(prepare_parts(w, st, n_parts, d_hits, d_counts, nr, &pv, &d_tot));

@@ -7,9 +7,7 @@
 
 #include <algorithm>
 #include <atomic>
-#include <condition_variable>
 #include <memory>
-#include <mutex>
 #include <string>
 #include <vector>
 
@@ -92,9 +90,20 @@ struct DevBuf {
   }
 };
 
+// segsort.cu
+// Sorts keys[seg_off[q] .. + seg_cnt[q]) ascending for each segment q < nq with more than min_count keys.  The sort
+// reserves its scratch, synchronising the stream first when it has to grow; reserve it in advance to avoid that.
+struct SegSortScratch {
+  DevBuf lists;   // three work lists of nq segments: one warp, one CTA in shared memory, one CTA in global memory
+  DevBuf counts;  // their lengths
+  int reserve(uint32_t nq);
+};
+int run_segmented_sort(cudaStream_t st, SegSortScratch& s, uint64_t* keys, const uint32_t* seg_off,
+                       const uint32_t* seg_cnt, uint32_t nq, uint32_t min_count);
+
 struct BatchCounters {  // device-side scalars of one sub-batch
   unsigned long long total_slots, total_hits, total_cands, total_out;
-  unsigned int max_len, overflow, n_warp, n_medium, n_large, bad_offsets, n_heavy, heavy_cursor, n_monster;
+  unsigned int max_len, overflow, bad_offsets, n_heavy, heavy_cursor, n_monster;
   unsigned int inv_min_len;  // ~(shortest read) so that a zeroed struct means "no read seen"
   unsigned int n_ssw_full, n_over_len;  // candidates of reads >= 254 bases that needed the full SW matrices; reads over the length limit
   unsigned long long verified[2];  // two-round verification: candidates verified in round 1 / round 2
@@ -179,8 +188,9 @@ struct BatchWorkspace {
   DevBuf cand_lead, cand_order2;  // two-round verification: leader of each candidate, compacted visiting order
   // bit-plane encoded reads of the sub-batch
   DevBuf enc;
-  // scan scratch, counters, worklists
+  // scan scratch, counters, coalesce's heavy and monster lists, the segmented sort's scratch
   DevBuf scan_tmp, counters, worklist;
+  SegSortScratch sort;
   // whole-batch results (device-resident API): mtsvgpu_hit or mtsvgpu_taxhit records
   DevBuf out_hits, out_hit_off;
   // staged inputs for the host API
@@ -196,14 +206,7 @@ struct Lane {
   PinnedPtr<BatchCounters> h_ctr;    // mapped: sub-batch scalars published by the device
   BatchCounters* h_ctr_dev = nullptr;
   cudaEvent_t emit_event = nullptr;  // recorded after each append to the batch output
-  bool has_turn = false;             // holds the output turnstile for its current slice
-  uint64_t slice = 0;                // index of the slice being processed
-  uint64_t chunk_reads = 0;          // reads per launch group; halves when a group overflows the seed-hit cap
-  mtsvgpu_batch_stats stats{};
-  // event pool for profiling
-  std::vector<cudaEvent_t> ev_pool;
-  std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> ev_used;
-  size_t ev_next = 0;
+  std::vector<cudaEvent_t> ev_pool;  // per-stage timing (profiling)
 };
 
 // What a batch call returns, CSR by read: the Hit records of every strand (mtsvgpu_hit), or per read each TaxID once
@@ -236,18 +239,13 @@ struct mtsvgpu_index {
   mtsv::Lane lanes[2];
   cudaStream_t lane1_stream = nullptr;
   cudaEvent_t fork_event = nullptr, join_event = nullptr;
-  // slices append to the batch output in order: a turnstile over the slice index
-  std::mutex emit_mu;
-  std::condition_variable emit_cv;
-  uint64_t emit_turn = 0;
-  int abort_rc = 0;
-  std::string abort_msg;
-  mtsvgpu_batch_stats stats{};
+  mtsvgpu_batch_stats stats{};  // of the last batch call
   // host API: copy streams, per-sub-batch "input landed" events, pinned result buffers
   cudaStream_t copy_in_stream = nullptr;
   std::vector<cudaEvent_t> in_events;
   cudaStream_t copy_out_stream = nullptr;
   cudaEvent_t out_event = nullptr;
+  std::vector<cudaEvent_t> trace_events;  // MTSV_B200_TRACE: the slice timeline
   mtsv::PinnedPtr<uint8_t> pin_hits;
   size_t pin_hits_cap = 0;
   mtsv::PinnedPtr<uint8_t> pin_off;
@@ -295,17 +293,15 @@ int locate_batch(mtsvgpu_index* h, const uint64_t* rows, uint64_t n_rows, uint64
 int edit_distance_batch(int device, const uint8_t* pats, const uint64_t* pat_off,
                         const uint8_t* texts, const uint64_t* text_off, uint64_t n_pairs,
                         uint32_t* edits);
-int run_segmented_sort(cudaStream_t st, DevBuf& worklist, uint64_t* keys, const uint32_t* seg_off,
-                       const uint32_t* seg_cnt, uint32_t nq, uint32_t min_count, BatchCounters* d_ctr);
 // collapse.cu
 // The (TaxID, edit) merge of keys tax << 32 | edit, read r's keys at [seg_off[r], seg_off[r] + seg_cnt[r])
 // (seg_off[n_reads] = the end).  taxid_merge_count sorts each segment (none when key_bound, a bound on the keys, is
 // 0), counts its records into tax_cnt and scans them into tax_off; the record total goes to *d_total.
 // taxid_merge_write then writes read r's records to out[out_base + tax_off[r]] on and out_off[read_base + r] =
 // out_base + tax_off[r] for r = 0 .. n_reads.
-int taxid_merge_count(cudaStream_t st, DevBuf& worklist, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
-                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, BatchCounters* d_ctr,
-                      uint32_t* tax_cnt, uint32_t* tax_off, uint64_t* d_total);
+int taxid_merge_count(cudaStream_t st, SegSortScratch& sort, DevBuf& scan_tmp, uint64_t* keys, const uint32_t* seg_off,
+                      const uint32_t* seg_cnt, uint32_t n_reads, uint64_t key_bound, uint32_t* tax_cnt,
+                      uint32_t* tax_off, uint64_t* d_total);
 void taxid_merge_write(cudaStream_t st, const uint64_t* keys, const uint32_t* seg_off, const uint32_t* tax_off,
                        uint32_t n_reads, mtsvgpu_taxhit* out, uint64_t out_base, uint64_t* out_off, uint64_t read_base);
 int collapse_device(int device, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
@@ -315,7 +311,8 @@ int collapse_device_long(int device, cudaStream_t st, uint32_t n_parts, const mt
                          const uint32_t* const* d_counts, uint64_t n_reads, mtsvgpu_hit** d_out,
                          uint64_t** d_out_off, uint64_t* n_out);
 struct CollapseScratch {
-  DevBuf offs[16], total, comb_off, keys, scan_tmp, counters, worklist, cnt_out, off_out32;
+  DevBuf offs[16], total, comb_off, comb_total, keys, scan_tmp, cnt_out, off_out32;  // comb_total: one u64
+  SegSortScratch sort;
 };
 int collapse_taxid_async(CollapseScratch& w, cudaStream_t st, uint32_t n_parts, const mtsvgpu_hit* const* d_hits,
                          const uint32_t* const* d_counts, uint32_t nr, uint64_t hit_cap, mtsvgpu_taxhit* out,

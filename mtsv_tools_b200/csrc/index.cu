@@ -257,6 +257,7 @@ void index_destroy(mtsvgpu_index* h) {
   if (h->fork_event) cudaEventDestroy(h->fork_event);
   if (h->join_event) cudaEventDestroy(h->join_event);
   for (cudaEvent_t e : h->in_events) cudaEventDestroy(e);
+  for (cudaEvent_t e : h->trace_events) cudaEventDestroy(e);
   if (h->copy_in_stream) cudaStreamDestroy(h->copy_in_stream);
   if (h->copy_out_stream) cudaStreamDestroy(h->copy_out_stream);
   if (h->out_event) cudaEventDestroy(h->out_event);
@@ -330,6 +331,8 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
 
   MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   h->stream = h->own_stream;
+  h->lanes[0].ws = &h->ws;
+  h->lanes[1].ws = &h->ws1;
   MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_in_stream, cudaStreamNonBlocking));
   MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_out_stream, cudaStreamNonBlocking));
   MTSV_CUDA_TRY(cudaEventCreateWithFlags(&h->out_event, cudaEventDisableTiming));

@@ -2,7 +2,7 @@
 references.
 
 * mtsvgpu_collapse_device (mode TaxId) takes arbitrary per-read hit lists, which makes it a direct harness for the
-  segmented sorts (binner.cu::run_segmented_sort: warp <= 32 keys, shared-memory bitonic <= 4096, in place in global
+  segmented sorts (segsort.cu::run_segmented_sort: warp <= 32 keys, shared-memory bitonic <= 4096, in place in global
   memory above), the merge (core.cuh::taxid_count / taxid_write) and the scan (util.cu::exclusive_scan_u32: 2048-entry
   tiles, a carry loop above 1024 tiles).  The reference is plain numpy.
 * mtsvgpu_collapse_device_taxid_gi against a numpy statement of its rule.
