@@ -1488,20 +1488,16 @@ struct SubBatch : BatchCall {
         rv{c.d_seqs, c.d_seq_off, read0, n_reads}, nq(n_reads * c.p.ns), qn((size_t)nq + 1) {}
   unsigned qgrid() const { return (nq + 255) / 256; }
   int fetch() { return fetch_counters(ln, d_ctr, &hc, st); }
-  // per-stage timing (profiling only)
-  cudaEvent_t next_event() {
-    if (lr.ev_next == ln.ev_pool.size()) {
-      cudaEvent_t e;
-      cudaEventCreate(&e);
-      ln.ev_pool.push_back(e);
-    }
-    return ln.ev_pool[lr.ev_next++];
-  }
-  void begin(int stage) {
-    if (!h->profiling) return;
-    cudaEvent_t a = next_event(), b = next_event();
+  // per-stage timing (profiling only): the next event pair of the lane's pool, which grows on demand.  Recording and
+  // reading the events is best-effort.
+  int begin(int stage) {
+    if (!h->profiling) return 0;
+    MTSV_TRY(events_reserve(ln.ev_pool, lr.ev_next + 2, cudaEventDefault));
+    cudaEvent_t a = ln.ev_pool[lr.ev_next].get(), b = ln.ev_pool[lr.ev_next + 1].get();
+    lr.ev_next += 2;
     cudaEventRecord(a, ln.stream);
     lr.ev_used.push_back({stage, {a, b}});
+    return 0;
   }
   void end() {
     if (!h->profiling) return;
@@ -1553,7 +1549,7 @@ int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pac
   MTSV_TRY(ws.enc.reserve(((size_t)total_words * p.ns + 1) * sizeof(ReadWord)));
   ev = EncView{ws.enc.as<ReadWord>(), total_words};
 
-  begin(ST_PREP);
+  MTSV_TRY(begin(ST_PREP));
   uint32_t* slot_off = ws.slot_off.as<uint32_t>();
   MTSV_LAUNCH(count_slots_kernel, qgrid(), 256, 0, st, rv, p, nq, slot_off, d_ctr);
   MTSV_TRY(exclusive_scan_u32(slot_off, slot_off, nq, ws.scan_tmp, (uint64_t*)&d_ctr->total_slots, st));
@@ -1571,7 +1567,7 @@ int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pac
   uniform = min_len == hc.max_len;
   lr.stats.n_seed_slots += n_slots;
   // (only now that the slot count is known to fit the buffers)
-  begin(ST_PREP);
+  MTSV_TRY(begin(ST_PREP));
   // all reads of one length: slots are addressed arithmetically, no slot -> query map needed
   uni_spq = (uniform && nq && n_slots % nq == 0) ? n_slots / nq : 0;
   if (!uni_spq) MTSV_LAUNCH(expand_slots_kernel, qgrid(), 256, 0, st, slot_off, nq, ws.slot_q.as<uint32_t>());
@@ -1603,13 +1599,13 @@ int SubBatch::slots_encode(uint64_t slot_bound, uint64_t sub_bytes, uint64_t pac
 int SubBatch::search() {
   for (DevBuf* b : {&ws.q_nseeds, &ws.q_nhits, &ws.hit_off}) MTSV_TRY(b->reserve(qn * 4));
   const uint32_t* slot_off = ws.slot_off.as<uint32_t>();
-  begin(ST_SEARCH);
+  MTSV_TRY(begin(ST_SEARCH));
   if (n_slots)
     MTSV_LAUNCH(seed_search_kernel, (n_slots + 255) / 256, 256, 0, st, h->ix.fm_view(), h->ix.ktab_view(), rv, ev, p,
                 slot_off, ws.slot_q.as<uint32_t>(), n_slots, ws.slot_lo.as<uint32_t>(),
                 ws.slot_cnt.as<uint32_t>(), d_ctr, h->profiling ? 1 : 0, hc.max_len, uni_spq);
   end();
-  begin(ST_SELECT);
+  MTSV_TRY(begin(ST_SELECT));
   MTSV_LAUNCH(seed_select_kernel, qgrid(), 256, 0, st, rv, ev, p, slot_off, nq, ws.slot_cnt.as<uint32_t>(),
               ws.slot_hoff.as<uint32_t>(), ws.q_nseeds.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), d_ctr);
   MTSV_TRY(exclusive_scan_u32(ws.q_nhits.as<uint32_t>(), ws.hit_off.as<uint32_t>(), nq, ws.scan_tmp,
@@ -1639,16 +1635,16 @@ int SubBatch::candidates() {
   MTSV_TRY(ws.sort.reserve(nq));
   MTSV_TRY(ws.hit_keys.reserve((size_t)n_hits * 8));
   MTSV_TRY(ws.cand_sparse.reserve((size_t)n_hits * sizeof(CandRec)));
-  begin(ST_LOCATE);
+  MTSV_TRY(begin(ST_LOCATE));
   MTSV_LAUNCH(locate_kernel, qgrid(), 256, 0, st, ix.fm_view(), ix.sa_view(), p, ws.slot_off.as<uint32_t>(), nq,
               ws.slot_lo.as<uint32_t>(), ws.slot_cnt.as<uint32_t>(), ws.slot_hoff.as<uint32_t>(),
               ws.hit_off.as<uint32_t>(), ws.q_nhits.as<uint32_t>(), ws.hit_keys.as<uint64_t>());
   end();
-  begin(ST_SORT);
+  MTSV_TRY(begin(ST_SORT));
   MTSV_TRY(run_segmented_sort(st, ws.sort, ws.hit_keys.as<uint64_t>(), ws.hit_off.as<uint32_t>(),
                               ws.q_nhits.as<uint32_t>(), nq, kLightItems));
   end();
-  begin(ST_COALESCE);
+  MTSV_TRY(begin(ST_COALESCE));
   MTSV_TRY(ws.cand_stage.reserve((size_t)n_hits * sizeof(CandRec)));
   MTSV_CUDA_TRY(cudaMemsetAsync(&d_ctr->n_heavy, 0, 3 * sizeof(unsigned int), st));
   MTSV_LAUNCH(coalesce_kernel, (rv.n_reads + 127) / 128, 128, 0, st, ix.bins_view(), rv, p, nq,
@@ -1670,7 +1666,7 @@ int SubBatch::candidates() {
   if (!n_cand) return 0;
   MTSV_TRY(ws.cand_dense.reserve((size_t)n_cand * sizeof(CandRec)));
   MTSV_TRY(ws.cand_q.reserve((size_t)n_cand * 4));
-  begin(ST_RANK);
+  MTSV_TRY(begin(ST_RANK));
   MTSV_LAUNCH(rank_emit_kernel, qgrid(), 256, 0, st, nq, ws.hit_off.as<uint32_t>(), ws.q_ncand.as<uint32_t>(),
               ws.cand_off.as<uint32_t>(), ws.cand_sparse.as<CandRec>(), ws.cand_dense.as<CandRec>(),
               ws.cand_q.as<uint32_t>());
@@ -1686,7 +1682,7 @@ int SubBatch::verify() {
   // windows of the same sequence) and the sub-batch has more candidates than strands.
   bool grouped = !ssw && (group_verify ? group_verify[0] != '0' : n_cand > nq && h->ix.n_bins > h->ix.n_taxids);
   MTSV_TRY(ws.cand_edit.reserve((size_t)n_cand * 4));
-  begin(ST_VERIFY);
+  MTSV_TRY(begin(ST_VERIFY));
   MTSV_TRY(ws.cand_flag.reserve(((size_t)n_cand + 1) * 4));
   MTSV_TRY(ws.cand_order.reserve((size_t)n_cand * 4));
   MTSV_LAUNCH(cand_class_kernel, (n_cand + 255) / 256, 256, 0, st, ws.cand_dense.as<CandRec>(), n_cand,
@@ -1808,7 +1804,7 @@ int SubBatch::select_append(uint64_t* out_total) {
   uint64_t sub_out = 0, sub_tax = 0;
   if (n_cand) {
     MTSV_TRY(ws.hit_tmp.reserve((size_t)n_cand * sizeof(HitRec)));
-    begin(ST_EMIT);
+    MTSV_TRY(begin(ST_EMIT));
     MTSV_LAUNCH(select_kernel, (nq + 127) / 128, 128, 0, st, h->ix.bins_view(), rv, p, nq, ws.cand_off.as<uint32_t>(),
                 ws.cand_dense.as<CandRec>(), ws.cand_edit.as<uint32_t>(), ws.hit_tmp.as<HitRec>(),
                 ws.q_nout.as<uint32_t>());
@@ -1830,12 +1826,12 @@ int SubBatch::select_append(uint64_t* out_total) {
   }
   MTSV_TRY(run.emit_acquire(lr));
   Lane& other = h->lanes[&ln == &h->lanes[0] ? 1 : 0];
-  if (other.emit_event) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, other.emit_event, 0));
+  MTSV_CUDA_TRY(cudaStreamWaitEvent(st, other.emit_event.get(), 0));
   BatchWorkspace& res = h->ws;  // batch results (shared, appended in slice order)
   const size_t rec = taxhits ? sizeof(mtsvgpu_taxhit) : sizeof(HitRec);
   const uint64_t sub_rec = taxhits ? sub_tax : sub_out;
   MTSV_TRY(grow_preserve(res.out_hits, *out_total * rec, (*out_total + sub_rec + 1) * rec, st));
-  begin(ST_EMIT);
+  MTSV_TRY(begin(ST_EMIT));
   if (taxhits) {
     taxid_merge_write(st, ws.hit_keys.as<uint64_t>(), seg_off(), tax_off(), rv.n_reads, res.out_hits.as<mtsvgpu_taxhit>(),
                       *out_total, res.out_hit_off.as<uint64_t>(), rv.read0);
@@ -1846,8 +1842,7 @@ int SubBatch::select_append(uint64_t* out_total) {
   }
   end();
   MTSV_CUDA_TRY(cudaGetLastError());
-  if (!ln.emit_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&ln.emit_event, cudaEventDisableTiming));
-  MTSV_CUDA_TRY(cudaEventRecord(ln.emit_event, st));
+  MTSV_CUDA_TRY(cudaEventRecord(ln.emit_event.get(), st));
   // host API: start copying this sub-batch's results out while the next one computes
   if (src) MTSV_TRY(src->results(*out_total, sub_rec, rv.read0, rv.n_reads, st));
   resolve();
@@ -1972,13 +1967,9 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
   const int n_lanes = n_sub >= 2 && two_lanes ? 2 : 1;
   h->lanes[0].stream = st;
   if (n_lanes == 2) {
-    if (!h->lane1_stream) MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->lane1_stream, cudaStreamNonBlocking));
-    if (!h->fork_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&h->fork_event, cudaEventDisableTiming));
-    if (!h->join_event) MTSV_CUDA_TRY(cudaEventCreateWithFlags(&h->join_event, cudaEventDisableTiming));
-    h->lanes[1].stream = h->lane1_stream;
     // lane 1 starts after whatever the caller queued on the handle's stream (its inputs)
-    MTSV_CUDA_TRY(cudaEventRecord(h->fork_event, st));
-    MTSV_CUDA_TRY(cudaStreamWaitEvent(h->lane1_stream, h->fork_event, 0));
+    MTSV_CUDA_TRY(cudaEventRecord(h->fork_event.get(), st));
+    MTSV_CUDA_TRY(cudaStreamWaitEvent(h->lane1_stream.get(), h->fork_event.get(), 0));
   }
   BatchRun run;
   const int device = h->ix.device;
@@ -2003,15 +1994,15 @@ int bin_batch_device(mtsvgpu_index* h, const uint8_t* d_seqs, const uint64_t* d_
     lane_main(0);
     helper.join();
     // everything lane 1 did is ordered before what follows on the handle's stream
-    MTSV_CUDA_TRY(cudaEventRecord(h->join_event, h->lane1_stream));
-    MTSV_CUDA_TRY(cudaStreamWaitEvent(st, h->join_event, 0));
+    MTSV_CUDA_TRY(cudaEventRecord(h->join_event.get(), h->lane1_stream.get()));
+    MTSV_CUDA_TRY(cudaStreamWaitEvent(st, h->join_event.get(), 0));
   } else {
     lane_main(0);
   }
   for (const LaneRun& lr : run.lanes) add_stats(h->stats, lr.stats);
   if (run.abort_rc != 0) {
     cudaStreamSynchronize(st);
-    if (h->lane1_stream) cudaStreamSynchronize(h->lane1_stream);
+    cudaStreamSynchronize(h->lane1_stream.get());
     return set_error(run.abort_rc, "%s", run.abort_msg.c_str());
   }
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));

@@ -128,12 +128,9 @@ int index_build(const uint8_t* seqs, const uint64_t* seq_off, const uint32_t* gi
     }
   }
 
-  cudaStream_t st = nullptr;
-  MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-  struct StreamGuard {
-    cudaStream_t s;
-    ~StreamGuard() { cudaStreamDestroy(s); }
-  } sg{st};
+  Stream stream;
+  MTSV_TRY(stream_create(stream));
+  const cudaStream_t st = stream.get();
   DevPtr<uint8_t> text_g, bwt_g;
   MTSV_TRY(dev_alloc(text_g, n + 16));
   uint8_t* d_text = text_g.get();

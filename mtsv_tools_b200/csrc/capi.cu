@@ -72,7 +72,7 @@ int mtsvgpu_index_get_info(const mtsvgpu_index* ix, mtsvgpu_index_info* info) {
 
 int mtsvgpu_set_stream(mtsvgpu_index* ix, void* cuda_stream) {
   if (!ix) return set_error(MTSVGPU_EINVAL, "index is NULL");
-  ix->stream = cuda_stream ? (cudaStream_t)cuda_stream : ix->own_stream;
+  ix->stream = cuda_stream ? (cudaStream_t)cuda_stream : ix->own_stream.get();
   return 0;
 }
 
@@ -123,8 +123,8 @@ struct HostUpload : BatchSource {
   size_t rec_bytes;  // result records: mtsvgpu_hit or mtsvgpu_taxhit
   // MTSV_B200_TRACE: per-slice timeline (when each slice landed, when its compute started), from the handle's pool
   cudaEvent_t trace_t0 = nullptr;
-  const cudaEvent_t* trace_landed = nullptr;
-  const cudaEvent_t* trace_started = nullptr;
+  const Event* trace_landed = nullptr;
+  const Event* trace_started = nullptr;
   HostUpload(mtsvgpu_index* h, size_t rec) : ix(h), rec_bytes(rec) {}
   int upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, uint64_t* h2d_bytes);
   int wait_slice(uint64_t i, cudaStream_t st) override;
@@ -137,8 +137,8 @@ int HostUpload::wait_slice(uint64_t i, cudaStream_t st) {
     if (upload_rc.load(std::memory_order_acquire) != 0) return set_error(upload_rc.load(), "%s", upload_msg.c_str());
     std::this_thread::yield();
   }
-  if (i < ix->in_events.size()) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, ix->in_events[i], 0));
-  if (trace_started) MTSV_CUDA_TRY(cudaEventRecord(trace_started[i], st));
+  if (i < ix->in_events.size()) MTSV_CUDA_TRY(cudaStreamWaitEvent(st, ix->in_events[i].get(), 0));
+  if (trace_started) MTSV_CUDA_TRY(cudaEventRecord(trace_started[i].get(), st));
   return 0;
 }
 
@@ -153,15 +153,15 @@ int HostUpload::results(uint64_t first_hit, uint64_t n_hits, uint64_t first_read
     out_overlap_ok = false;  // does not fit / unexpected order: the caller copies everything at the end
     return 0;
   }
-  MTSV_CUDA_TRY(cudaEventRecord(ix->out_event, st));
-  MTSV_CUDA_TRY(cudaStreamWaitEvent(ix->copy_out_stream, ix->out_event, 0));
+  MTSV_CUDA_TRY(cudaEventRecord(ix->out_event.get(), st));
+  MTSV_CUDA_TRY(cudaStreamWaitEvent(ix->copy_out_stream.get(), ix->out_event.get(), 0));
   const uint8_t* d_recs = ix->ws.out_hits.as<uint8_t>();
   const uint64_t* d_off = ix->ws.out_hit_off.as<uint64_t>();
   if (n_hits)
     MTSV_CUDA_TRY(cudaMemcpyAsync(ix->pin_hits.get() + first_hit * rec_bytes, d_recs + first_hit * rec_bytes,
-                                  n_hits * rec_bytes, cudaMemcpyDeviceToHost, ix->copy_out_stream));
+                                  n_hits * rec_bytes, cudaMemcpyDeviceToHost, ix->copy_out_stream.get()));
   MTSV_CUDA_TRY(cudaMemcpyAsync((uint64_t*)ix->pin_off.get() + first_read, d_off + first_read,
-                                (n_reads + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out_stream));
+                                (n_reads + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->copy_out_stream.get()));
   out_copied_hits = first_hit + n_hits;
   out_copied_reads = first_read + n_reads;
   return 0;
@@ -186,7 +186,7 @@ static bool uniform_lengths(const uint64_t* o, uint64_t n_reads) {  // o[0 .. n_
 int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, uint64_t* h2d_bytes) {
   MTSV_CUDA_TRY(cudaSetDevice(ix->ix.device));
   BatchWorkspace& ws = ix->ws;
-  cudaStream_t cin = ix->copy_in_stream;
+  cudaStream_t cin = ix->copy_in_stream.get();
   const uint64_t* offs = seq_off;
   const bool packed = !pack_base.empty();
   const uint64_t n_sub = bounds.size() - 1;
@@ -228,8 +228,8 @@ int HostUpload::upload(const uint8_t* seqs, uint64_t base, uint64_t bytes, uint6
     if (cn)
       MTSV_CUDA_TRY(cudaMemcpyAsync(ws.d_seqs.as<uint8_t>() + c0, seqs + base + c0, cn, cudaMemcpyHostToDevice, cin));
     *h2d_bytes += cn;
-    MTSV_CUDA_TRY(cudaEventRecord(ix->in_events[i], cin));
-    if (trace_landed) MTSV_CUDA_TRY(cudaEventRecord(trace_landed[i], cin));
+    MTSV_CUDA_TRY(cudaEventRecord(ix->in_events[i].get(), cin));
+    if (trace_landed) MTSV_CUDA_TRY(cudaEventRecord(trace_landed[i].get(), cin));
     slices_enqueued.store(i + 1, std::memory_order_release);
   }
   return 0;
@@ -246,7 +246,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   *hits = nullptr;
   *hit_off = nullptr;
   MTSV_CUDA_TRY(cudaSetDevice(ix->ix.device));
-  cudaStream_t st = ix->stream, cin = ix->copy_in_stream;
+  cudaStream_t st = ix->stream, cin = ix->copy_in_stream.get();
   static const bool trace = getenv("MTSV_B200_TRACE") != nullptr;  // host-side phase times on stderr
   auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t_begin = trace ? now() : 0;
@@ -271,18 +271,10 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   up.bounds = slice_bounds(n_reads, ix->opts.batch_reads, true, true);
   const uint64_t n_sub = up.bounds.size() - 1;
   if (packed) up.pack_base.assign(n_sub, 0);
-  while (ix->in_events.size() < n_sub) {
-    cudaEvent_t e;
-    MTSV_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    ix->in_events.push_back(e);
-  }
+  MTSV_TRY(events_reserve(ix->in_events, n_sub, cudaEventDisableTiming));
   if (trace) {
-    while (ix->trace_events.size() < 2 * n_sub + 1) {
-      cudaEvent_t e;
-      MTSV_CUDA_TRY(cudaEventCreate(&e));
-      ix->trace_events.push_back(e);
-    }
-    up.trace_t0 = ix->trace_events[0];
+    MTSV_TRY(events_reserve(ix->trace_events, 2 * n_sub + 1, cudaEventDefault));
+    up.trace_t0 = ix->trace_events[0].get();
     up.trace_landed = ix->trace_events.data() + 1;
     up.trace_started = ix->trace_events.data() + 1 + n_sub;
     MTSV_CUDA_TRY(cudaEventRecord(up.trace_t0, cin));
@@ -316,7 +308,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   ix->stats.h2d_bytes = h2d_bytes;
   if (rc != 0) {
     cudaStreamSynchronize(cin);
-    cudaStreamSynchronize(ix->copy_out_stream);
+    cudaStreamSynchronize(ix->copy_out_stream.get());
     return rc;
   }
   const double t_comp = trace ? now() : 0;
@@ -327,7 +319,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
   const size_t hb = (n_hits ? n_hits : 1) * rec, ob = (n_reads + 1) * sizeof(uint64_t);
   if (pinned_result) {
     // slices may still be on their way into the buffers ensure_pinned is about to replace
-    MTSV_CUDA_TRY(cudaStreamSynchronize(ix->copy_out_stream));
+    MTSV_CUDA_TRY(cudaStreamSynchronize(ix->copy_out_stream.get()));
     MTSV_TRY(ensure_pinned(ix->pin_hits, ix->pin_hits_cap, hb));
     MTSV_TRY(ensure_pinned(ix->pin_off, ix->pin_off_cap, ob));
     h_hits = ix->pin_hits.get();
@@ -341,7 +333,7 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
       return set_error(MTSVGPU_ENOMEM, "host allocation of the result failed");
     }
   }
-  cudaError_t e = cudaStreamSynchronize(ix->copy_out_stream);
+  cudaError_t e = cudaStreamSynchronize(ix->copy_out_stream.get());
   // (nothing more to copy when everything was copied slice by slice)
   if (!(pinned_result && up.out_overlap_ok && up.out_copied_hits == n_hits && up.out_copied_reads == n_reads)) {
     if (e == cudaSuccess && n_hits)
@@ -365,8 +357,8 @@ static int bin_batch_host(mtsvgpu_index* ix, const uint8_t* seqs, const uint64_t
     char line[256];
     for (uint64_t i = 0; i < n_sub; ++i) {
       float a = 0, b = 0;
-      cudaEventElapsedTime(&a, up.trace_t0, up.trace_landed[i]);  // (every slice's events have completed)
-      cudaEventElapsedTime(&b, up.trace_t0, up.trace_started[i]);
+      cudaEventElapsedTime(&a, up.trace_t0, up.trace_landed[i].get());  // (every slice's events have completed)
+      cudaEventElapsedTime(&b, up.trace_t0, up.trace_started[i].get());
       snprintf(line, sizeof line, "[mtsv_b200 trace]   %2llu: %8llu  %7.2f  %7.2f\n", (unsigned long long)i,
                (unsigned long long)(up.bounds[i + 1] - up.bounds[i]), a, b);
       out += line;

@@ -286,10 +286,10 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
   const mtsvgpu_hit* d_hits = static_cast<const mtsvgpu_hit*>(d_recs);
   cudaStream_t st = h->stream;
   static const bool trace = getenv("MTSV_B200_TRACE") != nullptr;  // phase times on stderr
-  cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+  Event ev[5];
   if (trace) {
-    for (auto& e : ev) cudaEventCreate(&e);
-    cudaEventRecord(ev[0], st);
+    for (Event& e : ev) MTSV_TRY(event_create(e, cudaEventDefault));
+    cudaEventRecord(ev[0].get(), st);
   }
   // ---- exchange: my hits of range d into rank d's buffer, flag, wait for everybody's flags here ----
   const uint32_t epoch = ++c->epoch, parity = epoch & 1u;
@@ -303,13 +303,13 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
     MTSV_LAUNCH(chunk_push_kernel, dim3(gx, c->world), 256, 0, st, c->peers, c->lay, d_hits, d_hit_off, n_reads, step,
                 c->rank, parity, d_overflow);
   }
-  if (trace) cudaEventRecord(ev[1], st);
+  if (trace) cudaEventRecord(ev[1].get(), st);
   MTSV_LAUNCH(chunk_signal_kernel, 1, 32, 0, st, c->peers, c->world, c->rank, epoch);
   const long long timeout_cycles = c->timeout_cycles;  // 30 s: a peer that never arrives is an error
-  if (trace) cudaEventRecord(ev[4], st);
+  if (trace) cudaEventRecord(ev[4].get(), st);
   MTSV_LAUNCH(chunk_wait_kernel, 1, 32, 0, st, c->base.get(), c->world, epoch, timeout_cycles, c->d_status.get(),
               c->h_status_dev);
-  if (trace) cudaEventRecord(ev[2], st);
+  if (trace) cudaEventRecord(ev[2].get(), st);
   // ---- merge epilogue over the world slots of my range (src/collapse.rs:597-602) ----
   const mtsvgpu_hit* part_hits[kMaxRanks];
   const uint32_t* part_counts[kMaxRanks];
@@ -321,19 +321,18 @@ int bin_batch_chunked(mtsvgpu_index* h, mtsvgpu_comm* c, const uint8_t* d_seqs, 
   // zeros they were created with, so the merge below stays in bounds; its result is discarded)
   MTSV_TRY(collapse_taxid_async(c->scratch, st, c->world, part_hits, part_counts, (uint32_t)(hi - lo),
                                 (uint64_t)c->world * c->lay.cap_hits, c->out.get(), c->out_off.get(), c->d_n_out.get()));
-  if (trace) cudaEventRecord(ev[3], st);
+  if (trace) cudaEventRecord(ev[3].get(), st);
   uint64_t total = 0;
   MTSV_CUDA_TRY(cudaMemcpyAsync(&total, c->d_n_out.get(), 8, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));  // the batch's one host synchronisation after the local binning
   if (trace) {
     float a = 0, b = 0, d = 0, sg = 0;
-    cudaEventElapsedTime(&a, ev[0], ev[1]);
-    cudaEventElapsedTime(&sg, ev[1], ev[4]);
-    cudaEventElapsedTime(&b, ev[4], ev[2]);
-    cudaEventElapsedTime(&d, ev[2], ev[3]);
+    cudaEventElapsedTime(&a, ev[0].get(), ev[1].get());
+    cudaEventElapsedTime(&sg, ev[1].get(), ev[4].get());
+    cudaEventElapsedTime(&b, ev[4].get(), ev[2].get());
+    cudaEventElapsedTime(&d, ev[2].get(), ev[3].get());
     fprintf(stderr, "[mtsv_b200 trace] rank %u chunked batch: %llu hits, push %.3f ms, signal %.3f ms, wait %.3f ms, merge %.3f ms\n",
             c->rank, (unsigned long long)n_hits, a, sg, b, d);
-    for (auto& e : ev) cudaEventDestroy(e);
   }
   const uint32_t status = *c->h_status;
   if (status == 1)

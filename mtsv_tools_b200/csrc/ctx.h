@@ -76,6 +76,23 @@ int pinned_alloc(PinnedPtr<T>& p, uint64_t count, unsigned flags = cudaHostAlloc
   return 0;
 }
 
+// owners of streams and events
+struct CudaStreamDestroy {
+  void operator()(cudaStream_t s) const;
+};
+struct CudaEventDestroy {
+  void operator()(cudaEvent_t e) const;
+};
+using Stream = std::unique_ptr<CUstream_st, CudaStreamDestroy>;
+using Event = std::unique_ptr<CUevent_st, CudaEventDestroy>;
+
+// The library's only stream and event creation: a non-blocking stream; an event with cudaEventCreateWithFlags's
+// flags.  A failure clears the runtime's last error and returns MTSVGPU_ECUDA.
+int stream_create(Stream& s);
+int event_create(Event& e, unsigned flags);
+// grows `pool` to at least n events created with `flags`
+int events_reserve(std::vector<Event>& pool, size_t n, unsigned flags);
+
 // MTSVGPU_ENODEVICE without a device, MTSVGPU_EINVAL for a number outside [0, count), else cudaSetDevice
 int use_device(int device);
 
@@ -201,12 +218,12 @@ struct BatchWorkspace {
 // scratch, own host thread): while one lane's host thread waits for the scalars of a stage, the other lane's
 // kernels keep the device busy, and the tails of memory-bound and ALU-bound kernels of different slices overlap.
 struct Lane {
-  cudaStream_t stream = nullptr;     // lane 0: the handle's stream; lane 1: a private non-blocking stream
-  BatchWorkspace* ws = nullptr;      // scratch of the lane (results and staged inputs live in the handle's ws)
-  PinnedPtr<BatchCounters> h_ctr;    // mapped: sub-batch scalars published by the device
+  cudaStream_t stream = nullptr;   // lane 0: the handle's stream; lane 1: the handle's lane1_stream
+  BatchWorkspace* ws = nullptr;    // scratch of the lane (results and staged inputs live in the handle's ws)
+  PinnedPtr<BatchCounters> h_ctr;  // mapped: sub-batch scalars published by the device
   BatchCounters* h_ctr_dev = nullptr;
-  cudaEvent_t emit_event = nullptr;  // recorded after each append to the batch output
-  std::vector<cudaEvent_t> ev_pool;  // per-stage timing (profiling)
+  Event emit_event;                // recorded after each append to the batch output
+  std::vector<Event> ev_pool;      // per-stage timing (profiling)
 };
 
 // What a batch call returns, CSR by read: the Hit records of every strand (mtsvgpu_hit), or per read each TaxID once
@@ -231,21 +248,21 @@ struct BatchSource {
 struct mtsvgpu_index {
   mtsv::DeviceIndex ix;
   mtsvgpu_index_opts opts{};
-  cudaStream_t own_stream = nullptr;
-  cudaStream_t stream = nullptr;
+  mtsv::Stream own_stream;
+  cudaStream_t stream = nullptr;  // own_stream or the caller's (mtsvgpu_set_stream)
   bool profiling = false;
   mtsv::BatchWorkspace ws;   // lane 0 scratch + the batch results + the staged inputs of the host API
   mtsv::BatchWorkspace ws1;  // lane 1 scratch
   mtsv::Lane lanes[2];
-  cudaStream_t lane1_stream = nullptr;
-  cudaEvent_t fork_event = nullptr, join_event = nullptr;
+  mtsv::Stream lane1_stream;
+  mtsv::Event fork_event, join_event;
   mtsvgpu_batch_stats stats{};  // of the last batch call
   // host API: copy streams, per-sub-batch "input landed" events, pinned result buffers
-  cudaStream_t copy_in_stream = nullptr;
-  std::vector<cudaEvent_t> in_events;
-  cudaStream_t copy_out_stream = nullptr;
-  cudaEvent_t out_event = nullptr;
-  std::vector<cudaEvent_t> trace_events;  // MTSV_B200_TRACE: the slice timeline
+  mtsv::Stream copy_in_stream;
+  std::vector<mtsv::Event> in_events;
+  mtsv::Stream copy_out_stream;
+  mtsv::Event out_event;
+  std::vector<mtsv::Event> trace_events;  // MTSV_B200_TRACE: the slice timeline
   mtsv::PinnedPtr<uint8_t> pin_hits;
   size_t pin_hits_cap = 0;
   mtsv::PinnedPtr<uint8_t> pin_off;

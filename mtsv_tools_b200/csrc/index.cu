@@ -248,21 +248,32 @@ __global__ void text_pack4_kernel(const uint8_t* __restrict__ text, uint64_t n, 
 
 void index_destroy(mtsvgpu_index* h) {
   if (!h) return;
-  cudaSetDevice(h->ix.device);  // the members' memory is freed by `delete h`, on this device
-  for (Lane& ln : h->lanes) {
-    if (ln.emit_event) cudaEventDestroy(ln.emit_event);
-    for (cudaEvent_t e : ln.ev_pool) cudaEventDestroy(e);
-  }
-  if (h->lane1_stream) cudaStreamDestroy(h->lane1_stream);
-  if (h->fork_event) cudaEventDestroy(h->fork_event);
-  if (h->join_event) cudaEventDestroy(h->join_event);
-  for (cudaEvent_t e : h->in_events) cudaEventDestroy(e);
-  for (cudaEvent_t e : h->trace_events) cudaEventDestroy(e);
-  if (h->copy_in_stream) cudaStreamDestroy(h->copy_in_stream);
-  if (h->copy_out_stream) cudaStreamDestroy(h->copy_out_stream);
-  if (h->out_event) cudaEventDestroy(h->out_event);
-  if (h->own_stream) cudaStreamDestroy(h->own_stream);
+  cudaSetDevice(h->ix.device);  // the members' memory, streams and events are freed by `delete h`, on this device
   delete h;
+}
+
+using IndexPtr = std::unique_ptr<mtsvgpu_index, void (*)(mtsvgpu_index*)>;
+
+// ---- the handle with the streams and events it keeps for its life: its own stream, the host API's copy streams and
+// result event, lane 1's stream with the events that fork it from and join it to the handle's stream, and each lane's
+// emit event.  The lanes are wired to their streams and workspaces. ----
+static int create_handle(int device, const mtsvgpu_index_opts* opts, IndexPtr& h) {
+  h.reset(new mtsvgpu_index);
+  h->ix.device = device;
+  if (opts) h->opts = *opts;
+  MTSV_TRY(stream_create(h->own_stream));
+  MTSV_TRY(stream_create(h->copy_in_stream));
+  MTSV_TRY(stream_create(h->copy_out_stream));
+  MTSV_TRY(event_create(h->out_event, cudaEventDisableTiming));
+  MTSV_TRY(stream_create(h->lane1_stream));
+  MTSV_TRY(event_create(h->fork_event, cudaEventDisableTiming));
+  MTSV_TRY(event_create(h->join_event, cudaEventDisableTiming));
+  for (Lane& ln : h->lanes) MTSV_TRY(event_create(ln.emit_event, cudaEventDisableTiming));
+  h->stream = h->own_stream.get();
+  h->lanes[0].ws = &h->ws;
+  h->lanes[1].ws = &h->ws1;
+  h->lanes[1].stream = h->lane1_stream.get();
+  return 0;
 }
 
 static uint32_t auto_ktab_k(uint64_t n) {
@@ -277,70 +288,44 @@ static uint32_t auto_ktab_k(uint64_t n) {
   return k;
 }
 
-int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out) {
-  double t0 = now_s();
-  const uint8_t* text = parts.text;
-  const uint64_t n = parts.n;
+// ---- validation of the MGIndex fields on the host (SURVEY §8b "loader must assert") ----
+static int check_parts(const IndexParts& parts) {
+  const uint64_t n = parts.n, n_bins = parts.n_bins, sa_rate = parts.sa_rate;
   const mtsvgpu_bin* bins = parts.bins;
-  const uint64_t n_bins = parts.n_bins;
-  const uint8_t* bwt = parts.bwt;
-  const uint64_t* sa_sample = parts.sa_sample;
-  const uint64_t sa_sample_len = parts.sa_sample_len;
-  const uint64_t sa_rate = parts.sa_rate;
-  if (!text || !bins || !bwt || (!sa_sample && !parts.d_sa_full) || !out)
-    return set_error(MTSVGPU_EINVAL, "null argument");
-  *out = nullptr;
-  // ---- validation of the MGIndex fields (SURVEY §8b "loader must assert") ----
   if (n < 2) return set_error(MTSVGPU_EFORMAT, "index text has %llu symbols", (unsigned long long)n);
   if (n >= (1ull << 32) - 64)
     return set_error(MTSVGPU_ELIMIT,
                      "index has %llu symbols; this build keeps 32-bit rows (limit 2^32-64)",
                      (unsigned long long)n);
-  if (!parts.text_on_device && text[n - 1] != '$') return set_error(MTSVGPU_EFORMAT, "sequences do not end with '$'");
+  if (!parts.text_on_device && parts.text[n - 1] != '$')
+    return set_error(MTSVGPU_EFORMAT, "sequences do not end with '$'");
   if (sa_rate == 0 || sa_rate > 0xffffffffull)
     return set_error(MTSVGPU_EFORMAT, "bad suffix-array sample rate");
-  if (!parts.d_sa_full && sa_sample_len != (n + sa_rate - 1) / sa_rate)
+  if (!parts.d_sa_full && parts.sa_sample_len != (n + sa_rate - 1) / sa_rate)
     return set_error(MTSVGPU_EFORMAT, "suffix-array sample has %llu entries, expected %llu",
-                     (unsigned long long)sa_sample_len,
+                     (unsigned long long)parts.sa_sample_len,
                      (unsigned long long)((n + sa_rate - 1) / sa_rate));
   if (n_bins == 0 || n_bins > 0xfffffff0ull) return set_error(MTSVGPU_EFORMAT, "bad bin count");
-  {
-    uint64_t prev_end = 0;
-    for (uint64_t i = 0; i < n_bins; ++i) {
-      if (bins[i].start != prev_end || bins[i].end < bins[i].start || bins[i].end > n - 1)
-        return set_error(MTSVGPU_EFORMAT, "bin %llu [%llu,%llu) is not contiguous within the text",
-                         (unsigned long long)i, (unsigned long long)bins[i].start,
-                         (unsigned long long)bins[i].end);
-      prev_end = bins[i].end;
-    }
-    if (prev_end != n - 1)
-      return set_error(MTSVGPU_EFORMAT, "bins end at %llu, text (without '$') at %llu",
-                       (unsigned long long)prev_end, (unsigned long long)(n - 1));
+  uint64_t prev_end = 0;
+  for (uint64_t i = 0; i < n_bins; ++i) {
+    if (bins[i].start != prev_end || bins[i].end < bins[i].start || bins[i].end > n - 1)
+      return set_error(MTSVGPU_EFORMAT, "bin %llu [%llu,%llu) is not contiguous within the text",
+                       (unsigned long long)i, (unsigned long long)bins[i].start,
+                       (unsigned long long)bins[i].end);
+    prev_end = bins[i].end;
   }
+  if (prev_end != n - 1)
+    return set_error(MTSVGPU_EFORMAT, "bins end at %llu, text (without '$') at %llu",
+                     (unsigned long long)prev_end, (unsigned long long)(n - 1));
+  return 0;
+}
 
-  MTSV_TRY(use_device(device));
-
-  std::unique_ptr<mtsvgpu_index, void (*)(mtsvgpu_index*)> guard(new mtsvgpu_index, index_destroy);
-  mtsvgpu_index* h = guard.get();
-  if (opts) h->opts = *opts;
-  DeviceIndex& d = h->ix;
-  d.device = device;
-  d.n = n;
-  d.n_bins = n_bins;
-  d.file_sa_rate = sa_rate;
-
-  MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-  h->stream = h->own_stream;
-  h->lanes[0].ws = &h->ws;
-  h->lanes[1].ws = &h->ws1;
-  MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_in_stream, cudaStreamNonBlocking));
-  MTSV_CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_out_stream, cudaStreamNonBlocking));
-  MTSV_CUDA_TRY(cudaEventCreateWithFlags(&h->out_event, cudaEventDisableTiming));
-  cudaStream_t st = h->stream;
-
-  // ---- text and bins ----
+// ---- text, its 4-bit match classes and the bins ----
+static int upload_text_bins(DeviceIndex& d, const IndexParts& parts, cudaStream_t st) {
+  const uint64_t n = d.n, n_bins = d.n_bins;
+  const mtsvgpu_bin* bins = parts.bins;
   MTSV_TRY(dev_alloc(d.text, n + 16, &d.device_bytes));
-  MTSV_CUDA_TRY(cudaMemcpyAsync(d.text.get(), text, n, cudaMemcpyDefault, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(d.text.get(), parts.text, n, cudaMemcpyDefault, st));
   MTSV_CUDA_TRY(cudaMemsetAsync(d.text.get() + n, 0, 16, st));
   if (parts.text_on_device) {
     uint8_t last = 0;
@@ -353,30 +338,34 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
   MTSV_TRY(dev_alloc(d.text4, d.text4_words, &d.device_bytes));
   MTSV_LAUNCH(text_pack4_kernel, (unsigned)((d.text4_words + 255) / 256), 256, 0, st, d.text.get(), n, d.text4.get(),
               d.text4_words);
-  {
-    std::vector<uint32_t> bs(n_bins), be(n_bins), bt(n_bins), bg(n_bins);
-    for (uint64_t i = 0; i < n_bins; ++i) {
-      bs[i] = (uint32_t)bins[i].start;
-      be[i] = (uint32_t)bins[i].end;
-      bt[i] = bins[i].tax_id;
-      bg[i] = bins[i].gi;
-    }
-    {
-      std::vector<uint32_t> t = bt;
-      std::sort(t.begin(), t.end());
-      d.n_taxids = (uint64_t)(std::unique(t.begin(), t.end()) - t.begin());
-    }
-    MTSV_TRY(dev_alloc(d.bin_start, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(d.bin_end, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(d.bin_tax, n_bins, &d.device_bytes));
-    MTSV_TRY(dev_alloc(d.bin_gi, n_bins, &d.device_bytes));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_start.get(), bs.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_end.get(), be.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_tax.get(), bt.data(), n_bins * 4, cudaMemcpyHostToDevice));
-    MTSV_CUDA_TRY(cudaMemcpy(d.bin_gi.get(), bg.data(), n_bins * 4, cudaMemcpyHostToDevice));
+  std::vector<uint32_t> bs(n_bins), be(n_bins), bt(n_bins), bg(n_bins);
+  for (uint64_t i = 0; i < n_bins; ++i) {
+    bs[i] = (uint32_t)bins[i].start;
+    be[i] = (uint32_t)bins[i].end;
+    bt[i] = bins[i].tax_id;
+    bg[i] = bins[i].gi;
   }
+  {
+    std::vector<uint32_t> t = bt;
+    std::sort(t.begin(), t.end());
+    d.n_taxids = (uint64_t)(std::unique(t.begin(), t.end()) - t.begin());
+  }
+  MTSV_TRY(dev_alloc(d.bin_start, n_bins, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.bin_end, n_bins, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.bin_tax, n_bins, &d.device_bytes));
+  MTSV_TRY(dev_alloc(d.bin_gi, n_bins, &d.device_bytes));
+  MTSV_CUDA_TRY(cudaMemcpy(d.bin_start.get(), bs.data(), n_bins * 4, cudaMemcpyHostToDevice));
+  MTSV_CUDA_TRY(cudaMemcpy(d.bin_end.get(), be.data(), n_bins * 4, cudaMemcpyHostToDevice));
+  MTSV_CUDA_TRY(cudaMemcpy(d.bin_tax.get(), bt.data(), n_bins * 4, cudaMemcpyHostToDevice));
+  MTSV_CUDA_TRY(cudaMemcpy(d.bin_gi.get(), bg.data(), n_bins * 4, cudaMemcpyHostToDevice));
+  return 0;
+}
 
-  // ---- BWT re-layout ----
+// ---- BWT re-layout and C.  *t_start: when the kernels start.  d_diag stays with the caller for the densify
+// stage.  The uploaded BWT and the other scratch are freed on return, before the suffix array is allocated. ----
+static int relayout_bwt(DeviceIndex& d, const IndexParts& parts, cudaStream_t st, DevPtr<PackDiag>& d_diag,
+                        double* t_start) {
+  const uint64_t n = d.n;
   d.n_blocks = n / kRowsPerBlock + 1;
   d.n_super = (d.n_blocks + kBlocksPerSuper - 1) / kBlocksPerSuper;
   MTSV_TRY(dev_alloc(d.blocks, d.n_super * kBlocksPerSuper, &d.device_bytes));
@@ -386,9 +375,8 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
   DevPtr<uint8_t> d_bwt;
   DevPtr<uint32_t> d_super_tot, d_super_n;
   DevPtr<unsigned long long> d_totals;
-  DevPtr<PackDiag> d_diag;
   // (a BWT that is already on the device is used where it lies: the caller pads it by 64 bytes)
-  const uint8_t* bwt_dev = bwt;
+  const uint8_t* bwt_dev = parts.bwt;
   if (!parts.bwt_on_device) {
     MTSV_TRY(dev_alloc(d_bwt, n + 64));
     bwt_dev = d_bwt.get();
@@ -398,9 +386,9 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
   MTSV_TRY(dev_alloc(d_totals, 5));
   MTSV_TRY(dev_alloc(d_diag, 1));
   MTSV_CUDA_TRY(cudaMemsetAsync(d_diag.get(), 0, sizeof(PackDiag), st));
-  if (!parts.bwt_on_device) MTSV_CUDA_TRY(cudaMemcpyAsync(d_bwt.get(), bwt, n, cudaMemcpyHostToDevice, st));
+  if (!parts.bwt_on_device) MTSV_CUDA_TRY(cudaMemcpyAsync(d_bwt.get(), parts.bwt, n, cudaMemcpyHostToDevice, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  double t_relayout0 = now_s();
+  *t_start = now_s();
 
   MTSV_LAUNCH(fm_pack_kernel, (unsigned)d.n_super, kBlocksPerSuper, 0, st, bwt_dev, n, d.n_blocks,
               d.blocks.get(), d.n_before.get(), d_super_tot.get(), d_diag.get());
@@ -429,29 +417,35 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
   d.C[SYM_T] = (uint32_t)(1 + totals[0] + totals[1] + totals[2] + totals[4]);
   MTSV_TRY(dev_alloc(d.d_C, 8, &d.device_bytes));
   MTSV_CUDA_TRY(cudaMemcpy(d.d_C.get(), d.C, 5 * sizeof(uint32_t), cudaMemcpyHostToDevice));
-  d_bwt.reset();
+  return 0;
+}
 
-  // ---- suffix array at the device rate ----
+// ---- suffix array at the device rate, built on this device (sufsort.cu): the complete array is adopted as it is,
+// or thinned to the requested rate and then freed ----
+static int sa_from_full(DeviceIndex& d, uint32_t rate, DevPtr<uint32_t>& full, cudaStream_t st) {
+  const uint64_t n = d.n;
+  if (rate <= 1) {
+    d.sa = std::move(full);
+    d.sa_rate = 1;
+    d.sa_len = n;
+    d.device_bytes += n * 4;
+    return 0;
+  }
+  d.sa_rate = rate;
+  d.sa_len = (n + rate - 1) / rate;
+  MTSV_TRY(dev_alloc(d.sa, d.sa_len, &d.device_bytes));
+  MTSV_LAUNCH(sa_thin_kernel, (unsigned)((d.sa_len + 255) / 256), 256, 0, st, full.get(), d.sa_len, rate, d.sa.get());
+  MTSV_CUDA_TRY(cudaStreamSynchronize(st));
+  full.reset();
+  return 0;
+}
+
+// ---- suffix array at the device rate, densified from the file's samples.  d_diag: the re-layout's, whose
+// sa_mismatch and rows_seen are still 0. ----
+static int sa_from_samples(DeviceIndex& d, uint32_t rate, const IndexParts& parts, PackDiag* d_diag, cudaStream_t st) {
+  const uint64_t n = d.n, sa_rate = parts.sa_rate, sa_sample_len = parts.sa_sample_len;
   size_t free_b = 0, total_b = 0;
   MTSV_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-  uint32_t rate = h->opts.sa_rate;
-  if (parts.d_sa_full) {
-    // built on this device (sufsort.cu): the complete array is adopted as it is, or thinned to the requested rate
-    if (rate <= 1) {
-      d.sa = std::move(parts.d_sa_full);
-      d.sa_rate = 1;
-      d.sa_len = n;
-      d.device_bytes += n * 4;
-    } else {
-      d.sa_rate = rate;
-      d.sa_len = (n + rate - 1) / rate;
-      MTSV_TRY(dev_alloc(d.sa, d.sa_len, &d.device_bytes));
-      MTSV_LAUNCH(sa_thin_kernel, (unsigned)((d.sa_len + 255) / 256), 256, 0, st, parts.d_sa_full.get(), d.sa_len, rate,
-                  d.sa.get());
-      MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-      parts.d_sa_full.reset();
-    }
-  } else {
   if (rate == 0) {
     rate = 1;
     // keep the dense array under a quarter of what is still free (the rest is for batches)
@@ -464,62 +458,89 @@ int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts,
   MTSV_TRY(dev_alloc(d.sa, d.sa_len, &d.device_bytes));
   DevPtr<uint64_t> d_sample;
   MTSV_TRY(dev_alloc(d_sample, sa_sample_len));
-  MTSV_CUDA_TRY(cudaMemcpyAsync(d_sample.get(), sa_sample, sa_sample_len * 8, cudaMemcpyHostToDevice, st));
+  MTSV_CUDA_TRY(cudaMemcpyAsync(d_sample.get(), parts.sa_sample, sa_sample_len * 8, cudaMemcpyHostToDevice, st));
   MTSV_CUDA_TRY(cudaMemsetAsync(d.sa.get(), 0xff, d.sa_len * 4, st));
   MTSV_LAUNCH(sa_densify_kernel, (unsigned)((sa_sample_len + 127) / 128), 128, 0, st, d.fm_view(),
-              d_sample.get(), sa_sample_len, (uint32_t)sa_rate, rate, d.sa.get(), d_diag.get());
+              d_sample.get(), sa_sample_len, (uint32_t)sa_rate, rate, d.sa.get(), d_diag);
   MTSV_CUDA_TRY(cudaGetLastError());
-  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag.get(), sizeof diag, cudaMemcpyDeviceToHost, st));
+  PackDiag diag;
+  MTSV_CUDA_TRY(cudaMemcpyAsync(&diag, d_diag, sizeof diag, cudaMemcpyDeviceToHost, st));
   MTSV_CUDA_TRY(cudaStreamSynchronize(st));
   if (diag.sa_mismatch != 0 || diag.rows_seen != n)
     return set_error(MTSVGPU_EFORMAT,
                      "suffix-array samples are inconsistent with the BWT (%llu LF walks disagree, "
                      "%llu of %llu rows reached)",
                      diag.sa_mismatch, diag.rows_seen, (unsigned long long)n);
-  }
+  return 0;
+}
 
-  // ---- k-mer interval table ----
-  uint32_t kk = h->opts.ktab_k;
+// ---- k-mer interval table of order kk (the option: 0 = auto, 0xffffffff = none) ----
+static int build_ktab(DeviceIndex& d, uint32_t kk, cudaStream_t st) {
+  const uint64_t n = d.n;
   if (kk == 0) kk = auto_ktab_k(n);
   if (kk == 0xffffffffu) kk = 0;
   if (kk > 16) kk = 16;
-  if (kk > 0) {
-    MTSV_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-    while (kk > 1 && (1ull << (2 * kk)) * 8ull * 5 / 4 > free_b / 3) --kk;
-    uint64_t size = 1ull << (2 * kk);
-    MTSV_TRY(dev_alloc(d.ktab, size, &d.device_bytes));
-    if (kk >= 1) {
-      DevPtr<uint2> d_ktmp;
-      MTSV_TRY(dev_alloc(d_ktmp, kk >= 2 ? (1ull << (2 * (kk - 1))) : 1));
-      // levels alternate between the two buffers so that level kk lands in d.ktab
-      uint2* bufs[2] = {d.ktab.get(), d_ktmp.get()};
-      int cur = (kk % 2 == 0) ? 0 : 1;  // level 0 buffer
-      MTSV_LAUNCH(ktab_init_kernel, 1, 1, 0, st, bufs[cur], (uint32_t)n);
-      uint64_t cur_size = 1;
-      for (uint32_t lev = 1; lev <= kk; ++lev) {
-        uint64_t threads = cur_size * 4;
-        MTSV_LAUNCH(ktab_level_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, d.fm_view(),
-                    bufs[cur], bufs[cur ^ 1], lev);
-        cur ^= 1;
-        cur_size *= 4;
-      }
-      // row indexes of ordinary entries must stay below the direct tag; MTSV_B200_KTAB_DIRECT=0 is an A/B knob
-      const char* de = getenv("MTSV_B200_KTAB_DIRECT");
-      if (n < ((uint64_t)kKtabDirectTag << 24) && !(de && de[0] == '0')) {
-        MTSV_LAUNCH(ktab_direct_kernel, (unsigned)((size + 255) / 256), 256, 0, st, d.fm_view(), d.sa_view(),
-                    d.text.get(), d.ktab.get(), size);
-        d.ktab_direct = 1;
-      }
-      MTSV_CUDA_TRY(cudaGetLastError());
-      MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-    }
+  if (kk == 0) return 0;
+  size_t free_b = 0, total_b = 0;
+  MTSV_CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+  while (kk > 1 && (1ull << (2 * kk)) * 8ull * 5 / 4 > free_b / 3) --kk;
+  const uint64_t size = 1ull << (2 * kk);
+  MTSV_TRY(dev_alloc(d.ktab, size, &d.device_bytes));
+  DevPtr<uint2> d_ktmp;
+  MTSV_TRY(dev_alloc(d_ktmp, kk >= 2 ? (1ull << (2 * (kk - 1))) : 1));
+  // levels alternate between the two buffers so that level kk lands in d.ktab
+  uint2* bufs[2] = {d.ktab.get(), d_ktmp.get()};
+  int cur = (kk % 2 == 0) ? 0 : 1;  // level 0 buffer
+  MTSV_LAUNCH(ktab_init_kernel, 1, 1, 0, st, bufs[cur], (uint32_t)n);
+  uint64_t cur_size = 1;
+  for (uint32_t lev = 1; lev <= kk; ++lev) {
+    uint64_t threads = cur_size * 4;
+    MTSV_LAUNCH(ktab_level_kernel, (unsigned)((threads + 255) / 256), 256, 0, st, d.fm_view(),
+                bufs[cur], bufs[cur ^ 1], lev);
+    cur ^= 1;
+    cur_size *= 4;
   }
+  // row indexes of ordinary entries must stay below the direct tag; MTSV_B200_KTAB_DIRECT=0 is an A/B knob
+  const char* de = getenv("MTSV_B200_KTAB_DIRECT");
+  if (n < ((uint64_t)kKtabDirectTag << 24) && !(de && de[0] == '0')) {
+    MTSV_LAUNCH(ktab_direct_kernel, (unsigned)((size + 255) / 256), 256, 0, st, d.fm_view(), d.sa_view(),
+                d.text.get(), d.ktab.get(), size);
+    d.ktab_direct = 1;
+  }
+  MTSV_CUDA_TRY(cudaGetLastError());
+  MTSV_CUDA_TRY(cudaStreamSynchronize(st));  // (before d_ktmp is freed)
   d.ktab_k = kk;
-  MTSV_CUDA_TRY(cudaStreamSynchronize(st));
-  double t1 = now_s();
+  return 0;
+}
+
+int index_assemble(IndexParts parts, int device, const mtsvgpu_index_opts* opts, mtsvgpu_index** out) {
+  const double t0 = now_s();
+  if (!parts.text || !parts.bins || !parts.bwt || (!parts.sa_sample && !parts.d_sa_full) || !out)
+    return set_error(MTSVGPU_EINVAL, "null argument");
+  *out = nullptr;
+  MTSV_TRY(check_parts(parts));
+  MTSV_TRY(use_device(device));
+  IndexPtr h(nullptr, index_destroy);
+  MTSV_TRY(create_handle(device, opts, h));
+  DeviceIndex& d = h->ix;
+  d.n = parts.n;
+  d.n_bins = parts.n_bins;
+  d.file_sa_rate = parts.sa_rate;
+  const cudaStream_t st = h->stream;
+  MTSV_TRY(upload_text_bins(d, parts, st));
+  DevPtr<PackDiag> d_diag;
+  double t_relayout0 = 0;
+  MTSV_TRY(relayout_bwt(d, parts, st, d_diag, &t_relayout0));
+  if (parts.d_sa_full)
+    MTSV_TRY(sa_from_full(d, h->opts.sa_rate, parts.d_sa_full, st));
+  else
+    MTSV_TRY(sa_from_samples(d, h->opts.sa_rate, parts, d_diag.get(), st));
+  MTSV_TRY(build_ktab(d, h->opts.ktab_k, st));
+  // (each stage from the re-layout on synchronises the stream after its last device work: the load is complete)
+  const double t1 = now_s();
   d.relayout_seconds = t1 - t_relayout0;
   d.load_seconds = t1 - t0;
-  *out = guard.release();
+  *out = h.release();
   return 0;
 }
 

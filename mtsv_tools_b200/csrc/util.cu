@@ -1,4 +1,5 @@
-// util.cu — error plumbing, device selection, memory allocation and the exclusive-scan primitive used between stages.
+// util.cu — error plumbing, device selection, memory allocation, stream and event creation and the exclusive-scan
+// primitive used between stages.
 #include <stdio.h>
 
 #include "ctx.h"
@@ -54,6 +55,40 @@ int pinned_alloc(void** p, size_t bytes, unsigned flags) {
   (void)cudaGetLastError();
   *p = nullptr;
   return set_error(MTSVGPU_ENOMEM, "cudaHostAlloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
+}
+
+void CudaStreamDestroy::operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+void CudaEventDestroy::operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+
+int stream_create(Stream& s) {
+  cudaStream_t q = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return set_error(MTSVGPU_ECUDA, "cudaStreamCreateWithFlags failed: %s", cudaGetErrorString(e));
+  }
+  s.reset(q);
+  return 0;
+}
+
+int event_create(Event& ev, unsigned flags) {
+  cudaEvent_t q = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&q, flags);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();
+    return set_error(MTSVGPU_ECUDA, "cudaEventCreateWithFlags(%#x) failed: %s", flags, cudaGetErrorString(e));
+  }
+  ev.reset(q);
+  return 0;
+}
+
+int events_reserve(std::vector<Event>& pool, size_t n, unsigned flags) {
+  while (pool.size() < n) {
+    Event e;
+    MTSV_TRY(event_create(e, flags));
+    pool.push_back(std::move(e));
+  }
+  return 0;
 }
 
 int use_device(int device) {

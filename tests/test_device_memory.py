@@ -92,7 +92,9 @@ def _free_bytes():
 def test_device_memory_comes_back(ref, reads):
     """Indexes that are opened, used and closed, an index rejected after its device allocations, and the collapse
     and edit-distance entry points: after a warm-up round, further rounds leave the free device memory where it
-    was, to well below the footprint of one open index."""
+    was, to well below the footprint of one open index.  One index runs host-API batches of several slices with
+    per-stage timing on, so that its streams and events (both lanes, the emit events, the profiling pool, the
+    overlapped copy-out) are in use when it is closed."""
     cat, off, gi, tax, oix = ref
     host, d_seqs, d_off, n = reads
     # two '$' in the BWT: found by the re-layout kernel, after the index's arrays are on the device
@@ -114,6 +116,11 @@ def test_device_memory_comes_back(ref, reads):
             footprint = max(footprint, base - _free_bytes())
         with MGIndex.build(cat, off, gi, tax) as g:
             g.bin_reads_device(d_seqs.data_ptr(), d_off.data_ptr(), n)
+            footprint = max(footprint, base - _free_bytes())
+        with _from_parts(oix, batch_reads=500) as g:  # 8 slices, alternating between the two lanes
+            g.set_profiling(True)
+            for _ in range(2):  # the second call copies its results out slice by slice
+                g.bin_reads_pinned(host)
             footprint = max(footprint, base - _free_bytes())
         with pytest.raises(LibraryError) as ei:
             _from_parts(oix, bwt=bwt2)
