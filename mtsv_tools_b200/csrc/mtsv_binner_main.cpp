@@ -14,7 +14,7 @@
 //                     bit planes the device consumes (mtsvgpu_pack_read: no intermediate copy of the bases);
 //                     the same pool later formats result lines
 //   one thread per GPU (--gpus) gathers parsed blocks into batches in page-locked memory, calls the library,
-//                     keeps the results; batches go to the GPUs round-robin
+//                     keeps the results; each GPU takes the next batch whenever it is free
 //   writer thread     appends the formatted batches in input order (so results are deterministic and
 //                     resume-by-results is exact)
 //
@@ -40,7 +40,6 @@
 #include <mutex>
 #include <string>
 #include <thread>
-#include <tuple>
 #include <unordered_set>
 #include <vector>
 
@@ -137,60 +136,51 @@ bool read_ids_from_results(const char* path, std::unordered_set<std::string>* id
   char* line = nullptr;
   size_t cap = 0;
   ssize_t n;
-  while ((n = getline(&line, &cap, f)) >= 0) {
+  bool ok = true;
+  while (ok && (n = getline(&line, &cap, f)) >= 0) {
     std::string s(line, (size_t)n);
     while (!s.empty() && isspace((unsigned char)s.back())) s.pop_back();
-    size_t b = 0;
-    while (b < s.size() && isspace((unsigned char)s[b])) ++b;
-    if (b == s.size()) continue;
-    size_t colon = s.rfind(':');  // rsplitn(2, ':')
-    if (colon == std::string::npos || colon == 0) {
-      *err = "Missing read id";
-      free(line);
-      fclose(f);
-      return false;
-    }
-    ids->insert(s.substr(0, colon));
+    if (s.empty()) continue;  // (a blank line)
+    const size_t colon = s.rfind(':');  // rsplitn(2, ':')
+    ok = colon != std::string::npos && colon != 0;
+    if (ok) ids->insert(s.substr(0, colon));
   }
   free(line);
   fclose(f);
-  return true;
+  if (!ok) *err = "Missing read id";
+  return ok;
 }
 
-bool resume_offset(const char* results, const char* input, bool fastq, uint64_t* offset, std::string* err) {
-  struct stat sb;
-  if (stat(results, &sb) != 0) {
-    *offset = 0;
-    return true;
-  }
-  std::unordered_set<std::string> ids;
-  if (!read_ids_from_results(results, &ids, err)) return false;
-  FastxBlocks in(input, fastq);
-  if (!in.ok()) {
-    *err = "cannot open input";
-    return false;
-  }
-  std::string text, id;
-  uint64_t n, idx = 0, last = 0;
-  bool any = false;
+// f(record) for every record of a FASTA / FASTQ file; 0 at its end, else FastxBlocks::next's error or -3 (no file)
+template <class F>
+int for_each_record(const char* path, bool fastq, F f) {
+  FastxBlocks in(path, fastq);
+  if (!in.ok()) return -3;
+  std::string text;
+  uint64_t n;
   int rc;
   while ((rc = in.next(&text, &n)) == 1) {
     Lines ln{text.data(), text.data() + text.size()};
     FastxRecord r;
-    while (next_record(ln, fastq, true, &r) == 1) {
-      if (ids.count(id.assign(r.id, r.id_end))) {
-        last = idx;
-        any = true;
-      }
-      ++idx;
-    }
+    while (next_record(ln, fastq, true, &r) == 1) f(r);
   }
-  if (rc < 0) {
-    *err = rc == -1 ? "parse error while scanning input" : "cannot read input";
-    return false;
-  }
-  *offset = any ? last + 1 : 0;
-  return true;
+  return rc;
+}
+
+// the number of input records up to the last one that has a line in the results file (0 when none has)
+bool resume_offset(const char* results, const char* input, bool fastq, uint64_t* offset, std::string* err) {
+  std::unordered_set<std::string> ids;
+  if (!read_ids_from_results(results, &ids, err)) return false;
+  std::string id;
+  uint64_t idx = 0;
+  *offset = 0;
+  const int rc = for_each_record(input, fastq, [&](const FastxRecord& r) {
+    if (ids.count(id.assign(r.id, r.id_end))) *offset = idx + 1;
+    ++idx;
+  });
+  if (rc == 0) return true;
+  *err = rc == -3 ? "cannot open input" : rc == -1 ? "parse error while scanning input" : "cannot read input";
+  return false;
 }
 
 void usage() {
@@ -218,10 +208,180 @@ void usage() {
           "                                 than 4096 bases get no assignments; default: warn and go on)\n");
 }
 
+struct Options {
+  const char *fasta = nullptr, *fastq = nullptr, *index = nullptr, *results = nullptr;
+  mtsvgpu_params p{0.13, 18, 15, 0.015, 2000, 200, -1, -1, 2, 0};
+  uint64_t read_offset = 0, batch_reads = 1u << 19;
+  bool long_fmt = false, force = false, dump_reads = false, strict_limits = false;
+  int device = 0, n_gpus = 1, n_threads = 0;
+  bool dump_mt = false;  // test hook: the pipeline without a GPU, printing "id<TAB>length" of each read to stdout
+  const char* input() const { return fasta ? fasta : fastq; }
+  bool is_fastq() const { return fastq != nullptr; }
+};
 
-// ------------------------------------------------------------------------------------------
-// pipeline
-// ------------------------------------------------------------------------------------------
+constexpr int kGoOn = -1;  // the steps of main return this when the run goes on, else the process's exit code
+
+int parse_args(int argc, char** argv, Options* o) {
+  auto need = [&](int& i) -> const char* {
+    if (i + 1 >= argc) {
+      fprintf(stderr, "error: %s requires a value\n", argv[i]);
+      exit(1);
+    }
+    return argv[++i];
+  };
+  mtsvgpu_params& p = o->p;
+  for (int i = 1; i < argc; ++i) {
+    std::string a = argv[i];
+    if (a == "--fasta" || a == "-fa" || a == "-f") o->fasta = need(i);
+    else if (a == "--fastq" || a == "-fq") o->fastq = need(i);
+    else if (a == "--index" || a == "-i") o->index = need(i);
+    else if (a == "--results" || a == "-m") o->results = need(i);
+    else if (a == "--threads" || a == "-t") o->n_threads = atoi(need(i));
+    else if (a == "--edit-rate" || a == "-e") p.edit_rate = atof(need(i));
+    else if (a == "--seed-size") p.seed_size = (uint32_t)strtoul(need(i), nullptr, 10);
+    else if (a == "--seed-interval") p.seed_gap = (uint32_t)strtoul(need(i), nullptr, 10);
+    else if (a == "--min-seed") p.min_seed = atof(need(i));
+    else if (a == "--max-hits") p.max_hits = strtoull(need(i), nullptr, 10);
+    else if (a == "--tune-max-hits") p.tune_max_hits = strtoull(need(i), nullptr, 10);
+    else if (a == "--max-assignments") p.max_assignments = strtoll(need(i), nullptr, 10);
+    else if (a == "--max-candidates") p.max_candidates = strtoll(need(i), nullptr, 10);
+    else if (a == "--read-offset") o->read_offset = strtoull(need(i), nullptr, 10);
+    else if (a == "--output-format") o->long_fmt = std::string(need(i)) == "long";
+    else if (a == "--force-overwrite") o->force = true;
+    else if (a == "-v") g_verbose = true;
+    else if (a == "--gpu") o->device = atoi(need(i));
+    else if (a == "--gpus") o->n_gpus = atoi(need(i));
+    else if (a == "--strict-limits") o->strict_limits = true;
+    else if (a == "--dump-reads") o->dump_reads = true;  // test hook: parse the input, print "id<TAB>seq", no GPU
+    else if (a == "--dump-reads-mt") o->dump_reads = true, o->n_threads = o->n_threads ? o->n_threads : -1;  // same through the pipeline's scanner + parser
+    else if (a == "--batch-reads") o->batch_reads = strtoull(need(i), nullptr, 10);
+    else if (a == "-h" || a == "--help") {
+      usage();
+      return 0;
+    } else {
+      fprintf(stderr, "error: unknown argument %s\n", a.c_str());
+      usage();
+      return 1;
+    }
+  }
+  o->dump_mt = o->dump_reads && o->n_threads != 0;
+  return kGoOn;
+}
+
+int check_options(Options* o) {
+  if ((!o->fasta && !o->fastq) || (o->fasta && o->fastq) || (!o->index && !o->dump_mt)) {
+    usage();
+    return 1;
+  }
+  // validation as src/bin/mtsv-binner.rs:151,195 (the reference panics; exit code 101 there)
+  if (o->p.edit_rate < 0.0 || o->p.edit_rate > 1.0) {
+    logf("ERROR", "Edit tolerance proportion must be between 0 and 1, inclusive");
+    return 101;
+  }
+  if (o->p.min_seed <= 0.0 || o->p.min_seed > 1.0) {
+    logf("ERROR", "Min seed percent must be between 0 and 1");
+    return 101;
+  }
+  if (o->p.seed_size < 16) logf("WARN", "Seed size may be small enough that it causes performance issues.");
+  else if (o->p.seed_size > 24) logf("WARN", "Seed size may be large enough that significant results are ignored.");
+  if (!o->results && !o->dump_mt) {
+    logf("ERROR", "No results path provided!");
+    return 3;  // :262-265
+  }
+  if (o->n_gpus < 1) o->n_gpus = 1;
+  if (o->n_threads <= 0) o->n_threads = (int)std::max(1u, std::thread::hardware_concurrency());
+  if (o->batch_reads == 0) o->batch_reads = 1;
+  return kGoOn;
+}
+
+// test hook --dump-reads: parse the input on this thread, print "id<TAB>seq" of every record from --read-offset on
+int dump_reads(const Options& o) {
+  uint64_t idx = 0;
+  const int rc = for_each_record(o.input(), o.is_fastq(), [&](const FastxRecord& r) {
+    if (idx++ < o.read_offset) return;
+    fwrite(r.id, 1, (size_t)(r.id_end - r.id), stdout);
+    putchar('\t');
+    Lines sl{r.seq, r.seq_end};
+    const char *b, *e;
+    while (sl.next(&b, &e)) fwrite(b, 1, (size_t)(e - b), stdout);
+    putchar('\n');
+  });
+  return rc == -3 ? 2 : rc < 0 ? 12 : 0;
+}
+
+// An existing results file is appended to, and the run resumes after the last read it holds, unless
+// --force-overwrite is given (src/binner.rs:54-61).  --dump-reads-mt writes to stdout.
+int open_results(Options* o, FILE** out) {
+  *out = stdout;
+  if (o->dump_mt) return kGoOn;
+  struct stat sb;
+  const bool append = !o->force && stat(o->results, &sb) == 0;
+  if (append) {
+    uint64_t resume = 0;
+    std::string err;
+    if (!resume_offset(o->results, o->input(), o->is_fastq(), &resume, &err)) {
+      logf("ERROR", "Error computing resume offset: %s", err.c_str());
+      return 4;  // :288-291
+    }
+    logf("INFO", "Existing results detected at %s; resuming after read offset %llu", o->results,
+         (unsigned long long)resume);
+    o->read_offset += resume;
+  }
+  if (!(*out = fopen(o->results, append ? "a" : "w"))) {
+    logf("ERROR", "Error running query: cannot open %s: %s", o->results, strerror(errno));
+    return 2;
+  }
+  return kGoOn;
+}
+
+struct IndexClose {
+  void operator()(mtsvgpu_index* ix) const { mtsvgpu_index_close(ix); }
+};
+struct HostFree {
+  void operator()(void* p) const { mtsvgpu_host_free(p); }
+};
+using Index = std::unique_ptr<mtsvgpu_index, IndexClose>;
+
+// A first small batch brings in what a fresh process pays once (kernel images, workspaces, page-locked result
+// buffers) while the other devices and the reader start up.  Its results are discarded.
+void warm_up(mtsvgpu_index* ix, int g, const Options& o) {
+  std::vector<uint8_t> seq(256 * 150);
+  std::vector<uint64_t> off(257);
+  uint32_t x = 12345u + (uint32_t)g;
+  for (auto& c : seq) c = (uint8_t)"ACGT"[(x = x * 1664525u + 1013904223u) >> 30];
+  for (size_t i = 0; i <= 256; ++i) off[i] = i * 150;
+  const mtsvgpu_hit* wh = nullptr;
+  const mtsvgpu_taxhit* wt = nullptr;
+  const uint64_t* wo = nullptr;
+  uint64_t wn = 0;
+  if (o.long_fmt) (void)mtsvgpu_bin_batch_pinned(ix, seq.data(), off.data(), 256, &o.p, &wh, &wo, &wn);
+  else (void)mtsvgpu_assign_batch_pinned(ix, seq.data(), off.data(), 256, &o.p, &wt, &wo, &wn);
+}
+
+// One handle per GPU, opened and warmed up side by side (null handles for --dump-reads-mt); none when one fails.
+std::vector<Index> open_indexes(const Options& o) {
+  std::vector<Index> ix((size_t)o.n_gpus);
+  if (o.dump_mt) return ix;
+  logf("INFO", "Deserializing candidate filter ...");
+  std::vector<std::thread> openers;
+  std::vector<std::string> errs((size_t)o.n_gpus);
+  for (int g = 0; g < o.n_gpus; ++g)
+    openers.emplace_back([&, g] {
+      mtsvgpu_index* h = nullptr;
+      if (mtsvgpu_index_open(o.index, o.device + g, nullptr, &h) == 0) warm_up(h, g, o);
+      else errs[(size_t)g] = mtsvgpu_last_error();
+      ix[(size_t)g].reset(h);
+    });
+  for (auto& t : openers) t.join();
+  for (int g = 0; g < o.n_gpus; ++g)
+    if (!ix[(size_t)g]) {
+      logf("ERROR", "Error running query: %s", errs[(size_t)g].c_str());
+      return {};
+    }
+  return ix;
+}
+
+// ---- pipeline ----
 struct TextBlock {  // whole records, as they stand in the file
   uint64_t seq = 0;
   std::string text;
@@ -234,7 +394,6 @@ struct ParsedBlock {
   std::vector<uint32_t> len;      // bases per read
   std::vector<uint32_t> id_end;   // end of each id inside `ids`
   std::string ids;
-  bool bad = false;
 };
 
 struct Batch {
@@ -246,73 +405,10 @@ struct Batch {
   std::vector<uint64_t> hit_off;
   std::vector<std::string> text;  // one per part, filled by the formatter tasks
   std::atomic<uint32_t> pending{0};
-  uint64_t lines = 0;
 };
 
-class Pool {  // fixed set of workers running queued tasks
- public:
-  explicit Pool(int n) {
-    for (int i = 0; i < n; ++i) th_.emplace_back([this] { run(); });
-  }
-  ~Pool() {
-    {
-      std::lock_guard<std::mutex> lk(mu_);
-      stop_ = true;
-    }
-    cv_.notify_all();
-    for (auto& t : th_) t.join();
-  }
-  void submit(std::function<void()> f) {
-    {
-      std::lock_guard<std::mutex> lk(mu_);
-      q_.push_back(std::move(f));
-    }
-    cv_.notify_one();
-  }
-
- private:
-  void run() {
-    for (;;) {
-      std::function<void()> f;
-      {
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_.wait(lk, [this] { return stop_ || !q_.empty(); });
-        if (q_.empty()) return;
-        f = std::move(q_.front());
-        q_.pop_front();
-      }
-      f();
-    }
-  }
-  std::mutex mu_;
-  std::condition_variable cv_;
-  std::deque<std::function<void()>> q_;
-  std::vector<std::thread> th_;
-  bool stop_ = false;
-};
-
-struct Shared {
-  std::mutex mu;
-  std::condition_variable cv;
-  int exit_code = 0;
-  std::string error;
-  void fail(int code, const std::string& msg) {
-    std::lock_guard<std::mutex> lk(mu);
-    if (exit_code == 0) {
-      exit_code = code;
-      error = msg;
-    }
-    cv.notify_all();
-  }
-  bool failed() {
-    std::lock_guard<std::mutex> lk(mu);
-    return exit_code != 0;
-  }
-};
-
-// parse + pack one block of whole records, all but the first `skip` (a pool task)
-void parse_block(const TextBlock& tb, bool fastq, uint64_t skip, ParsedBlock* out) {
-  out->n = 0;
+// parse + pack one block of whole records, all but the first `skip` (a worker's task); false at a read too long
+bool parse_block(const TextBlock& tb, bool fastq, uint64_t skip, ParsedBlock* out) {
   out->len.reserve(tb.n_records - skip);
   out->id_end.reserve(tb.n_records - skip);
   out->packed.reserve(tb.text.size() / 4);
@@ -321,10 +417,7 @@ void parse_block(const TextBlock& tb, bool fastq, uint64_t skip, ParsedBlock* ou
   std::string multi;
   for (uint64_t i = 0; next_record(ln, fastq, true, &r) == 1; ++i) {
     if (i < skip) continue;
-    if (r.len > 0xfffffff0ull) {
-      out->bad = true;
-      return;
-    }
+    if (r.len > 0xfffffff0ull) return false;
     out->ids.append(r.id, r.id_end);
     out->id_end.push_back((uint32_t)out->ids.size());
     const char* seq = r.seq;
@@ -341,416 +434,323 @@ void parse_block(const TextBlock& tb, bool fastq, uint64_t skip, ParsedBlock* ou
     out->len.push_back((uint32_t)r.len);
     ++out->n;
   }
+  return true;
 }
 
-}  // namespace
+// page-locked memory for a GPU thread's batch input
+struct PinnedBuf {
+  std::unique_ptr<void, HostFree> p;
+  size_t cap = 0;
+  bool fit(size_t need, size_t grown) {  // false: `need` bytes do not fit and `grown` bytes cannot be allocated
+    if (need > cap) {
+      p.reset();  // (the old buffer is freed before the new one is allocated)
+      p.reset(mtsvgpu_host_alloc(cap = grown));
+    }
+    return p != nullptr;
+  }
+};
 
-int main(int argc, char** argv) {
-  const char *fasta = nullptr, *fastq = nullptr, *index = nullptr, *results = nullptr;
-  mtsvgpu_params p{0.13, 18, 15, 0.015, 2000, 200, -1, -1, 2, 0};
-  uint64_t read_offset = 0, batch_reads = 1u << 19;
-  bool long_fmt = false, force = false, dump_reads = false, strict_limits = false;
-  int device = 0, n_gpus = 1, n_threads = 0;
-  auto need = [&](int& i) -> const char* {
-    if (i + 1 >= argc) {
-      fprintf(stderr, "error: %s requires a value\n", argv[i]);
-      exit(1);
-    }
-    return argv[++i];
-  };
-  for (int i = 1; i < argc; ++i) {
-    std::string a = argv[i];
-    if (a == "--fasta" || a == "-fa" || a == "-f") fasta = need(i);
-    else if (a == "--fastq" || a == "-fq") fastq = need(i);
-    else if (a == "--index" || a == "-i") index = need(i);
-    else if (a == "--results" || a == "-m") results = need(i);
-    else if (a == "--threads" || a == "-t") n_threads = atoi(need(i));
-    else if (a == "--edit-rate" || a == "-e") p.edit_rate = atof(need(i));
-    else if (a == "--seed-size") p.seed_size = (uint32_t)strtoul(need(i), nullptr, 10);
-    else if (a == "--seed-interval") p.seed_gap = (uint32_t)strtoul(need(i), nullptr, 10);
-    else if (a == "--min-seed") p.min_seed = atof(need(i));
-    else if (a == "--max-hits") p.max_hits = strtoull(need(i), nullptr, 10);
-    else if (a == "--tune-max-hits") p.tune_max_hits = strtoull(need(i), nullptr, 10);
-    else if (a == "--max-assignments") p.max_assignments = strtoll(need(i), nullptr, 10);
-    else if (a == "--max-candidates") p.max_candidates = strtoll(need(i), nullptr, 10);
-    else if (a == "--read-offset") read_offset = strtoull(need(i), nullptr, 10);
-    else if (a == "--output-format") long_fmt = std::string(need(i)) == "long";
-    else if (a == "--force-overwrite") force = true;
-    else if (a == "-v") g_verbose = true;
-    else if (a == "--gpu") device = atoi(need(i));
-    else if (a == "--gpus") n_gpus = atoi(need(i));
-    else if (a == "--strict-limits") strict_limits = true;
-    else if (a == "--dump-reads") dump_reads = true;  // test hook: parse the input, print "id<TAB>seq", no GPU
-    else if (a == "--dump-reads-mt") dump_reads = true, n_threads = n_threads ? n_threads : -1;  // same through the pipeline's scanner + parser
-    else if (a == "--batch-reads") batch_reads = strtoull(need(i), nullptr, 10);
-    else if (a == "-h" || a == "--help") {
-      usage();
-      return 0;
-    } else {
-      fprintf(stderr, "error: unknown argument %s\n", a.c_str());
-      usage();
-      return 1;
-    }
-  }
-  const bool dump_mt = dump_reads && n_threads != 0;
-  if (dump_reads && !dump_mt && (fasta || fastq)) {
-    FastxBlocks in(fasta ? fasta : fastq, fastq != nullptr);
-    if (!in.ok()) return 2;
-    std::string text;
-    uint64_t n, idx = 0;
-    int rc;
-    while ((rc = in.next(&text, &n)) == 1) {
-      Lines ln{text.data(), text.data() + text.size()};
-      FastxRecord r;
-      while (next_record(ln, fastq != nullptr, true, &r) == 1) {
-        if (idx++ < read_offset) continue;
-        fwrite(r.id, 1, (size_t)(r.id_end - r.id), stdout);
-        putchar('\t');
-        Lines sl{r.seq, r.seq_end};
-        const char *b, *e;
-        while (sl.next(&b, &e)) fwrite(b, 1, (size_t)(e - b), stdout);
-        putchar('\n');
-      }
-    }
-    return rc < 0 ? 12 : 0;
-  }
-  if ((!fasta && !fastq) || (fasta && fastq) || (!index && !dump_mt)) {
-    usage();
-    return 1;
-  }
-  // validation as src/bin/mtsv-binner.rs:151,195 (the reference panics; exit code 101 there)
-  if (p.edit_rate < 0.0 || p.edit_rate > 1.0) {
-    logf("ERROR", "Edit tolerance proportion must be between 0 and 1, inclusive");
-    return 101;
-  }
-  if (p.min_seed <= 0.0 || p.min_seed > 1.0) {
-    logf("ERROR", "Min seed percent must be between 0 and 1");
-    return 101;
-  }
-  if (p.seed_size < 16) logf("WARN", "Seed size may be small enough that it causes performance issues.");
-  else if (p.seed_size > 24) logf("WARN", "Seed size may be large enough that significant results are ignored.");
-  if (!results && !dump_mt) {
-    logf("ERROR", "No results path provided!");
-    return 3;  // :262-265
-  }
-  if (n_gpus < 1) n_gpus = 1;
-  if (n_threads <= 0) n_threads = (int)std::max(1u, std::thread::hardware_concurrency());
-  if (batch_reads == 0) batch_reads = 1;
-  const char* input = fasta ? fasta : fastq;
-  const bool is_fastq = fastq != nullptr;
-  struct stat sb;
-  const bool append = !dump_mt && !force && stat(results, &sb) == 0;
-  uint64_t resume = 0;
-  if (!force && !dump_mt) {
-    std::string err;
-    if (!resume_offset(results, input, is_fastq, &resume, &err)) {
-      logf("ERROR", "Error computing resume offset: %s", err.c_str());
-      return 4;  // :288-291
-    }
-    if (append) logf("INFO", "Existing results detected at %s; resuming after read offset %llu", results,
-                     (unsigned long long)resume);
-  }
-  read_offset += resume;
+// The threads of one run (see the top of the file), their shared state and their stages.  One mutex guards the queues
+// and the failure, so a failure wakes every wait.  run() returns once all threads, workers included, have ended.
+class Pipeline {
+ public:
+  Pipeline(const Options& o, FastxBlocks& blocks, FILE* out, const std::vector<Index>& ix)
+      : o_(o), blocks_(blocks), out_(out), ix_(ix) {}
+  std::atomic<uint64_t> total_reads{0}, total_lines{0}, over_len{0}, over_hits{0};
 
-  FILE* out = dump_mt ? stdout : fopen(results, append ? "a" : "w");  // src/binner.rs:54-61
-  if (!out) {
-    logf("ERROR", "Error running query: cannot open %s: %s", results, strerror(errno));
-    return 2;
-  }
-  FastxBlocks blocks(input, is_fastq);  // src/binner.rs:21-33
-  if (!blocks.ok()) {
-    logf("ERROR", "Error running query: cannot open %s", input);
-    if (!dump_mt) fclose(out);
-    return 2;
-  }
-  std::vector<mtsvgpu_index*> handles((size_t)n_gpus, nullptr);
-  if (!dump_mt) {
-    logf("INFO", "Deserializing candidate filter ...");
-    std::vector<std::thread> openers;
-    std::vector<std::string> errs((size_t)n_gpus);
-    for (int g = 0; g < n_gpus; ++g)
-      openers.emplace_back([&, g] {
-        if (mtsvgpu_index_open(index, device + g, nullptr, &handles[(size_t)g]) != 0) {
-          errs[(size_t)g] = mtsvgpu_last_error();
-          return;
-        }
-        // a first small batch brings in what a fresh process pays once (kernel images, workspaces, page-locked
-        // result buffers) while the other devices and the reader start up; its results are discarded
-        std::vector<uint8_t> wseq(256 * 150);
-        std::vector<uint64_t> woff(257);
-        uint32_t x = 12345u + (uint32_t)g;
-        for (auto& c : wseq) c = (uint8_t)"ACGT"[(x = x * 1664525u + 1013904223u) >> 30];
-        for (size_t i = 0; i <= 256; ++i) woff[i] = i * 150;
-        const uint64_t* wo = nullptr;
-        uint64_t wn = 0;
-        if (long_fmt) {
-          const mtsvgpu_hit* wh = nullptr;
-          (void)mtsvgpu_bin_batch_pinned(handles[(size_t)g], wseq.data(), woff.data(), 256, &p, &wh, &wo, &wn);
-        } else {
-          const mtsvgpu_taxhit* wt = nullptr;
-          (void)mtsvgpu_assign_batch_pinned(handles[(size_t)g], wseq.data(), woff.data(), 256, &p, &wt, &wo, &wn);
+  int run() {
+    std::vector<std::thread> workers, gpus;
+    for (int i = 0; i < o_.n_threads; ++i) workers.emplace_back([this] { work(); });
+    std::thread reader([this] { read_blocks(); });
+    std::thread writer([this] { write_batches(); });
+    for (int g = 0; g < o_.n_gpus; ++g)
+      gpus.emplace_back([this, g] {
+        PinnedBuf packed, off;
+        while (std::shared_ptr<Batch> b = take_batch()) {
+          if (!o_.dump_mt && !compute(g, b.get(), &packed, &off)) break;
+          queue_format(b);
         }
       });
-    for (auto& t : openers) t.join();
-    for (int g = 0; g < n_gpus; ++g)
-      if (!handles[(size_t)g]) {
-        logf("ERROR", "Error running query: %s", errs[(size_t)g].c_str());
-        for (auto h : handles) mtsvgpu_index_close(h);
-        fclose(out);
-        return 2;
-      }
+    for (auto& t : gpus) t.join();
+    reader.join();
+    {
+      std::lock_guard<std::mutex> lk(mu_);  // no task is queued after this: the workers end once the queue is empty
+      batches_total_ = batch_seq_;
+      stop_ = true;
+      done_cv_.notify_all();
+      task_cv_.notify_all();
+    }
+    writer.join();
+    for (auto& t : workers) t.join();
+    if (code_) logf("ERROR", "%s", error_.c_str());
+    return code_;
   }
-  logf("INFO", "Beginning queries.");
-  auto t0 = std::chrono::steady_clock::now();
 
-  Shared sh;
-  // a failure anywhere in the pipeline is raised through `sh`, not through every stage's condition variable: waits
-  // re-check it at short intervals
-  auto wait_on = [](std::condition_variable& cv, std::unique_lock<std::mutex>& lk, auto pred) {
-    while (!pred()) cv.wait_for(lk, std::chrono::milliseconds(50));
-  };
-  Pool pool(n_threads);
-  // ---- reader -> parsed blocks (ordered by block sequence number) ----
-  std::mutex pmu;
-  std::condition_variable pcv;
-  std::map<uint64_t, std::unique_ptr<ParsedBlock>> parsed;  // finished blocks waiting for their turn
-  uint64_t blocks_issued = 0, blocks_taken = 0;
-  bool reader_done = false;
-  const uint64_t max_blocks_in_flight = (uint64_t)std::max(8, 4 * n_threads) + batch_reads / 8192;
-  std::thread reader([&] {
+ private:
+  void fail(int code, const std::string& msg) {
+    std::lock_guard<std::mutex> lk(mu_);
+    if (code_ == 0) {
+      error_ = msg;
+      code_ = code;
+    }
+    parsed_cv_.notify_all();
+    done_cv_.notify_all();
+  }
+
+  void submit(std::function<void()> task) {
+    std::lock_guard<std::mutex> lk(mu_);
+    tasks_.push_back(std::move(task));
+    task_cv_.notify_one();
+  }
+  void work() {
+    for (;;) {
+      std::function<void()> task;
+      {
+        std::unique_lock<std::mutex> lk(mu_);
+        task_cv_.wait(lk, [this] { return stop_ || !tasks_.empty(); });
+        if (tasks_.empty()) return;
+        task = std::move(tasks_.front());
+        tasks_.pop_front();
+      }
+      task();
+    }
+  }
+
+  // blocks of whole records to the parser tasks, with at most max_in_flight of them issued and not yet taken
+  void read_blocks() {
+    const uint64_t max_in_flight = (uint64_t)std::max(8, 4 * o_.n_threads) + o_.batch_reads / 8192;
     uint64_t records_seen = 0;  // complete records read so far (including skipped ones)
-    while (!sh.failed()) {
+    while (!code_) {
       auto tb = std::make_shared<TextBlock>();
-      const int rc = blocks.next(&tb->text, &tb->n_records);
+      const int rc = blocks_.next(&tb->text, &tb->n_records);
       if (rc == 0) break;
-      if (rc < 0 || blocks.malformed_next()) {  // (the records of a block that ends at a malformed one are not binned)
+      if (rc < 0 || blocks_.malformed_next()) {  // (the records of a block that ends at a malformed one are not binned)
         std::string msg = "Unable to read from input file";
         if (rc != -2) msg += ": malformed record after " + std::to_string(records_seen) + " reads";
-        sh.fail(12, msg);  // src/binner.rs:81-84
+        fail(12, msg);  // src/binner.rs:81-84
         break;
       }
       // .skip(read_offset) (src/binner.rs:176,199): whole blocks are dropped, the parser skips the first records of
       // a straddling block
       const uint64_t first = records_seen;
       records_seen += tb->n_records;
-      if (records_seen <= read_offset) continue;
-      const uint64_t skip = read_offset > first ? read_offset - first : 0;
-      uint64_t seq;
+      if (records_seen <= o_.read_offset) continue;
+      const uint64_t skip = o_.read_offset > first ? o_.read_offset - first : 0;
       {
-        std::unique_lock<std::mutex> lk(pmu);
-        wait_on(pcv, lk, [&] { return blocks_issued - blocks_taken < max_blocks_in_flight || sh.failed(); });
-        seq = blocks_issued++;
+        std::unique_lock<std::mutex> lk(mu_);
+        parsed_cv_.wait(lk, [&] { return issued_ - taken_ < max_in_flight || code_; });
+        tb->seq = issued_++;
       }
-      tb->seq = seq;
-      pool.submit([&, tb, skip] {
+      submit([this, tb, skip] {
         auto pb = std::make_unique<ParsedBlock>();
-        if (!sh.failed()) parse_block(*tb, is_fastq, skip, pb.get());
-        if (pb->bad) sh.fail(12, "Unable to read from input file: malformed record");
-        std::lock_guard<std::mutex> lk(pmu);
-        parsed[tb->seq] = std::move(pb);
-        pcv.notify_all();
+        if (!code_ && !parse_block(*tb, o_.is_fastq(), skip, pb.get()))
+          fail(12, "Unable to read from input file: malformed record");
+        std::lock_guard<std::mutex> lk(mu_);
+        parsed_[tb->seq] = std::move(pb);
+        parsed_cv_.notify_all();
       });
     }
-    std::lock_guard<std::mutex> lk(pmu);
-    reader_done = true;
-    pcv.notify_all();
-  });
+    std::lock_guard<std::mutex> lk(mu_);
+    reader_done_ = true;
+    parsed_cv_.notify_all();
+  }
 
-  // ---- batches: GPU threads take consecutive parsed blocks; formatted batches are written in order ----
-  std::mutex bmu;  // serialises "take the next blocks" so that batches are consecutive runs of blocks
-  uint64_t batch_seq = 0;
-  std::mutex wmu;
-  std::condition_variable wcv;
-  std::map<uint64_t, std::shared_ptr<Batch>> done;  // formatted (or empty) batches by sequence number
-  uint64_t batches_total = ~0ull;                   // known once the input is exhausted
-  std::atomic<uint64_t> total_reads{0}, total_lines{0}, over_len{0}, over_hits{0};
-
-  auto take_batch = [&]() -> std::shared_ptr<Batch> {
-    std::lock_guard<std::mutex> blk(bmu);
+  // consecutive parsed blocks until they hold batch_reads reads or the input ends; null when none is left or failed
+  std::shared_ptr<Batch> take_batch() {
+    std::lock_guard<std::mutex> tlk(take_mu_);
     auto b = std::make_shared<Batch>();
-    std::unique_lock<std::mutex> lk(pmu);
+    std::unique_lock<std::mutex> lk(mu_);
     for (;;) {
-      wait_on(pcv, lk, [&] { return parsed.count(blocks_taken) || (reader_done && blocks_taken == blocks_issued) || sh.failed(); });
-      if (sh.failed()) return nullptr;
-      if (!parsed.count(blocks_taken)) break;  // input exhausted
-      auto it = parsed.find(blocks_taken);
+      parsed_cv_.wait(lk, [&] { return parsed_.count(taken_) || (reader_done_ && taken_ == issued_) || code_; });
+      if (code_) return nullptr;
+      auto it = parsed_.find(taken_);
+      if (it == parsed_.end()) break;  // input exhausted
       b->n_reads += it->second->n;
       b->parts.push_back(std::move(it->second));
-      parsed.erase(it);
-      ++blocks_taken;
-      pcv.notify_all();
-      if (b->n_reads >= batch_reads) break;
+      parsed_.erase(it);
+      ++taken_;
+      parsed_cv_.notify_all();
+      if (b->n_reads >= o_.batch_reads) break;
     }
     if (b->parts.empty()) return nullptr;
-    b->seq = batch_seq++;
+    b->seq = batch_seq_++;
     return b;
-  };
+  }
 
-  auto gpu_main = [&](int g) {
-    mtsvgpu_index* ix = handles[(size_t)g];
-    uint8_t* pin_packed = nullptr;
-    uint64_t* pin_off = nullptr;
-    size_t cap_packed = 0, cap_off = 0;
-    for (;;) {
-      std::shared_ptr<Batch> b = take_batch();
-      if (!b) break;
-      size_t pbytes = 0;
-      for (auto& part : b->parts) pbytes += part->packed.size();
-      const auto tb0 = std::chrono::steady_clock::now();
-      auto since = [&](std::chrono::steady_clock::time_point t) {
-        return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
-      };
-      double ms_gather = 0, ms_call = 0;
-      if (!dump_mt) {
-        if (pbytes + 64 > cap_packed) {
-          mtsvgpu_host_free(pin_packed);
-          cap_packed = pbytes + pbytes / 4 + 4096;
-          pin_packed = (uint8_t*)mtsvgpu_host_alloc(cap_packed);
-        }
-        if ((b->n_reads + 1) * 8 > cap_off) {
-          mtsvgpu_host_free(pin_off);
-          cap_off = (b->n_reads + 1) * 8 + (b->n_reads / 4) * 8 + 4096;
-          pin_off = (uint64_t*)mtsvgpu_host_alloc(cap_off);
-        }
-        if (!pin_packed || !pin_off) {
-          sh.fail(2, std::string("Error running query: ") + mtsvgpu_last_error());
-          break;
-        }
-        size_t at = 0;
-        uint64_t r = 0, bases = 0;
-        pin_off[0] = 0;
-        for (auto& part : b->parts) {
-          memcpy(pin_packed + at, part->packed.data(), part->packed.size());
-          at += part->packed.size();
-          for (uint32_t i = 0; i < part->n; ++i) pin_off[++r] = (bases += part->len[i]);
-          std::vector<uint8_t>().swap(part->packed);
-        }
-        // default format: the library merges each read's hits into its TaxID=edit list; long: the Hit records
-        const mtsvgpu_hit* hits = nullptr;
-        const mtsvgpu_taxhit* taxhits = nullptr;
-        const uint64_t* hit_off = nullptr;
-        uint64_t n_hits = 0;
-        ms_gather = since(tb0);
-        const auto tc0 = std::chrono::steady_clock::now();
-        const int rc = long_fmt ? mtsvgpu_bin_batch_packed(ix, pin_packed, pbytes, pin_off, b->n_reads, &p, &hits,
-                                                           &hit_off, &n_hits)
-                                : mtsvgpu_assign_batch_packed(ix, pin_packed, pbytes, pin_off, b->n_reads, &p, &taxhits,
-                                                              &hit_off, &n_hits);
-        if (rc != 0) {
-          sh.fail(2, std::string("Error running query: ") + mtsvgpu_last_error());
-          break;
-        }
-        ms_call = since(tc0);
-        mtsvgpu_batch_stats bst;
-        if (mtsvgpu_last_batch_stats(ix, &bst) == 0) {
-          over_len += bst.n_reads_over_limit;
-          over_hits += bst.n_strands_over_hits;
-        }
-        if (long_fmt)  // (the handle's buffers are reused by its next batch)
-          b->hits.assign(hits, hits + n_hits);
-        else
-          b->taxhits.assign(taxhits, taxhits + n_hits);
-        b->hit_off.assign(hit_off, hit_off + b->n_reads + 1);
-        logf("DEBUG", "gpu %d batch %llu: %llu reads, %llu %s; waited+gathered %.1f ms, library call %.1f ms, results copied %.1f ms",
-             g, (unsigned long long)b->seq, (unsigned long long)b->n_reads, (unsigned long long)n_hits,
-             long_fmt ? "hits" : "assignments", ms_gather, ms_call,
-             since(tc0) - ms_call);
-      }
-      // format: one pool task per parsed block of the batch
-      b->text.resize(b->parts.size());
-      b->pending.store((uint32_t)b->parts.size());
-      uint64_t first = 0;
-      for (size_t k = 0; k < b->parts.size(); ++k) {
-        const uint64_t r0 = first;
-        first += b->parts[k]->n;
-        pool.submit([&, b, k, r0] {
-          const ParsedBlock& part = *b->parts[k];
-          std::string& text = b->text[k];
-          uint64_t lines = 0;
-          uint32_t id0 = 0;
-          for (uint32_t i = 0; i < part.n; ++i) {
-            const uint32_t id1 = part.id_end[i];
-            if (dump_mt) {
-              text.append(part.ids, id0, id1 - id0);
-              text.push_back('\t');
-              put_u64(&text, part.len[i]);
-              text.push_back('\n');
-            } else {
-              const uint64_t h0 = b->hit_off[r0 + i], h1 = b->hit_off[r0 + i + 1];
-              const size_t before = text.size();
-              if (long_fmt)
-                format_hits_long(part.ids.data() + id0, id1 - id0, b->hits.data() + h0, h1 - h0, &text);
-              else
-                format_taxhits(part.ids.data() + id0, id1 - id0, b->taxhits.data() + h0, h1 - h0, &text);
-              lines += text.size() != before;
-            }
-            id0 = id1;
-          }
-          total_lines += lines;
-          if (b->pending.fetch_sub(1) == 1) {
-            std::lock_guard<std::mutex> lk(wmu);
-            done[b->seq] = b;
-            wcv.notify_all();
-          }
-        });
-      }
-      total_reads += b->n_reads;
+  // gathers the batch into page-locked memory, runs it on GPU g, copies the results out of the handle's buffers
+  bool compute(int g, Batch* b, PinnedBuf* pin_packed, PinnedBuf* pin_off) {
+    size_t pbytes = 0;
+    for (auto& part : b->parts) pbytes += part->packed.size();
+    const auto tb0 = std::chrono::steady_clock::now();
+    auto since = [](std::chrono::steady_clock::time_point t) {
+      return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t).count();
+    };
+    const uint64_t n = b->n_reads;
+    if (!pin_packed->fit(pbytes + 64, pbytes + pbytes / 4 + 4096) ||
+        !pin_off->fit((n + 1) * 8, (n + 1) * 8 + (n / 4) * 8 + 4096)) {
+      fail(2, std::string("Error running query: ") + mtsvgpu_last_error());
+      return false;
     }
-    mtsvgpu_host_free(pin_packed);
-    mtsvgpu_host_free(pin_off);
-  };
+    uint8_t* packed = (uint8_t*)pin_packed->p.get();
+    uint64_t* off = (uint64_t*)pin_off->p.get();
+    size_t at = 0;
+    uint64_t r = 0, bases = 0;
+    off[0] = 0;
+    for (auto& part : b->parts) {
+      memcpy(packed + at, part->packed.data(), part->packed.size());
+      at += part->packed.size();
+      for (uint32_t i = 0; i < part->n; ++i) off[++r] = (bases += part->len[i]);
+      std::vector<uint8_t>().swap(part->packed);
+    }
+    // default format: the library merges each read's hits into its TaxID=edit list; long: the Hit records
+    mtsvgpu_index* ix = ix_[(size_t)g].get();
+    const mtsvgpu_hit* hits = nullptr;
+    const mtsvgpu_taxhit* taxhits = nullptr;
+    const uint64_t* hit_off = nullptr;
+    uint64_t n_hits = 0;
+    const double ms_gather = since(tb0);
+    const auto tc0 = std::chrono::steady_clock::now();
+    const int rc = o_.long_fmt ? mtsvgpu_bin_batch_packed(ix, packed, pbytes, off, n, &o_.p, &hits, &hit_off, &n_hits)
+                               : mtsvgpu_assign_batch_packed(ix, packed, pbytes, off, n, &o_.p, &taxhits, &hit_off,
+                                                             &n_hits);
+    if (rc != 0) {
+      fail(2, std::string("Error running query: ") + mtsvgpu_last_error());
+      return false;
+    }
+    const double ms_call = since(tc0);
+    mtsvgpu_batch_stats bst;
+    if (mtsvgpu_last_batch_stats(ix, &bst) == 0) {
+      over_len += bst.n_reads_over_limit;
+      over_hits += bst.n_strands_over_hits;
+    }
+    if (o_.long_fmt)
+      b->hits.assign(hits, hits + n_hits);
+    else
+      b->taxhits.assign(taxhits, taxhits + n_hits);
+    b->hit_off.assign(hit_off, hit_off + n + 1);
+    logf("DEBUG", "gpu %d batch %llu: %llu reads, %llu %s; waited+gathered %.1f ms, library call %.1f ms, results copied %.1f ms",
+         g, (unsigned long long)b->seq, (unsigned long long)n, (unsigned long long)n_hits,
+         o_.long_fmt ? "hits" : "assignments", ms_gather, ms_call, since(tc0) - ms_call);
+    return true;
+  }
 
-  std::thread writer([&] {
-    uint64_t next = 0;
-    for (;;) {
+  // one format task per parsed block of the batch; the last one to finish hands the batch to the writer
+  void queue_format(const std::shared_ptr<Batch>& b) {
+    b->text.resize(b->parts.size());
+    b->pending.store((uint32_t)b->parts.size());
+    uint64_t r0 = 0;  // the part's first read in the batch
+    for (size_t k = 0; k < b->parts.size(); ++k) {
+      submit([this, b, k, r0] {
+        const ParsedBlock& part = *b->parts[k];
+        std::string& text = b->text[k];
+        uint64_t lines = 0;
+        uint32_t id0 = 0;
+        for (uint32_t i = 0; i < part.n; ++i) {
+          const uint32_t id1 = part.id_end[i];
+          if (o_.dump_mt) {
+            text.append(part.ids, id0, id1 - id0);
+            text.push_back('\t');
+            put_u64(&text, part.len[i]);
+            text.push_back('\n');
+          } else {
+            const uint64_t h0 = b->hit_off[r0 + i], h1 = b->hit_off[r0 + i + 1];
+            const size_t before = text.size();
+            if (o_.long_fmt)
+              format_hits_long(part.ids.data() + id0, id1 - id0, b->hits.data() + h0, h1 - h0, &text);
+            else
+              format_taxhits(part.ids.data() + id0, id1 - id0, b->taxhits.data() + h0, h1 - h0, &text);
+            lines += text.size() != before;
+          }
+          id0 = id1;
+        }
+        total_lines += lines;
+        if (b->pending.fetch_sub(1) == 1) {
+          std::lock_guard<std::mutex> lk(mu_);
+          done_[b->seq] = b;
+          done_cv_.notify_all();
+        }
+      });
+      r0 += b->parts[k]->n;
+    }
+    total_reads += b->n_reads;
+  }
+
+  void write_batches() {
+    for (uint64_t next = 0;; ++next) {
       std::shared_ptr<Batch> b;
       {
-        std::unique_lock<std::mutex> lk(wmu);
-        wait_on(wcv, lk, [&] { return done.count(next) || next == batches_total || sh.failed(); });
-        if (!done.count(next)) return;
-        b = done[next];
-        done.erase(next);
+        std::unique_lock<std::mutex> lk(mu_);
+        done_cv_.wait(lk, [&] { return done_.count(next) || next == batches_total_ || code_; });
+        auto it = done_.find(next);
+        if (it == done_.end()) return;
+        b = std::move(it->second);
+        done_.erase(it);
       }
       for (const std::string& t : b->text)
-        if (!t.empty() && fwrite(t.data(), 1, t.size(), out) != t.size()) {
-          sh.fail(11, std::string("Error writing to result file (") + strerror(errno) + ")");  // src/binner.rs:136-139
+        if (!t.empty() && fwrite(t.data(), 1, t.size(), out_) != t.size()) {
+          fail(11, std::string("Error writing to result file (") + strerror(errno) + ")");  // src/binner.rs:136-139
           return;
         }
-      ++next;
     }
-  });
+  }
 
-  std::vector<std::thread> gpus;
-  for (int g = 0; g < n_gpus; ++g) gpus.emplace_back(gpu_main, g);
-  for (auto& t : gpus) t.join();
-  reader.join();
-  {
-    std::lock_guard<std::mutex> lk(wmu);
-    batches_total = batch_seq;
-    wcv.notify_all();
+  const Options& o_;
+  FastxBlocks& blocks_;
+  FILE* out_;
+  const std::vector<Index>& ix_;
+  std::mutex mu_;
+  std::atomic<int> code_{0};  // exit code of the first failure (set under mu_), and its message
+  std::string error_;
+  std::condition_variable task_cv_;          // the workers' queue of parse and format tasks
+  std::deque<std::function<void()>> tasks_;
+  bool stop_ = false;
+  std::condition_variable parsed_cv_;                        // a block was parsed or taken, or the reader is done
+  std::map<uint64_t, std::unique_ptr<ParsedBlock>> parsed_;  // parsed blocks waiting for their turn, by sequence
+  uint64_t issued_ = 0, taken_ = 0;                          // blocks handed to the parser / taken into batches
+  bool reader_done_ = false;
+  std::mutex take_mu_;  // serialises take_batch, so that batches are consecutive runs of blocks
+  uint64_t batch_seq_ = 0;
+  std::condition_variable done_cv_;                  // a batch was formatted, or the number of batches is known
+  std::map<uint64_t, std::shared_ptr<Batch>> done_;  // formatted (or empty) batches by sequence number
+  uint64_t batches_total_ = ~0ull;                   // known once the GPU threads are done
+};
+
+}  // namespace
+
+int main(int argc, char** argv) {
+  Options o;
+  int code = parse_args(argc, argv, &o);
+  if (code != kGoOn) return code;
+  if (o.dump_reads && !o.dump_mt && o.input()) return dump_reads(o);
+  if ((code = check_options(&o)) != kGoOn) return code;
+  FILE* out;  // (on an early return, exit() closes it)
+  if ((code = open_results(&o, &out)) != kGoOn) return code;
+  FastxBlocks blocks(o.input(), o.is_fastq());  // src/binner.rs:21-33
+  if (!blocks.ok()) {
+    logf("ERROR", "Error running query: cannot open %s", o.input());
+    return 2;
   }
-  writer.join();
-  for (auto h : handles) mtsvgpu_index_close(h);
-  int code = 0;
-  {
-    std::lock_guard<std::mutex> lk(sh.mu);
-    code = sh.exit_code;
-    if (code) logf("ERROR", "%s", sh.error.c_str());
-  }
-  if (!dump_mt && fclose(out) != 0 && code == 0) {
+  std::vector<Index> ix = open_indexes(o);
+  if (ix.empty()) return 2;
+  logf("INFO", "Beginning queries.");
+  const auto t0 = std::chrono::steady_clock::now();
+  Pipeline pipe(o, blocks, out, ix);
+  code = pipe.run();
+  ix.clear();
+  if (!o.dump_mt && fclose(out) != 0 && code == 0) {
     logf("ERROR", "Error writing to result file (%s)", strerror(errno));
     code = 11;
   }
   if (code) return code;
-  if (over_len.load() || over_hits.load()) {
+  if (pipe.over_len.load() || pipe.over_hits.load()) {
     // the reference has no such limits: say so loudly (README "Limits"); --strict-limits turns it into a failure
     logf("WARN", "%llu read(s) longer than %d bases and %llu read strand(s) with more than 2^26 seed hits were reported "
                  "without assignments (limits of this implementation)",
-         (unsigned long long)over_len.load(), MTSVGPU_MAX_READ_LEN, (unsigned long long)over_hits.load());
-    if (strict_limits) return 2;
+         (unsigned long long)pipe.over_len.load(), MTSVGPU_MAX_READ_LEN, (unsigned long long)pipe.over_hits.load());
+    if (o.strict_limits) return 2;
   }
   double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   logf("INFO", "All reads binned: %llu reads, %llu result lines. Took %.3f seconds.",
-       (unsigned long long)total_reads.load(), (unsigned long long)total_lines.load(), secs);
+       (unsigned long long)pipe.total_reads.load(), (unsigned long long)pipe.total_lines.load(), secs);
   return 0;
 }
